@@ -2,6 +2,7 @@
 """bench.py -- TCE policy-update throughput on B200 (BASELINE.json: "TCE policy-update episodes/sec").
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torch.distributed.run)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR     (also writes the last step's outputs)
     python bench.py --impl reference --gpus N --steps K --warmup W
 
 A *step* is ONE policy epoch of ``TemporalCorrelatedAgent.update_policy``
@@ -268,8 +269,8 @@ def capture_epoch(agent, dataset, times, pairs, rank=0):
         box = [agent.policy_epoch(dataset, times, pairs)]
         launches = _lib.LAUNCHES - l0
 
-        def step_fn():
-            box[0] = agent.policy_epoch(dataset, times, pairs)
+        def step_fn():                                           # in place: the returned metrics track the last step
+            box[0].copy_(agent.policy_epoch(dataset, times, pairs))
         return step_fn, box[0], launches, "eager", None, None
 
 
@@ -555,6 +556,18 @@ def _mark(msg):
         print(f"[bench r{os.environ.get('RANK', '0')}] {msg}", file=sys.stderr, flush=True)
 
 
+def dump_outputs(out_dir, metrics, policy):
+    """What the last timed step handed its caller, as ``out_dir/<name>.npy``: the metrics vector (fp64, the agent's
+    loss keys then its KL keys) and every policy parameter after that step's Adam update (fp32, in
+    ``policy.parameters`` order).  The workload is seeded, so the same arguments give the same inputs on every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"metrics": metrics.double()}
+    arrays.update((f"policy_param_{i:02d}", p.detach().float()) for i, p in enumerate(policy.parameters))
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def run_ours(args):
     import torch.distributed as dist
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -593,6 +606,8 @@ def run_ours(args):
     value = world * B_PER_GPU / (ms_per_step * 1e-3)
     _mark("timed region done")
     final = metrics.cpu()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, final, agent.policy)
     if not torch.isfinite(final).all():
         raise SystemExit("non-finite loss in the timed region")
 
@@ -933,7 +948,14 @@ def main():
     ap.add_argument("--multi-extras", action="store_true",
                     help="N > 1: also run config.variants / also on every rank (by default they are N = 1 lines: at "
                          "N > 1 the run is the headline step, e2e and the roofline, i.e. what the scaling curve needs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (metrics vector and updated policy "
+                         "parameters) to DIR/<name>.npy, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
     if int(os.environ.get("WORLD_SIZE", "1")) > 1 and not args.multi_extras:
         args.no_variants = args.no_also = True
     if args.impl == "reference":

@@ -15,8 +15,7 @@ What is produced (all tiny, float64 unless the reference's own test uses float32
                        the box-pushing config; its ``mp`` is the oracle ProDMP through the shim in
                        ``oracle/ref_loader.py``) : policy(), Gaussian helpers, sample(use_mean),
                        log_prob -- pins the tensor plumbing of the oracle policy.
-* ``oracle_path.pt`` -- oracle-generated (PARITY UNPINNED) end-to-end vectors for three MP shapes:
-                       tables, trajectories, segment log-probs + gradients, projections.
+* ``oracle_path.pt`` -- oracle-generated (PARITY UNPINNED) ProDMP tables for three MP shapes.
 """
 from __future__ import annotations
 
@@ -203,45 +202,18 @@ def util_times(init_time, T, dt):
 
 
 def gen_oracle_path():
-    """PARITY UNPINNED vectors straight from the oracle (regression fixtures for the CUDA path)."""
-    from . import policy as opol, projection as oproj, util as ou
+    """PARITY UNPINNED ProDMP tables straight from the oracle (regression fixtures for the CUDA tables).  Only what a
+    test reads is stored: every fixture file stays under 1 MB."""
+    from . import policy as opol
     out = {}
     for name in ("box", "metaworld", "table_tennis"):
         cfg = MP_CONFIGS[name]
-        D, K1, T = cfg["num_dof"], cfg["num_basis"] + 1, NUM_TIMES[name]
-        Dp, B = D * K1, 4
+        Dp = cfg["num_dof"] * (cfg["num_basis"] + 1)
         pol = opol.TemporalCorrelatedPolicy(Dp, mp=dict(type="prodmp", args=dict(cfg, dtype=torch.float64)),
                                             contextual=True, min_std=1e-4)
         tb = pol.mp.tables
-        inp = synthetic_inputs(name, B, seed=1234)
-        times = ou.get_times(inp["init_time"], T, cfg["dt"])
-        torch.manual_seed(0)
-        pairs = ou.get_time_pairs(T, dict(num_select=25, fixed_interval=True))
-        smp = pol.sample(False, inp["mean"], inp["L"], times, inp["init_time"], inp["init_pos"],
-                         inp["init_vel"], eps=inp["eps"])
-        mean = inp["mean"].clone().requires_grad_(True)
-        L = inp["L"].clone().requires_grad_(True)
-        lp, tmean, tcov, reg = pol.log_prob(smp, mean, L, times, inp["init_time"], inp["init_pos"],
-                                            inp["init_vel"], pred_pairs=pairs, return_parts=True)
-        w = torch.linspace(0.5, 1.5, lp.numel(), dtype=torch.float64).reshape(lp.shape)
-        gm, gL = torch.autograd.grad((lp * w).sum(), [mean, L])
-        rec = dict(tables=dict(y1=tb.y1, y2=tb.y2, dy1=tb.dy1, dy2=tb.dy2, pos_basis=tb.pos_basis,
-                               vel_basis=tb.vel_basis, scale=pol.mp.weights_goal_scale),
-                   inputs=inp, times=times, pred_pairs=pairs, smp_traj=smp, log_prob=lp.detach(),
-                   traj_mean=tmean.detach(), traj_cov=tcov.detach(), reg=reg, grad_w=w,
-                   grad_mean=gm, grad_L_tril=torch.tril(gL))
-        for typ, kw in (("KLProjectionLayer", dict(mean_bound=0.05, cov_bound=5e-4)),
-                        ("FrobeniusProjectionLayer", dict(mean_bound=0.05, cov_bound=5e-4)),
-                        ("WassersteinProjectionLayer", dict(mean_bound=0.005, cov_bound=2.5e-4))):
-            layer = oproj.projection_factory(typ, proj_type=typ, trust_region_coeff=1.0, scale_prec=True,
-                                             entropy_schedule="linear", action_dim=Dp, total_train_steps=7500,
-                                             target_entropy=0.0, temperature=0.7, dtype=torch.float64, **kw)
-            layer.initial_entropy = pol.entropy([inp["mean_old"], inp["L_old"]]).mean()
-            pm, pL = layer(pol, (inp["mean"], inp["L"]), (inp["mean_old"], inp["L_old"]), 100)
-            rec[typ] = dict(proj_mean=pm, proj_L=pL, initial_entropy=layer.initial_entropy,
-                            tr_loss=layer.get_trust_region_loss(pol, (inp["mean"], inp["L"]), (pm, pL),
-                                                                set_variance=False))
-        out[name] = rec
+        out[name] = dict(tables=dict(y1=tb.y1, y2=tb.y2, dy1=tb.dy1, dy2=tb.dy2, pos_basis=tb.pos_basis,
+                                     vel_basis=tb.vel_basis, scale=pol.mp.weights_goal_scale))
     return out
 
 
