@@ -111,6 +111,13 @@ int tce_policy_head_fwd(const float *vec, int64_t ldb_vec, float min_std, float 
 /* grad_vec [Bv, nvec]: Bv = B (ldb_vec != 0) or 1 (sum over the batch, ldb_vec == 0)               */
 int tce_policy_head_bwd(const float *vec, int64_t ldb_vec, const float *grad_L, float *grad_vec,
                         int64_t B, int n, void *stream);
+/* diagonal policy head (std_only): vec [B or 1, n] -> L [B, n, n] = diag(softplus(v) + min_std), zeros
+ * elsewhere; ldb_vec = 0 broadcasts one vector.  The backward reads the diagonal of grad_L; grad_vec [Bv, n]
+ * with Bv = 1 (ldb_vec == 0: summed over the batch in a fixed order) or B.                             */
+int tce_policy_head_diag_fwd(const float *vec, int64_t ldb_vec, float min_std, float *L, int64_t B, int n,
+                             void *stream);
+int tce_policy_head_diag_bwd(const float *vec, int64_t ldb_vec, const float *grad_L, float *grad_vec,
+                             int64_t B, int n, void *stream);
 /* per-episode Gaussian scalars used by every projection / KL / entropy call
  * (black_box_policy.py:130-224, projection_utils.gaussian_kl):
  *   out[b, 0] = maha(mean, mean_o, L_o) = |L_o^-1 (mean - mean_o)|^2
@@ -167,6 +174,20 @@ int tce_proj_entropy_fwd(const float *L, const double *beta, int64_t ldb_beta, i
                          double *entropy, int64_t B, int n, void *stream);
 int tce_proj_entropy_bwd(const float *L, const double *beta, int64_t ldb_beta, int equality,
                          const float *grad_out, float *grad_L, int64_t B, int n, void *stream);
+/* Diagonal KL covariance projection (std_only policies), optionally followed by the entropy control of
+ * tce_proj_entropy_fwd (beta == NULL: none).  Every diagonal is a strided vector: element i of episode b is
+ * s[b * ldb + i * inc] (dense factor: ldb = n*n, inc = n+1; packed [B, n]: inc = 1; one shared vector: ldb = 0
+ * on the inputs).  With lam_i = (s_old,i / s_i)^2 the projected variance is s_old,i^2 (1+eta) / (lam_i+eta), eta
+ * the root of KL_cov(eta) = eps_cov where the KL before the projection exceeds eps_cov.  state [B, 4] fp64
+ * {eta, active, alpha, entropy active} feeds the backward; info [B] (optional): 1 if a standard deviation is not
+ * positive and finite.  The backward returns d loss / d s (s_old is a constant).  One warp per episode, n <= 1024. */
+int tce_proj_kl_diag_fwd(const float *s, int64_t ldb_s, int64_t inc_s, const float *s_old, int64_t ldb_so,
+                         int64_t inc_so, double eps_cov, const double *beta, int64_t ldb_beta, int equality,
+                         float *out, int64_t ldb_o, int64_t inc_o, double *state, int32_t *info, int64_t B, int n,
+                         void *stream);
+int tce_proj_kl_diag_bwd(const float *s, int64_t ldb_s, int64_t inc_s, const float *s_old, int64_t ldb_so,
+                         int64_t inc_so, const double *state, const float *grad_out, int64_t ldb_g, int64_t inc_g,
+                         float *grad_s, int64_t ldb_gs, int64_t inc_gs, int64_t B, int n, void *stream);
 /* KL covariance projection: min KL(N(.,S)||N(.,S~)) s.t. KL_cov(S||S_old) <= eps_cov, solved exactly on
  * the generalised eigenvalues (CTA-per-matrix one-sided Jacobi + Newton for eta); proj_L = chol(S_proj).
  * `save` (tce_proj_kl_save_doubles(B, n) doubles) carries M = L_old Q, U = L~^-1 M, L~^-1, Sigma_proj, lambda,
@@ -299,6 +320,26 @@ int tce_seglik_bwd_dsigma(const tce_tables_t *tables, const void *work, const fl
                           const float *init_time, const int64_t *pred_pairs, const float *upstream,
                           float *grad_mean, float *grad_sigma, int64_t B, int64_t T, int64_t P, void *stream);
 int tce_dsigma_to_dl(const float *grad_sigma, int64_t B, const float *L, float *grad_L, int n, void *stream);
+/* Diagonal covariance (std_only policies, per-episode standard deviations s, strided as for tce_proj_kl_diag_*):
+ * C is block diagonal with one 2 x 2 block per (pair, DoF), C_d[k,k'] = sum_j h_kj h_k'j s_{d,j}^2 + reg.
+ * tce_seglik_diag_max: the regulariser seed diag_max = max over the batch of diag C (atomic max into *diag_max,
+ * zero it first; all-reduce(MAX) it between the launches at > 1 GPU).  tce_seglik_diag_fwd: logp [B, P], info [B, P]
+ * (optional; first non-positive pivot as in tce_seglik_chol).  tce_seglik_diag_bwd: from grad_logp [B, P],
+ * grad_mean [B, Dp] and grad_s (strided, ldb_gs > 0), either may be NULL.  fp64 arithmetic, fixed summation order. */
+int tce_seglik_diag_max(const tce_tables_t *tables, const float *s, int64_t ldb_s, int64_t inc_s,
+                        const float *times, const float *init_time, const int64_t *pred_pairs, double *diag_max,
+                        int64_t B, int64_t T, int64_t P, void *stream);
+int tce_seglik_diag_fwd(const tce_tables_t *tables, const float *smp_traj, const float *mean, const float *s,
+                        int64_t ldb_s, int64_t inc_s, const float *times, const float *init_time,
+                        const float *init_pos, const float *init_vel, const int64_t *pred_pairs,
+                        const double *diag_max, double reg_rel, float *logp, int32_t *info, int64_t B, int64_t T,
+                        int64_t P, void *stream);
+int tce_seglik_diag_bwd(const tce_tables_t *tables, const float *smp_traj, const float *mean, const float *s,
+                        int64_t ldb_s, int64_t inc_s, const float *times, const float *init_time,
+                        const float *init_pos, const float *init_vel, const int64_t *pred_pairs,
+                        const double *diag_max, double reg_rel, const float *grad_logp, float *grad_mean,
+                        float *grad_s, int64_t ldb_gs, int64_t inc_gs, int64_t B, int64_t T, int64_t P,
+                        void *stream);
 
 /* ---- (3') the same likelihood, fused: product path of TemporalCorrelatedPolicy.log_prob / segment_surrogate --------
  * (temporal_correlated_policy.py:104-203 + temporal_correlated_agent.py:718-739).

@@ -45,6 +45,17 @@ SIGNATURES = {
     "tce_chol_bwd": (C.c_int, [_P, _P, _P, _I64, _I32, _P]),
     "tce_policy_head_fwd": (C.c_int, [_P, _I64, _F, _P, _I64, _I32, _P]),
     "tce_policy_head_bwd": (C.c_int, [_P, _I64, _P, _P, _I64, _I32, _P]),
+    "tce_policy_head_diag_fwd": (C.c_int, [_P, _I64, _F, _P, _I64, _I32, _P]),
+    "tce_policy_head_diag_bwd": (C.c_int, [_P, _I64, _P, _P, _I64, _I32, _P]),
+    "tce_proj_kl_diag_fwd": (C.c_int, [_P, _I64, _I64, _P, _I64, _I64, _D, _P, _I64, _I32, _P, _I64, _I64, _P, _P, _I64,
+                                       _I32, _P]),
+    "tce_proj_kl_diag_bwd": (C.c_int, [_P, _I64, _I64, _P, _I64, _I64, _P, _P, _I64, _I64, _P, _I64, _I64, _I64, _I32,
+                                       _P]),
+    "tce_seglik_diag_max": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
+    "tce_seglik_diag_fwd": (C.c_int, [_P, _P, _P, _P, _I64, _I64, _P, _P, _P, _P, _P, _P, _D, _P, _P, _I64, _I64, _I64,
+                                      _P]),
+    "tce_seglik_diag_bwd": (C.c_int, [_P, _P, _P, _P, _I64, _I64, _P, _P, _P, _P, _P, _P, _D, _P, _P, _P, _I64, _I64,
+                                      _I64, _I64, _I64, _P]),
     "tce_gauss_stats": (C.c_int, [_P, _P, _I64, _P, _P, _I64, _P, _I64, _I32, _P]),
     "tce_gauss_stats_bwd": (C.c_int, [_P, _P, _I64, _P, _P, _I64, _P, _P, _P, _I64, _I32, _P]),
     "tce_gauss_maha": (C.c_int, [_P, _P, _P, _I64, _P, _P, _P, _I64, _I32, _P]),

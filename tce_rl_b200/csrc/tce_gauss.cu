@@ -294,6 +294,46 @@ __global__ void head_bwd_kernel(const float *__restrict__ vec, long long ldb_vec
   }
 }
 
+// Diagonal head (std_only): L = diag(softplus(v) + min_std), zeros elsewhere; one thread per entry of the dense factor
+__global__ void __launch_bounds__(256)
+head_diag_fwd_kernel(const float *__restrict__ vec, long long ldb_vec, float min_std, float *__restrict__ L,
+                     long long B, int n) {
+  const long long nn = (long long)n * n, total = B * nn;
+  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+    const long long b = e / nn;
+    const int r = (int)(e - b * nn), i = r / n;
+    L[e] = (r == i * (n + 1)) ? softplus_f(vec[b * ldb_vec + i]) + min_std : 0.f;
+  }
+}
+
+// grad_vec[b, i] = grad_L[b, i, i] * sigmoid(v[b, i]).  ldb_vec == 0 (one shared vector): CTA per i sums the batch in a
+// fixed order (strided partial sums, then a tree) -- deterministic, no atomics.
+__global__ void __launch_bounds__(256)
+head_diag_bwd_kernel(const float *__restrict__ vec, long long ldb_vec, const float *__restrict__ gL,
+                     float *__restrict__ gvec, long long B, int n) {
+  const long long nn = (long long)n * n;
+  if (ldb_vec != 0) {
+    const long long total = B * n;
+    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+      const long long b = e / n;
+      const int i = (int)(e - b * n);
+      gvec[e] = gL[b * nn + (long long)i * (n + 1)] / (1.f + expf(-vec[b * ldb_vec + i]));
+    }
+    return;
+  }
+  __shared__ float red[256];
+  const int i = blockIdx.x;
+  float acc = 0.f;
+  for (long long b = threadIdx.x; b < B; b += blockDim.x) acc += gL[b * nn + (long long)i * (n + 1)];
+  red[threadIdx.x] = acc;
+  __syncthreads();
+  for (int s = blockDim.x >> 1; s > 0; s >>= 1) {
+    if ((int)threadIdx.x < s) red[threadIdx.x] += red[threadIdx.x + s];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) gvec[i] = red[0] / (1.f + expf(-vec[i]));
+}
+
 }  // namespace
 
 static int gauss_num_sms() {
@@ -387,5 +427,31 @@ extern "C" int tce_policy_head_bwd(const float *vec, int64_t ldb_vec, const floa
   dim3 grid((nvec + 127) / 128, (unsigned)((B + chunk - 1) / chunk));
   head_bwd_kernel<<<grid, 128, 0, st>>>(vec, ldb_vec, grad_L, grad_vec, B, n, chunk);
   TCE_CHECK_LAUNCH("head_bwd_kernel");
+  return TCE_OK;
+}
+
+extern "C" int tce_policy_head_diag_fwd(const float *vec, int64_t ldb_vec, float min_std, float *L, int64_t B, int n,
+                                        void *stream) {
+  if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
+  if (!vec || !L || B < 0 || n < 1 || ldb_vec < 0) return TCE_ERR_INVALID_ARGUMENT;
+  const long long blocks = (B * n * n + 255) / 256, cap = 8LL * gauss_num_sms();
+  head_diag_fwd_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, (cudaStream_t)stream>>>(vec, ldb_vec, min_std,
+                                                                                                 L, B, n);
+  TCE_CHECK_LAUNCH("head_diag_fwd_kernel");
+  return TCE_OK;
+}
+
+extern "C" int tce_policy_head_diag_bwd(const float *vec, int64_t ldb_vec, const float *grad_L, float *grad_vec,
+                                        int64_t B, int n, void *stream) {
+  if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
+  if (!vec || !grad_L || !grad_vec || B < 0 || n < 1 || ldb_vec < 0) return TCE_ERR_INVALID_ARGUMENT;
+  long long blocks = n;
+  if (ldb_vec != 0) {
+    const long long cap = 8LL * gauss_num_sms();
+    blocks = (B * n + 255) / 256;
+    blocks = blocks < cap ? blocks : cap;
+  }
+  head_diag_bwd_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(vec, ldb_vec, grad_L, grad_vec, B, n);
+  TCE_CHECK_LAUNCH("head_diag_bwd_kernel");
   return TCE_OK;
 }

@@ -596,6 +596,116 @@ __device__ inline double kl_solve_eta(const double *lam, int n, double eps, doub
   return eta;
 }
 
+// -----------------------------------------------------------------------------------------------------
+// Diagonal KL projection (std_only policies).  With lam_i = (s_old,i / s_i)^2 the dual is the same scalar function
+// kl_of_eta, and the projected variance is elementwise: s_old,i^2 (1 + eta) / (lam_i + eta)  -- no eigen-solve, so
+// equal standard deviations (a fresh policy) are not a degenerate case.  One warp per episode.
+// -----------------------------------------------------------------------------------------------------
+constexpr int KD_WARPS = 4;
+constexpr int KD_SC = 4;      // state per episode: eta, KL step active, alpha, entropy control active
+
+// Root of KL_cov(eta) = eps for one warp (kl_of_eta hands every lane the same value, so the control flow is
+// warp-uniform): bracket by doubling, then Newton steps safeguarded by bisection.
+__device__ inline double kl_solve_eta_warp(const double *lam, int n, double eps) {
+  double lo = 0.0, hi = 1.0;
+  for (int it = 0; it < 1000 && kl_of_eta(lam, n, hi, nullptr) > eps; ++it) { lo = hi; hi *= 2.0; }
+  double eta = 0.5 * (lo + hi);
+  for (int it = 0; it < 200; ++it) {
+    double df;
+    const double f = kl_of_eta(lam, n, eta, &df) - eps;
+    if (f > 0.0) lo = eta; else hi = eta;
+    double nxt = (df < 0.0) ? eta - f / df : 0.5 * (lo + hi);
+    if (!(nxt > lo && nxt < hi)) nxt = 0.5 * (lo + hi);
+    const bool done = fabs(nxt - eta) <= 4e-16 * fmax(1.0, eta) || hi - lo <= 4e-16 * fmax(1.0, hi);
+    eta = nxt;
+    if (done) break;
+  }
+  return eta;
+}
+
+// Forward (gout == NULL): out = alpha * s_proj and the state {eta, active, alpha, entropy active}.
+// Backward: out = d loss / d s from gout = d loss / d out; implicit differentiation of eta,
+// d eta / d lam_j = -(d KL / d lam_j) / (d KL / d eta), and the alpha term of the entropy control.
+__global__ void __launch_bounds__(KD_WARPS * 32)
+proj_kl_diag_kernel(const float *__restrict__ s, long long ldb_s, long long inc_s, const float *__restrict__ so,
+                    long long ldb_so, long long inc_so, double eps, const double *__restrict__ beta, long long ldb_beta,
+                    int equality, const float *__restrict__ gout, long long ldb_g, long long inc_g,
+                    float *__restrict__ out, long long ldb_o, long long inc_o, double *__restrict__ state,
+                    int32_t *__restrict__ info, long long B, int n) {
+  extern __shared__ double kd_lam[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long b = (long long)blockIdx.x * KD_WARPS + warp;
+  if (b >= B) return;                                   // warp-uniform, no CTA barrier below
+  double *lam = kd_lam + warp * n;
+  const float *sb = s + b * ldb_s, *sob = so + b * ldb_so;
+  int bad = 0;
+  for (int i = lane; i < n; i += 32) {
+    const double v = sb[i * inc_s], vo = sob[i * inc_so];
+    if (!(v > 0.0) || !(vo > 0.0) || !(v < INFINITY) || !(vo < INFINITY)) bad = 1;
+    const double r = vo / v;
+    lam[i] = r * r;
+  }
+  bad = __any_sync(0xffffffffu, bad);
+  __syncwarp();
+  double *sc = state + b * KD_SC;
+  float *ob = out + b * ldb_o;
+  if (!gout) {
+    const bool active = !bad && kl_of_eta(lam, n, 0.0, nullptr) > eps;
+    const double eta = active ? kl_solve_eta_warp(lam, n, eps) : 0.0;
+    double ls = 0.0;
+    for (int i = lane; i < n; i += 32)
+      ls += active ? log((double)sob[i * inc_so]) + 0.5 * log((1.0 + eta) / (lam[i] + eta)) : log((double)sb[i * inc_s]);
+    ls = warp_sum(ls);
+    const double H = 0.5 * n * (1.0 + LOG_2PI) + ls;
+    const double bt = beta ? beta[b * ldb_beta] : 0.0;
+    const bool ent = beta != nullptr && (equality || H < bt);
+    const double alpha = ent ? exp((bt - H) / n) : 1.0;
+    for (int i = lane; i < n; i += 32) {
+      const double p = active ? (double)sob[i * inc_so] * sqrt((1.0 + eta) / (lam[i] + eta)) : (double)sb[i * inc_s];
+      ob[i * inc_o] = (float)(alpha * p);
+    }
+    if (lane == 0) {
+      sc[0] = eta; sc[1] = active ? 1.0 : 0.0; sc[2] = alpha; sc[3] = ent ? 1.0 : 0.0;
+      if (info) info[b] = bad;
+    }
+    return;
+  }
+  const double eta = sc[0], alpha = sc[2];
+  const bool active = sc[1] != 0.0, ent = sc[3] != 0.0;
+  const float *gb = gout + b * ldb_g;
+  // entropy control: out = alpha(p) p with d alpha / d p_j = -alpha / (n p_j)
+  double dot = 0.0;
+  for (int i = lane; i < n; i += 32) {
+    const double p = active ? (double)sob[i * inc_so] * sqrt((1.0 + eta) / (lam[i] + eta)) : (double)sb[i * inc_s];
+    dot = fma((double)gb[i * inc_g], p, dot);
+  }
+  dot = ent ? warp_sum(dot) : 0.0;
+  if (!active) {
+    for (int i = lane; i < n; i += 32) {
+      const double p = sb[i * inc_s];
+      ob[i * inc_o] = (float)(alpha * gb[i * inc_g] - alpha * dot / (n * p));
+    }
+    return;
+  }
+  // p_i = s_old,i sqrt((1+eta)/(lam_i+eta)):  d p_i / d lam_i = -p_i / (2 (lam_i+eta)),
+  // d p_i / d eta = p_i (lam_i - 1) / (2 (1+eta) (lam_i+eta));  d KL / d lam_j = (lam_j - 1) / (2 (lam_j+eta)^2)
+  double geta = 0.0;
+  for (int i = lane; i < n; i += 32) {
+    const double l = lam[i], p = (double)sob[i * inc_so] * sqrt((1.0 + eta) / (l + eta));
+    const double gp = alpha * gb[i * inc_g] - alpha * dot / (n * p);
+    geta += gp * p * (l - 1.0) / (2.0 * (1.0 + eta) * (l + eta));
+  }
+  geta = warp_sum(geta);
+  double dfde;
+  kl_of_eta(lam, n, eta, &dfde);
+  for (int i = lane; i < n; i += 32) {
+    const double l = lam[i], p = (double)sob[i * inc_so] * sqrt((1.0 + eta) / (l + eta));
+    const double gp = alpha * gb[i * inc_g] - alpha * dot / (n * p);
+    const double glam = -gp * p / (2.0 * (l + eta)) - geta * (l - 1.0) / (2.0 * (l + eta) * (l + eta) * dfde);
+    ob[i * inc_o] = (float)(glam * (-2.0 * l / (double)sb[i * inc_s]));     // d lam_i / d s_i = -2 lam_i / s_i
+  }
+}
+
 // Forward.  With W = Lt^-1 Lo, one-sided Jacobi rotates the columns of W into U~ = W Q (orthogonal columns,
 // |U~_j|^2 = lam_j = eigenvalues of W^T W); then M := Lo Q = Lt U~ and
 //   Sigma_proj = Lo Q diag((1+eta)/(lam+eta)) Q^T Lo^T = M D M^T ,   proj_L = chol(Sigma_proj).
@@ -1637,6 +1747,37 @@ extern "C" int tce_proj_entropy_bwd(const float *L, const double *beta, int64_t 
   if (!L || !beta || !grad_out || !grad_L || B < 0 || n < 1) return TCE_ERR_INVALID_ARGUMENT;
   proj_entropy_kernel<<<(unsigned)B, 256, 0, (cudaStream_t)stream>>>(L, beta, ldb_beta, equality, grad_out, grad_L, nullptr, n);
   TCE_CHECK_LAUNCH("proj_entropy_kernel(bwd)");
+  return TCE_OK;
+}
+
+extern "C" int tce_proj_kl_diag_fwd(const float *s, int64_t ldb_s, int64_t inc_s, const float *s_old, int64_t ldb_so,
+                                    int64_t inc_so, double eps_cov, const double *beta, int64_t ldb_beta, int equality,
+                                    float *out, int64_t ldb_o, int64_t inc_o, double *state, int32_t *info, int64_t B,
+                                    int n, void *stream) {
+  if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
+  if (!s || !s_old || !out || !state || B < 0 || n < 1 || n > 1024 || !(eps_cov > 0) || ldb_s < 0 || ldb_so < 0 ||
+      ldb_beta < 0 || (ldb_o == 0 && B > 1) || ldb_o < 0)
+    return TCE_ERR_INVALID_ARGUMENT;
+  proj_kl_diag_kernel<<<(unsigned)((B + KD_WARPS - 1) / KD_WARPS), KD_WARPS * 32, KD_WARPS * n * sizeof(double),
+                        (cudaStream_t)stream>>>(s, ldb_s, inc_s, s_old, ldb_so, inc_so, eps_cov, beta, ldb_beta, equality,
+                                                nullptr, 0, 0, out, ldb_o, inc_o, state, info, B, n);
+  TCE_CHECK_LAUNCH("proj_kl_diag_kernel");
+  return TCE_OK;
+}
+
+extern "C" int tce_proj_kl_diag_bwd(const float *s, int64_t ldb_s, int64_t inc_s, const float *s_old, int64_t ldb_so,
+                                    int64_t inc_so, const double *state, const float *grad_out, int64_t ldb_g,
+                                    int64_t inc_g, float *grad_s, int64_t ldb_gs, int64_t inc_gs, int64_t B, int n,
+                                    void *stream) {
+  if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
+  if (!s || !s_old || !state || !grad_out || !grad_s || B < 0 || n < 1 || n > 1024 || ldb_s < 0 || ldb_so < 0 ||
+      ldb_g < 0 || (ldb_gs == 0 && B > 1) || ldb_gs < 0)
+    return TCE_ERR_INVALID_ARGUMENT;
+  proj_kl_diag_kernel<<<(unsigned)((B + KD_WARPS - 1) / KD_WARPS), KD_WARPS * 32, KD_WARPS * n * sizeof(double),
+                        (cudaStream_t)stream>>>(s, ldb_s, inc_s, s_old, ldb_so, inc_so, 0.0, nullptr, 0, 0, grad_out,
+                                                ldb_g, inc_g, grad_s, ldb_gs, inc_gs, const_cast<double *>(state),
+                                                nullptr, B, n);
+  TCE_CHECK_LAUNCH("proj_kl_diag_kernel(bwd)");
   return TCE_OK;
 }
 

@@ -597,7 +597,153 @@ dsigma_to_dl_kernel(const float *__restrict__ dS, long long B, const float *__re
   }
 }
 
+// =====================================================================================================
+// Diagonal covariance (std_only policies), per-episode standard deviations s [B, Dp] (strided: s[b ldb + i inc]).
+// H is block diagonal per DoF, so C is block diagonal with one 2 x 2 block per (pair, DoF):
+//   C_d[k,k'] = sum_j h_kj h_k'j s_{d,j}^2 + reg delta_kk',   lp = sum_d log N(r_d; 0, C_d)
+// backward: d/d theta_{d,j} = sum_{p,k} h_pk[j] (g alpha)_{d,k},
+//           d/d s_{d,j} = 2 s_{d,j} sum_{p,k,k'} G_d[k,k'] h_pk[j] h_pk'[j],  G = g/2 (alpha alpha^T - C^-1).
+// One CTA per episode.  MODE 0: batch-global max of diag C (the regulariser seed; its own launch so that an
+// all-reduce(MAX) can run in between at >1 GPU), 1: log-probs, 2: gradients.  fp64 throughout (as the dense path);
+// the sums over segments run in a fixed order.
+// =====================================================================================================
+constexpr int SD_THREADS = 128;
+
+template <int D, int K1, int MODE>
+__global__ void __launch_bounds__(SD_THREADS)
+seglik_diag_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *__restrict__ mean,
+                   const float *__restrict__ s, long long ldb_s, long long inc_s, const float *__restrict__ times,
+                   const float *__restrict__ init_time, const float *__restrict__ init_pos,
+                   const float *__restrict__ init_vel, const int64_t *__restrict__ pairs, double *__restrict__ diag_max,
+                   double reg_rel, const float *__restrict__ grad_logp, float *__restrict__ logp,
+                   int32_t *__restrict__ info, float *__restrict__ grad_mean, float *__restrict__ grad_s,
+                   long long ldb_gs, long long inc_gs, int T, int P) {
+  constexpr int Dp = D * K1;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  double *hs = reinterpret_cast<double *>(smem_raw);             // [2P][K1]
+  double *xi = hs + 2 * P * K1;                                   // [2P][2]
+  double *init_row = xi + 4 * P;                                  // [5 + 2 K1]
+  double *s2 = init_row + 5 + 2 * K1;                             // [Dp] variances
+  double *part = s2 + Dp;                                         // MODE 1: [D][P] log-prob parts; MODE 2: [D][5][P]
+  int *bad_s = reinterpret_cast<int *>(part + (MODE == 2 ? 5 : 1) * D * P);   // MODE 1: [D][P]
+  __shared__ double s_max[SD_THREADS / 32];
+
+  const long long b = blockIdx.x;
+  const float *sb = s + b * ldb_s;
+  for (int i = threadIdx.x; i < Dp; i += blockDim.x) {
+    const double v = sb[i * inc_s];
+    s2[i] = v * v;
+  }
+  basis_points<K1>(tb, (double)init_time[b], times + b * T, pairs, P, hs, xi, init_row);   // ends with a barrier
+
+  if (MODE == 0) {
+    double my_max = 0.0;
+    for (int task = threadIdx.x; task < 2 * P * D; task += blockDim.x) {
+      const int d = task / (2 * P), q = task - d * 2 * P;
+      double c = 0.0;
+#pragma unroll
+      for (int j = 0; j < K1; ++j) c = fma(hs[q * K1 + j] * hs[q * K1 + j], s2[d * K1 + j], c);
+      my_max = fmax(my_max, c);
+    }
+    my_max = warp_max(my_max);
+    if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = my_max;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      double m = 0.0;
+      for (int w = 0; w < SD_THREADS / 32; ++w) m = fmax(m, s_max[w]);
+      atomic_max_pos_double(diag_max, m);
+    }
+    return;
+  }
+
+  const double reg = reg_rel * (*diag_max), tau = tb.tau;
+  for (int task = threadIdx.x; task < P * D; task += blockDim.x) {
+    const int d = task / P, p = task - d * P;
+    const double *h0 = hs + (2 * p) * K1, *h1 = h0 + K1;
+    double c00 = 0.0, c01 = 0.0, c11 = 0.0;
+#pragma unroll
+    for (int j = 0; j < K1; ++j) {
+      const double v = s2[d * K1 + j];
+      c00 = fma(h0[j] * h0[j], v, c00);
+      c01 = fma(h0[j] * h1[j], v, c01);
+      c11 = fma(h1[j] * h1[j], v, c11);
+    }
+    c00 += reg;
+    c11 += reg;
+    // residual r_k = x - mu (as the dense path)
+    const double y0 = (double)init_pos[b * D + d], v0 = (double)init_vel[b * D + d] * tau;
+    const float *th = mean + b * Dp + d * K1;
+    double r[2];
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int q = 2 * p + k;
+      double mu = xi[2 * q] * y0 + xi[2 * q + 1] * v0;
+#pragma unroll
+      for (int j = 0; j < K1; ++j) mu = fma(hs[q * K1 + j], (double)th[j], mu);
+      if (tb.relative_goal) {
+        const double shift = tb.relative_goal_scaled ? y0 : y0 / tb.scale[K1 - 1];
+        mu = fma(hs[q * K1 + K1 - 1], shift, mu);
+      }
+      r[k] = (double)smp_traj[(b * T + pairs[q]) * (2 * D) + d] - mu;
+    }
+    // 2 x 2 Cholesky; bad = first non-positive pivot as row (2 d + k) + 1 of the full matrix
+    int bad = 0;
+    if (!(c00 > 0.0)) bad = 2 * d + 1;
+    const double l00 = sqrt(c00), l10 = c01 / l00, d11 = c11 - l10 * l10;
+    if (!(d11 > 0.0) && bad == 0) bad = 2 * d + 2;
+    const double l11 = sqrt(d11);
+    const double z0 = r[0] / l00, z1 = (r[1] - l10 * z0) / l11;
+    if (MODE == 1) {
+      part[d * P + p] = -0.5 * (2.0 * 1.8378770664093453 + z0 * z0 + z1 * z1) - 0.5 * (log(c00) + log(d11));
+      bad_s[d * P + p] = bad;
+    } else {
+      const double g = (double)grad_logp[b * P + p];
+      const double idet = 1.0 / (c00 * c11 - c01 * c01);
+      const double i00 = c11 * idet, i01 = -c01 * idet, i11 = c00 * idet;          // C^-1
+      const double a0 = i00 * r[0] + i01 * r[1], a1 = i01 * r[0] + i11 * r[1];      // alpha = C^-1 r
+      double *pd = part + (size_t)d * 5 * P + p;
+      pd[0] = g * a0;
+      pd[P] = g * a1;
+      pd[2 * P] = 0.5 * g * (a0 * a0 - i00);
+      pd[3 * P] = 0.5 * g * (a0 * a1 - i01);
+      pd[4 * P] = 0.5 * g * (a1 * a1 - i11);
+    }
+  }
+  __syncthreads();
+  if (MODE == 1) {
+    for (int p = threadIdx.x; p < P; p += blockDim.x) {
+      double lp = 0.0;
+      int bad = 0;
+      for (int d = 0; d < D; ++d) {
+        lp += part[d * P + p];
+        if (bad == 0) bad = bad_s[d * P + p];
+      }
+      logp[b * P + p] = (float)lp;
+      if (info) info[b * P + p] = bad;
+    }
+    return;
+  }
+  for (int o = threadIdx.x; o < Dp; o += blockDim.x) {
+    const int d = o / K1, j = o - d * K1;
+    const double *pd = part + (size_t)d * 5 * P;
+    double gm = 0.0, gv = 0.0;
+    for (int p = 0; p < P; ++p) {
+      const double h0 = hs[(2 * p) * K1 + j], h1 = hs[(2 * p + 1) * K1 + j];
+      gm = fma(h0, pd[p], fma(h1, pd[P + p], gm));
+      gv = fma(h0 * h0, pd[2 * P + p], fma(2.0 * h0 * h1, pd[3 * P + p], fma(h1 * h1, pd[4 * P + p], gv)));
+    }
+    if (grad_mean) grad_mean[b * Dp + o] = (float)gm;
+    if (grad_s) grad_s[b * ldb_gs + o * inc_gs] = (float)(2.0 * (double)sb[o * inc_s] * gv);
+  }
+}
+
 // ---- host side ---------------------------------------------------------------------------------------
+template <int D, int K1>
+size_t diag_smem(int P, int mode) {
+  return sizeof(double) * (2 * P * K1 + 4 * P + 5 + 2 * K1 + D * K1 + (mode == 2 ? 5 : 1) * D * P) +
+         (mode == 1 ? sizeof(int) * D * P : 0) + 16;
+}
+
 template <int D, int K1>
 size_t gram_smem(int P) {
   constexpr int Dp = D * K1, NR = (Dp + 1) & ~1, NR4 = (Dp + 3) & ~3, LD = NR4 + 1, SD = NR + 1;
@@ -758,6 +904,68 @@ extern "C" int tce_seglik_bwd_dsigma(const tce_tables_t *t, const void *work, co
   if (B != 0 && !grad_sigma) return TCE_ERR_INVALID_ARGUMENT;
   return seglik_bwd_launch<true>(t, work, nullptr, 0, times, init_time, pred_pairs, upstream, grad_mean, grad_sigma,
                                  B, T, P, stream);
+}
+
+template <int MODE>
+static int seglik_diag_launch(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *s,
+                              int64_t ldb_s, int64_t inc_s, const float *times, const float *init_time,
+                              const float *init_pos, const float *init_vel, const int64_t *pred_pairs, double *diag_max,
+                              double reg_rel, const float *grad_logp, float *logp, int32_t *info, float *grad_mean,
+                              float *grad_s, int64_t ldb_gs, int64_t inc_gs, int64_t B, int64_t T, int64_t P,
+                              void *stream) {
+  if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
+  if (!t || !s || !times || !init_time || !pred_pairs || !diag_max || B < 0 || T < 1 || P < 1 || P > 4096 ||
+      ldb_s < 0)
+    return TCE_ERR_INVALID_ARGUMENT;
+  if (MODE >= 1 && (!smp_traj || !mean || !init_pos || !init_vel)) return TCE_ERR_INVALID_ARGUMENT;
+  if (MODE == 1 && !logp) return TCE_ERR_INVALID_ARGUMENT;
+  if (MODE == 2 && (!grad_logp || (!grad_mean && !grad_s) || (grad_s && (ldb_gs < 0 || (ldb_gs == 0 && B > 1)))))
+    return TCE_ERR_INVALID_ARGUMENT;
+  cudaStream_t st = (cudaStream_t)stream;
+#define X(Dv, Kv)                                                                                                  \
+  if (t->D == Dv && t->K1 == Kv) {                                                                                 \
+    const size_t smem = diag_smem<Dv, Kv>((int)P, MODE);                                                           \
+    if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;                                                       \
+    if (smem > 48 * 1024)                                                                                          \
+      TCE_CUDA(cudaFuncSetAttribute(seglik_diag_kernel<Dv, Kv, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                    (int)smem), "diag smem attr");                                                 \
+    seglik_diag_kernel<Dv, Kv, MODE><<<(unsigned)B, SD_THREADS, smem, st>>>(                                        \
+        tab_dev(t), smp_traj, mean, s, ldb_s, inc_s, times, init_time, init_pos, init_vel, pred_pairs, diag_max,   \
+        reg_rel, grad_logp, logp, info, grad_mean, grad_s, ldb_gs, inc_gs, (int)T, (int)P);                        \
+    TCE_CHECK_LAUNCH("seglik_diag_kernel");                                                                        \
+    return TCE_OK;                                                                                                 \
+  }
+  TCE_FOR_SHAPES(X)
+#undef X
+  return TCE_ERR_UNSUPPORTED_SHAPE;
+}
+
+extern "C" int tce_seglik_diag_max(const tce_tables_t *t, const float *s, int64_t ldb_s, int64_t inc_s,
+                                   const float *times, const float *init_time, const int64_t *pred_pairs,
+                                   double *diag_max, int64_t B, int64_t T, int64_t P, void *stream) {
+  return seglik_diag_launch<0>(t, nullptr, nullptr, s, ldb_s, inc_s, times, init_time, nullptr, nullptr, pred_pairs,
+                               diag_max, 0.0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, B, T, P, stream);
+}
+
+extern "C" int tce_seglik_diag_fwd(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *s,
+                                   int64_t ldb_s, int64_t inc_s, const float *times, const float *init_time,
+                                   const float *init_pos, const float *init_vel, const int64_t *pred_pairs,
+                                   const double *diag_max, double reg_rel, float *logp, int32_t *info, int64_t B,
+                                   int64_t T, int64_t P, void *stream) {
+  return seglik_diag_launch<1>(t, smp_traj, mean, s, ldb_s, inc_s, times, init_time, init_pos, init_vel, pred_pairs,
+                               const_cast<double *>(diag_max), reg_rel, nullptr, logp, info, nullptr, nullptr, 0, 0, B,
+                               T, P, stream);
+}
+
+extern "C" int tce_seglik_diag_bwd(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *s,
+                                   int64_t ldb_s, int64_t inc_s, const float *times, const float *init_time,
+                                   const float *init_pos, const float *init_vel, const int64_t *pred_pairs,
+                                   const double *diag_max, double reg_rel, const float *grad_logp, float *grad_mean,
+                                   float *grad_s, int64_t ldb_gs, int64_t inc_gs, int64_t B, int64_t T, int64_t P,
+                                   void *stream) {
+  return seglik_diag_launch<2>(t, smp_traj, mean, s, ldb_s, inc_s, times, init_time, init_pos, init_vel, pred_pairs,
+                               const_cast<double *>(diag_max), reg_rel, grad_logp, nullptr, nullptr, grad_mean, grad_s,
+                               ldb_gs, inc_gs, B, T, P, stream);
 }
 
 extern "C" int tce_dsigma_to_dl(const float *grad_sigma, int64_t B, const float *L, float *grad_L, int n,

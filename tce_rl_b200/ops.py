@@ -260,6 +260,43 @@ def _head_backward(ctx, gL):
 policy_head.register_autograd(_head_backward, setup_context=_head_setup)
 
 
+@torch.library.custom_op("tce::policy_head_diag", mutates_args=())
+def policy_head_diag(vec: Tensor, batch: int, dim: int, min_std: float) -> Tensor:
+    """std vector [dim] (shared) or [B, dim] -> L [B, dim, dim] = diag(softplus(vec) + min_std)."""
+    vec = _chk(vec, name="std vector")
+    ldb = 0 if vec.dim() == 1 else vec.shape[-1]
+    L = torch.empty(batch, dim, dim, device=vec.device, dtype=torch.float32)
+    _lib.call("tce_policy_head_diag_fwd", _p(vec), ldb, float(min_std), _p(L), batch, dim, _stream())
+    return L
+
+
+@policy_head_diag.register_fake
+def _(vec, batch, dim, min_std):
+    return vec.new_empty(batch, dim, dim)
+
+
+@torch.library.custom_op("tce::policy_head_diag_bwd", mutates_args=())
+def policy_head_diag_bwd(vec: Tensor, grad_L: Tensor) -> Tensor:
+    vec, grad_L = _chk(vec), _chk(grad_L)
+    ldb = 0 if vec.dim() == 1 else vec.shape[-1]
+    g = torch.empty_like(vec)
+    _lib.call("tce_policy_head_diag_bwd", _p(vec), ldb, _p(grad_L), _p(g), grad_L.shape[0], grad_L.shape[-1], _stream())
+    return g
+
+
+@policy_head_diag_bwd.register_fake
+def _(vec, grad_L):
+    return torch.empty_like(vec)
+
+
+def _head_diag_backward(ctx, gL):
+    (vec,) = ctx.saved_tensors
+    return policy_head_diag_bwd(vec, gL), None, None, None
+
+
+policy_head_diag.register_autograd(_head_diag_backward, setup_context=_head_setup)
+
+
 @torch.library.custom_op("tce::gauss_stats", mutates_args=())
 def gauss_stats(mean: Tensor, L: Tensor, mean_o: Tensor, L_o: Tensor) -> Tensor:
     """[B, 5] float64: maha, tr(Sigma_o^-1 Sigma), logdet Sigma, logdet Sigma_o, entropy(mean, L)."""
@@ -283,7 +320,8 @@ def _(mean, L, mean_o, L_o):
 # The product path of the likelihood is the fused implementation in ops_seglik.py (re-exported at the end of this
 # module); the STAGED ops below (gram / chol / bwd with an fp64 HBM workspace) are kept as an independent
 # implementation for cross-checks (tests) and for mp.ProDMP.get_traj_pos_cov.
-from .ops_seglik import set_regulariser_group, _reduce_diag_max, unit_seed, sync_uniform  # noqa: E402
+from .ops_seglik import (set_regulariser_group, _reduce_diag_max, unit_seed, sync_uniform,  # noqa: E402
+                         diag_strides, _dense_diag_grad)
 
 
 def _work(tables: int, B: int, P: int, device) -> Tensor:
@@ -1138,6 +1176,71 @@ def proj_kl_cov(L: Tensor, L_o: Tensor, eps_cov: float, state: Tensor, warm: boo
     return _ProjKLCov.apply(L, L_o, eps_cov, state, warm, holder)
 
 
+KL_DIAG_STATE = 4       # per matrix: eta, KL step active, alpha, entropy control active
+
+
+@torch.library.custom_op("tce::proj_kl_diag", mutates_args=())
+def proj_kl_diag(L: Tensor, L_o: Tensor, eps_cov: float, beta: Optional[Tensor],
+                 equality: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """KL covariance projection of DIAGONAL factors (std_only policy), closed form, optionally followed by the entropy
+    control of ``proj_entropy`` (``beta`` [Bc] or [1] fp64; None = none).  L [Bc, n, n] and L_o [Bc or 1, n, n] are
+    read on their diagonals only (any strides) -> (out [Bc, n, n] diagonal, state [Bc, 4] fp64, info [Bc] int32)."""
+    ldb, inc = diag_strides(L)
+    ldb_o, inc_o = diag_strides(L_o, "L_o")
+    Bc, n = L.shape[0], L.shape[-1]
+    if L_o.shape[0] not in (1, Bc) or L_o.shape[-1] != n:
+        raise TceError("L_o must be [Bc, n, n] or [1, n, n]")
+    out, ldb_out, inc_out = _dense_diag_grad(L)
+    state = torch.empty(Bc, KL_DIAG_STATE, device=L.device, dtype=torch.float64)
+    info = torch.empty(Bc, device=L.device, dtype=torch.int32)
+    if beta is not None:
+        beta = _chk(beta, torch.float64, "beta")
+    _lib.call("tce_proj_kl_diag_fwd", _p(L), ldb, inc, _p(L_o), ldb_o, inc_o, float(eps_cov), _p(beta),
+              0 if beta is None or beta.numel() == 1 else 1, int(equality), _p(out), ldb_out, inc_out, _p(state),
+              _p(info), Bc, n, _stream())
+    return out, state, info
+
+
+@proj_kl_diag.register_fake
+def _(L, L_o, eps_cov, beta, equality):
+    Bc = L.shape[0]
+    return (L.new_empty(Bc, L.shape[-1], L.shape[-1]), L.new_empty(Bc, KL_DIAG_STATE, dtype=torch.float64),
+            L.new_empty(Bc, dtype=torch.int32))
+
+
+@torch.library.custom_op("tce::proj_kl_diag_bwd", mutates_args=())
+def proj_kl_diag_bwd(grad_out: Tensor, L: Tensor, L_o: Tensor, state: Tensor) -> Tensor:
+    """d loss / d L [Bc, n, n] (diagonal) from d loss / d out; L_o is a constant."""
+    ldb, inc = diag_strides(L)
+    ldb_o, inc_o = diag_strides(L_o, "L_o")
+    ldb_g, inc_g = diag_strides(grad_out, "grad_out")
+    state = _chk(state, torch.float64, "state")
+    g, ldb_gs, inc_gs = _dense_diag_grad(L)
+    _lib.call("tce_proj_kl_diag_bwd", _p(L), ldb, inc, _p(L_o), ldb_o, inc_o, _p(state), _p(grad_out), ldb_g, inc_g,
+              _p(g), ldb_gs, inc_gs, L.shape[0], L.shape[-1], _stream())
+    return g
+
+
+@proj_kl_diag_bwd.register_fake
+def _(grad_out, L, L_o, state):
+    return L.new_empty(L.shape[0], L.shape[-1], L.shape[-1])
+
+
+def _pkd_setup(ctx, inputs, output):
+    ctx.save_for_backward(inputs[0], inputs[1], output[1])
+    ctx.set_materialize_grads(False)
+
+
+def _pkd_backward(ctx, g, g_state, g_info):
+    if g is None:
+        return None, None, None, None, None
+    L, L_o, state = ctx.saved_tensors
+    return proj_kl_diag_bwd(g, L, L_o, state), None, None, None, None
+
+
+proj_kl_diag.register_autograd(_pkd_backward, setup_context=_pkd_setup)
+
+
 @torch.library.custom_op("tce::proj_frob_cov", mutates_args=())
 def proj_frob_cov(L: Tensor, L_o: Tensor, eps_cov: float) -> Tuple[Tensor, Tensor, Tensor]:
     L = _chk(L, name="L")
@@ -1280,4 +1383,4 @@ cov_distance.register_autograd(_cd_backward, setup_context=_cd_setup)
 # (3) product path of the segment likelihood: fused kernels
 # --------------------------------------------------------------------------------------------------
 from .ops_seglik import (seg_logprob, seg_surrogate, seglik, pairs_chained, times_uniform, declare_uniform,  # noqa: E402,F401
-                         shared_factor)
+                         shared_factor, seg_logprob_diag)

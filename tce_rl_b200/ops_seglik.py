@@ -425,6 +425,106 @@ def seg_logprob(smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pa
     return (logp, info, diag_max) if return_info else logp
 
 
+def diag_strides(L: Tensor, name: str = "L") -> Tuple[int, int]:
+    """(ldb, inc) of the diagonals of a [B, n, n] float32 CUDA factor as a strided vector: element i of episode b is
+    at ``data_ptr + b * ldb + i * inc`` (any strides; a single matrix or a stride-0 batch expand gives ldb = 0)."""
+    if not L.is_cuda or L.dtype != torch.float32 or L.dim() != 3 or L.shape[-1] != L.shape[-2]:
+        raise TceError(f"{name} must be a CUDA float32 [B, n, n] tensor")
+    return (0 if L.shape[0] == 1 else L.stride(0)), L.stride(1) + L.stride(2)
+
+
+def _dense_diag_grad(L: Tensor) -> Tuple[Tensor, int, int]:
+    """Zero [B, n, n] gradient buffer whose diagonal a kernel writes (ldb = n^2, inc = n + 1)."""
+    n = L.shape[-1]
+    return torch.zeros(L.shape[0], n, n, device=L.device, dtype=torch.float32), n * n, n + 1
+
+
+@torch.library.custom_op("tce::seglik_diag_fwd", mutates_args=())
+def seglik_diag_fwd(smp_traj: Tensor, mean: Tensor, L: Tensor, times: Tensor, init_time: Tensor, init_pos: Tensor,
+                    init_vel: Tensor, pred_pairs: Tensor, tables: int, reg_rel: float) -> Tuple[Tensor, Tensor, Tensor]:
+    """Diagonal per-episode factors L [B, Dp, Dp] (only the diagonal is read) -> (logp [B, P], diag_max [1] fp64,
+    info [B, P] int32)."""
+    smp_traj, mean, times = _chk(smp_traj, name="smp_traj"), _chk(mean, name="mean"), _chk(times, name="times")
+    init_time, init_pos, init_vel = _chk(init_time), _chk(init_pos), _chk(init_vel)
+    pairs = _chk(pred_pairs, torch.int64, "pred_pairs")
+    ldb, inc = diag_strides(L)
+    B, T = times.shape
+    P = pairs.shape[0]
+    dev = mean.device
+    diag_max = torch.zeros(1, device=dev, dtype=torch.float64)
+    logp = torch.empty(B, P, device=dev, dtype=torch.float32)
+    info = torch.empty(B, P, device=dev, dtype=torch.int32)
+    if B == 0:
+        return logp, diag_max, info
+    st = _stream()
+    _lib.call("tce_seglik_diag_max", tables, _p(L), ldb, inc, _p(times), _p(init_time), _p(pairs), _p(diag_max), B, T,
+              P, st)
+    _reduce_diag_max(diag_max)
+    _lib.call("tce_seglik_diag_fwd", tables, _p(smp_traj), _p(mean), _p(L), ldb, inc, _p(times), _p(init_time),
+              _p(init_pos), _p(init_vel), _p(pairs), _p(diag_max), float(reg_rel), _p(logp), _p(info), B, T, P, st)
+    return logp, diag_max, info
+
+
+@seglik_diag_fwd.register_fake
+def _(smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs, tables, reg_rel):
+    B, P = times.shape[0], pred_pairs.shape[0]
+    return mean.new_empty(B, P), mean.new_empty(1, dtype=torch.float64), mean.new_empty(B, P, dtype=torch.int32)
+
+
+@torch.library.custom_op("tce::seglik_diag_bwd", mutates_args=())
+def seglik_diag_bwd(grad_logp: Tensor, smp_traj: Tensor, mean: Tensor, L: Tensor, times: Tensor, init_time: Tensor,
+                    init_pos: Tensor, init_vel: Tensor, pred_pairs: Tensor, diag_max: Tensor, tables: int,
+                    reg_rel: float) -> Tuple[Tensor, Tensor]:
+    """-> (grad_mean [B, Dp], grad_L [B, Dp, Dp], non-zero on the diagonal only)."""
+    grad_logp = _chk(grad_logp, name="grad_logp")
+    smp_traj, mean, times = _chk(smp_traj), _chk(mean), _chk(times)
+    init_time, init_pos, init_vel = _chk(init_time), _chk(init_pos), _chk(init_vel)
+    pairs = _chk(pred_pairs, torch.int64, "pred_pairs")
+    ldb, inc = diag_strides(L)
+    B, T = times.shape
+    g_mean = torch.empty(B, mean.shape[-1], device=mean.device, dtype=torch.float32)
+    g_L, ldb_g, inc_g = _dense_diag_grad(L)
+    if B == 0:
+        return g_mean, g_L
+    _lib.call("tce_seglik_diag_bwd", tables, _p(smp_traj), _p(mean), _p(L), ldb, inc, _p(times), _p(init_time),
+              _p(init_pos), _p(init_vel), _p(pairs), _p(diag_max), float(reg_rel), _p(grad_logp), _p(g_mean), _p(g_L),
+              ldb_g, inc_g, B, T, pairs.shape[0], _stream())
+    return g_mean, g_L
+
+
+@seglik_diag_bwd.register_fake
+def _(grad_logp, smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs, diag_max, tables, reg_rel):
+    return mean.new_empty(mean.shape), L.new_empty(L.shape)
+
+
+def _seglik_diag_setup(ctx, inputs, output):
+    ctx.save_for_backward(*inputs[:8], output[1])
+    ctx.tables, ctx.reg_rel = inputs[8], inputs[9]
+    ctx.set_materialize_grads(False)
+
+
+def _seglik_diag_backward(ctx, g_logp, g_diag, g_info):
+    if g_logp is None:
+        return (None,) * 10
+    smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs, diag_max = ctx.saved_tensors
+    g_mean, g_L = seglik_diag_bwd(g_logp.contiguous(), smp_traj, mean, L, times, init_time, init_pos, init_vel,
+                                  pred_pairs, diag_max, ctx.tables, ctx.reg_rel)
+    return (None, g_mean if ctx.needs_input_grad[1] else None, g_L if ctx.needs_input_grad[2] else None) + (None,) * 7
+
+
+seglik_diag_fwd.register_autograd(_seglik_diag_backward, setup_context=_seglik_diag_setup)
+
+
+def seg_logprob_diag(smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs, tables, reg_rel: float = 1e-4,
+                     return_info: bool = False):
+    """Segment-wise log-likelihood [B, P] of a diagonal covariance (std_only policy) with per-episode factors
+    L [B, Dp, Dp]: only the diagonal of L is read, C is block diagonal per DoF (2 x 2 blocks), O(Dp) per segment.
+    Differentiable w.r.t. ``mean`` and ``L`` (the gradient w.r.t. L is zero off the diagonal)."""
+    logp, diag_max, info = seglik_diag_fwd(smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs,
+                                           tables.handle, float(reg_rel))
+    return (logp, info, diag_max) if return_info else logp
+
+
 def seg_surrogate(smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs, logp_old, advantage, tables,
                   reg_rel: float = 1e-4, uniform: Optional[bool] = None, sigma=None):
     """-> (surrogate loss = -mean(exp(lp - lp_old) * adv) [fp32 scalar, differentiable], mean ratio, logp).

@@ -25,8 +25,6 @@ class AbstractGaussianPolicy:
         if self.dtype != torch.float32:
             raise NotImplementedError("the sm_100a kernels take fp32 tensors (fp64 is used internally where "
                                       "the arithmetic is ill conditioned); pass dtype=float32")
-        if self.std_only:
-            raise NotImplementedError("std_only policies are not used by any TCE config and are not built")
         self.num_dof = dim_out
         self.min_std = float(kwargs.get("min_std", 1e-2))
         self.mean_net = self.variance_net = None
@@ -41,7 +39,7 @@ class AbstractGaussianPolicy:
                                                   device=self.device)
         cls = self.__class__.__name__
         self.mean_net = mk(cls + "_mean", self.dim_out, self.mean_net_args)
-        dim_var = self.dim_out + self.dim_out * (self.dim_out - 1) // 2
+        dim_var = self.dim_out if self.std_only else self.dim_out + self.dim_out * (self.dim_out - 1) // 2
         if self.contextual_cov:
             self.variance_net = mk(cls + "_variance", dim_var, self.variance_net_args)
         else:
@@ -83,14 +81,17 @@ class AbstractGaussianPolicy:
         rollout.load_net(self.variance_net, log_dir, epoch)
 
     def _vector_to_cholesky(self, cov_val: torch.Tensor, batch: int | None = None):
-        """softplus(diag) + min_std, strictly-lower row-major fill -- one fused kernel (``tce::policy_head``)."""
+        """softplus(diag) + min_std, strictly-lower row-major fill (std_only: diagonal only) -- one fused kernel
+        (``tce::policy_head`` / ``tce::policy_head_diag``)."""
+        head = ops.policy_head_diag if self.std_only else ops.policy_head
         if cov_val.dim() == 1:
-            return ops.policy_head(cov_val, int(batch), self.dim_out, self.min_std)
-        return ops.policy_head(cov_val, cov_val.shape[0], self.dim_out, self.min_std)
+            return head(cov_val, int(batch), self.dim_out, self.min_std)
+        return head(cov_val, cov_val.shape[0], self.dim_out, self.min_std)
 
     def _cholesky_to_vector(self, params_L: torch.Tensor):
-        diag, off = util.reverse_build_matrix(params_L, True)
-        return torch.cat([util.reverse_from_softplus_space(diag, self.min_std), off], dim=-1)
+        diag, off = util.reverse_build_matrix(params_L, not self.std_only)
+        diag = util.reverse_from_softplus_space(diag, self.min_std)
+        return diag if self.std_only else torch.cat([diag, off], dim=-1)
 
     def set_cov_variable(self, param_L: torch.Tensor):
         assert self.contextual_std is False, "Variance is a net instead of a variable."
@@ -168,13 +169,27 @@ class TemporalCorrelatedPolicy(BlackBoxPolicy):
     def log_prob(self, smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel, **kwargs):
         """TCE segment-wise likelihood [B, P] (temporal_correlated_policy.py:104-203)."""
         pred_pairs = kwargs["pred_pairs"]
+        if self._per_episode_diag(params_L, times.shape[0]):
+            return ops.seg_logprob_diag(smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel,
+                                        pred_pairs, self.mp.tables)
         return ops.seg_logprob(smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel, pred_pairs,
                                self.mp.tables)
+
+    def _per_episode_diag(self, params_L, batch):
+        """std_only with one factor per episode: the block-diagonal (2 x 2 per DoF) likelihood.  A factor shared by
+        the batch keeps the shared-covariance path, which forms the trajectory covariance once per batch."""
+        return self.is_diag and ops.shared_factor(params_L, batch) is None
 
     def segment_surrogate(self, smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel, pred_pairs,
                           log_prob_old, advantages):
         """Fused ``log_prob`` + ``surrogate_loss`` (temporal_correlated_agent.py:538-550,718-739): returns
-        (-mean(exp(lp_new - lp_old) * adv), mean importance ratio, lp_new) from two kernels, backward = one."""
+        (-mean(exp(lp_new - lp_old) * adv), mean importance ratio, lp_new) from two kernels, backward = one.
+        Per-episode diagonal factors: the diagonal likelihood, then the surrogate formula of the agent on its log-probs."""
+        if self._per_episode_diag(params_L, times.shape[0]):
+            lp = ops.seg_logprob_diag(smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel, pred_pairs,
+                                      self.mp.tables)
+            ratio = (lp - log_prob_old).exp()
+            return -(ratio * advantages).mean(), ratio.mean().detach(), lp.detach()
         return ops.seg_surrogate(smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel, pred_pairs,
                                  log_prob_old, advantages, self.mp.tables)
 

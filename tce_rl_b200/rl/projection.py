@@ -462,13 +462,16 @@ class KLProjectionLayer(BaseProjectionLayer):
         in the state: the covariance terms of the trust-region loss and of the logging decomposition are closed forms
         of it (``cache``: no gauss_stats launches), the trust-region covariance gradient is added inside the backward
         kernel (``get_trust_region_loss(fold=True)``)."""
-        if (not policy.contextual_std or policy.is_diag or not self.fuse_entropy or not p[1].is_cuda
-                or p[1].shape[-1] > 64):
+        if (not policy.contextual_std or not self.fuse_entropy or not p[1].is_cuda
+                or (p[1].shape[-1] > 64 and not policy.is_diag)):
             return None
         mean, L = p
         old_mean, old_L = q
         mean_part = self._mean_part(policy, p, q)
         proj_mean = ops.proj_mean(mean, old_mean, mean_part, self.mean_bound)
+        if policy.is_diag:
+            self.cache = {"new_old_mean": mean_part.detach()}
+            return proj_mean, self._diag_projection(L, old_L, beta)
         Lc = L.contiguous()
         state = self._state_for(Lc)
         self._last_state = state
@@ -512,16 +515,24 @@ class KLProjectionLayer(BaseProjectionLayer):
         self._old_linv = linv                                   # reused by the logging branch of the same epoch
         return 0.5 * _maha(policy, p[0], q[0], q[1], linv=linv)
 
+    def _diag_projection(self, L, L_old, beta):
+        """Diagonal factors (std_only policy): closed-form projection [+ entropy control], one warp per matrix.  No
+        eigen-system is kept, so nothing can be folded into its backward and no Sigma is handed to the likelihood."""
+        self._last_state = self._last_call = None
+        return ops.proj_kl_diag(L, L_old, self.cov_bound, beta, self.entropy_eq)[0]
+
     def _cov_projection(self, policy, L, L_old):
         if policy.is_diag:
-            raise NotImplementedError("diagonal KL projection is outside the TCE configs")
+            return self._diag_projection(L, L_old, None)
         Lc = L.contiguous()
         state = self._state_for(Lc)
         return ops.proj_kl_cov(Lc, L_old.contiguous(), self.cov_bound, state, self.warm_start, self)[0]
 
     def _cov_projection_with_entropy(self, policy, L, L_old, beta):
-        if policy.is_diag or not self.fuse_entropy:
+        if not self.fuse_entropy:
             return None
+        if policy.is_diag:
+            return self._diag_projection(L, L_old, beta)
         Lc = L.contiguous()
         state = self._state_for(Lc)
         self._last_state = state
