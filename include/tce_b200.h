@@ -248,7 +248,7 @@ int tce_proj_kl_bwd_sigma_k(const float *L, const double *grad_sigma, const doub
 /* tce_proj_kl_entropy_fwd in two launches: _sigma writes the state (Sigma_proj, alpha = entropy scale from the
  * closed-form log-determinant, ...; for an inactive projection also the outputs); _chol forms
  * proj_L = chol(Sigma_proj) and out_L = alpha proj_L from the state.  What only needs the covariance
- * (tce_seglik_gram_sigma) can be ordered after the first launch alone.                                    */
+ * (the likelihood's Sigma0 inputs) can be ordered after the first launch alone.                            */
 int tce_proj_kl_entropy_fwd_sigma(const float *L, const float *L_o, double eps_cov, const double *beta,
                                   int64_t ldb_beta, int equality, float *proj_L, float *out_L, double *save,
                                   int32_t *info, int warm_start, int64_t B, int n, void *stream);
@@ -297,14 +297,6 @@ int tce_seglik_gram(const tce_tables_t *tables, const float *smp_traj, const flo
                     int64_t ldb_L, const float *times, const float *init_time, const float *init_pos,
                     const float *init_vel, const int64_t *pred_pairs, void *work, double *diag_max,
                     int64_t B, int64_t T, int64_t P, void *stream);
-/* Stage 1 for ONE covariance shared by the batch, given as Sigma = (*sigma_scale) * Sigma0 [Dp, Dp] fp64 (device
- * pointers; sigma_scale may be NULL = 1) instead of its factor -- e.g. straight out of tce_proj_kl_entropy_fwd's
- * state: no L load and no L L^T per episode.                                                              */
-int tce_seglik_gram_sigma(const tce_tables_t *tables, const float *smp_traj, const float *mean,
-                          const double *Sigma0, const double *sigma_scale, const float *times,
-                          const float *init_time, const float *init_pos, const float *init_vel,
-                          const int64_t *pred_pairs, void *work, double *diag_max, int64_t B, int64_t T, int64_t P,
-                          void *stream);
 int tce_seglik_chol(const tce_tables_t *tables, const void *work, void *adj, const double *diag_max, double reg_rel,
                     const float *grad_logp, const float *logp_old, const float *advantage,
                     double grad_scale, double *loss_acc, float *logp, int32_t *info, int64_t B,
@@ -313,13 +305,6 @@ int tce_seglik_bwd(const tce_tables_t *tables, const void *work, const float *L,
                    const float *times, const float *init_time, const int64_t *pred_pairs,
                    const float *upstream, float *grad_mean, float *grad_L, int64_t B, int64_t T, int64_t P,
                    void *stream);
-/* ONE covariance for the batch (ldb_L = 0): grad_L = 2 tril(dSigma L) is linear in dSigma, so stage 3 can write
- * upstream * d logp / d Sigma [B, Dp, Dp] (symmetric) without touching L; tce_dsigma_to_dl sums it over the
- * batch (fixed order) and applies the product once: grad_L [n, n] = 2 tril((sum_b grad_sigma_b) L).       */
-int tce_seglik_bwd_dsigma(const tce_tables_t *tables, const void *work, const float *times,
-                          const float *init_time, const int64_t *pred_pairs, const float *upstream,
-                          float *grad_mean, float *grad_sigma, int64_t B, int64_t T, int64_t P, void *stream);
-int tce_dsigma_to_dl(const float *grad_sigma, int64_t B, const float *L, float *grad_L, int n, void *stream);
 /* Diagonal covariance (std_only policies, per-episode standard deviations s, strided as for tce_proj_kl_diag_*):
  * C is block diagonal with one 2 x 2 block per (pair, DoF), C_d[k,k'] = sum_j h_kj h_k'j s_{d,j}^2 + reg.
  * tce_seglik_diag_max: the regulariser seed diag_max = max over the batch of diag C (atomic max into *diag_max,

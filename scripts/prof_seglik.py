@@ -29,16 +29,6 @@ for _ in range(3):
     _lib.call("tce_seglik_gram", tabs.handle, p(traj), p(g["mean"]), p(g["L"]), Dp * Dp, p(times_g), p(g["init_time"]), p(g["init_pos"]), p(g["init_vel"]), p(pairs_g), p(work), p(dmax), B, T, P, st)
     _lib.call("tce_seglik_chol", tabs.handle, p(work), p(adj), p(dmax), 1e-4, p(glp), None, None, 0.0, None, p(logp), p(info), B, P, st)
     _lib.call("tce_seglik_bwd", tabs.handle, p(adj), p(g["L"]), Dp * Dp, p(times_g), p(g["init_time"]), p(pairs_g), None, p(gm), p(gL), B, T, P, st)
-# the shared-covariance variants that run inside the policy epoch of a non-contextual policy (Sigma in, dSigma out)
-L1 = g["L"][:1].contiguous()
-Sigma = (L1[0].double() @ L1[0].double().T).contiguous()
-one = torch.ones(1, device=dev, dtype=torch.float64)
-gS = torch.empty(B, Dp, Dp, device=dev); gL1 = torch.empty(1, Dp, Dp, device=dev)
-for _ in range(3):
-    _lib.call("tce_seglik_gram_sigma", tabs.handle, p(traj), p(g["mean"]), p(Sigma), p(one), p(times_g), p(g["init_time"]), p(g["init_pos"]), p(g["init_vel"]), p(pairs_g), p(work), p(dmax), B, T, P, st)
-    _lib.call("tce_seglik_chol", tabs.handle, p(work), p(adj), p(dmax), 1e-4, p(glp), None, None, 0.0, None, p(logp), p(info), B, P, st)
-    _lib.call("tce_seglik_bwd_dsigma", tabs.handle, p(adj), p(times_g), p(g["init_time"]), p(pairs_g), None, p(gm), p(gS), B, T, P, st)
-    _lib.call("tce_dsigma_to_dl", p(gS), B, p(L1), p(gL1), Dp, st)
 torch.cuda.synchronize()
 print("ok", float(logp.sum()))
 

@@ -90,11 +90,8 @@ SIGNATURES = {
     "tce_cov_distance": (C.c_int, [_I32, _P, _P, _I64, _I32, _P, _P, _P, _I64, _I32, _P]),
     "tce_seglik_work_bytes": (C.c_size_t, [_P, _I64, _I64]),
     "tce_seglik_gram": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
-    "tce_seglik_gram_sigma": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
     "tce_seglik_chol": (C.c_int, [_P, _P, _P, _P, _D, _P, _P, _P, _D, _P, _P, _P, _I64, _I64, _P]),
     "tce_seglik_bwd": (C.c_int, [_P, _P, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
-    "tce_seglik_bwd_dsigma": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
-    "tce_dsigma_to_dl": (C.c_int, [_P, _I64, _P, _P, _I32, _P]),
     "tce_seglik_fused_config": (C.c_int, [_P, _I64, _I64, _I32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                           C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "tce_seglik_prepass": (C.c_int, [_P] * 4 + [_I64] + [_P] * 9 + [_I32, _I64, _I64, _I64, _P]),

@@ -1571,15 +1571,6 @@ int num_sms_proj() {
   return sms;
 }
 
-bool kl_compact_enabled() {             // TCE_KL_COMPACT=0: always one 512-thread CTA per SM (cross-check)
-  static int on = -1;
-  if (on < 0) {
-    const char *e = getenv("TCE_KL_COMPACT");
-    on = !(e && e[0] == '0');
-  }
-  return on != 0;
-}
-
 template <typename K>
 int set_smem(K kernel, size_t smem) {
   if (smem > 220 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;
@@ -1808,7 +1799,7 @@ static int kl_fwd_launch(const float *L, const float *L_o, double eps_cov, const
     return TCE_ERR_INVALID_ARGUMENT;
   PJ_CHECK_N(n);
   // more matrices than SMs: two CTAs of 256 threads per SM on three buffers each (`compact`), else one of 512 on four
-  const int compact = B > num_sms_proj() && kl_compact_enabled();
+  const int compact = B > num_sms_proj();
   const size_t smem = pj_smem_exclusive(pj_smem(n, compact ? 3 : 4) + sizeof(double) * LA_JACOBI_SCRATCH, B);
   int rc = set_smem(proj_kl_cov_fwd_kernel, compact ? pj_smem(n, 4) + sizeof(double) * LA_JACOBI_SCRATCH : smem);
   if (rc) return rc;
@@ -1827,7 +1818,7 @@ static int kl_bwd_launch(const float *L, const float *proj_L, const float *grad_
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if (!L || !proj_L || !grad_out || !save || !grad_L || B < 0) return TCE_ERR_INVALID_ARGUMENT;
   PJ_CHECK_N(n);
-  const int compact = B > num_sms_proj() && kl_compact_enabled();      // as kl_fwd_launch: two 256-thread CTAs per SM
+  const int compact = B > num_sms_proj();      // as kl_fwd_launch: two 256-thread CTAs per SM
   const size_t smem = pj_smem_exclusive(pj_smem(n, compact ? 3 : 4), B);
   int rc = set_smem(proj_kl_cov_bwd_kernel, compact ? pj_smem(n, 4) : smem);
   if (rc) return rc;

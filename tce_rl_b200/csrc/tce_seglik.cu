@@ -97,13 +97,10 @@ __device__ void load_lower(const float *__restrict__ L, float *Ls, int n, int NR
 // =====================================================================================================
 // Stage 1: gram.  One CTA per episode.
 // =====================================================================================================
-// SIGMA_IN: the covariance Sigma = scale * Sigma0 ([Dp, Dp] fp64, ONE matrix for the batch, e.g. straight out of the
-// KL projection) is given instead of its factor: no L load and no L L^T per episode.
-template <int D, int K1, bool SIGMA_IN>
+template <int D, int K1>
 __global__ void __launch_bounds__(SL_THREADS, 4)
 seglik_gram_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *__restrict__ mean,
-                   const float *__restrict__ L, long long ldb_L, const double *__restrict__ Sigma0,
-                   const double *__restrict__ sigma_scale, const float *__restrict__ times,
+                   const float *__restrict__ L, long long ldb_L, const float *__restrict__ times,
                    const float *__restrict__ init_time, const float *__restrict__ init_pos,
                    const float *__restrict__ init_vel, const int64_t *__restrict__ pairs, double *__restrict__ Cmat,
                    double *__restrict__ Rres, double *__restrict__ diag_max, int T, int P) {
@@ -124,23 +121,7 @@ seglik_gram_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *_
   const float *times_b = times + b * T;
 
   SL_STAMP(0);
-  if (SIGMA_IN) {
-    const double sc = sigma_scale ? *sigma_scale : 1.0;
-    for (int e0 = threadIdx.x; e0 < Dp * Dp; e0 += 4 * SL_THREADS) {     // four loads in flight per thread
-      double v[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) v[u] = (e0 + u * SL_THREADS < Dp * Dp) ? Sigma0[e0 + u * SL_THREADS] : 0.0;
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const int e = e0 + u * SL_THREADS;
-        if (e < Dp * Dp) Sg[(e / Dp) * SD + (e % Dp)] = sc * v[u];
-      }
-    }
-    if (NR > Dp)                                                          // zero padding row / column
-      for (int t = threadIdx.x; t < NR; t += blockDim.x) { Sg[Dp * SD + t] = 0.0; Sg[t * SD + Dp] = 0.0; }
-  } else {
-    load_lower(L + b * ldb_L, Ls, Dp, NR4, LD);
-  }
+  load_lower(L + b * ldb_L, Ls, Dp, NR4, LD);
   __syncthreads();
   SL_STAMP(1);
   basis_points<K1>(tb, (double)init_time[b], times_b, pairs, P, hs, xi, init_row);   // ends with a barrier
@@ -148,7 +129,7 @@ seglik_gram_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *_
 
   // ---- Sigma = L L^T (fp32 FFMA, 4x4 register tiles over the lower triangle: 8 LDS per 16 FFMA) -> Sg (fp64,
   //      mirrored).  Rows/cols are padded to NR4 (multiple of 4) with zeros.
-  if (!SIGMA_IN) {
+  {
     constexpr int NT4 = NR4 / 4;
     for (int t = threadIdx.x; t < tri(NT4); t += blockDim.x) {
       int I, J;
@@ -428,10 +409,7 @@ seglik_chol_kernel(const double *Cmat, const double *Rres, double *Gout, double 
 // =====================================================================================================
 // Stage 3: backward accumulation.  One CTA per episode.
 // =====================================================================================================
-// DSIGMA: write up * d logp / d Sigma (symmetric [Dp, Dp]) instead of grad_L = 2 up tril(dSigma L).  With ONE
-// covariance for the batch the product with L is linear in dSigma, so it is applied once to the batch sum
-// (dsigma_to_dl_kernel) instead of once per episode, and L is not loaded at all.
-template <int D, int K1, bool DSIGMA>
+template <int D, int K1>
 __global__ void __launch_bounds__(SL_THREADS, 4)
 seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__restrict__ Alpha,
                   const float *__restrict__ L, long long ldb_L, const float *__restrict__ times,
@@ -456,7 +434,7 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
   const float up = upstream ? *upstream : 1.0f;       // scalar gradient of the fused surrogate loss
 
   SL_STAMP(16);
-  if (!DSIGMA) load_lower(L + b * ldb_L, Ls, Dp, NR, LD);
+  load_lower(L + b * ldb_L, Ls, Dp, NR, LD);
   for (int e = threadIdx.x; e < NT * P; e += blockDim.x) Gs[e] = (float)Gb[e];
   for (int e = threadIdx.x; e < NR * LD; e += blockDim.x) Ms[e] = 0.f;
   basis_points<K1>(tb, (double)init_time[b], times + b * T, pairs, P, hs, xi, init_row);
@@ -505,11 +483,6 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
   __syncthreads();
 
   SL_STAMP(19);
-  if (DSIGMA) {                                   // up * dSigma, symmetric, dense [Dp][Dp]
-    float *gS = grad_L + (size_t)b * Dp * Dp;
-    for (int e = threadIdx.x; e < Dp * Dp; e += blockDim.x) gS[e] = up * Ms[(e / Dp) * LD + (e % Dp)];
-    return;
-  }
   // ---- grad_L = 2 * tril(M L)  (fp32 FFMA, 4x4 tiles over the lower triangle), staged in the Gs buffer
   float *out = Gs;                                // [Dp][Dp] dense (the Gs region is sized for it)
   for (int e = threadIdx.x; e < Dp * Dp; e += blockDim.x) out[e] = 0.f;
@@ -548,53 +521,6 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
   float *gL = grad_L + (size_t)b * Dp * Dp;
   for (int e = threadIdx.x; e < Dp * Dp; e += blockDim.x) gL[e] = out[e];
   SL_STAMP(21);
-}
-
-// grad_L = 2 tril((sum_b dSigma_b) L): CTA per row i.  Stage 1: the row of the batch sum (B x n values, four
-// interleaved partial sums per column, fixed order -> deterministic); stage 2: thread per column j, fp32 as the
-// per-episode product it replaces, L read coalesced straight from L2 with eight loads in flight.
-constexpr int DS_PARTS = 16;                                      // 1024 threads = 16 batch slices x 64 columns
-__global__ void __launch_bounds__(DS_PARTS * 64)
-dsigma_to_dl_kernel(const float *__restrict__ dS, long long B, const float *__restrict__ L, float *__restrict__ out,
-                    int n) {
-  extern __shared__ float sm_f[];
-  float *part = sm_f, *srow = sm_f + DS_PARTS * 64;               // [16][64] partial sums, [n] row
-  const int i = blockIdx.x, k = threadIdx.x & 63, q = threadIdx.x >> 6;
-  const size_t nn = (size_t)n * n;
-  for (int k0 = 0; k0 < n; k0 += 64) {                              // n <= 128: at most two passes
-    float a[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};          // eight loads in flight per thread
-    if (k0 + k < n) {
-      const float *src = dS + (size_t)i * n + k0 + k;
-      long long b = q;
-      for (; b + 7 * DS_PARTS < B; b += 8 * DS_PARTS) {
-#pragma unroll
-        for (int u = 0; u < 8; ++u) a[u] += src[(size_t)(b + u * DS_PARTS) * nn];
-      }
-      for (; b < B; b += DS_PARTS) a[0] += src[(size_t)b * nn];
-    }
-    part[q * 64 + k] = ((a[0] + a[1]) + (a[2] + a[3])) + ((a[4] + a[5]) + (a[6] + a[7]));
-    __syncthreads();
-    if (threadIdx.x < 64 && k0 + k < n) {
-      float t = 0.f;
-#pragma unroll
-      for (int u = 0; u < DS_PARTS; ++u) t += part[u * 64 + k];
-      srow[k0 + k] = t;
-    }
-    __syncthreads();
-  }
-  for (int j = threadIdx.x; j < n; j += blockDim.x) {
-    float acc[4] = {0.f, 0.f, 0.f, 0.f};
-    if (j <= i) {
-      int kk = j;                                                   // L[k][j] = 0 for k < j
-#pragma unroll 2
-      for (; kk + 3 < n; kk += 4) {
-#pragma unroll
-        for (int u = 0; u < 4; ++u) acc[u] = fmaf(srow[kk + u], L[(size_t)(kk + u) * n + j], acc[u]);
-      }
-      for (; kk < n; ++kk) acc[0] = fmaf(srow[kk], L[(size_t)kk * n + j], acc[0]);
-    }
-    out[(size_t)i * n + j] = j <= i ? 2.f * ((acc[0] + acc[1]) + (acc[2] + acc[3])) : 0.f;
-  }
 }
 
 // =====================================================================================================
@@ -785,14 +711,12 @@ static inline double *work_R(const tce_tables_t *t, void *work, int64_t B, int64
   return (double *)work + (size_t)B * (size_t)P * (N * (N + 1) / 2);
 }
 
-template <bool SIGMA_IN>
-static int seglik_gram_launch(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *L,
-                              int64_t ldb_L, const double *Sigma0, const double *sigma_scale, const float *times,
-                              const float *init_time, const float *init_pos, const float *init_vel,
-                              const int64_t *pred_pairs, void *work, double *diag_max, int64_t B, int64_t T, int64_t P,
-                              void *stream) {
+extern "C" int tce_seglik_gram(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *L,
+                               int64_t ldb_L, const float *times, const float *init_time, const float *init_pos,
+                               const float *init_vel, const int64_t *pred_pairs, void *work, double *diag_max,
+                               int64_t B, int64_t T, int64_t P, void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
-  if (!t || !smp_traj || !mean || (SIGMA_IN ? !Sigma0 : !L) || !times || !init_time || !init_pos || !init_vel ||
+  if (!t || !smp_traj || !mean || !L || !times || !init_time || !init_pos || !init_vel ||
       !pred_pairs || !work || !diag_max || B < 0 || T < 1 || P < 1 || P > 4096)
     return TCE_ERR_INVALID_ARGUMENT;
   cudaStream_t st = (cudaStream_t)stream;
@@ -801,36 +725,19 @@ static int seglik_gram_launch(const tce_tables_t *t, const float *smp_traj, cons
   if (t->D == Dv && t->K1 == Kv) {                                                                                \
     const size_t smem = gram_smem<Dv, Kv>((int)P);                                                                \
     if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;                                                      \
-    TCE_CUDA(cudaFuncSetAttribute(seglik_gram_kernel<Dv, Kv, SIGMA_IN>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+    TCE_CUDA(cudaFuncSetAttribute(seglik_gram_kernel<Dv, Kv>, cudaFuncAttributeMaxDynamicSharedMemorySize,       \
                                   (int)smem), "gram smem attr");                                                  \
-    cudaFuncSetAttribute(seglik_gram_kernel<Dv, Kv, SIGMA_IN>, cudaFuncAttributePreferredSharedMemoryCarveout,    \
+    cudaFuncSetAttribute(seglik_gram_kernel<Dv, Kv>, cudaFuncAttributePreferredSharedMemoryCarveout,              \
                          cudaSharedmemCarveoutMaxShared);                                                         \
-    seglik_gram_kernel<Dv, Kv, SIGMA_IN><<<(unsigned)B, SL_THREADS, smem, st>>>(                                   \
-        tab_dev(t), smp_traj, mean, L, ldb_L, Sigma0, sigma_scale, times, init_time, init_pos, init_vel, pred_pairs, \
-        Cmat, R, diag_max, (int)T, (int)P);                                                                       \
+    seglik_gram_kernel<Dv, Kv><<<(unsigned)B, SL_THREADS, smem, st>>>(                                             \
+        tab_dev(t), smp_traj, mean, L, ldb_L, times, init_time, init_pos, init_vel, pred_pairs, Cmat, R, diag_max, \
+        (int)T, (int)P);                                                                                          \
     TCE_CHECK_LAUNCH("seglik_gram_kernel");                                                                       \
     return TCE_OK;                                                                                                \
   }
   TCE_FOR_SHAPES(X)
 #undef X
   return TCE_ERR_UNSUPPORTED_SHAPE;
-}
-
-extern "C" int tce_seglik_gram(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *L,
-                               int64_t ldb_L, const float *times, const float *init_time, const float *init_pos,
-                               const float *init_vel, const int64_t *pred_pairs, void *work, double *diag_max,
-                               int64_t B, int64_t T, int64_t P, void *stream) {
-  return seglik_gram_launch<false>(t, smp_traj, mean, L, ldb_L, nullptr, nullptr, times, init_time, init_pos, init_vel,
-                                   pred_pairs, work, diag_max, B, T, P, stream);
-}
-
-extern "C" int tce_seglik_gram_sigma(const tce_tables_t *t, const float *smp_traj, const float *mean,
-                                     const double *Sigma0, const double *sigma_scale, const float *times,
-                                     const float *init_time, const float *init_pos, const float *init_vel,
-                                     const int64_t *pred_pairs, void *work, double *diag_max, int64_t B, int64_t T,
-                                     int64_t P, void *stream) {
-  return seglik_gram_launch<true>(t, smp_traj, mean, nullptr, 0, Sigma0, sigma_scale, times, init_time, init_pos,
-                                  init_vel, pred_pairs, work, diag_max, B, T, P, stream);
 }
 
 extern "C" int tce_seglik_chol(const tce_tables_t *t, const void *work, void *adj, const double *diag_max, double reg_rel,
@@ -862,12 +769,12 @@ extern "C" int tce_seglik_chol(const tce_tables_t *t, const void *work, void *ad
   return TCE_OK;
 }
 
-template <bool DSIGMA>
-static int seglik_bwd_launch(const tce_tables_t *t, const void *work, const float *L, int64_t ldb_L, const float *times,
-                             const float *init_time, const int64_t *pred_pairs, const float *upstream,
-                             float *grad_mean, float *grad_out, int64_t B, int64_t T, int64_t P, void *stream) {
+extern "C" int tce_seglik_bwd(const tce_tables_t *t, const void *work, const float *L, int64_t ldb_L,
+                              const float *times, const float *init_time, const int64_t *pred_pairs,
+                              const float *upstream, float *grad_mean, float *grad_L, int64_t B, int64_t T,
+                              int64_t P, void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
-  if (!t || !work || (!DSIGMA && !L) || !times || !init_time || !pred_pairs || B < 0 || T < 1 || P < 1)
+  if (!t || !work || !L || !times || !init_time || !pred_pairs || B < 0 || T < 1 || P < 1)
     return TCE_ERR_INVALID_ARGUMENT;
   cudaStream_t st = (cudaStream_t)stream;
   const double *G = (const double *)work, *A = work_R(t, const_cast<void *>(work), B, P);
@@ -875,35 +782,18 @@ static int seglik_bwd_launch(const tce_tables_t *t, const void *work, const floa
   if (t->D == Dv && t->K1 == Kv) {                                                                               \
     const size_t smem = bwd_smem<Dv, Kv>((int)P);                                                                \
     if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;                                                     \
-    TCE_CUDA(cudaFuncSetAttribute(seglik_bwd_kernel<Dv, Kv, DSIGMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+    TCE_CUDA(cudaFuncSetAttribute(seglik_bwd_kernel<Dv, Kv>, cudaFuncAttributeMaxDynamicSharedMemorySize,        \
                                   (int)smem), "bwd smem attr");                                                  \
-    cudaFuncSetAttribute(seglik_bwd_kernel<Dv, Kv, DSIGMA>, cudaFuncAttributePreferredSharedMemoryCarveout,      \
+    cudaFuncSetAttribute(seglik_bwd_kernel<Dv, Kv>, cudaFuncAttributePreferredSharedMemoryCarveout,              \
                          cudaSharedmemCarveoutMaxShared);                                                        \
-    seglik_bwd_kernel<Dv, Kv, DSIGMA><<<(unsigned)B, SL_THREADS, smem, st>>>(                                     \
-        tab_dev(t), G, A, L, ldb_L, times, init_time, pred_pairs, upstream, grad_mean, grad_out, (int)T, (int)P); \
+    seglik_bwd_kernel<Dv, Kv><<<(unsigned)B, SL_THREADS, smem, st>>>(                                             \
+        tab_dev(t), G, A, L, ldb_L, times, init_time, pred_pairs, upstream, grad_mean, grad_L, (int)T, (int)P);   \
     TCE_CHECK_LAUNCH("seglik_bwd_kernel");                                                                       \
     return TCE_OK;                                                                                               \
   }
   TCE_FOR_SHAPES(X)
 #undef X
   return TCE_ERR_UNSUPPORTED_SHAPE;
-}
-
-extern "C" int tce_seglik_bwd(const tce_tables_t *t, const void *work, const float *L, int64_t ldb_L,
-                              const float *times, const float *init_time, const int64_t *pred_pairs,
-                              const float *upstream, float *grad_mean, float *grad_L, int64_t B, int64_t T,
-                              int64_t P, void *stream) {
-  return seglik_bwd_launch<false>(t, work, L, ldb_L, times, init_time, pred_pairs, upstream, grad_mean, grad_L, B, T,
-                                  P, stream);
-}
-
-extern "C" int tce_seglik_bwd_dsigma(const tce_tables_t *t, const void *work, const float *times,
-                                     const float *init_time, const int64_t *pred_pairs, const float *upstream,
-                                     float *grad_mean, float *grad_sigma, int64_t B, int64_t T, int64_t P,
-                                     void *stream) {
-  if (B != 0 && !grad_sigma) return TCE_ERR_INVALID_ARGUMENT;
-  return seglik_bwd_launch<true>(t, work, nullptr, 0, times, init_time, pred_pairs, upstream, grad_mean, grad_sigma,
-                                 B, T, P, stream);
 }
 
 template <int MODE>
@@ -966,13 +856,4 @@ extern "C" int tce_seglik_diag_bwd(const tce_tables_t *t, const float *smp_traj,
   return seglik_diag_launch<2>(t, smp_traj, mean, s, ldb_s, inc_s, times, init_time, init_pos, init_vel, pred_pairs,
                                const_cast<double *>(diag_max), reg_rel, grad_logp, nullptr, nullptr, grad_mean, grad_s,
                                ldb_gs, inc_gs, B, T, P, stream);
-}
-
-extern "C" int tce_dsigma_to_dl(const float *grad_sigma, int64_t B, const float *L, float *grad_L, int n,
-                                void *stream) {
-  if (!grad_sigma || !L || !grad_L || n < 1 || n > 128 || B < 1) return TCE_ERR_INVALID_ARGUMENT;
-  dsigma_to_dl_kernel<<<(unsigned)n, DS_PARTS * 64, sizeof(float) * (DS_PARTS * 64 + 128), (cudaStream_t)stream>>>(
-      grad_sigma, (long long)B, L, grad_L, n);
-  TCE_CHECK_LAUNCH("dsigma_to_dl_kernel");
-  return TCE_OK;
 }

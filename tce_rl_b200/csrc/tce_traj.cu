@@ -2,26 +2,11 @@
 // Replaces ProDMP.get_traj_pos / get_traj_vel behind TemporalCorrelatedPolicy.sample
 // (mprl/rl/policy/temporal_correlated_policy.py:76-100); math: SURVEY App. A.5.
 //
-// HBM-bound (algorithmic bytes/episode = 4*[Dp + (1+2D) + T + 2D*T]).  The fp32 basis rows are staged
-// in shared memory once per (persistent) CTA; every thread owns one (episode, time) point, results go
-// through a shared tile so that the global stores are contiguous float4.
-#include <stdlib.h>
-
+// HBM-bound (algorithmic bytes/episode = 4*[Dp + (1+2D) + T + 2D*T]).  General time grids run
+// traj_fwd_warp_kernel; a time grid common to the whole batch runs traj_rows_kernel + traj_uniform_kernel.
 #include "tce_common.cuh"
 
 namespace {
-
-constexpr int TRAJ_THREADS = 256;
-constexpr int MAX_EP_PER_CHUNK = 32;   // chunk of 256 time points spans <= 256/T + 2 episodes
-
-struct EpInit {     // per-episode values at init_time
-  float y1b, y2b, dy1b, dy2b, inv_det;
-  float pb[TCE_MAX_K1], vb[TCE_MAX_K1];
-};
-
-__device__ __forceinline__ const float *tab_row(const TabDev &tb, const float *srow, int staged_rows, int i) {
-  return i < staged_rows ? srow + (size_t)i * tb.row32_stride : tb.row32 + (size_t)i * tb.row32_stride;
-}
 
 // index of a time in the pre-computed grid without divisions (inv_tau = 1 / tau, fp64)
 __device__ __forceinline__ void time_to_index_fast(const TabDev &tb, double inv_tau, float t, int &i0, float &w) {
@@ -34,114 +19,7 @@ __device__ __forceinline__ void time_to_index_fast(const TabDev &tb, double inv_
   w = (float)(idx - (double)f);
 }
 
-template <int K1>
-__global__ void __launch_bounds__(TRAJ_THREADS)
-traj_fwd_kernel(TabDev tb, const float *__restrict__ params, const float *__restrict__ times,
-                const float *__restrict__ init_time, const float *__restrict__ init_pos,
-                const float *__restrict__ init_vel, float *__restrict__ traj, long long B, int T,
-                int staged_rows, int chunk) {
-  extern __shared__ __align__(16) float smem[];
-  const int D = tb.D, D2 = 2 * D, Dp = D * K1, stride = tb.row32_stride;
-  const int ep_floats = Dp + D2;                                  // theta | y0 | v0 * tau  per episode
-  float *tile = smem;                                             // [TRAJ_THREADS][2D] output tile (16B aligned)
-  EpInit *eps = reinterpret_cast<EpInit *>(tile + TRAJ_THREADS * D2);
-  float *epd = reinterpret_cast<float *>(eps + MAX_EP_PER_CHUNK);  // [MAX_EP_PER_CHUNK][ep_floats]
-  float *srow = epd + MAX_EP_PER_CHUNK * ep_floats;               // staged table rows
-  __shared__ float s_scale[TCE_MAX_K1];
-
-  for (int i = threadIdx.x; i < staged_rows * stride; i += blockDim.x) srow[i] = tb.row32[i];
-  if (threadIdx.x < K1) s_scale[threadIdx.x] = (float)tb.scale[threadIdx.x];
-  __syncthreads();
-
-  const long long total = B * (long long)T;
-  const float tau = (float)tb.tau, inv_tau_f = 1.0f / tau;
-  const double inv_tau = 1.0 / tb.tau;
-  const float goal_shift_scale = tb.relative_goal ? (tb.relative_goal_scaled ? 1.0f : 1.0f / s_scale[K1 - 1]) : 0.0f;
-  // chunk = time points per CTA iteration: TRAJ_THREADS, or fewer for very short trajectories (T < 9: the time
-  // PAIRS of the mp_pytorch surface) so that a chunk never spans more than MAX_EP_PER_CHUNK episodes
-  for (long long g0 = (long long)blockIdx.x * chunk; g0 < total; g0 += (long long)gridDim.x * chunk) {
-    const long long b_first = g0 / T;
-    long long g_last = g0 + chunk - 1;
-    if (g_last >= total) g_last = total - 1;
-    const int n_ep = (int)(g_last / T - b_first) + 1;
-    // per-episode data: initial-condition basis values, parameters, y0, v0 * tau
-    for (int e = threadIdx.x; e < n_ep; e += blockDim.x) {
-      int i0; float wf;
-      time_to_index_fast(tb, inv_tau, init_time[b_first + e], i0, wf);
-      const float *r0 = tab_row(tb, srow, staged_rows, i0), *r1 = tab_row(tb, srow, staged_rows, i0 + 1);
-      EpInit &E = eps[e];
-      E.y1b = lerp_t(r0[0], r1[0], wf); E.y2b = lerp_t(r0[1], r1[1], wf);
-      E.dy1b = lerp_t(r0[2], r1[2], wf); E.dy2b = lerp_t(r0[3], r1[3], wf);
-      E.inv_det = 1.0f / (E.y1b * E.dy2b - E.y2b * E.dy1b);
-#pragma unroll
-      for (int j = 0; j < K1; ++j) {
-        E.pb[j] = lerp_t(r0[4 + j], r1[4 + j], wf);
-        E.vb[j] = lerp_t(r0[4 + K1 + j], r1[4 + K1 + j], wf);
-      }
-    }
-    for (int i = threadIdx.x; i < n_ep * ep_floats; i += blockDim.x) {
-      const int e = i / ep_floats, k = i - e * ep_floats;
-      const long long bb = b_first + e;
-      float v;
-      if (k < Dp) v = params[bb * Dp + k];
-      else if (k < Dp + D) v = init_pos[bb * D + (k - Dp)];
-      else v = init_vel[bb * D + (k - Dp - D)] * tau;
-      epd[i] = v;
-    }
-    __syncthreads();
-    const long long g = g0 + threadIdx.x;
-    if (g < total && (int)threadIdx.x < chunk) {
-      const int e = (int)(g / T - b_first);
-      const EpInit &E = eps[e];
-      const float *ed = epd + e * ep_floats;
-      int i0; float wf;
-      time_to_index_fast(tb, inv_tau, times[g], i0, wf);
-      const float *r0 = tab_row(tb, srow, staged_rows, i0), *r1 = tab_row(tb, srow, staged_rows, i0 + 1);
-      const float y1 = lerp_t(r0[0], r1[0], wf), y2 = lerp_t(r0[1], r1[1], wf);
-      const float dy1 = lerp_t(r0[2], r1[2], wf), dy2 = lerp_t(r0[3], r1[3], wf);
-      const float xi1 = (E.dy2b * y1 - E.dy1b * y2) * E.inv_det, xi2 = (E.y1b * y2 - E.y2b * y1) * E.inv_det;
-      const float xi3 = (E.dy2b * dy1 - E.dy1b * dy2) * E.inv_det, xi4 = (E.y1b * dy2 - E.y2b * dy1) * E.inv_det;
-      float hp[K1], hv[K1];
-#pragma unroll
-      for (int j = 0; j < K1; ++j) {
-        const float pj = lerp_t(r0[4 + j], r1[4 + j], wf), vj = lerp_t(r0[4 + K1 + j], r1[4 + K1 + j], wf);
-        hp[j] = (pj - xi1 * E.pb[j] - xi2 * E.vb[j]) * s_scale[j];
-        hv[j] = (vj - xi3 * E.pb[j] - xi4 * E.vb[j]) * s_scale[j];
-      }
-      float *o = tile + threadIdx.x * D2;
-      for (int d = 0; d < D; ++d) {
-        const float y0 = ed[Dp + d], v0 = ed[Dp + D + d];
-        float p = xi1 * y0 + xi2 * v0, v = xi3 * y0 + xi4 * v0;
-        const float *th = ed + d * K1;
-#pragma unroll
-        for (int j = 0; j < K1; ++j) {
-          p = fmaf(hp[j], th[j], p);
-          v = fmaf(hv[j], th[j], v);
-        }
-        const float shift = goal_shift_scale * y0;         // relative goal (0 otherwise)
-        p = fmaf(hp[K1 - 1], shift, p);
-        v = fmaf(hv[K1 - 1], shift, v);
-        o[d] = p;
-        o[D + d] = v * inv_tau_f;
-      }
-    }
-    __syncthreads();
-    // contiguous store of the tile
-    const long long n_out = ((g_last - g0) + 1) * D2;
-    float *dst = traj + g0 * D2;
-    if ((n_out & 3) == 0 && ((g0 * D2) & 3) == 0) {
-      const float4 *s4 = reinterpret_cast<const float4 *>(tile);
-      float4 *d4 = reinterpret_cast<float4 *>(dst);
-      for (int i = threadIdx.x; i < n_out / 4; i += blockDim.x) d4[i] = s4[i];
-    } else {
-      for (int i = threadIdx.x; i < n_out; i += blockDim.x) dst[i] = tile[i];
-    }
-    __syncthreads();
-  }
-}
-
-
-// Warp-per-slab variant (the product path): a warp owns 32 consecutive time points of ONE episode, so everything
+// Warp-per-slab kernel (any time grid): a warp owns 32 consecutive time points of ONE episode, so everything
 // per-episode (basis values at the initial time, parameters, initial conditions) is warp-uniform: the initial-condition
 // row is built cooperatively (lane j -> basis column j) and broadcast by shuffles, the parameters are warp-uniform
 // (broadcast) loads through L1, the table rows are read through L1 as well (44 KB of fp32 rows: resident).  No shared
@@ -474,61 +352,18 @@ int launch_traj_uniform(const tce_tables *t, const float *params, const float *t
   return TCE_OK;
 }
 
-bool g_traj_cta = false;
-int g_traj_stage = -1;      // TCE_TRAJ_STAGE: 0 = read the basis rows through L1, 1 = stage them in smem (default)
-
 template <int K1>
 int launch_traj_fwd(const tce_tables *t, const float *params, const float *times, const float *init_time,
                     const float *init_pos, const float *init_vel, float *traj, int64_t B, int64_t T,
                     cudaStream_t st) {
-  if (g_traj_stage < 0) {
-    const char *e = getenv("TCE_TRAJ_STAGE");
-    g_traj_stage = e ? atoi(e) : 1;
-    const char *k = getenv("TCE_TRAJ_KERNEL");
-    g_traj_cta = k && k[0] == 'c';                 // "cta": the chunk-per-CTA kernel (kept for cross-checks)
-  }
-  if (!g_traj_cta) {
-    const long long slabs = B * ((T + 31) / 32);
-    long long grid = (slabs + TW_WARPS - 1) / TW_WARPS;
-    const long long cap = 8LL * num_sms();
-    if (grid > cap) grid = cap;
-    const size_t smem_w = (size_t)TW_WARPS * (32 * 2 * t->D + 4) * sizeof(float);
-    traj_fwd_warp_kernel<K1, TCE_MAX_DOF><<<(unsigned)grid, TW_WARPS * 32, smem_w, st>>>(
-        tab_dev(t), params, times, init_time, init_pos, init_vel, traj, B, (int)T);
-    TCE_CHECK_LAUNCH("traj_fwd_warp_kernel");
-    return TCE_OK;
-  }
-  const int stride = t->row32_stride;
-  const size_t row_bytes = (size_t)stride * sizeof(float);
-  int chunk = TRAJ_THREADS;
-  if ((TRAJ_THREADS + T - 1) / T + 2 > MAX_EP_PER_CHUNK) chunk = (int)((MAX_EP_PER_CHUNK - 2) * T);   // T < 9
-  const long long chunks = (B * T + chunk - 1) / chunk;
-  // Staging the rows pays only when a persistent CTA reuses them over several chunks; short-lived
-  // CTAs read the (few, hot) rows through L1 instead.
-  int staged = (int)((64 * 1024) / row_bytes);
-  if (staged > t->num_pc) staged = t->num_pc;
-  const size_t base_smem = (size_t)TRAJ_THREADS * 2 * t->D * sizeof(float) + MAX_EP_PER_CHUNK * sizeof(EpInit) +
-                           (size_t)MAX_EP_PER_CHUNK * (t->D * K1 + 2 * t->D) * sizeof(float) + 16;
-  int ctas_per_sm = (int)((220 * 1024) / (base_smem + (size_t)staged * row_bytes));
-  if (ctas_per_sm > 8) ctas_per_sm = 8;
-  long long grid = (long long)ctas_per_sm * num_sms();
-  if (!g_traj_stage || chunks < 4 * grid) {
-    staged = 0;
-    grid = 8LL * num_sms();
-  }
-  if (grid > chunks) grid = chunks;
-  const size_t smem = base_smem + (size_t)staged * row_bytes;
-  static bool attr_set = false;
-  if (!attr_set) {
-    TCE_CUDA(cudaFuncSetAttribute(traj_fwd_kernel<K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024),
-             "traj smem attr");
-    cudaFuncSetAttribute(traj_fwd_kernel<K1>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                         cudaSharedmemCarveoutMaxShared);
-    attr_set = true;
-  }
-  traj_fwd_kernel<K1><<<(unsigned)grid, TRAJ_THREADS, smem, st>>>(tab_dev(t), params, times, init_time, init_pos,
-                                                                  init_vel, traj, B, (int)T, staged, chunk);
-  TCE_CHECK_LAUNCH("traj_fwd_kernel");
+  const long long slabs = B * ((T + 31) / 32);
+  long long grid = (slabs + TW_WARPS - 1) / TW_WARPS;
+  const long long cap = 8LL * num_sms();
+  if (grid > cap) grid = cap;
+  const size_t smem_w = (size_t)TW_WARPS * (32 * 2 * t->D + 4) * sizeof(float);
+  traj_fwd_warp_kernel<K1, TCE_MAX_DOF><<<(unsigned)grid, TW_WARPS * 32, smem_w, st>>>(
+      tab_dev(t), params, times, init_time, init_pos, init_vel, traj, B, (int)T);
+  TCE_CHECK_LAUNCH("traj_fwd_warp_kernel");
   return TCE_OK;
 }
 

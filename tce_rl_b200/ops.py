@@ -317,11 +317,20 @@ def _(mean, L, mean_o, L_o):
 # --------------------------------------------------------------------------------------------------
 # (3) segment-wise trajectory likelihood
 # --------------------------------------------------------------------------------------------------
-# The product path of the likelihood is the fused implementation in ops_seglik.py (re-exported at the end of this
-# module); the STAGED ops below (gram / chol / bwd with an fp64 HBM workspace) are kept as an independent
-# implementation for cross-checks (tests) and for mp.ProDMP.get_traj_pos_cov.
+# Two implementations of the likelihood.  A shared covariance runs the fused kernels in ops_seglik.py (re-exported at
+# the end of this module); per-episode factors run the STAGED ops below (gram / chol / bwd with an fp64 HBM workspace,
+# see ops_seglik.PER_EPISODE_STAGED).  The staged gram kernel also serves mp.ProDMP.get_traj_pos_cov, and the tests use
+# the staged ops as an independent reference for the fused kernels.
 from .ops_seglik import (set_regulariser_group, _reduce_diag_max, unit_seed, sync_uniform,  # noqa: E402
                          diag_strides, _dense_diag_grad)
+
+
+def _episode_factors(L: Tensor, B: int, n: int) -> Tuple[Tensor, int]:
+    """(storage, batch stride) of the per-episode factors L [B, n, n] read by the staged kernels; a stride-0 batch
+    expand of one matrix is fine.  A [1, n, n] factor with B > 1 is refused: the kernels would read past its end."""
+    if tuple(L.shape) != (B, n, n):
+        raise TceError(f"L must be [B, n, n] = [{B}, {n}, {n}], got {list(L.shape)}")
+    return _batched_matrix(L)
 
 
 def _work(tables: int, B: int, P: int, device) -> Tensor:
@@ -336,8 +345,8 @@ def seglik_fwd(smp_traj: Tensor, mean: Tensor, L: Tensor, times: Tensor, init_ti
     smp_traj, mean, times = _chk(smp_traj, name="smp_traj"), _chk(mean, name="mean"), _chk(times, name="times")
     init_time, init_pos, init_vel = _chk(init_time), _chk(init_pos), _chk(init_vel)
     pairs = _chk(pred_pairs, torch.int64, "pred_pairs")
-    L, ldb = _batched_matrix(L)
     B, T = times.shape
+    L, ldb = _episode_factors(L, B, mean.shape[-1])
     P = pairs.shape[0]
     dev = mean.device
     work = _work(tables, B, P, dev)
@@ -366,8 +375,8 @@ def seglik_bwd(grad_logp: Tensor, work: Tensor, diag_max: Tensor, L: Tensor, tim
                pred_pairs: Tensor, tables: int, reg_rel: float, dim_params: int) -> Tuple[Tensor, Tensor]:
     grad_logp, times, init_time = _chk(grad_logp), _chk(times), _chk(init_time)
     pairs = _chk(pred_pairs, torch.int64)
-    L, ldb = _batched_matrix(L)
     B, T = times.shape
+    L, ldb = _episode_factors(L, B, dim_params)
     P = pairs.shape[0]
     dev = times.device
     adj = torch.empty_like(work)
@@ -419,8 +428,7 @@ def seg_logprob_staged(smp_traj, mean, L, times, init_time, init_pos, init_vel, 
 @torch.library.custom_op("tce::seglik_surrogate_fwd", mutates_args=())
 def seglik_surrogate_fwd(smp_traj: Tensor, mean: Tensor, L: Tensor, times: Tensor, init_time: Tensor,
                          init_pos: Tensor, init_vel: Tensor, pred_pairs: Tensor, logp_old: Tensor, advantage: Tensor,
-                         tables: int, reg_rel: float, sigma: Optional[Tensor] = None,
-                         sigma_scale: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+                         tables: int, reg_rel: float) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """Fused segment likelihood + importance-sampling surrogate (temporal_correlated_agent.py:718-739).
 
     -> (stats [2] fp64 = {-mean(ratio * adv), mean(ratio)}, logp [B,P], adj (per-segment adjoints for the
@@ -431,7 +439,7 @@ def seglik_surrogate_fwd(smp_traj: Tensor, mean: Tensor, L: Tensor, times: Tenso
     logp_old, advantage = _chk(logp_old, name="logp_old"), _chk(advantage, name="advantage")
     pairs = _chk(pred_pairs, torch.int64, "pred_pairs")
     B, T = times.shape
-    L, ldb = _batched_matrix(L, batch=B)
+    L, ldb = _episode_factors(L, B, mean.shape[-1])
     P = pairs.shape[0]
     dev = mean.device
     work = _work(tables, B, P, dev)
@@ -440,15 +448,8 @@ def seglik_surrogate_fwd(smp_traj: Tensor, mean: Tensor, L: Tensor, times: Tenso
     logp = torch.empty(B, P, device=dev, dtype=torch.float32)
     info = torch.empty(B, P, device=dev, dtype=torch.int32)
     st = _stream()
-    if sigma is not None:          # ONE covariance for the batch, given as sigma_scale * sigma [Dp, Dp] fp64
-        n = mean.shape[-1]
-        if sigma.dtype != torch.float64 or not sigma.is_cuda or not sigma.is_contiguous() or sigma.numel() != n * n:
-            raise TceError("sigma must be a contiguous CUDA float64 [Dp, Dp] tensor")
-        _lib.call("tce_seglik_gram_sigma", tables, _p(smp_traj), _p(mean), _p(sigma), _p(sigma_scale), _p(times),
-                  _p(init_time), _p(init_pos), _p(init_vel), _p(pairs), _p(work), _p(diag_max), B, T, P, st)
-    else:
-        _lib.call("tce_seglik_gram", tables, _p(smp_traj), _p(mean), _p(L), ldb, _p(times), _p(init_time),
-                  _p(init_pos), _p(init_vel), _p(pairs), _p(work), _p(diag_max), B, T, P, st)
+    _lib.call("tce_seglik_gram", tables, _p(smp_traj), _p(mean), _p(L), ldb, _p(times), _p(init_time), _p(init_pos),
+              _p(init_vel), _p(pairs), _p(work), _p(diag_max), B, T, P, st)
     _reduce_diag_max(diag_max)
     _lib.call("tce_seglik_chol", tables, _p(work), _p(work), _p(diag_max), float(reg_rel), None, _p(logp_old),
               _p(advantage), 1.0 / (B * P), _p(stats), _p(logp), _p(info), B, P, st)
@@ -456,8 +457,7 @@ def seglik_surrogate_fwd(smp_traj: Tensor, mean: Tensor, L: Tensor, times: Tenso
 
 
 @seglik_surrogate_fwd.register_fake
-def _(smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs, logp_old, advantage, tables, reg_rel,
-      sigma=None, sigma_scale=None):
+def _(smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs, logp_old, advantage, tables, reg_rel):
     B, P = times.shape[0], pred_pairs.shape[0]
     n = smp_traj.shape[-1]
     return (mean.new_empty(2, dtype=torch.float64), mean.new_empty(B, P),
@@ -471,43 +471,23 @@ def seglik_surrogate_bwd(upstream: Tensor, adj: Tensor, L: Tensor, times: Tensor
     pairs = _chk(pred_pairs, torch.int64)
     up = _chk(upstream, torch.float32, "upstream")
     B, T = times.shape
-    single = L.dim() == 3 and L.shape[0] == 1 and B > 1     # ONE factor [1, n, n] shared by the batch
-    L, ldb = _batched_matrix(L, batch=B)
+    L, ldb = _episode_factors(L, B, dim_params)
     P = pairs.shape[0]
     g_mean = torch.empty(B, dim_params, device=times.device, dtype=torch.float32)
     g_L = torch.empty(B, dim_params, dim_params, device=times.device, dtype=torch.float32)
-    if single:
-        # grad_L = 2 tril(dSigma L) is linear in dSigma: stage 3 writes dSigma per episode (no L, no product),
-        # one small kernel sums over the batch and applies the product once
-        _lib.call("tce_seglik_bwd_dsigma", tables, _p(adj), _p(times), _p(init_time), _p(pairs), _p(up), _p(g_mean),
-                  _p(g_L), B, T, P, _stream())
-        out = torch.empty(1, dim_params, dim_params, device=times.device, dtype=torch.float32)
-        _lib.call("tce_dsigma_to_dl", _p(g_L), B, _p(L), _p(out), dim_params, _stream())
-        return g_mean, out
     _lib.call("tce_seglik_bwd", tables, _p(adj), _p(L), ldb, _p(times), _p(init_time), _p(pairs), _p(up), _p(g_mean),
               _p(g_L), B, T, P, _stream())
     return g_mean, g_L
 
 
-_ONES = {}
-
-
-def _ones(n: int, device) -> Tensor:
-    key = (n, str(device))
-    if key not in _ONES:
-        _ONES[key] = torch.ones(n, device=device, dtype=torch.float32)
-    return _ONES[key]
-
-
 @seglik_surrogate_bwd.register_fake
 def _(upstream, adj, L, times, init_time, pred_pairs, tables, dim_params):
     B = times.shape[0]
-    Bl = 1 if (L.dim() == 3 and L.shape[0] == 1) else B
-    return times.new_empty(B, dim_params), times.new_empty(Bl, dim_params, dim_params)
+    return times.new_empty(B, dim_params), times.new_empty(B, dim_params, dim_params)
 
 
 def _sur_setup(ctx, inputs, output):
-    (smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs, logp_old, advantage, tables, reg_rel) = inputs[:12]
+    (smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs, logp_old, advantage, tables, reg_rel) = inputs
     ctx.save_for_backward(output[2], L, times, init_time, pred_pairs)
     ctx.tables, ctx.dim_params = tables, mean.shape[-1]
     ctx.set_materialize_grads(False)
@@ -515,7 +495,7 @@ def _sur_setup(ctx, inputs, output):
 
 def _sur_backward(ctx, g_stats, g_logp, g_adj, g_info):
     adj, L, times, init_time, pred_pairs = ctx.saved_tensors
-    none = (None,) * 14
+    none = (None,) * 12
     if g_stats is None:
         return none
     if g_stats is _E0.get(str(g_stats.device)):            # unit seed (see unit_seed): d total / d surrogate = 1
@@ -523,7 +503,7 @@ def _sur_backward(ctx, g_stats, g_logp, g_adj, g_info):
     else:
         up = g_stats[0].to(torch.float32).reshape(1)       # d total / d surrogate loss (device scalar, no sync)
     g_mean, g_L = seglik_surrogate_bwd(up, adj, L, times, init_time, pred_pairs, ctx.tables, ctx.dim_params)
-    return None, g_mean, g_L, None, None, None, None, None, None, None, None, None, None, None
+    return None, g_mean, g_L, None, None, None, None, None, None, None, None, None
 
 
 seglik_surrogate_fwd.register_autograd(_sur_backward, setup_context=_sur_setup)
@@ -532,15 +512,8 @@ seglik_surrogate_fwd.register_autograd(_sur_backward, setup_context=_sur_setup)
 def seg_surrogate_staged(smp_traj, mean, L, times, init_time, init_pos, init_vel, pred_pairs, logp_old, advantage,
                          tables: Tables, reg_rel: float = 1e-4):
     """Staged kernels -> (surrogate loss = -mean(exp(lp - lp_old) * adv) [fp32 scalar, differentiable], mean ratio, logp)."""
-    first = getattr(L, "_tce_first", None)       # a broadcast factor: differentiate w.r.t. the ONE matrix behind it
-    sig = getattr(L, "_tce_sigma", None)          # (Sigma0 [Dp, Dp] fp64, scale [1] fp64): Sigma = scale * Sigma0 = L L^T
-    if first is not None and first.shape[0] == 1:
-        L = first
-    else:
-        sig = None
     stats, logp, _adj, _info = seglik_surrogate_fwd(smp_traj, mean, L, times, init_time, init_pos, init_vel,
-                                                    pred_pairs, logp_old, advantage, tables.handle, reg_rel,
-                                                    None if sig is None else sig[0], None if sig is None else sig[1])
+                                                    pred_pairs, logp_old, advantage, tables.handle, reg_rel)
     loss, ratio = _StatsToFloat.apply(stats)
     return loss, ratio.detach(), logp.detach()
 

@@ -343,6 +343,40 @@ def test_surrogate_single_factor_path_equals_broadcast_path():
     assert (gL0 - gL1).abs().max() <= 1e-4 * gL1.abs().max()
 
 
+def test_staged_ops_refuse_one_factor_for_many_episodes():
+    """The staged likelihood ops read L[b] for every episode b: a contiguous [1, n, n] factor with B > 1 is refused
+    (shared factors go through the fused kernels).  The factor is the first matrix of a [B, n, n] buffer, so a missing
+    check would read valid memory and fail the assertion rather than read out of bounds."""
+    from tce_rl_b200._lib import TceError
+    name, B = "box", 8
+    cfg, T, inp, times, pairs = setup_case(name, B)
+    tabs = ops.Tables(**cfg)
+    c = lambda t: t.to(DEV)
+    Dp, P = inp["mean"].shape[-1], pairs.shape[0]
+    full = c(inp["L"])
+    one = full[:1]
+    assert one.is_contiguous() and one.shape == (1, Dp, Dp)
+    smp = ops.prodmp_traj(c(inp["mean"]), c(times), c(inp["init_time"]), c(inp["init_pos"]), c(inp["init_vel"]),
+                          tabs.handle, cfg["num_dof"])
+    args = (c(times), c(inp["init_time"]), c(inp["init_pos"]), c(inp["init_vel"]), c(pairs))
+    lp_old, adv = torch.zeros(B, P, device=DEV), torch.ones(B, P, device=DEV)
+    _, work, diag_max, _ = ops.seglik_fwd(smp, c(inp["mean"]), full, *args, tabs.handle, 1e-4)
+    _, _, adj, _ = ops.seglik_surrogate_fwd(smp, c(inp["mean"]), full, *args, lp_old, adv, tabs.handle, 1e-4)
+    with pytest.raises(TceError, match=r"\[B, n, n\]"):
+        ops.seglik_fwd(smp, c(inp["mean"]), one, *args, tabs.handle, 1e-4)
+    with pytest.raises(TceError, match=r"\[B, n, n\]"):
+        ops.seglik_surrogate_fwd(smp, c(inp["mean"]), one, *args, lp_old, adv, tabs.handle, 1e-4)
+    with pytest.raises(TceError, match=r"\[B, n, n\]"):
+        ops.seglik_bwd(torch.ones(B, P, device=DEV), work, diag_max, one, c(times), c(inp["init_time"]), c(pairs),
+                       tabs.handle, 1e-4, Dp)
+    with pytest.raises(TceError, match=r"\[B, n, n\]"):
+        ops.seglik_surrogate_bwd(torch.ones(1, device=DEV), adj, one, c(times), c(inp["init_time"]), c(pairs),
+                                 tabs.handle, Dp)
+    # a stride-0 expand of the same matrix is one factor per episode and still accepted
+    lp, _, _, _ = ops.seglik_fwd(smp, c(inp["mean"]), one.expand(B, -1, -1), *args, tabs.handle, 1e-4)
+    assert torch.isfinite(lp).all()
+
+
 @pytest.mark.parametrize("n,B", [(63, 200), (63, 203), (63, 9), (63, 3), (28, 37), (6, 64), (64, 16), (100, 12)])
 def test_gauss_maha_values_and_gradients(n, B):
     """tce_gauss_maha / tce_gauss_maha_bwd_full (black_box_policy.py:183-224 ``maha``) against fp64 torch: value and the
