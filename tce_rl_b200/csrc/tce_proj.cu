@@ -555,7 +555,8 @@ __device__ inline double kl_solve_eta(const double *lam, int n, double eps, doub
     __syncthreads();
     if (ok) return eta;
   }
-  // round 1: geometric grid eta_w = 2^(w - 10), w = 0..31  (1e-3 .. 2e6)
+  // round 1: geometric grid eta_w = 2^(w - 10), w = 0..31  (1e-3 .. 2.1e6); a root above the grid is bracketed by
+  // doubling from there (rare: the new standard deviations ~100x below the old ones), then two refinement rounds
   double lo = 0.0, hi = ldexp(1.0, 32 - 10);
   for (int round = 0; round < 3; ++round) {
     for (int w = warp; w < 32; w += nwarp) {
@@ -573,6 +574,14 @@ __device__ inline double kl_solve_eta(const double *lam, int n, double eps, doub
       cand[32] = nlo; cand[33] = nhi;
     }
     __syncthreads();
+    if (round == 0 && cand[31] > eps) {      // f(2^21) > eps (uniform over the CTA): hi = 2^22 is not known to bound
+      if (warp == 0) {
+        double l = ldexp(1.0, 21), h = 2.0 * l;
+        for (int it = 0; it < 1000 && kl_of_eta(lam, n, h, nullptr) > eps; ++it) { l = h; h *= 2.0; }
+        if (lane == 0) { cand[32] = l; cand[33] = h; }
+      }
+      __syncthreads();
+    }
     lo = cand[32]; hi = cand[33];
     __syncthreads();
   }
