@@ -305,6 +305,33 @@ int tce_seglik_bwd(const tce_tables_t *tables, const void *work, const float *L,
                    const float *times, const float *init_time, const int64_t *pred_pairs,
                    const float *upstream, float *grad_mean, float *grad_L, int64_t B, int64_t T, int64_t P,
                    void *stream);
+/* Shapes.  The staged entry points above and below (and the diagonal likelihood) serve every supported shape:
+ * 1 <= num_dof <= 8, 2 <= K1 <= 16, Dp = num_dof K1 <= 64.  The five (num_dof, K1) pairs (7, 9), (4, 9), (7, 4), (3, 4)
+ * and (2, 3) have kernels specialised on num_dof and are the only shapes of the fused and uniform-grid entry points
+ * (tce_seglik_fused_config ... tce_seglik_uniform_finish); other shapes run the staged kernels with num_dof read from
+ * the tables.  Anything else returns TCE_ERR_UNSUPPORTED_SHAPE.
+ * tce_seglik_compiled: 1 = one of the five specialised shapes, 0 = supported by the staged path only,
+ * TCE_ERR_UNSUPPORTED_SHAPE = outside the supported set.  Host only, no launch.                                      */
+int tce_seglik_compiled(const tce_tables_t *tables);
+/* Stage 1 for ONE covariance shared by the batch, given as Sigma = (*sigma_scale) * Sigma0 [Dp, Dp] fp64 (device
+ * pointers; sigma_scale may be NULL = 1) instead of its factor -- e.g. straight out of tce_proj_kl_entropy_fwd's
+ * state.  Stages 2 and 3 as for tce_seglik_gram (stage 3 through tce_seglik_bwd_shared).                       */
+int tce_seglik_gram_sigma(const tce_tables_t *tables, const float *smp_traj, const float *mean,
+                          const double *Sigma0, const double *sigma_scale, const float *times,
+                          const float *init_time, const float *init_pos, const float *init_vel,
+                          const int64_t *pred_pairs, void *work, double *diag_max, int64_t B, int64_t T, int64_t P,
+                          void *stream);
+/* Stage 3 for ONE covariance shared by the batch (a factor L [Dp, Dp] given to tce_seglik_gram with ldb_L = 0, or
+ * tce_seglik_gram_sigma): grad_mean [B, Dp] (may be NULL) per episode as tce_seglik_bwd; the gradient w.r.t. the
+ * covariance is summed over the batch in a fixed order (per-CTA partials, then one reduce; no atomics), so two calls
+ * on the same inputs give the same bits.  grad_sigma [Dp, Dp] fp64 = upstream * sum_b d lp_b / d Sigma (symmetric),
+ * grad_L [Dp, Dp] fp32 = 2 tril(grad_sigma L) (needs L); either may be NULL, not both.  part: workspace of
+ * tce_seglik_shared_part_doubles(tables, B) doubles (0: unsupported shape or B < 1).  Three launches.        */
+size_t tce_seglik_shared_part_doubles(const tce_tables_t *tables, int64_t B);
+int tce_seglik_bwd_shared(const tce_tables_t *tables, const void *work, const float *L, const float *times,
+                          const float *init_time, const int64_t *pred_pairs, const float *upstream, float *grad_mean,
+                          double *part, float *grad_L, double *grad_sigma, int64_t B, int64_t T, int64_t P,
+                          void *stream);
 /* Diagonal covariance (std_only policies, per-episode standard deviations s, strided as for tce_proj_kl_diag_*):
  * C is block diagonal with one 2 x 2 block per (pair, DoF), C_d[k,k'] = sum_j h_kj h_k'j s_{d,j}^2 + reg.
  * tce_seglik_diag_max: the regulariser seed diag_max = max over the batch of diag C (atomic max into *diag_max,

@@ -92,6 +92,10 @@ SIGNATURES = {
     "tce_seglik_gram": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
     "tce_seglik_chol": (C.c_int, [_P, _P, _P, _P, _D, _P, _P, _P, _D, _P, _P, _P, _I64, _I64, _P]),
     "tce_seglik_bwd": (C.c_int, [_P, _P, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
+    "tce_seglik_compiled": (C.c_int, [_P]),
+    "tce_seglik_gram_sigma": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
+    "tce_seglik_shared_part_doubles": (C.c_size_t, [_P, _I64]),
+    "tce_seglik_bwd_shared": (C.c_int, [_P] * 11 + [_I64, _I64, _I64, _P]),
     "tce_seglik_fused_config": (C.c_int, [_P, _I64, _I64, _I32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                           C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "tce_seglik_prepass": (C.c_int, [_P] * 4 + [_I64] + [_P] * 9 + [_I32, _I64, _I64, _I64, _P]),
@@ -149,7 +153,7 @@ def check(status: int, what: str = "") -> None:
 
 
 LAUNCHES = 0          # kernel launches issued through the C ABI (bench.py reports them as gpu_launches)
-_NO_KERNEL = {"tce_seglik_fused_config", "tce_seglik_uniform_parts", "tce_prodmp_tables_export", "tce_prodmp_tables_create", "tce_debug_kl_phase_cycles", "tce_debug_seglik_phase_cycles"}
+_NO_KERNEL = {"tce_seglik_fused_config", "tce_seglik_compiled", "tce_seglik_shared_part_doubles", "tce_seglik_uniform_parts", "tce_prodmp_tables_export", "tce_prodmp_tables_create", "tce_debug_kl_phase_cycles", "tce_debug_seglik_phase_cycles"}
 
 
 # Optional per-launch timing (bench.py's roofline report): when TIMING is a list, every kernel-launching ABI call is

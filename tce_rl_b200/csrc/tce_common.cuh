@@ -8,6 +8,29 @@
 
 #define TCE_MAX_K1 16   // max parameters per DoF (num_basis + 1)
 #define TCE_MAX_DOF 8
+#define TCE_MAX_DP 64   // max parameters per episode (num_dof * K1) of the likelihood and the projections
+
+// CALL with `K1` a compile-time constant for every K1 the tables accept (2..TCE_MAX_K1); returns
+// TCE_ERR_UNSUPPORTED_SHAPE for anything else.
+#define TCE_DISPATCH_K1(K1v, CALL)                   \
+  switch (K1v) {                                     \
+    case 2: { constexpr int K1 = 2; CALL; } break;   \
+    case 3: { constexpr int K1 = 3; CALL; } break;   \
+    case 4: { constexpr int K1 = 4; CALL; } break;   \
+    case 5: { constexpr int K1 = 5; CALL; } break;   \
+    case 6: { constexpr int K1 = 6; CALL; } break;   \
+    case 7: { constexpr int K1 = 7; CALL; } break;   \
+    case 8: { constexpr int K1 = 8; CALL; } break;   \
+    case 9: { constexpr int K1 = 9; CALL; } break;   \
+    case 10: { constexpr int K1 = 10; CALL; } break; \
+    case 11: { constexpr int K1 = 11; CALL; } break; \
+    case 12: { constexpr int K1 = 12; CALL; } break; \
+    case 13: { constexpr int K1 = 13; CALL; } break; \
+    case 14: { constexpr int K1 = 14; CALL; } break; \
+    case 15: { constexpr int K1 = 15; CALL; } break; \
+    case 16: { constexpr int K1 = 16; CALL; } break; \
+    default: return TCE_ERR_UNSUPPORTED_SHAPE;       \
+  }
 
 // Opaque tables handle (device pointers + the scalars every kernel needs).
 struct tce_tables {

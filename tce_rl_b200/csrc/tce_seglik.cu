@@ -96,19 +96,25 @@ __device__ void load_lower(const float *__restrict__ L, float *Ls, int n, int NR
 
 // =====================================================================================================
 // Stage 1: gram.  One CTA per episode.
+// DC > 0: the number of DoF is the compile-time DC (the shapes of TCE_FOR_SHAPES); DC = 0: it is read from the tables
+// (every other supported shape, K1 still a template parameter).  Only the DC = 0 instantiations take the covariance
+// itself (Sigma = *sigma_scale * Sigma0, [Dp, Dp] fp64, ONE matrix for the batch) instead of its factor.
 // =====================================================================================================
-template <int D, int K1>
-__global__ void __launch_bounds__(SL_THREADS, 4)
+template <int DC, int K1>
+__global__ void __launch_bounds__(SL_THREADS, DC ? 4 : 2)
 seglik_gram_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *__restrict__ mean,
                    const float *__restrict__ L, long long ldb_L, const float *__restrict__ times,
                    const float *__restrict__ init_time, const float *__restrict__ init_pos,
                    const float *__restrict__ init_vel, const int64_t *__restrict__ pairs, double *__restrict__ Cmat,
-                   double *__restrict__ Rres, double *__restrict__ diag_max, int T, int P) {
-  constexpr int Dp = D * K1, N = 2 * D, NT = tri(N);
-  constexpr int NR = (Dp + 1) & ~1;          // Sg rows / cols (even)
-  constexpr int NR4 = (Dp + 3) & ~3;         // Ls rows padded to a multiple of 4 for the 4x4 tiles
-  constexpr int LD = NR4 + 1;                // padded row stride of Ls (floats)
-  constexpr int SD = NR + 1;                 // row stride of Sg (doubles), odd, >= NR (tile padding)
+                   double *__restrict__ Rres, double *__restrict__ diag_max, int T, int P,
+                   const double *__restrict__ Sigma0, const double *__restrict__ sigma_scale) {
+  const int D = DC ? DC : tb.D;
+  const int Dp = D * K1, N = 2 * D, NT = tri(N);
+  const int NR = (Dp + 1) & ~1;              // Sg rows / cols (even)
+  const int NR4 = (Dp + 3) & ~3;             // Ls rows padded to a multiple of 4 for the 4x4 tiles
+  const int LD = NR4 + 1;                    // padded row stride of Ls (floats)
+  const int SD = NR + 1;                     // row stride of Sg (doubles), odd, >= NR (tile padding)
+  const bool sigma_in = DC == 0 && Sigma0 != nullptr;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double *Sg = reinterpret_cast<double *>(smem_raw);              // [NR][SD]
   double *hs = Sg + NR * SD;                                      // [2P][K1]
@@ -121,7 +127,15 @@ seglik_gram_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *_
   const float *times_b = times + b * T;
 
   SL_STAMP(0);
-  load_lower(L + b * ldb_L, Ls, Dp, NR4, LD);
+  if (sigma_in) {
+    const double sc = sigma_scale ? *sigma_scale : 1.0;
+    for (int e = threadIdx.x; e < NR * NR; e += blockDim.x) {
+      const int i = e / NR, c = e - i * NR;
+      Sg[i * SD + c] = (i < Dp && c < Dp) ? sc * Sigma0[i * Dp + c] : 0.0;
+    }
+  } else {
+    load_lower(L + b * ldb_L, Ls, Dp, NR4, LD);
+  }
   __syncthreads();
   SL_STAMP(1);
   basis_points<K1>(tb, (double)init_time[b], times_b, pairs, P, hs, xi, init_row);   // ends with a barrier
@@ -129,8 +143,8 @@ seglik_gram_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *_
 
   // ---- Sigma = L L^T (fp32 FFMA, 4x4 register tiles over the lower triangle: 8 LDS per 16 FFMA) -> Sg (fp64,
   //      mirrored).  Rows/cols are padded to NR4 (multiple of 4) with zeros.
-  {
-    constexpr int NT4 = NR4 / 4;
+  if (!sigma_in) {
+    const int NT4 = NR4 / 4;
     for (int t = threadIdx.x; t < tri(NT4); t += blockDim.x) {
       int I, J;
       tri_decode(t, I, J);
@@ -406,37 +420,177 @@ seglik_chol_kernel(const double *Cmat, const double *Rres, double *Gout, double 
   }
 }
 
+// The same for N = 16 (D = 8): its 136-entry triangle does not fit the 255-register budget (seglik_chol_kernel spills
+// 44 bytes at N = 14 already).  The triangle and z live in shared memory as [entry][thread] (conflict free, 39 KB), the
+// loops stay rolled (unrolled, the compiler caches the shared values in registers and spills ~2 KB per thread).
+template <int N>
+__global__ void __launch_bounds__(CH_THREADS)
+seglik_chol_smem_kernel(const double *Cmat, const double *Rres, double *Gout, double *Aout, const double *__restrict__ diag_max,
+                   double reg_rel, const float *__restrict__ grad_logp, const float *__restrict__ logp_old,
+                   const float *__restrict__ advantage, double grad_scale, double *__restrict__ loss_acc,
+                   float *__restrict__ logp, int32_t *__restrict__ info, long long BP, int P, int want_grad) {
+  constexpr int NT = tri(N);
+  __shared__ double sm[(NT + N) * CH_THREADS];
+  const long long gid = (long long)blockIdx.x * CH_THREADS + threadIdx.x;
+  const bool active = gid < BP;
+  double loss_part = 0.0, ratio_part = 0.0;
+  if (active) {
+    const long long b = gid / P;
+    const int p = (int)(gid % P);
+    const double *Cb = Cmat + (size_t)b * NT * P + p;
+    const double *Rb = Rres + (size_t)b * N * P + p;
+    double *Gb = Gout + (size_t)b * NT * P + p;
+    double *Ab = Aout + (size_t)b * N * P + p;
+#define CLIN(e) sm[(e) * CH_THREADS + threadIdx.x]
+#define CE(r, q) CLIN(tri_idx(r, q))
+#define ZE(i) sm[(NT + (i)) * CH_THREADS + threadIdx.x]
+    const double reg = reg_rel * (*diag_max);
+#pragma unroll 1
+    for (int e = 0; e < NT; ++e) CLIN(e) = Cb[(size_t)e * P];
+#pragma unroll 1
+    for (int i = 0; i < N; ++i) ZE(i) = Rb[(size_t)i * P];
+    // Cholesky (in place, lower), forward substitution and log-determinant
+    int bad = 0;
+    double half_logdet = 0.0, maha = 0.0;
+#pragma unroll 1
+    for (int j = 0; j < N; ++j) {
+      double dj = CE(j, j) + reg;
+#pragma unroll 1
+      for (int k = 0; k < j; ++k) dj = fma(-CE(j, k), CE(j, k), dj);
+      if (!(dj > 0.0) && bad == 0) bad = j + 1;
+      // 1/sqrt(dj): fp32 MUFU seed + two fp64 Newton steps (1e-7 -> 1e-14 -> rounding).  The DIAGONAL STORES THE
+      // RECIPROCAL 1/S_jj: every later division (substitutions, inverse) becomes a multiplication -- fp64 divide
+      // and sqrt are ~40-instruction subroutines and there were ~130 of them per segment.
+      double inv = (double)rsqrtf((float)dj);
+      inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
+      inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
+      CE(j, j) = inv;
+      half_logdet += 0.5 * log(dj);
+#pragma unroll 1
+      for (int i = j + 1; i < N; ++i) {
+        double v = CE(i, j);
+#pragma unroll 1
+        for (int k = 0; k < j; ++k) v = fma(-CE(i, k), CE(j, k), v);
+        CE(i, j) = v * inv;
+      }
+      double zj = ZE(j);
+#pragma unroll 1
+      for (int k = 0; k < j; ++k) zj = fma(-CE(j, k), ZE(k), zj);
+      zj *= inv;
+      ZE(j) = zj;
+      maha = fma(zj, zj, maha);
+    }
+    const double lp = -0.5 * ((double)N * 1.8378770664093453 + maha) - half_logdet;
+    if (logp) logp[gid] = (float)lp;
+    if (info) info[gid] = bad;
+    if (want_grad) {
+      double g;
+      if (logp_old) {                      // fused surrogate: loss = -grad_scale * sum ratio * adv
+        const double ratio = exp(lp - (double)logp_old[gid]);
+        g = -ratio * (double)advantage[gid] * grad_scale;
+        loss_part = g;
+        ratio_part = ratio * grad_scale;
+      } else {
+        g = (double)grad_logp[gid];
+      }
+      // alpha = S^-T z (back substitution)
+#pragma unroll 1
+      for (int i = N - 1; i >= 0; --i) {
+        double v = ZE(i);
+#pragma unroll 1
+        for (int k = i + 1; k < N; ++k) v = fma(-CE(k, i), ZE(k), v);
+        ZE(i) = v * CE(i, i);
+      }
+      // S <- S^-1 (lower, in place; the diagonal already holds 1/S_jj = X_jj)
+#pragma unroll 1
+      for (int j = 0; j < N; ++j) {
+#pragma unroll 1
+        for (int i = j + 1; i < N; ++i) {
+          double v = 0.0;
+#pragma unroll 1
+          for (int k = j; k < i; ++k) v = fma(CE(i, k), CE(k, j), v);
+          CE(i, j) = -v * CE(i, i);
+        }
+      }
+      // (column j: S[i][k], j <= k < i, are still the Cholesky entries; X[k][j], k < i, are done)
+      // C^-1 = X^T X (lower, in place, row by row: entry (i,j) only reads rows k >= i, and within row i
+      // the diagonal X[i][i] is consumed last), then G = g/2 (alpha alpha^T - C^-1)
+#pragma unroll 1
+      for (int i = 0; i < N; ++i) {
+#pragma unroll 1
+        for (int j = 0; j <= i; ++j) {
+          double v = 0.0;
+#pragma unroll 1
+          for (int k = i; k < N; ++k) v = fma(CE(k, i), CE(k, j), v);
+          CE(i, j) = 0.5 * g * (ZE(i) * ZE(j) - v);
+        }
+      }
+#pragma unroll 1
+      for (int e = 0; e < NT; ++e) Gb[(size_t)e * P] = CLIN(e);
+#pragma unroll 1
+      for (int i = 0; i < N; ++i) Ab[(size_t)i * P] = g * ZE(i);
+    }
+#undef CE
+#undef CLIN
+#undef ZE
+  }
+  if (loss_acc) {
+    loss_part = warp_sum(loss_part);
+    ratio_part = warp_sum(ratio_part);
+    if ((threadIdx.x & 31) == 0 && ratio_part != 0.0) {
+      atomicAdd(loss_acc, loss_part);
+      atomicAdd(loss_acc + 1, ratio_part);
+    }
+  }
+}
+
 // =====================================================================================================
 // Stage 3: backward accumulation.  One CTA per episode.
 // =====================================================================================================
-template <int D, int K1>
-__global__ void __launch_bounds__(SL_THREADS, 4)
+// DC as for the gram kernel.  With dsig_part != NULL (DC = 0 only) the covariance is ONE matrix for the batch: CTA c
+// owns episodes c, c + gridDim.x, ... (< B), sums upstream * d lp / d Sigma over them in that order and writes the sum
+// in block layout to dsig_part[c][tri(D) K1 K1] (fp64, entry (blk, i, j) = M_{d d'}[i][j], (d, d') = tri_decode(blk));
+// seglik_dsigma_sum_kernel then adds the partials in a fixed order.  No L is read and grad_L is not written.
+template <int DC, int K1>
+__global__ void __launch_bounds__(SL_THREADS, DC ? 4 : 2)
 seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__restrict__ Alpha,
                   const float *__restrict__ L, long long ldb_L, const float *__restrict__ times,
                   const float *__restrict__ init_time, const int64_t *__restrict__ pairs,
                   const float *__restrict__ upstream, float *__restrict__ grad_mean, float *__restrict__ grad_L,
-                  int T, int P) {
-  constexpr int Dp = D * K1, N = 2 * D, NT = tri(N);
-  constexpr int NR = (Dp + 3) & ~3;          // rows padded to a multiple of 4 for the 4x4 tiles
-  constexpr int LD = NR + 1;
+                  int T, int P, double *__restrict__ dsig_part, long long B) {
+  const int D = DC ? DC : tb.D;
+  const int Dp = D * K1, N = 2 * D, NT = tri(N);
+  const int NR = (Dp + 3) & ~3;              // rows padded to a multiple of 4 for the 4x4 tiles
+  const int LD = NR + 1;
+  const bool multi = DC == 0 && dsig_part != nullptr;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float *Gs = reinterpret_cast<float *>(smem_raw);                // [NT][P] staged adjoints, fp32 (later: out tile)
-  const int gs_floats = (NT * P > Dp * Dp ? NT * P : Dp * Dp + 1) & ~1;              // same rule as bwd_smem()
+  // Gs holds NT * P staged adjoints (and later the Dp x Dp output tile); its size is made even so that hs is 8-byte
+  // aligned.  DC = 0 rounds up.  The DC > 0 instantiations keep their original rounding, which rounds an odd NT * P
+  // down: hs[0] then overwrites the last staged adjoint (reachable at (7, 4) and (3, 4) with an odd P large enough
+  // that NT * P > Dp * Dp); bwd_smem() sizes the buffer for the rounded-up layout.
+  const int gs_need = NT * P > Dp * Dp ? NT * P : Dp * Dp + 1;
+  const int gs_floats = DC ? (gs_need & ~1) : ((gs_need + 1) & ~1);
   double *hs = reinterpret_cast<double *>(Gs + gs_floats);       // [2P][K1]
   double *xi = hs + 2 * P * K1;                                   // [2P][2]
   double *init_row = xi + 4 * P;                                  // [5 + 2 K1]
   float *Ls = reinterpret_cast<float *>(init_row + 5 + 2 * K1 + 1);  // [NR][LD]
   float *Ms = Ls + NR * LD;                                       // [NR][LD]  dlp/dSigma (symmetric)
+  double *Pacc = reinterpret_cast<double *>(Ms + NR * LD);        // multi: [tri(D) K1][K1] running sum
 
-  const long long b = blockIdx.x;
+  const float up = upstream ? *upstream : 1.0f;       // scalar gradient of the fused surrogate loss
+  if (multi)
+    for (int e = threadIdx.x; e < tri(D) * K1 * K1; e += blockDim.x) Pacc[e] = 0.0;
+  for (long long b = blockIdx.x;; b += gridDim.x) {
   const double *Gb = Gmat + (size_t)b * NT * P;
   const double *Ab = Alpha + (size_t)b * N * P;
-  const float up = upstream ? *upstream : 1.0f;       // scalar gradient of the fused surrogate loss
 
   SL_STAMP(16);
-  load_lower(L + b * ldb_L, Ls, Dp, NR, LD);
-  for (int e = threadIdx.x; e < NT * P; e += blockDim.x) Gs[e] = (float)Gb[e];
-  for (int e = threadIdx.x; e < NR * LD; e += blockDim.x) Ms[e] = 0.f;
+  if (!multi) load_lower(L + b * ldb_L, Ls, Dp, NR, LD);
+  if (!multi)
+    for (int e = threadIdx.x; e < NT * P; e += blockDim.x) Gs[e] = (float)Gb[e];
+  if (!multi)
+    for (int e = threadIdx.x; e < NR * LD; e += blockDim.x) Ms[e] = 0.f;
   basis_points<K1>(tb, (double)init_time[b], times + b * T, pairs, P, hs, xi, init_row);
 
   SL_STAMP(17);
@@ -449,7 +603,7 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
       grad_mean[b * Dp + o] = up * (float)acc;
     }
   }
-  if (!grad_L) return;
+  if (!grad_L && !multi) return;
 
   SL_STAMP(18);
   // ---- M_{dd'}[i][:] = sum_p sum_{k,k'} G[(d,k),(d',k')] h_pk[i] h_pk'[:]   (fp64), task (blk, i)
@@ -465,13 +619,23 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
     const float *g10 = Gs + (size_t)tri_idx(r0 + 1, q0) * P;
     const float *g11 = Gs + (size_t)tri_idx(r0 + 1, q0 + 1) * P;
     const float *g01 = (d != dd) ? Gs + (size_t)tri_idx(r0, q0 + 1) * P : g10;    // symmetric inside a diagonal block
+    // multi: the adjoints are read in fp64 from the workspace.  The batch sum of a shared covariance's gradient
+    // cancels (advantages of both signs) far below the size of its terms; fp32-staged adjoints then cost ~1e-3 of it.
+    const double *G00 = Gb + (size_t)tri_idx(r0, q0) * P, *G10 = Gb + (size_t)tri_idx(r0 + 1, q0) * P;
+    const double *G11 = Gb + (size_t)tri_idx(r0 + 1, q0 + 1) * P;
+    const double *G01 = (d != dd) ? Gb + (size_t)tri_idx(r0, q0 + 1) * P : G10;
     for (int p = 0; p < P; ++p) {
       const double a0 = hs[(2 * p) * K1 + i], a1 = hs[(2 * p + 1) * K1 + i];
-      const double w0 = a0 * (double)g00[p] + a1 * (double)g10[p];      // coefficient of h_p0[:]
-      const double w1 = a0 * (double)g01[p] + a1 * (double)g11[p];      // coefficient of h_p1[:]
+      const double w0 = multi ? a0 * G00[p] + a1 * G10[p] : a0 * (double)g00[p] + a1 * (double)g10[p];   // coefficient of h_p0[:]
+      const double w1 = multi ? a0 * G01[p] + a1 * G11[p] : a0 * (double)g01[p] + a1 * (double)g11[p];   // coefficient of h_p1[:]
 #pragma unroll
       for (int j = 0; j < K1; ++j)
         acc[j] = fma(w0, hs[(2 * p) * K1 + j], fma(w1, hs[(2 * p + 1) * K1 + j], acc[j]));
+    }
+    if (multi) {                                  // this thread owns these entries for every episode: fixed order
+#pragma unroll
+      for (int j = 0; j < K1; ++j) Pacc[task * K1 + j] += (double)up * acc[j];
+      continue;
     }
 #pragma unroll
     for (int j = 0; j < K1; ++j) {
@@ -481,6 +645,12 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
     }
   }
   __syncthreads();
+  if (multi) {                                    // (the barrier above: Gs / hs are free for the next episode)
+    if (b + gridDim.x < B) continue;
+    for (int e = threadIdx.x; e < tri(D) * K1 * K1; e += blockDim.x)
+      dsig_part[(size_t)blockIdx.x * tri(D) * K1 * K1 + e] = Pacc[e];
+    return;
+  }
 
   SL_STAMP(19);
   // ---- grad_L = 2 * tril(M L)  (fp32 FFMA, 4x4 tiles over the lower triangle), staged in the Gs buffer
@@ -488,7 +658,7 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
   for (int e = threadIdx.x; e < Dp * Dp; e += blockDim.x) out[e] = 0.f;
   __syncthreads();
   {
-    constexpr int NT4 = NR / 4;
+    const int NT4 = NR / 4;
     for (int t = threadIdx.x; t < tri(NT4); t += blockDim.x) {
       int I, J;
       tri_decode(t, I, J);
@@ -521,6 +691,35 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
   float *gL = grad_L + (size_t)b * Dp * Dp;
   for (int e = threadIdx.x; e < Dp * Dp; e += blockDim.x) gL[e] = out[e];
   SL_STAMP(21);
+  return;
+  }
+}
+
+// dS [Dp][Dp] fp64 = sum over the nparts partials of seglik_bwd_kernel (fixed order), mirrored: thread per entry.
+__global__ void __launch_bounds__(256)
+seglik_dsigma_sum_kernel(const double *__restrict__ part, int nparts, int D, int K1, double *__restrict__ dS) {
+  const int NE = tri(D) * K1 * K1, Dp = D * K1;
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= NE) return;
+  double s = 0.0;
+  for (int c = 0; c < nparts; ++c) s += part[(size_t)c * NE + e];
+  const int blk = e / (K1 * K1), r = e - blk * K1 * K1, i = r / K1, j = r - i * K1;
+  int d, dd;
+  tri_decode(blk, d, dd);
+  dS[(d * K1 + i) * Dp + dd * K1 + j] = s;
+  if (d != dd) dS[(dd * K1 + j) * Dp + d * K1 + i] = s;
+}
+
+// grad_L [n][n] = 2 tril(dS L) for ONE shared factor L (dS symmetric, fp64): CTA per row, thread per column.
+__global__ void __launch_bounds__(64)
+seglik_dsigma_to_dl_kernel(const double *__restrict__ dS, const float *__restrict__ L, int n, float *__restrict__ grad_L) {
+  const int i = blockIdx.x;
+  for (int j = threadIdx.x; j < n; j += blockDim.x) {
+    double acc = 0.0;
+    if (j <= i)
+      for (int k = j; k < n; ++k) acc = fma(dS[(size_t)i * n + k], (double)L[(size_t)k * n + j], acc);
+    grad_L[(size_t)i * n + j] = (float)(2.0 * acc);
+  }
 }
 
 // =====================================================================================================
@@ -535,7 +734,7 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
 // =====================================================================================================
 constexpr int SD_THREADS = 128;
 
-template <int D, int K1, int MODE>
+template <int DC, int K1, int MODE>           // DC as for the gram kernel
 __global__ void __launch_bounds__(SD_THREADS)
 seglik_diag_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *__restrict__ mean,
                    const float *__restrict__ s, long long ldb_s, long long inc_s, const float *__restrict__ times,
@@ -544,7 +743,8 @@ seglik_diag_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *_
                    double reg_rel, const float *__restrict__ grad_logp, float *__restrict__ logp,
                    int32_t *__restrict__ info, float *__restrict__ grad_mean, float *__restrict__ grad_s,
                    long long ldb_gs, long long inc_gs, int T, int P) {
-  constexpr int Dp = D * K1;
+  const int D = DC ? DC : tb.D;
+  const int Dp = D * K1;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double *hs = reinterpret_cast<double *>(smem_raw);             // [2P][K1]
   double *xi = hs + 2 * P * K1;                                   // [2P][2]
@@ -664,29 +864,112 @@ seglik_diag_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *_
 }
 
 // ---- host side ---------------------------------------------------------------------------------------
-template <int D, int K1>
-size_t diag_smem(int P, int mode) {
+size_t diag_smem(int D, int K1, int P, int mode) {
   return sizeof(double) * (2 * P * K1 + 4 * P + 5 + 2 * K1 + D * K1 + (mode == 2 ? 5 : 1) * D * P) +
          (mode == 1 ? sizeof(int) * D * P : 0) + 16;
 }
 
-template <int D, int K1>
-size_t gram_smem(int P) {
-  constexpr int Dp = D * K1, NR = (Dp + 1) & ~1, NR4 = (Dp + 3) & ~3, LD = NR4 + 1, SD = NR + 1;
+size_t gram_smem(int D, int K1, int P) {
+  const int Dp = D * K1, NR = (Dp + 1) & ~1, NR4 = (Dp + 3) & ~3, LD = NR4 + 1, SD = NR + 1;
   return sizeof(double) * ((size_t)NR * SD + 2 * P * K1 + 4 * P + 5 + 2 * K1 + 1) + sizeof(float) * NR4 * LD + 16;
 }
-template <int D, int K1>
-size_t bwd_smem(int P) {
-  constexpr int Dp = D * K1, N = 2 * D, NT = tri(N), NR = (Dp + 3) & ~3, LD = NR + 1;
-  const size_t gs_floats = (size_t)((NT * P > Dp * Dp ? NT * P : Dp * Dp + 1) & ~1);
+size_t bwd_smem(int D, int K1, int P, bool multi) {
+  const int Dp = D * K1, N = 2 * D, NT = tri(N), NR = (Dp + 3) & ~3, LD = NR + 1;
+  const size_t gs_floats = (size_t)(((NT * P > Dp * Dp ? NT * P : Dp * Dp + 1) + 1) & ~1);   // >= the kernel's
   const size_t g = sizeof(float) * gs_floats;
-  return g + sizeof(double) * (2 * P * K1 + 4 * P + 5 + 2 * K1 + 1) + sizeof(float) * 2 * NR * LD + 16;
+  return g + sizeof(double) * (2 * P * K1 + 4 * P + 5 + 2 * K1 + 1) + sizeof(float) * 2 * NR * LD +
+         (multi ? sizeof(double) * tri(D) * K1 * K1 : 0) + 16;
+}
+
+int g_sms = 0;
+int sm_count() {
+  if (!g_sms) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&g_sms, cudaDevAttrMultiProcessorCount, dev);
+    if (g_sms <= 0) g_sms = 148;
+  }
+  return g_sms;
+}
+
+// CTAs (= partials) of the shared-covariance backward: a function of B and the device only, so that the summation
+// order -- and the result -- is the same on every call
+int64_t shared_parts(int64_t B) {
+  const int64_t cap = 2LL * sm_count();
+  return B < cap ? B : cap;
+}
+
+template <int DC, int K1>
+int gram_launch(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *L, int64_t ldb_L,
+                const double *Sigma0, const double *sigma_scale, const float *times, const float *init_time,
+                const float *init_pos, const float *init_vel, const int64_t *pred_pairs, double *Cmat, double *R,
+                double *diag_max, int64_t B, int64_t T, int64_t P, cudaStream_t st) {
+  const size_t smem = gram_smem(t->D, K1, (int)P);
+  if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;
+  TCE_CUDA(cudaFuncSetAttribute(seglik_gram_kernel<DC, K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
+           "gram smem attr");
+  cudaFuncSetAttribute(seglik_gram_kernel<DC, K1>, cudaFuncAttributePreferredSharedMemoryCarveout,
+                       cudaSharedmemCarveoutMaxShared);
+  seglik_gram_kernel<DC, K1><<<(unsigned)B, SL_THREADS, smem, st>>>(
+      tab_dev(t), smp_traj, mean, L, ldb_L, times, init_time, init_pos, init_vel, pred_pairs, Cmat, R, diag_max, (int)T,
+      (int)P, Sigma0, sigma_scale);
+  TCE_CHECK_LAUNCH("seglik_gram_kernel");
+  return TCE_OK;
+}
+
+template <int DC, int K1>
+int bwd_launch(const tce_tables_t *t, const double *G, const double *A, const float *L, int64_t ldb_L,
+               const float *times, const float *init_time, const int64_t *pred_pairs, const float *upstream,
+               float *grad_mean, float *grad_L, double *dsig_part, int64_t B, int64_t T, int64_t P, cudaStream_t st) {
+  const size_t smem = bwd_smem(t->D, K1, (int)P, dsig_part != nullptr);
+  if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;
+  TCE_CUDA(cudaFuncSetAttribute(seglik_bwd_kernel<DC, K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
+           "bwd smem attr");
+  cudaFuncSetAttribute(seglik_bwd_kernel<DC, K1>, cudaFuncAttributePreferredSharedMemoryCarveout,
+                       cudaSharedmemCarveoutMaxShared);
+  const int64_t grid = dsig_part ? shared_parts(B) : B;
+  seglik_bwd_kernel<DC, K1><<<(unsigned)grid, SL_THREADS, smem, st>>>(
+      tab_dev(t), G, A, L, ldb_L, times, init_time, pred_pairs, upstream, grad_mean, grad_L, (int)T, (int)P, dsig_part,
+      (long long)B);
+  TCE_CHECK_LAUNCH("seglik_bwd_kernel");
+  return TCE_OK;
+}
+
+template <int DC, int K1, int MODE>
+int diag_launch(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *s, int64_t ldb_s,
+                int64_t inc_s, const float *times, const float *init_time, const float *init_pos,
+                const float *init_vel, const int64_t *pred_pairs, double *diag_max, double reg_rel,
+                const float *grad_logp, float *logp, int32_t *info, float *grad_mean, float *grad_s, int64_t ldb_gs,
+                int64_t inc_gs, int64_t B, int64_t T, int64_t P, cudaStream_t st) {
+  const size_t smem = diag_smem(t->D, K1, (int)P, MODE);
+  if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;
+  if (smem > 48 * 1024)
+    TCE_CUDA(cudaFuncSetAttribute(seglik_diag_kernel<DC, K1, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)smem), "diag smem attr");
+  seglik_diag_kernel<DC, K1, MODE><<<(unsigned)B, SD_THREADS, smem, st>>>(
+      tab_dev(t), smp_traj, mean, s, ldb_s, inc_s, times, init_time, init_pos, init_vel, pred_pairs, diag_max, reg_rel,
+      grad_logp, logp, info, grad_mean, grad_s, ldb_gs, inc_gs, (int)T, (int)P);
+  TCE_CHECK_LAUNCH("seglik_diag_kernel");
+  return TCE_OK;
 }
 
 }  // namespace
 
-// (D, K1) combinations with instantiated kernels
+// (D, K1) combinations with instantiations specialised on D (and the fused / uniform-grid kernels of
+// tce_seglik_fused.cu); every other shape with 1 <= D <= 8, 2 <= K1 <= 16, D K1 <= 64 runs the DC = 0 instantiations
 #define TCE_FOR_SHAPES(X) X(7, 9) X(4, 9) X(7, 4) X(3, 4) X(2, 3)
+
+static bool shape_supported(const tce_tables_t *t) {
+  return t->D >= 1 && t->D <= TCE_MAX_DOF && t->K1 >= 2 && t->K1 <= TCE_MAX_K1 && t->D * t->K1 <= TCE_MAX_DP;
+}
+
+extern "C" int tce_seglik_compiled(const tce_tables_t *t) {
+  if (!t) return TCE_ERR_INVALID_ARGUMENT;
+#define X(Dv, Kv) if (t->D == Dv && t->K1 == Kv) return 1;
+  TCE_FOR_SHAPES(X)
+#undef X
+  return shape_supported(t) ? 0 : TCE_ERR_UNSUPPORTED_SHAPE;
+}
 
 // debugging aid: SM-clock stamps of block 0 of the last gram ([0..6]) and bwd ([16..21]) launches (synchronises)
 extern "C" int tce_debug_seglik_phase_cycles(long long *out32) {
@@ -711,33 +994,48 @@ static inline double *work_R(const tce_tables_t *t, void *work, int64_t B, int64
   return (double *)work + (size_t)B * (size_t)P * (N * (N + 1) / 2);
 }
 
-extern "C" int tce_seglik_gram(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *L,
-                               int64_t ldb_L, const float *times, const float *init_time, const float *init_pos,
-                               const float *init_vel, const int64_t *pred_pairs, void *work, double *diag_max,
-                               int64_t B, int64_t T, int64_t P, void *stream) {
+static int seglik_gram_any(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *L,
+                           int64_t ldb_L, const double *Sigma0, const double *sigma_scale, const float *times,
+                           const float *init_time, const float *init_pos, const float *init_vel,
+                           const int64_t *pred_pairs, void *work, double *diag_max, int64_t B, int64_t T, int64_t P,
+                           void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
-  if (!t || !smp_traj || !mean || !L || !times || !init_time || !init_pos || !init_vel ||
+  if (!t || !smp_traj || !mean || (Sigma0 ? false : !L) || !times || !init_time || !init_pos || !init_vel ||
       !pred_pairs || !work || !diag_max || B < 0 || T < 1 || P < 1 || P > 4096)
     return TCE_ERR_INVALID_ARGUMENT;
   cudaStream_t st = (cudaStream_t)stream;
   double *Cmat = (double *)work, *R = work_R(t, work, B, P);
-#define X(Dv, Kv)                                                                                                 \
-  if (t->D == Dv && t->K1 == Kv) {                                                                                \
-    const size_t smem = gram_smem<Dv, Kv>((int)P);                                                                \
-    if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;                                                      \
-    TCE_CUDA(cudaFuncSetAttribute(seglik_gram_kernel<Dv, Kv>, cudaFuncAttributeMaxDynamicSharedMemorySize,       \
-                                  (int)smem), "gram smem attr");                                                  \
-    cudaFuncSetAttribute(seglik_gram_kernel<Dv, Kv>, cudaFuncAttributePreferredSharedMemoryCarveout,              \
-                         cudaSharedmemCarveoutMaxShared);                                                         \
-    seglik_gram_kernel<Dv, Kv><<<(unsigned)B, SL_THREADS, smem, st>>>(                                             \
-        tab_dev(t), smp_traj, mean, L, ldb_L, times, init_time, init_pos, init_vel, pred_pairs, Cmat, R, diag_max, \
-        (int)T, (int)P);                                                                                          \
-    TCE_CHECK_LAUNCH("seglik_gram_kernel");                                                                       \
-    return TCE_OK;                                                                                                \
-  }
-  TCE_FOR_SHAPES(X)
+  if (!Sigma0) {
+#define X(Dv, Kv)                                                                                                  \
+    if (t->D == Dv && t->K1 == Kv)                                                                                 \
+      return gram_launch<Dv, Kv>(t, smp_traj, mean, L, ldb_L, nullptr, nullptr, times, init_time, init_pos,       \
+                                 init_vel, pred_pairs, Cmat, R, diag_max, B, T, P, st);
+    TCE_FOR_SHAPES(X)
 #undef X
+  }
+  if (!shape_supported(t)) return TCE_ERR_UNSUPPORTED_SHAPE;
+  TCE_DISPATCH_K1(t->K1, return (gram_launch<0, K1>(t, smp_traj, mean, L, ldb_L, Sigma0, sigma_scale, times, init_time,
+                                                    init_pos, init_vel, pred_pairs, Cmat, R, diag_max, B, T, P, st)));
   return TCE_ERR_UNSUPPORTED_SHAPE;
+}
+
+extern "C" int tce_seglik_gram(const tce_tables_t *t, const float *smp_traj, const float *mean, const float *L,
+                               int64_t ldb_L, const float *times, const float *init_time, const float *init_pos,
+                               const float *init_vel, const int64_t *pred_pairs, void *work, double *diag_max,
+                               int64_t B, int64_t T, int64_t P, void *stream) {
+  if (B != 0 && !L) return TCE_ERR_INVALID_ARGUMENT;
+  return seglik_gram_any(t, smp_traj, mean, L, ldb_L, nullptr, nullptr, times, init_time, init_pos, init_vel,
+                         pred_pairs, work, diag_max, B, T, P, stream);
+}
+
+extern "C" int tce_seglik_gram_sigma(const tce_tables_t *t, const float *smp_traj, const float *mean,
+                                     const double *Sigma0, const double *sigma_scale, const float *times,
+                                     const float *init_time, const float *init_pos, const float *init_vel,
+                                     const int64_t *pred_pairs, void *work, double *diag_max, int64_t B, int64_t T,
+                                     int64_t P, void *stream) {
+  if (B != 0 && !Sigma0) return TCE_ERR_INVALID_ARGUMENT;
+  return seglik_gram_any(t, smp_traj, mean, nullptr, 0, Sigma0, sigma_scale, times, init_time, init_pos, init_vel,
+                         pred_pairs, work, diag_max, B, T, P, stream);
 }
 
 extern "C" int tce_seglik_chol(const tce_tables_t *t, const void *work, void *adj, const double *diag_max, double reg_rel,
@@ -747,6 +1045,7 @@ extern "C" int tce_seglik_chol(const tce_tables_t *t, const void *work, void *ad
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if (!t || !work || !diag_max || B < 0 || P < 1) return TCE_ERR_INVALID_ARGUMENT;
   if (logp_old && !advantage) return TCE_ERR_INVALID_ARGUMENT;
+  if (!shape_supported(t)) return TCE_ERR_UNSUPPORTED_SHAPE;
   cudaStream_t st = (cudaStream_t)stream;
   const double *Cmat = (const double *)work, *R = work_R(t, const_cast<void *>(work), B, P);
   double *G = (double *)adj, *A = adj ? work_R(t, adj, B, P) : nullptr;
@@ -761,8 +1060,13 @@ extern "C" int tce_seglik_chol(const tce_tables_t *t, const void *work, void *ad
                                                             advantage, grad_scale, loss_acc, logp, info, BP,   \
                                                             (int)P, want_grad);                                \
     break;
-    Y(2) Y(3) Y(4) Y(7)
+    Y(1) Y(2) Y(3) Y(4) Y(5) Y(6) Y(7)
 #undef Y
+    case 8:
+      seglik_chol_smem_kernel<16><<<grid, CH_THREADS, 0, st>>>(Cmat, R, G, A, diag_max, reg_rel, grad_logp, logp_old,
+                                                               advantage, grad_scale, loss_acc, logp, info, BP, (int)P,
+                                                               want_grad);
+      break;
     default: return TCE_ERR_UNSUPPORTED_SHAPE;
   }
   TCE_CHECK_LAUNCH("seglik_chol_kernel");
@@ -779,21 +1083,47 @@ extern "C" int tce_seglik_bwd(const tce_tables_t *t, const void *work, const flo
   cudaStream_t st = (cudaStream_t)stream;
   const double *G = (const double *)work, *A = work_R(t, const_cast<void *>(work), B, P);
 #define X(Dv, Kv)                                                                                                \
-  if (t->D == Dv && t->K1 == Kv) {                                                                               \
-    const size_t smem = bwd_smem<Dv, Kv>((int)P);                                                                \
-    if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;                                                     \
-    TCE_CUDA(cudaFuncSetAttribute(seglik_bwd_kernel<Dv, Kv>, cudaFuncAttributeMaxDynamicSharedMemorySize,        \
-                                  (int)smem), "bwd smem attr");                                                  \
-    cudaFuncSetAttribute(seglik_bwd_kernel<Dv, Kv>, cudaFuncAttributePreferredSharedMemoryCarveout,              \
-                         cudaSharedmemCarveoutMaxShared);                                                        \
-    seglik_bwd_kernel<Dv, Kv><<<(unsigned)B, SL_THREADS, smem, st>>>(                                             \
-        tab_dev(t), G, A, L, ldb_L, times, init_time, pred_pairs, upstream, grad_mean, grad_L, (int)T, (int)P);   \
-    TCE_CHECK_LAUNCH("seglik_bwd_kernel");                                                                       \
-    return TCE_OK;                                                                                               \
-  }
+  if (t->D == Dv && t->K1 == Kv)                                                                                 \
+    return bwd_launch<Dv, Kv>(t, G, A, L, ldb_L, times, init_time, pred_pairs, upstream, grad_mean, grad_L,       \
+                              nullptr, B, T, P, st);
   TCE_FOR_SHAPES(X)
 #undef X
+  if (!shape_supported(t)) return TCE_ERR_UNSUPPORTED_SHAPE;
+  TCE_DISPATCH_K1(t->K1, return (bwd_launch<0, K1>(t, G, A, L, ldb_L, times, init_time, pred_pairs, upstream, grad_mean,
+                                                   grad_L, nullptr, B, T, P, st)));
   return TCE_ERR_UNSUPPORTED_SHAPE;
+}
+
+extern "C" size_t tce_seglik_shared_part_doubles(const tce_tables_t *t, int64_t B) {
+  if (!t || B < 1 || !shape_supported(t)) return 0;
+  const int64_t Dp = (int64_t)t->D * t->K1;
+  return (size_t)(shared_parts(B) * (int64_t)(t->D * (t->D + 1) / 2) * t->K1 * t->K1 + Dp * Dp);
+}
+
+extern "C" int tce_seglik_bwd_shared(const tce_tables_t *t, const void *work, const float *L, const float *times,
+                                     const float *init_time, const int64_t *pred_pairs, const float *upstream,
+                                     float *grad_mean, double *part, float *grad_L, double *grad_sigma, int64_t B,
+                                     int64_t T, int64_t P, void *stream) {
+  if (!t || !part || (!grad_L && !grad_sigma) || (grad_L && !L) || B < 1 || T < 1 || P < 1 || !work || !times ||
+      !init_time || !pred_pairs)
+    return TCE_ERR_INVALID_ARGUMENT;
+  if (!shape_supported(t)) return TCE_ERR_UNSUPPORTED_SHAPE;
+  cudaStream_t st = (cudaStream_t)stream;
+  const double *G = (const double *)work, *A = work_R(t, const_cast<void *>(work), B, P);
+  const int D = t->D, K1 = t->K1, Dp = D * K1, NE = tri(D) * K1 * K1;
+  const int64_t nparts = shared_parts(B);
+  double *dS = grad_sigma ? grad_sigma : part + (size_t)nparts * NE;
+  int rc = TCE_ERR_UNSUPPORTED_SHAPE;
+  TCE_DISPATCH_K1(K1, rc = (bwd_launch<0, K1>(t, G, A, nullptr, 0, times, init_time, pred_pairs, upstream, grad_mean,
+                                              nullptr, part, B, T, P, st)));
+  if (rc != TCE_OK) return rc;
+  seglik_dsigma_sum_kernel<<<(NE + 255) / 256, 256, 0, st>>>(part, (int)nparts, D, K1, dS);
+  TCE_CHECK_LAUNCH("seglik_dsigma_sum_kernel");
+  if (grad_L) {
+    seglik_dsigma_to_dl_kernel<<<Dp, 64, 0, st>>>(dS, L, Dp, grad_L);
+    TCE_CHECK_LAUNCH("seglik_dsigma_to_dl_kernel");
+  }
+  return TCE_OK;
 }
 
 template <int MODE>
@@ -813,20 +1143,16 @@ static int seglik_diag_launch(const tce_tables_t *t, const float *smp_traj, cons
     return TCE_ERR_INVALID_ARGUMENT;
   cudaStream_t st = (cudaStream_t)stream;
 #define X(Dv, Kv)                                                                                                  \
-  if (t->D == Dv && t->K1 == Kv) {                                                                                 \
-    const size_t smem = diag_smem<Dv, Kv>((int)P, MODE);                                                           \
-    if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;                                                       \
-    if (smem > 48 * 1024)                                                                                          \
-      TCE_CUDA(cudaFuncSetAttribute(seglik_diag_kernel<Dv, Kv, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                    (int)smem), "diag smem attr");                                                 \
-    seglik_diag_kernel<Dv, Kv, MODE><<<(unsigned)B, SD_THREADS, smem, st>>>(                                        \
-        tab_dev(t), smp_traj, mean, s, ldb_s, inc_s, times, init_time, init_pos, init_vel, pred_pairs, diag_max,   \
-        reg_rel, grad_logp, logp, info, grad_mean, grad_s, ldb_gs, inc_gs, (int)T, (int)P);                        \
-    TCE_CHECK_LAUNCH("seglik_diag_kernel");                                                                        \
-    return TCE_OK;                                                                                                 \
-  }
+  if (t->D == Dv && t->K1 == Kv)                                                                                   \
+    return diag_launch<Dv, Kv, MODE>(t, smp_traj, mean, s, ldb_s, inc_s, times, init_time, init_pos, init_vel,     \
+                                     pred_pairs, diag_max, reg_rel, grad_logp, logp, info, grad_mean, grad_s,      \
+                                     ldb_gs, inc_gs, B, T, P, st);
   TCE_FOR_SHAPES(X)
 #undef X
+  if (!shape_supported(t)) return TCE_ERR_UNSUPPORTED_SHAPE;
+  TCE_DISPATCH_K1(t->K1, return (diag_launch<0, K1, MODE>(t, smp_traj, mean, s, ldb_s, inc_s, times, init_time,
+                                                          init_pos, init_vel, pred_pairs, diag_max, reg_rel, grad_logp,
+                                                          logp, info, grad_mean, grad_s, ldb_gs, inc_gs, B, T, P, st)));
   return TCE_ERR_UNSUPPORTED_SHAPE;
 }
 

@@ -369,16 +369,6 @@ int launch_traj_fwd(const tce_tables *t, const float *params, const float *times
 
 }  // namespace
 
-#define TCE_DISPATCH_K1(K1v, CALL)                   \
-  switch (K1v) {                                     \
-    case 3: { constexpr int K1 = 3; CALL; } break;   \
-    case 4: { constexpr int K1 = 4; CALL; } break;   \
-    case 6: { constexpr int K1 = 6; CALL; } break;   \
-    case 9: { constexpr int K1 = 9; CALL; } break;   \
-    case 11: { constexpr int K1 = 11; CALL; } break; \
-    default: return TCE_ERR_UNSUPPORTED_SHAPE;       \
-  }
-
 extern "C" int tce_prodmp_traj_fwd(const tce_tables_t *t, const float *params, const float *times,
                                    const float *init_time, const float *init_pos, const float *init_vel,
                                    float *traj, int64_t B, int64_t T, void *stream) {

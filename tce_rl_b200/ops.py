@@ -72,6 +72,8 @@ class Tables:
         _lib.call("tce_prodmp_tables_create", C.byref(self.cfg), _stream(), C.byref(handle))
         self.handle = handle.value
         self.num_pc = _lib.load().tce_prodmp_tables_num_pc(self.handle)
+        # one of the five shapes with fused / uniform-grid likelihood kernels (else: staged kernels, see ops_seglik.compiled)
+        self.compiled = _lib.load().tce_seglik_compiled(self.handle) == 1
 
     def export(self):
         """fp64 tables as CPU tensors (for tests / inspection)."""

@@ -176,6 +176,13 @@ def shared_factor(L: Tensor, batch: int) -> Optional[Tensor]:
     return None
 
 
+def compiled(tables: int) -> bool:
+    """True for the five (num_dof, K1) shapes with specialised kernels (fused and uniform-grid paths), False for every
+    other supported shape, which runs the staged kernels (``tce_seglik_compiled``: one host query, no launch; NOT
+    cached by handle, see ``fused_config``).  Shapes outside the supported set fail in the kernels' entry points."""
+    return _lib.load().tce_seglik_compiled(tables) == 1
+
+
 def fused_config(tables: int, B: int, P: int, chained: bool) -> dict:
     """Launch geometry / buffer sizes of the fused path for these shapes (host integers; NOT cached by handle: a
     freed tables handle can be re-issued for another MP shape)."""
@@ -244,6 +251,11 @@ def seglik(smp_traj: Tensor, mean: Tensor, L: Optional[Tensor], sigma: Optional[
         return logp, info, acc, g_mean, g_L, g_S
     if need_L and shared and L is None:
         raise TceError("grad_L of a shared covariance needs its factor L")
+    if not compiled(tables):
+        g_L, g_S = _seglik_staged(smp_traj, mean, L, sigma, sigma_scale, times, init_time, init_pos, init_vel, pairs,
+                                  tables, reg_rel, grad_mode, grad_logp, logp_old, advantage, shared, need_L, need_S,
+                                  logp, info, acc, g_mean)
+        return logp, info, acc, g_mean, g_L, g_S
     st = _stream()
     cfg = fused_config(tables, B, P, chained)
     scale = 1.0 / (B * P)
@@ -296,6 +308,52 @@ def seglik(smp_traj: Tensor, mean: Tensor, L: Optional[Tensor], sigma: Optional[
         _lib.call("tce_seglik_dsigma_reduce", tables, _p(part), cfg["grid"], _p(L) if need_L else None, None,
                   _p(g_L) if need_L else None, _p(g_S) if need_S else None, st)
     return logp, info, acc, g_mean, g_L, g_S
+
+
+def _seglik_staged(smp_traj, mean, L, sigma, sigma_scale, times, init_time, init_pos, init_vel, pairs, tables, reg_rel,
+                   grad_mode, grad_logp, logp_old, advantage, shared, need_L, need_S, logp, info, acc, g_mean):
+    """``seglik`` on the staged kernels (shapes without fused / uniform-grid kernels): gram -> [all-reduce(MAX) of the
+    regulariser seed] -> per-segment Cholesky (+ surrogate) -> backward.  A shared covariance sums its gradient over the
+    batch in a fixed order (``tce_seglik_bwd_shared``).  Fills logp / info / acc / g_mean, returns (g_L, g_S)."""
+    lib = _lib.load()
+    B, T = times.shape
+    P, Dp = pairs.shape[0], mean.shape[-1]
+    dev = mean.device
+    diag_max, stats = acc[:1], acc[1:]
+    st = _stream()
+    work = torch.empty(max(lib.tce_seglik_work_bytes(tables, B, P) // 8, 1), device=dev, dtype=torch.float64)
+    if sigma is not None:
+        _lib.call("tce_seglik_gram_sigma", tables, _p(smp_traj), _p(mean), _p(sigma), _p(sigma_scale), _p(times),
+                  _p(init_time), _p(init_pos), _p(init_vel), _p(pairs), _p(work), _p(diag_max), B, T, P, st)
+    else:
+        _lib.call("tce_seglik_gram", tables, _p(smp_traj), _p(mean), _p(L), 0 if shared else Dp * Dp, _p(times),
+                  _p(init_time), _p(init_pos), _p(init_vel), _p(pairs), _p(work), _p(diag_max), B, T, P, st)
+    _reduce_diag_max(diag_max)
+    want = grad_mode != 0
+    _lib.call("tce_seglik_chol", tables, _p(work), _p(work) if want else None, _p(diag_max), float(reg_rel),
+              _p(grad_logp) if grad_mode == 1 else None, _p(logp_old) if grad_mode == 2 else None,
+              _p(advantage) if grad_mode == 2 else None, 1.0 / (B * P), _p(stats) if grad_mode == 2 else None,
+              _p(logp), _p(info), B, P, st)
+    g_L = mean.new_empty(0)
+    g_S = mean.new_empty(0, dtype=torch.float64)
+    if not want:
+        return g_L, g_S
+    if not shared:
+        if need_L:
+            g_L = torch.empty(B, Dp, Dp, device=dev, dtype=torch.float32)
+        _lib.call("tce_seglik_bwd", tables, _p(work), _p(L), Dp * Dp, _p(times), _p(init_time), _p(pairs), None,
+                  _p(g_mean), _p(g_L) if need_L else None, B, T, P, st)
+        return g_L, g_S
+    if need_L:
+        g_L = torch.empty(1, Dp, Dp, device=dev, dtype=torch.float32)
+    # the covariance gradient is formed even when only grad_mean is wanted: the shared backward needs a destination
+    sig_out = torch.empty(Dp, Dp, device=dev, dtype=torch.float64) if (need_S or not need_L) else None
+    part = torch.empty(lib.tce_seglik_shared_part_doubles(tables, B), device=dev, dtype=torch.float64)
+    _lib.call("tce_seglik_bwd_shared", tables, _p(work), _p(L) if need_L else None, _p(times), _p(init_time),
+              _p(pairs), None, _p(g_mean), _p(part), _p(g_L) if need_L else None, _p(sig_out), B, T, P, st)
+    if need_S:
+        g_S = sig_out
+    return g_L, g_S
 
 
 @seglik.register_fake
