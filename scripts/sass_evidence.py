@@ -4,10 +4,11 @@ import collections, re, sys
 txt = sys.stdin.read()
 funcs = re.split(r'\n\s*Function : ', txt)
 out = ["# SASS evidence (cuobjdump -sass tce_rl_b200/libtce_b200.so, sm_100a); scripts/sass_evidence.py",
-       "# per-kernel counts (kernels with bulk copies, cp.async, or > 300 FMAs):",
+       "# per-kernel counts (kernels with bulk copies, cp.async, MMA, or > 300 FMAs):",
        "#   UBLKCP.S.G = cp.async.bulk global -> shared (TMA, non-tensor form); SYNCS.* = mbarrier (ARRIVE.TRANS64 = expect_tx,",
        "#   PHASECHK.TRANS64.TRYWAIT = try_wait.parity); LDGSTS = cp.async (Ampere form); DFMA/FFMA = fp64 / fp32 FMA; FFMA2 = packed fp32x2 FMA (sm_100);",
-       "#   no *MMA / UTC*MMA / LDTM / STTM anywhere: the path is not on the tensor cores (profiles/r02_precision.txt says why)",
+       "#   MMA = DMMA.8x8x4 (fp64 tensor cores: the projection kernels' shared-memory matrix products, la_gemm); no HMMA /",
+       "#   UTC*MMA / LDTM / STTM anywhere: nothing runs on the fp16 / tf32 tensor-core paths (profiles/r02_precision.txt says why)",
        f"{'kernel':58s} {'UBLKCP':>7s} {'SYNCS':>6s} {'LDGSTS':>7s} {'DFMA':>6s} {'FFMA':>6s} {'FFMA2':>6s} {'SHFL':>6s} {'BAR':>5s} {'MMA':>4s}"]
 KEYS = ("UBLKCP", "SYNCS", "LDGSTS", "DFMA", "FFMA2", "SHFL", "BAR")
 fmt = lambda n, c: f"{n[:58]:58s} {c['UBLKCP']:7d} {c['SYNCS']:6d} {c['LDGSTS']:7d} {c['DFMA']:6d} {c['FFMA']:6d} {c['FFMA2']:6d} {c['SHFL']:6d} {c['BAR']:5d} {c['MMA']:4d}"
@@ -30,7 +31,7 @@ for f in funcs[1:]:
     tot.update(c)
     short = re.sub(r'^_ZN\d+_GLOBAL__N__[0-9a-f]+_\d+_', '', name)
     short = re.sub(r'^(tce_\w+?_cu)_[0-9a-f]{8}\d+', '', short)
-    if c["UBLKCP"] or c["DFMA"] > 300 or c["FFMA"] > 300 or c["LDGSTS"] or c["FFMA2"]:
+    if c["UBLKCP"] or c["DFMA"] > 300 or c["FFMA"] > 300 or c["LDGSTS"] or c["FFMA2"] or c["MMA"]:
         out.append(fmt(short, c))
 out.append(fmt(f"TOTAL (all {len(funcs) - 1} kernels)", tot))
 for f in funcs[1:]:

@@ -24,7 +24,7 @@ __device__ long long g_kl_prof[32];
 namespace {
 
 constexpr int PJ_THREADS = 512;
-constexpr int KL_THREADS = 512;   // 128 registers per thread: 4x4 fp64 GEMM tiles and the register-resident Jacobi
+constexpr int KL_THREADS = 512;   // 128 registers per thread: the register-resident Jacobi
 constexpr double LOG_2PI = 1.8378770664093453;
 constexpr int KL_SC = 16;     // scalars saved per matrix by the KL projection: eta, active, kl0, fingerprint, alpha, ent_active,
                               // alpha^2, [7] trust-region shape part, [8] trust-region volume part (KL(new || out)),
@@ -1015,7 +1015,7 @@ kl_chol_kernel(const double *__restrict__ save_Sig, const double *__restrict__ s
 //   Nt_ij = -(1+eta) rho_i rho_j Ft_ij - delta_ij etabar (df/dlam_i) / (df/deta) ,
 //   etabar = sum_i Ft_ii (rho_i - (1+eta) rho_i^2) ;  grad_Lt = -2 tril(Lt^-T U~ Nt U~^T)
 // with U~ = Lt^-1 M and Lt^-1 saved by the forward.  No triangular solves: P^-1 by recursive doubling
-// (la_tri_inverse), everything else is 4x4-tile GEMMs on four shared buffers.
+// (la_tri_inverse), everything else is fp64 tensor-core GEMMs (la_gemm) on four shared buffers.
 __global__ void __launch_bounds__(KL_THREADS)
 proj_kl_cov_bwd_kernel(const float *__restrict__ L, const float *__restrict__ proj_L, const float *__restrict__ gout,
                        const double *__restrict__ save_M, const double *__restrict__ save_U,

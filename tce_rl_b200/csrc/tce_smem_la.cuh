@@ -25,53 +25,65 @@ __device__ __forceinline__ float la_rcp_approx(float x) {
 }
 
 
-// C = beta * C + alpha * A B (m x n x k, all <= 64) with 4x4 register tiles: thread (I, J) of the first
-// 16 * ceil(m/4) threads owns rows 4I..4I+3 and the INTERLEAVED columns J, J+16, J+32, J+48, so that per k step
-// a warp (two I, sixteen J) reads A as four broadcasts and B as four conflict-free rows: 8 shared-memory
-// wavefronts per 16 DFMA per lane (the 2x2 version needed 6 per 4 and was shared-memory bound at ~13k cycles
-// for 64^3; this one is bound by the fp64 pipe at ~4-5k).  Needs >= 48 registers of tile state: callers run
-// with <= 512 threads per CTA.
+// D += A B for one 8x8x4 fp64 tile on the tensor cores (SASS DMMA.8x8x4).  Lane l holds A(l / 4, l % 4),
+// B(l % 4, l / 4) and D(l / 4, 2 (l % 4) + {0, 1}).
+__device__ __forceinline__ void la_dmma(double (&d)[2], double a, double b) {
+  asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};"
+      : "+d"(d[0]), "+d"(d[1]) : "d"(a), "d"(b));
+}
+
+// C = beta * C + alpha * A B (m x n x k, all <= 64) on the fp64 tensor cores: each warp owns a 16 x 16 block of
+// C as 2 x 2 DMMA tiles, so per k step of 4 it loads two A and two B fragments (one LDS.64 each) for four DMMA
+// (1024 FMA); the scalar 4x4-tile version issued 8 shared-memory wavefronts per 16 DFMA per lane and ran the
+// fp64 pipe at about half its rate.  Tile rows (and columns) are INTERLEAVED: fragment row g of tile t is row
+// 4 (g % 4) + g / 4 + 2 t of the block, so that a half-warp's four rows lie 4 apart; with the odd leading
+// dimensions of the callers' buffers the 16 addresses of every fragment load then fall in 16 distinct 8-byte
+// banks, for A and B, transposed or not.  Each output is summed in ascending k with one rounded FMA per product,
+// the same arithmetic as a scalar loop (scripts/ubench/gemm.cu checks this bit for bit).
 // a_tri / b_tri describe the structure of A and B and only clip the k range: the unused triangle of a
-// triangular operand MUST hold zeros.  c_tri is a hint that only that triangle of C is read afterwards (the
-// whole of C may be written).
+// triangular operand MUST hold zeros.  Fragment elements outside [0, m) x [0, k) of A and [0, k) x [0, n) of B
+// are never read (they may be another buffer, or C itself in la_chol).  c_tri is a hint that only that triangle
+// of C is read afterwards; all of the m x n C is written.
 __device__ inline void la_gemm(Mat C, Mat A, Mat B, int m, int n, int k, int a_tri, int b_tri, int c_tri,
                                double alpha, double beta) {
   (void)c_tri;
-  const int TI = (m + 3) >> 2;
-  for (int t = threadIdx.x; t < TI * 16; t += blockDim.x) {
-    const int I = t >> 4, J = t & 15, i0 = 4 * I;
-    int lo = 0, hi = k;
-    if (a_tri == TRI_LOWER) hi = min(hi, i0 + 4);
-    if (a_tri == TRI_UPPER) lo = max(lo, i0);
-    if (b_tri == TRI_LOWER) lo = max(lo, J);
-    const double *ap[4], *bp[4];
-#pragma unroll
-    for (int r = 0; r < 4; ++r) ap[r] = &A(min(i0 + r, m - 1), 0);
-#pragma unroll
-    for (int c = 0; c < 4; ++c) bp[c] = &B(0, min(J + 16 * c, n - 1));
-    double acc[4][4];
-#pragma unroll
-    for (int r = 0; r < 4; ++r)
-#pragma unroll
-      for (int c = 0; c < 4; ++c) acc[r][c] = 0.0;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarp = (int)(blockDim.x >> 5);
+  const int g = lane >> 2, q = lane & 3, pg = 4 * (g & 3) + (g >> 2);
+  const int TN = (n + 15) >> 4, nblk = ((m + 15) >> 4) * TN;
+  for (int t = warp; t < nblk; t += nwarp) {
+    const int r0 = (t / TN) << 4, c0 = (t - (t / TN) * TN) << 4;
+    int lo = 0, hi = k;                                  // multiples of 16, or k
+    if (a_tri == TRI_LOWER) hi = min(hi, r0 + 16);
+    if (a_tri == TRI_UPPER) lo = max(lo, r0);
+    if (b_tri == TRI_LOWER) lo = max(lo, c0);
+    if (b_tri == TRI_UPPER) hi = min(hi, c0 + 16);
+    const int ra = r0 + pg, cb = c0 + pg;
+    const bool va0 = ra < m, va1 = ra + 2 < m, vb0 = cb < n, vb1 = cb + 2 < n;
+    const double *pa0 = &A(va0 ? ra : 0, 0), *pa1 = &A(va1 ? ra + 2 : 0, 0);
+    const double *pb0 = &B(0, vb0 ? cb : 0), *pb1 = &B(0, vb1 ? cb + 2 : 0);
+    double d[2][2][2] = {};
 #pragma unroll 2
-    for (int q = lo; q < hi; ++q) {
-      double a[4], b[4];
-#pragma unroll
-      for (int r = 0; r < 4; ++r) a[r] = ap[r][q * A.cs];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) b[c] = bp[c][q * B.rs];
-#pragma unroll
-      for (int r = 0; r < 4; ++r)
-#pragma unroll
-        for (int c = 0; c < 4; ++c) acc[r][c] = fma(a[r], b[c], acc[r][c]);
+    for (int k0 = lo; k0 < hi; k0 += 4) {
+      const int kk = k0 + q;
+      const bool vk = kk < hi;
+      const double a0 = (vk && va0) ? pa0[kk * A.cs] : 0.0, a1 = (vk && va1) ? pa1[kk * A.cs] : 0.0;
+      const double b0 = (vk && vb0) ? pb0[kk * B.rs] : 0.0, b1 = (vk && vb1) ? pb1[kk * B.rs] : 0.0;
+      la_dmma(d[0][0], a0, b0);
+      la_dmma(d[0][1], a0, b1);
+      la_dmma(d[1][0], a1, b0);
+      la_dmma(d[1][1], a1, b1);
     }
 #pragma unroll
-    for (int r = 0; r < 4; ++r) {
+    for (int ti = 0; ti < 2; ++ti) {
+      const int i = ra + 2 * ti;
 #pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        const int i = i0 + r, jj = J + 16 * c;
-        if (i < m && jj < n) C(i, jj) = beta == 0.0 ? alpha * acc[r][c] : fma(beta, C(i, jj), alpha * acc[r][c]);
+      for (int tj = 0; tj < 2; ++tj) {
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const int f = 2 * q + e, j = c0 + 4 * (f & 3) + (f >> 2) + 2 * tj;
+          const double v = d[ti][tj][e];
+          if (i < m && j < n) C(i, j) = beta == 0.0 ? alpha * v : fma(beta, C(i, j), alpha * v);
+        }
       }
     }
   }
@@ -113,9 +125,9 @@ __device__ inline void la_diag_block_inverses(Mat L, double *dinv, int n) {
 // Recursive doubling instead of forward substitution: the 8x8 diagonal blocks are inverted directly, then
 // blocks of width w = 8, 16, 32 are merged pairwise,
 //   [A1 0; C A2]^-1 = [A1^-1 0; -A2^-1 C A1^-1  A2^-1],
-// two small products per level with every output element on its own thread: 3 levels x 3 barriers, ~4k cycles,
-// where the blocked substitution needs 8 dependent block rows (~25k cycles with n right-hand sides).  A solve
-// with n right-hand sides is then ONE triangular GEMM.  For the factors met here (covariance factors,
+// two small products per level with every output element on its own thread: 3 levels x 3 barriers
+// (scripts/ubench/gemm.cu gives the cycles), where the blocked substitution needs 8 dependent block rows (~25k
+// cycles with n right-hand sides).  A solve with n right-hand sides is then ONE triangular GEMM.  For the factors met here (covariance factors,
 // condition ~1e2) the explicit inverse loses nothing measurable in fp64.  Needs blockDim.x >= 256.
 __device__ inline void la_tri_inverse(Mat L, Mat X, double *dinv, int n) {
   la_diag_block_inverses(L, dinv, n);
@@ -136,10 +148,11 @@ __device__ inline void la_tri_inverse(Mat L, Mat X, double *dinv, int n) {
         const int pr = o >> (2 * lw), rem = o & ((1 << (2 * lw)) - 1), ii = rem >> lw, jj = rem & (w - 1);
         const int c0 = pr << (lw + 1), i = c0 + w + ii, j = c0 + jj;
         if (i < n) {
-          double a0 = 0.0, a1 = 0.0;
-          int k = jj;
-          for (; k + 1 < w; k += 2) { a0 = fma(L(i, c0 + k), X(c0 + k, j), a0); a1 = fma(L(i, c0 + k + 1), X(c0 + k + 1, j), a1); }
-          if (k < w) a0 = fma(L(i, c0 + k), X(c0 + k, j), a0);
+          // k runs over the WHOLE block (A1inv(k, j) = 0 for k < j, exact zeros that leave the sums unchanged): the
+          // lanes of a warp then read L(i, k) as a broadcast and A1inv(k, .) as a row.  Starting at k = j would give
+          // each lane its own k: a diagonal walk through X with a 4-way bank conflict on every load.
+          double a0 = 0.0, a1 = 0.0;                                  // even k, odd k
+          for (int k = 0; k < w; k += 2) { a0 = fma(L(i, c0 + k), X(c0 + k, j), a0); a1 = fma(L(i, c0 + k + 1), X(c0 + k + 1, j), a1); }
           v[u] = a0 + a1;
         }
       }
@@ -283,7 +296,7 @@ __device__ inline void la_trsm_lower_t(Mat L, const double *dinv, Mat X, int n, 
 // (shared int, pre-set to 0) receives the 1-based index of the first non-positive pivot.  Per block of 8
 // columns: warp 0 factors the whole panel (rows r0..n-1) in REGISTERS -- lane l holds rows l and l + 32, pivots
 // and multipliers travel by shuffle, one rsqrt per column -- then everybody applies the rank-8 update to the
-// trailing matrix with the 4x4-tile GEMM.  Two barriers per 8 columns, ~2.3k cycles per block.
+// trailing matrix with la_gemm (k = 8).  Two barriers per 8 columns.
 __device__ inline void la_chol(Mat A, int n, int *bad) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int r0 = 0; r0 < n; r0 += LA_NB) {
