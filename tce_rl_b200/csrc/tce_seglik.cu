@@ -565,12 +565,10 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
   const bool multi = DC == 0 && dsig_part != nullptr;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float *Gs = reinterpret_cast<float *>(smem_raw);                // [NT][P] staged adjoints, fp32 (later: out tile)
-  // Gs holds NT * P staged adjoints (and later the Dp x Dp output tile); its size is made even so that hs is 8-byte
-  // aligned.  DC = 0 rounds up.  The DC > 0 instantiations keep their original rounding, which rounds an odd NT * P
-  // down: hs[0] then overwrites the last staged adjoint (reachable at (7, 4) and (3, 4) with an odd P large enough
-  // that NT * P > Dp * Dp); bwd_smem() sizes the buffer for the rounded-up layout.
+  // Gs holds NT * P staged adjoints (and later the Dp x Dp output tile); its size is rounded UP to an even number of
+  // floats so that hs is 8-byte aligned and starts after the last adjoint, as bwd_smem() sizes it.
   const int gs_need = NT * P > Dp * Dp ? NT * P : Dp * Dp + 1;
-  const int gs_floats = DC ? (gs_need & ~1) : ((gs_need + 1) & ~1);
+  const int gs_floats = (gs_need + 1) & ~1;
   double *hs = reinterpret_cast<double *>(Gs + gs_floats);       // [2P][K1]
   double *xi = hs + 2 * P * K1;                                   // [2P][2]
   double *init_row = xi + 4 * P;                                  // [5 + 2 K1]

@@ -1703,9 +1703,17 @@ extern "C" size_t tce_seglik_uniform_ws_doubles(const tce_tables_t *t, int64_t P
   return 0;
 }
 
-static int uniform_ep(int64_t B) { return B <= 8 * (int64_t)sm_count() ? 8 : 32; }   /* episodes per chunk */
-static int uniform_grid(int64_t B) {
-  const int ep = uniform_ep(B);
+/* episodes per chunk of tce_seglik_uniform_main: 32 once 8 would give every SM more than one chunk, unless the
+   32-episode layout does not fit in shared memory at this P (large P: the 8-episode CTAs then loop over chunks) */
+static int uniform_ep(const tce_tables_t *t, int64_t B, int64_t P) {
+  if (B <= 8 * (int64_t)sm_count()) return 8;
+#define X(Dv, Kv) \
+  if (t->D == Dv && t->K1 == Kv) return UniMainSmem<Dv, Kv, 32>((int)P).total <= SMEM_LIMIT ? 32 : 8;
+  TCE_FOR_SHAPES(X)
+#undef X
+  return 32;
+}
+static int uniform_grid(int ep, int64_t B) {
   const int64_t chunks = (B + ep - 1) / ep;
   const int64_t cap = (int64_t)sm_count();
   return (int)(chunks < cap ? (chunks < 1 ? 1 : chunks) : cap);
@@ -1715,7 +1723,7 @@ static int uniform_grid(int64_t B) {
 extern "C" int tce_seglik_uniform_parts(const tce_tables_t *t, int64_t B, int64_t P, int32_t *nparts,
                                         int64_t *apart_doubles) {
   if (!t || P < 1 || B < 0) return TCE_ERR_INVALID_ARGUMENT;
-  const int g = uniform_grid(B);
+  const int g = uniform_grid(uniform_ep(t, B, P), B);
   const int64_t N = 2 * (int64_t)t->D, NT = N * (N + 1) / 2;
   if (P * (NT + 1) > 12 * UM_THREADS) return TCE_ERR_UNSUPPORTED_SHAPE;
   if (nparts) *nparts = g;
@@ -1769,12 +1777,13 @@ extern "C" int tce_seglik_uniform_main(const tce_tables_t *t, const double *ws, 
     return TCE_ERR_INVALID_ARGUMENT;
   if (grad_mode == 1 && !grad_logp) return TCE_ERR_INVALID_ARGUMENT;
   if (grad_mode == 2 && (!logp_old || !advantage)) return TCE_ERR_INVALID_ARGUMENT;
-  const unsigned grid = (unsigned)uniform_grid(B);
+  const int ep = uniform_ep(t, B, P);
+  const unsigned grid = (unsigned)uniform_grid(ep, B);
 #define X(Dv, Kv)                                                                                                  \
   if (t->D == Dv && t->K1 == Kv) {                                                                                 \
     constexpr int N = 2 * Dv, NT = N * (N + 1) / 2;                                                                \
     if (P * (NT + 1) > 12 * UM_THREADS) return TCE_ERR_UNSUPPORTED_SHAPE;                                          \
-    if (uniform_ep(B) == 8) {                                                                                      \
+    if (ep == 8) {                                                                                                 \
       const size_t smem = UniMainSmem<Dv, Kv, 8>((int)P).total;                                                    \
       if (smem > SMEM_LIMIT) return TCE_ERR_UNSUPPORTED_SHAPE;                                                     \
       auto kern = uniform_main_kernel<Dv, Kv, 8>;                                                                  \

@@ -8,6 +8,8 @@ Two device paths, same results:
              kernel, forward + backward, no HBM workspace) -> ``tce_seglik_dsigma_reduce`` (shared covariance only);
 * uniform  : every episode has the same time grid and the covariance is shared (all shipped TCE configs):
              ``tce_seglik_uniform_prep / _main / _finish`` + ``tce_seglik_dsigma_reduce``.
+A segment count that neither takes (P > 256, or no episode group of the fused kernel fits in shared memory) runs the
+staged kernels of ``csrc/tce_seglik.cu``, as every shape without specialised kernels does.
 
 The gradient of the fused surrogate is produced in the FORWARD call (the upstream gradient of a scalar loss is known:
 ``-ratio * adv / (B P)``); the autograd backward only scales it.
@@ -183,18 +185,25 @@ def compiled(tables: int) -> bool:
     return _lib.load().tce_seglik_compiled(tables) == 1
 
 
+def uniform_config(tables: int, B: int, P: int) -> dict:
+    """Buffer sizes of the uniform-grid path; ``uni_parts`` = 0: its kernels do not take this P."""
+    lib = _lib.load()
+    nparts, apart = C.c_int32(), C.c_int64()
+    rc = lib.tce_seglik_uniform_parts(tables, max(B, 1), P, C.byref(nparts), C.byref(apart))
+    return {"ws_doubles": lib.tce_seglik_uniform_ws_doubles(tables, P),
+            "uni_parts": nparts.value if rc == 0 else 0, "apart_doubles": apart.value if rc == 0 else 0}
+
+
 def fused_config(tables: int, B: int, P: int, chained: bool) -> dict:
     """Launch geometry / buffer sizes of the fused path for these shapes (host integers; NOT cached by handle: a
-    freed tables handle can be re-issued for another MP shape)."""
+    freed tables handle can be re-issued for another MP shape), and those of ``uniform_config``.  Raises
+    ``TceError`` when the fused kernel does not take P (P > 256, or no episode group fits in shared memory)."""
     lib = _lib.load()
     E, grid, part, pre = C.c_int32(), C.c_int32(), C.c_int64(), C.c_int64()
     _lib.check(lib.tce_seglik_fused_config(tables, max(B, 1), P, int(chained), C.byref(E), C.byref(grid),
                                            C.byref(part), C.byref(pre)), "tce_seglik_fused_config")
-    nparts, apart = C.c_int32(), C.c_int64()
-    rc = lib.tce_seglik_uniform_parts(tables, max(B, 1), P, C.byref(nparts), C.byref(apart))
     return {"E": E.value, "grid": grid.value, "part_floats": part.value, "pre_doubles": pre.value,
-            "ws_doubles": lib.tce_seglik_uniform_ws_doubles(tables, P),
-            "uni_parts": nparts.value if rc == 0 else 0, "apart_doubles": apart.value if rc == 0 else 0}
+            **uniform_config(tables, B, P)}
 
 
 @torch.library.custom_op("tce::seglik", mutates_args=())
@@ -251,16 +260,23 @@ def seglik(smp_traj: Tensor, mean: Tensor, L: Optional[Tensor], sigma: Optional[
         return logp, info, acc, g_mean, g_L, g_S
     if need_L and shared and L is None:
         raise TceError("grad_L of a shared covariance needs its factor L")
-    if not compiled(tables):
+    cfg = None
+    if compiled(tables):
+        if uniform:
+            cfg = uniform_config(tables, B, P)
+            uniform = cfg["uni_parts"] > 0                   # P outside the uniform kernels: general path
+        if not uniform:
+            try:
+                cfg = fused_config(tables, B, P, chained)
+            except TceError:                                 # P outside the fused kernel: staged kernels
+                cfg = None
+    if cfg is None:
         g_L, g_S = _seglik_staged(smp_traj, mean, L, sigma, sigma_scale, times, init_time, init_pos, init_vel, pairs,
                                   tables, reg_rel, grad_mode, grad_logp, logp_old, advantage, shared, need_L, need_S,
                                   logp, info, acc, g_mean)
         return logp, info, acc, g_mean, g_L, g_S
     st = _stream()
-    cfg = fused_config(tables, B, P, chained)
     scale = 1.0 / (B * P)
-    if uniform and cfg["uni_parts"] == 0:
-        uniform = False                                      # shape outside the uniform kernels: general path
     if uniform:
         ws = torch.empty(cfg["ws_doubles"], device=dev, dtype=torch.float64)
         Lp = None if sigma is not None else _p(L)
@@ -312,7 +328,8 @@ def seglik(smp_traj: Tensor, mean: Tensor, L: Optional[Tensor], sigma: Optional[
 
 def _seglik_staged(smp_traj, mean, L, sigma, sigma_scale, times, init_time, init_pos, init_vel, pairs, tables, reg_rel,
                    grad_mode, grad_logp, logp_old, advantage, shared, need_L, need_S, logp, info, acc, g_mean):
-    """``seglik`` on the staged kernels (shapes without fused / uniform-grid kernels): gram -> [all-reduce(MAX) of the
+    """``seglik`` on the staged kernels (shapes without fused / uniform-grid kernels, and segment counts that neither
+    takes on the shapes with them, e.g. P > 256 segments): gram -> [all-reduce(MAX) of the
     regulariser seed] -> per-segment Cholesky (+ surrogate) -> backward.  A shared covariance sums its gradient over the
     batch in a fixed order (``tce_seglik_bwd_shared``).  Fills logp / info / acc / g_mean, returns (g_L, g_S)."""
     lib = _lib.load()
