@@ -17,9 +17,7 @@
 // (cond(C) ~ 1e4 because neighbouring time points are almost perfectly correlated); fp32
 // accumulation there costs ~3e-4 absolute on the log-prob, above the 1e-4 parity bound.  They run in
 // fp64 (B200 DFMA = 1/2 FFMA rate); the two O(Dp^3) products Sigma = L L^T and (dSigma) L run in fp32.
-#include <math.h>
-
-#include "tce_common.cuh"
+#include "tce_seglik.cuh"
 
 // profiling scaffolding (-DTCE_PROFILE only): SM-clock stamps of block 0 of the last gram [0..15] / bwd [16..31] kernel
 #ifdef TCE_PROFILE
@@ -33,56 +31,22 @@ namespace {
 
 constexpr int SL_THREADS = 256;
 
-__host__ __device__ constexpr int tri(int n) { return n * (n + 1) / 2; }
-__device__ __forceinline__ int tri_idx(int r, int c) { return r * (r + 1) / 2 + c; }  // r >= c
-
 // ---- basis rows of the 2P time points of one episode (fp64) -----------------------------------------
 // hs [2P][K1]  : scaled H_pos row of time point q = 2p + k
 // xi [2P][2]   : xi1, xi2
+// init_row [5 + 2 K1] as for init_row_entry.  The three regions are disjoint (__restrict__): the loop then reads the
+// first five entries of init_row once per thread instead of once per basis entry.
 template <int K1>
 __device__ void basis_points(const TabDev &tb, double t_init, const float *__restrict__ times_b,
-                             const int64_t *__restrict__ pairs, int P, double *hs, double *xi, double *init_row) {
-  // init_row: [0..3] y1b,y2b,dy1b,dy2b ; [4] 1/det ; [5..5+K1) pos_b ; [5+K1 .. 5+2K1) vel_b
-  if (threadIdx.x <= K1) {
-    int i0; double w;
-    time_to_index(tb, t_init, i0, w);
-    if (threadIdx.x < K1) {
-      const int j = threadIdx.x;
-      init_row[5 + j] = lerp_t(tb.pos[(size_t)i0 * K1 + j], tb.pos[(size_t)(i0 + 1) * K1 + j], w);
-      init_row[5 + K1 + j] = lerp_t(tb.vel[(size_t)i0 * K1 + j], tb.vel[(size_t)(i0 + 1) * K1 + j], w);
-    } else {
-      const double a = lerp_t(tb.y1[i0], tb.y1[i0 + 1], w), b = lerp_t(tb.y2[i0], tb.y2[i0 + 1], w);
-      const double c = lerp_t(tb.dy1[i0], tb.dy1[i0 + 1], w), d = lerp_t(tb.dy2[i0], tb.dy2[i0 + 1], w);
-      init_row[0] = a; init_row[1] = b; init_row[2] = c; init_row[3] = d;
-      init_row[4] = 1.0 / (a * d - b * c);
-    }
-  }
+                             const int64_t *__restrict__ pairs, int P, double *__restrict__ hs,
+                             double *__restrict__ xi, double *__restrict__ init_row) {
+  if (threadIdx.x <= K1) init_row_entry<K1>(tb, t_init, threadIdx.x, init_row);
   __syncthreads();
-  const double y1b = init_row[0], y2b = init_row[1], dy1b = init_row[2], dy2b = init_row[3], idet = init_row[4];
   for (int it = threadIdx.x; it < 2 * P * (K1 + 1); it += blockDim.x) {
-    const int q = it / (K1 + 1), j = it - q * (K1 + 1);
-    int i0; double w;
-    time_to_index(tb, (double)times_b[pairs[q]], i0, w);           // pairs is [P][2] row-major -> q = 2p + k
-    const double y1 = lerp_t(tb.y1[i0], tb.y1[i0 + 1], w), y2 = lerp_t(tb.y2[i0], tb.y2[i0 + 1], w);
-    const double xi1 = (dy2b * y1 - dy1b * y2) * idet, xi2 = (y1b * y2 - y2b * y1) * idet;
-    if (j < K1) {
-      const double pj = lerp_t(tb.pos[(size_t)i0 * K1 + j], tb.pos[(size_t)(i0 + 1) * K1 + j], w);
-      hs[q * K1 + j] = (pj - xi1 * init_row[5 + j] - xi2 * init_row[5 + K1 + j]) * tb.scale[j];
-    } else {
-      xi[2 * q] = xi1;
-      xi[2 * q + 1] = xi2;
-    }
+    const int q = it / (K1 + 1), j = it - q * (K1 + 1);       // pairs is [P][2] row-major -> q = 2p + k
+    basis_entry<K1>(tb, init_row, (double)times_b[pairs[q]], j, hs + q * K1, xi + 2 * q);
   }
   __syncthreads();
-}
-
-// decode a lower-triangular tile index t -> (I, J), I >= J
-__device__ __forceinline__ void tri_decode(int t, int &I, int &J) {
-  int i = (int)((sqrtf(8.0f * (float)t + 1.0f) - 1.0f) * 0.5f);
-  while (i * (i + 1) / 2 > t) --i;
-  while ((i + 1) * (i + 2) / 2 <= t) ++i;
-  I = i;
-  J = t - i * (i + 1) / 2;
 }
 
 // load the lower triangle of a dense [n, n] matrix into padded shared memory (row stride LD), upper = 0,
@@ -285,10 +249,13 @@ seglik_gram_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *_
 }
 
 // =====================================================================================================
-// Stage 2: per-segment Cholesky / log-prob / adjoints.  One thread per (b, p); the packed lower
-// triangle lives in shared memory as [entry][thread] (conflict free, compile-time offsets).
+// Stage 2: per-segment Cholesky / log-prob / adjoints (seg_* of tce_seglik.cuh).  One thread per (b, p).
+// N <= 14: the packed triangle and z live in registers, every loop fully unrolled.  N = 16 (D = 8): its 136-entry
+// triangle does not fit the 255-register budget (N = 14 spills 44 bytes already); the triangle and z live in shared
+// memory as [entry][thread] (conflict free, 39 KB), the loops stay rolled (unrolled, the compiler caches the shared
+// values in registers and spills ~2 KB per thread).
 // =====================================================================================================
-constexpr int CH_THREADS = 32;   // NT * CH_THREADS doubles of static shared memory (27 KB at n = 14)
+constexpr int CH_THREADS = 32;
 
 template <int N>
 __global__ void __launch_bounds__(CH_THREADS)
@@ -297,242 +264,39 @@ seglik_chol_kernel(const double *Cmat, const double *Rres, double *Gout, double 
                    const float *__restrict__ advantage, double grad_scale, double *__restrict__ loss_acc,
                    float *__restrict__ logp, int32_t *__restrict__ info, long long BP, int P, int want_grad) {
   constexpr int NT = tri(N);
-#ifndef SEGLIK_CHOL_SMEM
-  double c[NT];                      // fully unrolled below: every index is a compile-time constant -> registers
-#else
-  __shared__ double sm[NT * CH_THREADS];
-#endif
+  constexpr bool IN_REGS = N <= 14;
   const long long gid = (long long)blockIdx.x * CH_THREADS + threadIdx.x;
-  const bool active = gid < BP;
   double loss_part = 0.0, ratio_part = 0.0;
-  if (active) {
+  auto segment = [&](auto &c, auto &z) {
     const long long b = gid / P;
     const int p = (int)(gid % P);
     const double *Cb = Cmat + (size_t)b * NT * P + p;
     const double *Rb = Rres + (size_t)b * N * P + p;
     double *Gb = Gout + (size_t)b * NT * P + p;
     double *Ab = Aout + (size_t)b * N * P + p;
-#ifndef SEGLIK_CHOL_SMEM
-#define CE(r, q) c[tri_idx(r, q)]
-#define CLIN(e) c[e]
-#else
-    double *c = sm + threadIdx.x;
-#define CE(r, q) c[(tri_idx(r, q)) * CH_THREADS]
-#define CLIN(e) c[(e) * CH_THREADS]
-#endif
     const double reg = reg_rel * (*diag_max);
-#pragma unroll
-    for (int e = 0; e < NT; ++e) CLIN(e) = Cb[(size_t)e * P];
-    double z[N];
-#pragma unroll
-    for (int i = 0; i < N; ++i) z[i] = Rb[(size_t)i * P];
-    // Cholesky (in place, lower), forward substitution and log-determinant
-    int bad = 0;
-    double half_logdet = 0.0, maha = 0.0;
-#pragma unroll
-    for (int j = 0; j < N; ++j) {
-      double dj = CE(j, j) + reg;
-#pragma unroll
-      for (int k = 0; k < j; ++k) dj = fma(-CE(j, k), CE(j, k), dj);
-      if (!(dj > 0.0) && bad == 0) bad = j + 1;
-      // 1/sqrt(dj): fp32 MUFU seed + two fp64 Newton steps (1e-7 -> 1e-14 -> rounding).  The DIAGONAL STORES THE
-      // RECIPROCAL 1/S_jj: every later division (substitutions, inverse) becomes a multiplication -- fp64 divide
-      // and sqrt are ~40-instruction subroutines and there were ~130 of them per segment.
-      double inv = (double)rsqrtf((float)dj);
-      inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
-      inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
-      CE(j, j) = inv;
-      half_logdet += 0.5 * log(dj);
-#pragma unroll
-      for (int i = j + 1; i < N; ++i) {
-        double v = CE(i, j);
-#pragma unroll
-        for (int k = 0; k < j; ++k) v = fma(-CE(i, k), CE(j, k), v);
-        CE(i, j) = v * inv;
-      }
-      double zj = z[j];
-#pragma unroll
-      for (int k = 0; k < j; ++k) zj = fma(-CE(j, k), z[k], zj);
-      zj *= inv;
-      z[j] = zj;
-      maha = fma(zj, zj, maha);
-    }
-    const double lp = -0.5 * ((double)N * 1.8378770664093453 + maha) - half_logdet;
+    seg_for<IN_REGS>(0, NT, [&](int e) { c[e] = Cb[(size_t)e * P]; });
+    seg_for<IN_REGS>(0, N, [&](int i) { z[i] = Rb[(size_t)i * P]; });
+    int bad;
+    const double lp = seg_factor<N, IN_REGS>(c, z, reg, bad);
     if (logp) logp[gid] = (float)lp;
     if (info) info[gid] = bad;
-    if (want_grad) {
-      double g;
-      if (logp_old) {                      // fused surrogate: loss = -grad_scale * sum ratio * adv
-        const double ratio = exp(lp - (double)logp_old[gid]);
-        g = -ratio * (double)advantage[gid] * grad_scale;
-        loss_part = g;
-        ratio_part = ratio * grad_scale;
-      } else {
-        g = (double)grad_logp[gid];
-      }
-      // alpha = S^-T z (back substitution)
-#pragma unroll
-      for (int i = N - 1; i >= 0; --i) {
-        double v = z[i];
-#pragma unroll
-        for (int k = i + 1; k < N; ++k) v = fma(-CE(k, i), z[k], v);
-        z[i] = v * CE(i, i);
-      }
-      // S <- S^-1 (lower, in place; the diagonal already holds 1/S_jj = X_jj)
-#pragma unroll
-      for (int j = 0; j < N; ++j) {
-#pragma unroll
-        for (int i = j + 1; i < N; ++i) {
-          double v = 0.0;
-#pragma unroll
-          for (int k = j; k < i; ++k) v = fma(CE(i, k), CE(k, j), v);
-          CE(i, j) = -v * CE(i, i);
-        }
-      }
-      // (column j: S[i][k], j <= k < i, are still the Cholesky entries; X[k][j], k < i, are done)
-      // C^-1 = X^T X (lower, in place, row by row: entry (i,j) only reads rows k >= i, and within row i
-      // the diagonal X[i][i] is consumed last), then G = g/2 (alpha alpha^T - C^-1)
-#pragma unroll
-      for (int i = 0; i < N; ++i) {
-#pragma unroll
-        for (int j = 0; j <= i; ++j) {
-          double v = 0.0;
-#pragma unroll
-          for (int k = i; k < N; ++k) v = fma(CE(k, i), CE(k, j), v);
-          CE(i, j) = 0.5 * g * (z[i] * z[j] - v);
-        }
-      }
-#pragma unroll
-      for (int e = 0; e < NT; ++e) Gb[(size_t)e * P] = CLIN(e);
-#pragma unroll
-      for (int i = 0; i < N; ++i) Ab[(size_t)i * P] = g * z[i];
+    if (!want_grad) return;
+    const SegIO io{grad_logp, logp_old, advantage, logp, info, grad_scale, reg, logp_old ? 2 : 1};
+    const double g = seg_upstream(io, lp, gid, loss_part, ratio_part);
+    seg_adjoint<N, IN_REGS>(c, z, g, c);
+    seg_for<IN_REGS>(0, NT, [&](int e) { Gb[(size_t)e * P] = c[e]; });
+    seg_for<IN_REGS>(0, N, [&](int i) { Ab[(size_t)i * P] = g * z[i]; });
+  };
+  if (gid < BP) {
+    if constexpr (IN_REGS) {
+      double c[NT], z[N];
+      segment(c, z);
+    } else {
+      __shared__ double sm[(NT + N) * CH_THREADS];
+      Strided c{sm + threadIdx.x, CH_THREADS}, z{sm + NT * CH_THREADS + threadIdx.x, CH_THREADS};
+      segment(c, z);
     }
-#undef CE
-#undef CLIN
-  }
-  if (loss_acc) {
-    loss_part = warp_sum(loss_part);
-    ratio_part = warp_sum(ratio_part);
-    if ((threadIdx.x & 31) == 0 && ratio_part != 0.0) {
-      atomicAdd(loss_acc, loss_part);
-      atomicAdd(loss_acc + 1, ratio_part);
-    }
-  }
-}
-
-// The same for N = 16 (D = 8): its 136-entry triangle does not fit the 255-register budget (seglik_chol_kernel spills
-// 44 bytes at N = 14 already).  The triangle and z live in shared memory as [entry][thread] (conflict free, 39 KB), the
-// loops stay rolled (unrolled, the compiler caches the shared values in registers and spills ~2 KB per thread).
-template <int N>
-__global__ void __launch_bounds__(CH_THREADS)
-seglik_chol_smem_kernel(const double *Cmat, const double *Rres, double *Gout, double *Aout, const double *__restrict__ diag_max,
-                   double reg_rel, const float *__restrict__ grad_logp, const float *__restrict__ logp_old,
-                   const float *__restrict__ advantage, double grad_scale, double *__restrict__ loss_acc,
-                   float *__restrict__ logp, int32_t *__restrict__ info, long long BP, int P, int want_grad) {
-  constexpr int NT = tri(N);
-  __shared__ double sm[(NT + N) * CH_THREADS];
-  const long long gid = (long long)blockIdx.x * CH_THREADS + threadIdx.x;
-  const bool active = gid < BP;
-  double loss_part = 0.0, ratio_part = 0.0;
-  if (active) {
-    const long long b = gid / P;
-    const int p = (int)(gid % P);
-    const double *Cb = Cmat + (size_t)b * NT * P + p;
-    const double *Rb = Rres + (size_t)b * N * P + p;
-    double *Gb = Gout + (size_t)b * NT * P + p;
-    double *Ab = Aout + (size_t)b * N * P + p;
-#define CLIN(e) sm[(e) * CH_THREADS + threadIdx.x]
-#define CE(r, q) CLIN(tri_idx(r, q))
-#define ZE(i) sm[(NT + (i)) * CH_THREADS + threadIdx.x]
-    const double reg = reg_rel * (*diag_max);
-#pragma unroll 1
-    for (int e = 0; e < NT; ++e) CLIN(e) = Cb[(size_t)e * P];
-#pragma unroll 1
-    for (int i = 0; i < N; ++i) ZE(i) = Rb[(size_t)i * P];
-    // Cholesky (in place, lower), forward substitution and log-determinant
-    int bad = 0;
-    double half_logdet = 0.0, maha = 0.0;
-#pragma unroll 1
-    for (int j = 0; j < N; ++j) {
-      double dj = CE(j, j) + reg;
-#pragma unroll 1
-      for (int k = 0; k < j; ++k) dj = fma(-CE(j, k), CE(j, k), dj);
-      if (!(dj > 0.0) && bad == 0) bad = j + 1;
-      // 1/sqrt(dj): fp32 MUFU seed + two fp64 Newton steps (1e-7 -> 1e-14 -> rounding).  The DIAGONAL STORES THE
-      // RECIPROCAL 1/S_jj: every later division (substitutions, inverse) becomes a multiplication -- fp64 divide
-      // and sqrt are ~40-instruction subroutines and there were ~130 of them per segment.
-      double inv = (double)rsqrtf((float)dj);
-      inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
-      inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
-      CE(j, j) = inv;
-      half_logdet += 0.5 * log(dj);
-#pragma unroll 1
-      for (int i = j + 1; i < N; ++i) {
-        double v = CE(i, j);
-#pragma unroll 1
-        for (int k = 0; k < j; ++k) v = fma(-CE(i, k), CE(j, k), v);
-        CE(i, j) = v * inv;
-      }
-      double zj = ZE(j);
-#pragma unroll 1
-      for (int k = 0; k < j; ++k) zj = fma(-CE(j, k), ZE(k), zj);
-      zj *= inv;
-      ZE(j) = zj;
-      maha = fma(zj, zj, maha);
-    }
-    const double lp = -0.5 * ((double)N * 1.8378770664093453 + maha) - half_logdet;
-    if (logp) logp[gid] = (float)lp;
-    if (info) info[gid] = bad;
-    if (want_grad) {
-      double g;
-      if (logp_old) {                      // fused surrogate: loss = -grad_scale * sum ratio * adv
-        const double ratio = exp(lp - (double)logp_old[gid]);
-        g = -ratio * (double)advantage[gid] * grad_scale;
-        loss_part = g;
-        ratio_part = ratio * grad_scale;
-      } else {
-        g = (double)grad_logp[gid];
-      }
-      // alpha = S^-T z (back substitution)
-#pragma unroll 1
-      for (int i = N - 1; i >= 0; --i) {
-        double v = ZE(i);
-#pragma unroll 1
-        for (int k = i + 1; k < N; ++k) v = fma(-CE(k, i), ZE(k), v);
-        ZE(i) = v * CE(i, i);
-      }
-      // S <- S^-1 (lower, in place; the diagonal already holds 1/S_jj = X_jj)
-#pragma unroll 1
-      for (int j = 0; j < N; ++j) {
-#pragma unroll 1
-        for (int i = j + 1; i < N; ++i) {
-          double v = 0.0;
-#pragma unroll 1
-          for (int k = j; k < i; ++k) v = fma(CE(i, k), CE(k, j), v);
-          CE(i, j) = -v * CE(i, i);
-        }
-      }
-      // (column j: S[i][k], j <= k < i, are still the Cholesky entries; X[k][j], k < i, are done)
-      // C^-1 = X^T X (lower, in place, row by row: entry (i,j) only reads rows k >= i, and within row i
-      // the diagonal X[i][i] is consumed last), then G = g/2 (alpha alpha^T - C^-1)
-#pragma unroll 1
-      for (int i = 0; i < N; ++i) {
-#pragma unroll 1
-        for (int j = 0; j <= i; ++j) {
-          double v = 0.0;
-#pragma unroll 1
-          for (int k = i; k < N; ++k) v = fma(CE(k, i), CE(k, j), v);
-          CE(i, j) = 0.5 * g * (ZE(i) * ZE(j) - v);
-        }
-      }
-#pragma unroll 1
-      for (int e = 0; e < NT; ++e) Gb[(size_t)e * P] = CLIN(e);
-#pragma unroll 1
-      for (int i = 0; i < N; ++i) Ab[(size_t)i * P] = g * ZE(i);
-    }
-#undef CE
-#undef CLIN
-#undef ZE
   }
   if (loss_acc) {
     loss_part = warp_sum(loss_part);
@@ -818,7 +582,7 @@ seglik_diag_kernel(TabDev tb, const float *__restrict__ smp_traj, const float *_
     const double l11 = sqrt(d11);
     const double z0 = r[0] / l00, z1 = (r[1] - l10 * z0) / l11;
     if (MODE == 1) {
-      part[d * P + p] = -0.5 * (2.0 * 1.8378770664093453 + z0 * z0 + z1 * z1) - 0.5 * (log(c00) + log(d11));
+      part[d * P + p] = -0.5 * (2.0 * LN_2PI + z0 * z0 + z1 * z1) - 0.5 * (log(c00) + log(d11));
       bad_s[d * P + p] = bad;
     } else {
       const double g = (double)grad_logp[b * P + p];
@@ -1058,13 +822,8 @@ extern "C" int tce_seglik_chol(const tce_tables_t *t, const void *work, void *ad
                                                             advantage, grad_scale, loss_acc, logp, info, BP,   \
                                                             (int)P, want_grad);                                \
     break;
-    Y(1) Y(2) Y(3) Y(4) Y(5) Y(6) Y(7)
+    Y(1) Y(2) Y(3) Y(4) Y(5) Y(6) Y(7) Y(8)
 #undef Y
-    case 8:
-      seglik_chol_smem_kernel<16><<<grid, CH_THREADS, 0, st>>>(Cmat, R, G, A, diag_max, reg_rel, grad_logp, logp_old,
-                                                               advantage, grad_scale, loss_acc, logp, info, BP, (int)P,
-                                                               want_grad);
-      break;
     default: return TCE_ERR_UNSUPPORTED_SHAPE;
   }
   TCE_CHECK_LAUNCH("seglik_chol_kernel");

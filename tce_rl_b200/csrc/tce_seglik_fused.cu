@@ -30,24 +30,11 @@
 // every shipped TCE config -- makes C_p, its factor and its inverse identical for all episodes:
 // tce_seglik_uniform_* evaluate them once and reduce the per-episode work to a residual, two 14 x 14 triangular
 // products and a rank-1 update (~50x fewer FLOPs).
-#include <math.h>
-
-#include "tce_common.cuh"
+#include "tce_seglik.cuh"
 
 namespace {
 
 constexpr int FT = 256;                      // threads of the fused kernel
-constexpr double LN_2PI = 1.8378770664093453;
-
-__host__ __device__ constexpr int tri(int n) { return n * (n + 1) / 2; }
-__device__ __forceinline__ int tri_idx(int r, int c) { return r * (r + 1) / 2 + c; }   // r >= c
-__device__ __forceinline__ void tri_decode(int t, int &I, int &J) {
-  int i = (int)((sqrtf(8.0f * (float)t + 1.0f) - 1.0f) * 0.5f);
-  while (i * (i + 1) / 2 > t) --i;
-  while ((i + 1) * (i + 2) / 2 <= t) ++i;
-  I = i;
-  J = t - i * (i + 1) / 2;
-}
 
 // ---- links between time points and pairs -------------------------------------------------------------
 // chained pairs (second time of pair p == first time of pair p + 1: the fixed-interval selection of every TCE
@@ -73,207 +60,31 @@ __device__ int block_chained(const int64_t *__restrict__ pairs, int P) {
   return __syncthreads_and(ok) != 0;
 }
 
-// ---- ProDMP basis rows with initial conditions (SURVEY App. A.3) ---------------------------------------------
-// init_row [5 + 2 K1]: y1b, y2b, dy1b, dy2b, 1/det, pos_b[K1], vel_b[K1] at the episode's initial time
-template <int K1>
-__device__ __forceinline__ void init_row_entry(const TabDev &tb, double t_init, int j, double *init_row) {
-  int i0; double w;
-  time_to_index(tb, t_init, i0, w);
-  if (j < K1) {
-    init_row[5 + j] = lerp_t(tb.pos[(size_t)i0 * K1 + j], tb.pos[(size_t)(i0 + 1) * K1 + j], w);
-    init_row[5 + K1 + j] = lerp_t(tb.vel[(size_t)i0 * K1 + j], tb.vel[(size_t)(i0 + 1) * K1 + j], w);
-  } else {
-    const double a = lerp_t(tb.y1[i0], tb.y1[i0 + 1], w), b = lerp_t(tb.y2[i0], tb.y2[i0 + 1], w);
-    const double c = lerp_t(tb.dy1[i0], tb.dy1[i0 + 1], w), d = lerp_t(tb.dy2[i0], tb.dy2[i0 + 1], w);
-    init_row[0] = a; init_row[1] = b; init_row[2] = c; init_row[3] = d;
-    init_row[4] = 1.0 / (a * d - b * c);
-  }
-}
-// entry j of the scaled basis row at time t (j < K1) or the pair (xi1, xi2) (j == K1)
-template <int K1>
-__device__ __forceinline__ void basis_entry(const TabDev &tb, const double *init_row, double t, int j, double *h_row,
-                                            double *xi_row) {
-  int i0; double w;
-  time_to_index(tb, t, i0, w);
-  const double y1 = lerp_t(tb.y1[i0], tb.y1[i0 + 1], w), y2 = lerp_t(tb.y2[i0], tb.y2[i0 + 1], w);
-  const double idet = init_row[4];
-  const double xi1 = (init_row[3] * y1 - init_row[2] * y2) * idet, xi2 = (init_row[0] * y2 - init_row[1] * y1) * idet;
-  if (j < K1) {
-    const double pj = lerp_t(tb.pos[(size_t)i0 * K1 + j], tb.pos[(size_t)(i0 + 1) * K1 + j], w);
-    h_row[j] = (pj - xi1 * init_row[5 + j] - xi2 * init_row[5 + K1 + j]) * tb.scale[j];
-  } else {
-    xi_row[0] = xi1;
-    xi_row[1] = xi2;
-  }
-}
-
-// ---- per-segment factorisation in registers -----------------------------------------------------------------
-// c: packed lower triangle of C (no regulariser), z: residual.  On return c holds the Cholesky factor with the
-// RECIPROCAL pivots on the diagonal, z = S^-1 r; returns log-prob, bad = index + 1 of the first non-positive pivot.
-template <int N>
-__device__ __forceinline__ double seg_factor(double (&c)[tri(N)], double (&z)[N], double reg, int &bad) {
-#define CE(r, q) c[(r) * ((r) + 1) / 2 + (q)]
-  bad = 0;
-  double half_logdet = 0.0, maha = 0.0;
-#pragma unroll
-  for (int j = 0; j < N; ++j) {
-    double dj = CE(j, j) + reg;
-#pragma unroll
-    for (int k = 0; k < j; ++k) dj = fma(-CE(j, k), CE(j, k), dj);
-    if (!(dj > 0.0) && bad == 0) bad = j + 1;
-    double inv = (double)rsqrtf((float)dj);             // fp32 MUFU seed + two fp64 Newton steps
-    inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
-    inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
-    CE(j, j) = inv;
-    half_logdet += 0.5 * log(dj);
-#pragma unroll
-    for (int i = j + 1; i < N; ++i) {
-      double v = CE(i, j);
-#pragma unroll
-      for (int k = 0; k < j; ++k) v = fma(-CE(i, k), CE(j, k), v);
-      CE(i, j) = v * inv;
-    }
-    double zj = z[j];
-#pragma unroll
-    for (int k = 0; k < j; ++k) zj = fma(-CE(j, k), z[k], zj);
-    zj *= inv;
-    z[j] = zj;
-    maha = fma(zj, zj, maha);
-  }
-  return -0.5 * ((double)N * LN_2PI + maha) - half_logdet;
-}
-// after seg_factor: c <- g/2 (alpha alpha^T - C^-1) (lower), z <- g alpha
-template <int N>
-__device__ __forceinline__ void seg_adjoint(double (&c)[tri(N)], double (&z)[N], double g) {
-#pragma unroll
-  for (int i = N - 1; i >= 0; --i) {                     // alpha = S^-T z
-    double v = z[i];
-#pragma unroll
-    for (int k = i + 1; k < N; ++k) v = fma(-CE(k, i), z[k], v);
-    z[i] = v * CE(i, i);
-  }
-#pragma unroll
-  for (int j = 0; j < N; ++j) {                          // S <- S^-1 (diagonal already holds 1 / S_jj)
-#pragma unroll
-    for (int i = j + 1; i < N; ++i) {
-      double v = 0.0;
-#pragma unroll
-      for (int k = j; k < i; ++k) v = fma(CE(i, k), CE(k, j), v);
-      CE(i, j) = -v * CE(i, i);
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < N; ++i) {                          // C^-1 = X^T X row by row, then G
-#pragma unroll
-    for (int j = 0; j <= i; ++j) {
-      double v = 0.0;
-#pragma unroll
-      for (int k = i; k < N; ++k) v = fma(CE(k, i), CE(k, j), v);
-      CE(i, j) = 0.5 * g * (z[i] * z[j] - v);
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < N; ++i) z[i] *= g;
-#undef CE
-}
-
 // phase 2 of the fused kernel for one segment: column `slot` of C [NT][S] / r [N][S] in shared memory -> log-prob,
 // upstream gradient, adjoints written back in place.  Deliberately NOT inlined: the packed triangle needs ~240
 // registers; as a separate function it gets the whole register file instead of competing with the kernel's
 // loop state (inlined: 4-6 KB of spill traffic per thread).
-struct SegIO {
-  const float *grad_logp, *logp_old, *advantage;
-  float *logp;
-  int32_t *info;
-  double grad_scale, reg;
-  int grad_mode;
-};
 template <int N>
 __device__ __noinline__ void segment_thread(double *Ccol, double *Rcol, int S, long long gid, const SegIO &io,
                                             double &loss_part, double &ratio_part) {
   // The packed triangle (N (N + 1) / 2 doubles = 210 registers at N = 14) lives in registers with compile-time
   // indices; the residual / z / alpha vector stays in the thread's shared-memory column (Rcol, stride S): with it in
   // registers too the function spills ~1.4 KB per thread, and with ~215 KB of the SM's L1 configured as shared
-  // memory those spills go to L2.
+  // memory those spills go to L2.  G goes straight to the column of C.
   constexpr int NT = tri(N);
   double c[NT];
-#define CE(r, q) c[(r) * ((r) + 1) / 2 + (q)]
-#define ZS(i) Rcol[(size_t)(i) * S]
+  Strided z{Rcol, S}, G{Ccol, S};
 #pragma unroll
   for (int t = 0; t < NT; ++t) c[t] = Ccol[(size_t)t * S];
-  int bad = 0;
-  double half_logdet = 0.0, maha = 0.0;
-#pragma unroll
-  for (int j = 0; j < N; ++j) {
-    double dj = CE(j, j) + io.reg;
-#pragma unroll
-    for (int k = 0; k < j; ++k) dj = fma(-CE(j, k), CE(j, k), dj);
-    if (!(dj > 0.0) && bad == 0) bad = j + 1;
-    double inv = (double)rsqrtf((float)dj);             // fp32 MUFU seed + two fp64 Newton steps
-    inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
-    inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
-    CE(j, j) = inv;                                     // the diagonal holds 1 / S_jj
-    half_logdet += 0.5 * log(dj);
-#pragma unroll
-    for (int i = j + 1; i < N; ++i) {
-      double v = CE(i, j);
-#pragma unroll
-      for (int k = 0; k < j; ++k) v = fma(-CE(i, k), CE(j, k), v);
-      CE(i, j) = v * inv;
-    }
-    double zj = ZS(j);
-#pragma unroll
-    for (int k = 0; k < j; ++k) zj = fma(-CE(j, k), ZS(k), zj);
-    zj *= inv;
-    ZS(j) = zj;
-    maha = fma(zj, zj, maha);
-  }
-  const double lp = -0.5 * ((double)N * LN_2PI + maha) - half_logdet;
+  int bad;
+  const double lp = seg_factor<N, true>(c, z, io.reg, bad);
   if (io.logp) io.logp[gid] = (float)lp;
   if (io.info) io.info[gid] = bad;
   if (io.grad_mode == 0) return;
-  double g;
-  if (io.grad_mode == 2) {
-    const double ratio = exp(lp - (double)io.logp_old[gid]);
-    g = -ratio * (double)io.advantage[gid] * io.grad_scale;
-    loss_part += g;
-    ratio_part += ratio * io.grad_scale;
-  } else {
-    g = (double)io.grad_logp[gid];
-  }
+  const double g = seg_upstream(io, lp, gid, loss_part, ratio_part);
+  seg_adjoint<N, true>(c, z, g, G);
 #pragma unroll
-  for (int i = N - 1; i >= 0; --i) {                     // alpha = S^-T z
-    double v = ZS(i);
-#pragma unroll
-    for (int k = i + 1; k < N; ++k) v = fma(-CE(k, i), ZS(k), v);
-    ZS(i) = v * CE(i, i);
-  }
-#pragma unroll
-  for (int j = 0; j < N; ++j) {                          // S <- S^-1
-#pragma unroll
-    for (int i = j + 1; i < N; ++i) {
-      double v = 0.0;
-#pragma unroll
-      for (int k = j; k < i; ++k) v = fma(CE(i, k), CE(k, j), v);
-      CE(i, j) = -v * CE(i, i);
-    }
-  }
-  const double hg = 0.5 * g;
-#pragma unroll
-  for (int i = 0; i < N; ++i) {                          // C^-1 = X^T X row by row, then G = g/2 (alpha alpha^T - C^-1)
-    const double ai = ZS(i);
-#pragma unroll
-    for (int j = 0; j <= i; ++j) {
-      double v = 0.0;
-#pragma unroll
-      for (int k = i; k < N; ++k) v = fma(CE(k, i), CE(k, j), v);
-      Ccol[(size_t)(i * (i + 1) / 2 + j) * S] = hg * (ai * ZS(j) - v);
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < N; ++i) ZS(i) = g * ZS(i);
-#undef CE
-#undef ZS
+  for (int i = 0; i < N; ++i) z[i] = g * z[i];
 }
 
 // phase 3b of the fused kernel: dSigma_dd'[i][j] = sum_q w_q[i] h_q[j] for one (episode, DoF block), 81 register
