@@ -336,8 +336,8 @@ int launch_traj_uniform(const tce_tables *t, const float *params, const float *t
   while (epc > 4 && (B + epc - 1) / epc < 2LL * num_sms()) epc >>= 1;
   int estride = (TU_TT * D2 + 3) & ~3;                 // multiple of 4 and = 8 (mod 32): conflict-light tile rows
   while ((estride & 31) != 8) estride += 4;
-  const size_t smem = sizeof(float) * ((size_t)T * RWP + (size_t)epc * estride);
-  if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;
+  const size_t smem = sizeof(float) * ((size_t)T * RWP + (size_t)epc * estride);   // ops.traj_uniform_layout mirrors
+  if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;                           // epc and smem: keep them in step
   if (smem > 48 * 1024)
     TCE_CUDA(cudaFuncSetAttribute(traj_uniform_kernel<K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
              "traj uniform smem attr");

@@ -100,6 +100,30 @@ class Tables:
 
 # --------------------------------------------------------------------------------------------------
 UNIFORM_TRAJ = True      # common-time-grid fast path of the trajectory synthesis (False: always the general kernel)
+_NUM_SMS = {}
+
+
+def _num_sms(device) -> int:
+    idx = torch.device(device).index
+    idx = torch.cuda.current_device() if idx is None else idx
+    if idx not in _NUM_SMS:
+        _NUM_SMS[idx] = torch.cuda.get_device_properties(idx).multi_processor_count
+    return _NUM_SMS[idx]
+
+
+def traj_uniform_layout(B: int, T: int, num_dof: int, k1: int, sms: int) -> Tuple[int, int]:
+    """(episodes per CTA, dynamic shared memory in bytes) of ``tce_prodmp_traj_fwd_uniform``: the same formula as
+    ``launch_traj_uniform`` (csrc/tce_traj.cu).  A CTA holds all T basis rows and one output tile."""
+    epc = min(256 // num_dof, 16)
+    while epc > 4 and -(-B // epc) < 2 * sms:
+        epc //= 2
+    estride = (20 * 2 * num_dof + 3) // 4 * 4
+    while estride % 32 != 8:
+        estride += 4
+    return epc, 4 * (T * ((2 * (k1 + 2) + 3) // 4 * 4) + epc * estride)
+
+
+TRAJ_UNIFORM_SMEM = 200 * 1024    # the uniform kernel's limit; longer horizons run the general kernel
 
 
 # (1) trajectory synthesis
@@ -112,9 +136,12 @@ def prodmp_traj(params: Tensor, times: Tensor, init_time: Tensor, init_pos: Tens
     B, T = times.shape
     traj = torch.empty(B, T, 2 * num_dof, device=params.device, dtype=torch.float32)
     # one time grid for the whole batch (a cached device read per tensor; never decided under graph capture): the
-    # basis rows are evaluated once and the batch becomes a small matrix product per episode
-    if UNIFORM_TRAJ and B >= 64 and times_uniform(init_time, times):
-        k1 = params.shape[-1] // num_dof
+    # basis rows are evaluated once and the batch becomes a small matrix product per episode.  The rows live in shared
+    # memory, so a horizon whose rows do not fit runs the general kernel.
+    k1 = params.shape[-1] // num_dof
+    if UNIFORM_TRAJ and B >= 64 and \
+            traj_uniform_layout(B, T, num_dof, k1, _num_sms(params.device))[1] <= TRAJ_UNIFORM_SMEM and \
+            times_uniform(init_time, times):
         rows = torch.empty(T * ((2 * (k1 + 2) + 3) // 4 * 4), device=params.device, dtype=torch.float32)
         _lib.call("tce_prodmp_traj_fwd_uniform", tables, _p(params), _p(times), _p(init_time), _p(init_pos), _p(init_vel),
                   _p(rows), _p(traj), B, T, _stream())
@@ -174,6 +201,32 @@ def mvn_rsample(mean: Tensor, L: Tensor, eps: Optional[Tensor], seed: int, offse
 @mvn_rsample.register_fake
 def _(mean, L, eps, seed, offset):
     return torch.empty_like(mean)
+
+
+def _rsample_setup(ctx, inputs, output):
+    mean, L, eps, seed, offset = inputs
+    ctx.save_for_backward(L if eps is not None and eps.requires_grad else None, eps)
+    ctx.seed, ctx.offset = seed, offset
+
+
+def _rsample_backward(ctx, g):
+    """out = mean + tril(L) eps: d/dmean = g, d/dL[b] = tril(g[b] eps[b]^T) (dense: autograd sums it for a stride-0
+    expanded factor), d/deps = tril(L)^T g.  In-kernel draws are regenerated from (seed, offset): the Philox counter
+    is the element index b * n + j whatever the factor, so the identity at stride 0 returns the forward's eps."""
+    L, eps = ctx.saved_tensors
+    g_L = g_eps = None
+    if ctx.needs_input_grad[1]:
+        if eps is None:
+            B, n = g.shape
+            eye = torch.eye(n, device=g.device, dtype=torch.float32).expand(B, n, n)
+            eps = mvn_rsample(g.new_zeros(B, n), eye, None, ctx.seed, ctx.offset)
+        g_L = torch.tril(g.unsqueeze(-1) * eps.unsqueeze(-2))
+    if ctx.needs_input_grad[2]:
+        g_eps = torch.einsum('bij,bi->bj', torch.tril(L), g)
+    return (g if ctx.needs_input_grad[0] else None), g_L, g_eps, None, None
+
+
+mvn_rsample.register_autograd(_rsample_backward, setup_context=_rsample_setup)
 
 
 @torch.library.custom_op("tce::chol_fwd", mutates_args=())

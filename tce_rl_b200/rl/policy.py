@@ -119,7 +119,8 @@ class BlackBoxPolicy(AbstractGaussianPolicy):
             smp = params_mean
         else:
             seed = int(torch.randint(0, 2 ** 62, [], device="cpu").item()) if eps is None else 0
-            smp = ops.mvn_rsample(params_mean, params_L, eps, seed, 0)
+            with torch.set_grad_enabled(bool(require_grad) and torch.is_grad_enabled()):   # nothing saved for a backward
+                smp = ops.mvn_rsample(params_mean, params_L, eps, seed, 0)
         return smp if require_grad else smp.detach()
 
     def log_prob(self, smp_params, params_mean, params_L, **kwargs):
@@ -158,12 +159,13 @@ class TemporalCorrelatedPolicy(BlackBoxPolicy):
                eps=None):
         """Trajectory [B, T, 2 D] (pos | vel) of sampled (or mean) ProDMP parameters
         (temporal_correlated_policy.py:34-102); ``eps`` [B, Dp] injects the normal draw."""
-        if use_mean:
-            theta = params_mean
-        else:
-            seed = int(torch.randint(0, 2 ** 62, [], device="cpu").item()) if eps is None else 0
-            theta = ops.mvn_rsample(params_mean, params_L, eps, seed, 0)
-        traj = ops.prodmp_traj(theta, times, init_time, init_pos, init_vel, self.mp.tables.handle, self.num_dof)
+        with torch.set_grad_enabled(bool(require_grad) and torch.is_grad_enabled()):      # nothing saved for a backward
+            if use_mean:
+                theta = params_mean
+            else:
+                seed = int(torch.randint(0, 2 ** 62, [], device="cpu").item()) if eps is None else 0
+                theta = ops.mvn_rsample(params_mean, params_L, eps, seed, 0)
+            traj = ops.prodmp_traj(theta, times, init_time, init_pos, init_vel, self.mp.tables.handle, self.num_dof)
         return traj if require_grad else traj.detach()
 
     def log_prob(self, smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel, **kwargs):
