@@ -271,6 +271,44 @@ int tce_proj_w2_cov_bwd(const float *L, const float *L_o, int64_t ldb_Lo, double
 int tce_cov_distance(int kind, const float *L, const float *L_o, int64_t ldb_Lo, int scale_prec,
                      const double *grad_val, double *val, float *grad_L, int64_t B, int n, void *stream);
 
+/* ---- (4b) the same for DIAGONAL factors (std_only policies) ---------------------------------------------------
+ * L = diag(s), L_o = diag(s_old), each a strided vector as for tce_proj_kl_diag_* (element i of episode b is
+ * s[b * ldb + i * inc]; ldb = 0 on an input broadcasts one vector).  Each entry point computes what the dense entry
+ * point above it computes on diag(s), elementwise: one warp per episode, n <= 1024, no shared memory.
+ * tce_gauss_stats_diag: out [B, 5] of tce_gauss_stats; s == NULL: the Mahalanobis term only, out [B] (no tce_tri_inverse
+ * for a shared factor); mean == mean_o == NULL: zero mean difference.  _bwd: grad_mean [B, n] (may be NULL) and grad_s
+ * (may be NULL) from grad_out [B, 5] (s == NULL: [B]).                                                               */
+int tce_gauss_stats_diag(const float *mean, const float *mean_o, const float *s, int64_t ldb_s, int64_t inc_s,
+                         const float *s_old, int64_t ldb_so, int64_t inc_so, double *out, int64_t B, int n,
+                         void *stream);
+int tce_gauss_stats_diag_bwd(const float *mean, const float *mean_o, const float *s, int64_t ldb_s, int64_t inc_s,
+                             const float *s_old, int64_t ldb_so, int64_t inc_so, const double *grad_out,
+                             float *grad_mean, float *grad_s, int64_t ldb_gs, int64_t inc_gs, int64_t B, int n,
+                             void *stream);
+/* Frobenius projection of the variances: out = sqrt((s^2 + eta s_old^2) / (1 + eta)); W2 (commutative) of the
+ * factors: out = (s + eta s_old) / (1 + eta); eta as in tce_proj_frob/w2_cov_fwd; save_sc [B, 4] = {eta, active, cp, 0}
+ * feeds the backward; info [B] (optional): 1 if a projected variance is not positive.  The backward returns
+ * d loss / d s (s_old is a constant).                                                                             */
+int tce_proj_frob_diag_fwd(const float *s, int64_t ldb_s, int64_t inc_s, const float *s_old, int64_t ldb_so,
+                           int64_t inc_so, double eps_cov, float *out, int64_t ldb_o, int64_t inc_o, double *save_sc,
+                           int32_t *info, int64_t B, int n, void *stream);
+int tce_proj_frob_diag_bwd(const float *s, int64_t ldb_s, int64_t inc_s, const float *s_old, int64_t ldb_so,
+                           int64_t inc_so, double eps_cov, const double *save_sc, const float *grad_out, int64_t ldb_g,
+                           int64_t inc_g, float *grad_s, int64_t ldb_gs, int64_t inc_gs, int64_t B, int n,
+                           void *stream);
+int tce_proj_w2_diag_fwd(const float *s, int64_t ldb_s, int64_t inc_s, const float *s_old, int64_t ldb_so,
+                         int64_t inc_so, double eps_cov, int scale_prec, float *out, int64_t ldb_o, int64_t inc_o,
+                         double *save_sc, int64_t B, int n, void *stream);
+int tce_proj_w2_diag_bwd(const float *s, int64_t ldb_s, int64_t inc_s, const float *s_old, int64_t ldb_so,
+                         int64_t inc_so, double eps_cov, int scale_prec, const double *save_sc, const float *grad_out,
+                         int64_t ldb_g, int64_t inc_g, float *grad_s, int64_t ldb_gs, int64_t inc_gs, int64_t B, int n,
+                         void *stream);
+/* covariance distance of tce_cov_distance (kind 0 Frobenius, 1 W2) on diagonal factors: val [B] when
+ * grad_val == NULL, otherwise grad_s = grad_val[b] * d val / d s.                                                 */
+int tce_cov_distance_diag(int kind, const float *s, int64_t ldb_s, int64_t inc_s, const float *s_old, int64_t ldb_so,
+                          int64_t inc_so, int scale_prec, const double *grad_val, double *val, float *grad_s,
+                          int64_t ldb_gs, int64_t inc_gs, int64_t B, int n, void *stream);
+
 /* ---- (3) TCE segment-wise trajectory likelihood -----------------------------------------------------
  * TemporalCorrelatedPolicy.log_prob (temporal_correlated_policy.py:104-203) = mp.update_inputs +
  * get_traj_pos(flat) + get_traj_pos_cov + MultivariateNormal(covariance_matrix).log_prob.
@@ -337,7 +375,8 @@ int tce_seglik_bwd_shared(const tce_tables_t *tables, const void *work, const fl
  * tce_seglik_diag_max: the regulariser seed diag_max = max over the batch of diag C (atomic max into *diag_max,
  * zero it first; all-reduce(MAX) it between the launches at > 1 GPU).  tce_seglik_diag_fwd: logp [B, P], info [B, P]
  * (optional; first non-positive pivot as in tce_seglik_chol).  tce_seglik_diag_bwd: from grad_logp [B, P],
- * grad_mean [B, Dp] and grad_s (strided, ldb_gs > 0), either may be NULL.  fp64 arithmetic, fixed summation order. */
+ * grad_mean [B, Dp] and grad_s (strided, ldb_gs > 0), either may be NULL.  fp64 arithmetic, fixed summation order.
+ * Every shape the tables accept (1 <= D <= 8, 2 <= K1 <= 16, Dp up to 128), not only the Dp <= 64 of the dense path. */
 int tce_seglik_diag_max(const tce_tables_t *tables, const float *s, int64_t ldb_s, int64_t inc_s,
                         const float *times, const float *init_time, const int64_t *pred_pairs, double *diag_max,
                         int64_t B, int64_t T, int64_t P, void *stream);

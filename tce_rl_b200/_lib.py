@@ -51,6 +51,17 @@ SIGNATURES = {
                                        _I32, _P]),
     "tce_proj_kl_diag_bwd": (C.c_int, [_P, _I64, _I64, _P, _I64, _I64, _P, _P, _I64, _I64, _P, _I64, _I64, _I64, _I32,
                                        _P]),
+    "tce_gauss_stats_diag": (C.c_int, [_P, _P, _P, _I64, _I64, _P, _I64, _I64, _P, _I64, _I32, _P]),
+    "tce_gauss_stats_diag_bwd": (C.c_int, [_P, _P, _P, _I64, _I64, _P, _I64, _I64, _P, _P, _P, _I64, _I64, _I64, _I32,
+                                           _P]),
+    "tce_proj_frob_diag_fwd": (C.c_int, [_P, _I64, _I64, _P, _I64, _I64, _D, _P, _I64, _I64, _P, _P, _I64, _I32, _P]),
+    "tce_proj_frob_diag_bwd": (C.c_int, [_P, _I64, _I64, _P, _I64, _I64, _D, _P, _P, _I64, _I64, _P, _I64, _I64, _I64,
+                                         _I32, _P]),
+    "tce_proj_w2_diag_fwd": (C.c_int, [_P, _I64, _I64, _P, _I64, _I64, _D, _I32, _P, _I64, _I64, _P, _I64, _I32, _P]),
+    "tce_proj_w2_diag_bwd": (C.c_int, [_P, _I64, _I64, _P, _I64, _I64, _D, _I32, _P, _P, _I64, _I64, _P, _I64, _I64,
+                                       _I64, _I32, _P]),
+    "tce_cov_distance_diag": (C.c_int, [_I32, _P, _I64, _I64, _P, _I64, _I64, _I32, _P, _P, _P, _I64, _I64, _I64, _I32,
+                                        _P]),
     "tce_seglik_diag_max": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
     "tce_seglik_diag_fwd": (C.c_int, [_P, _P, _P, _P, _I64, _I64, _P, _P, _P, _P, _P, _P, _D, _P, _P, _I64, _I64, _I64,
                                       _P]),

@@ -725,6 +725,12 @@ static bool shape_supported(const tce_tables_t *t) {
   return t->D >= 1 && t->D <= TCE_MAX_DOF && t->K1 >= 2 && t->K1 <= TCE_MAX_K1 && t->D * t->K1 <= TCE_MAX_DP;
 }
 
+// The diagonal likelihood keeps no Dp x Dp matrix: its work per (pair, DoF) depends on K1 only, so it takes every
+// shape the tables accept
+static bool diag_shape_supported(const tce_tables_t *t) {
+  return t->D >= 1 && t->D <= TCE_MAX_DOF && t->K1 >= 2 && t->K1 <= TCE_MAX_K1;
+}
+
 extern "C" int tce_seglik_compiled(const tce_tables_t *t) {
   if (!t) return TCE_ERR_INVALID_ARGUMENT;
 #define X(Dv, Kv) if (t->D == Dv && t->K1 == Kv) return 1;
@@ -906,7 +912,7 @@ static int seglik_diag_launch(const tce_tables_t *t, const float *smp_traj, cons
                                      ldb_gs, inc_gs, B, T, P, st);
   TCE_FOR_SHAPES(X)
 #undef X
-  if (!shape_supported(t)) return TCE_ERR_UNSUPPORTED_SHAPE;
+  if (!diag_shape_supported(t)) return TCE_ERR_UNSUPPORTED_SHAPE;
   TCE_DISPATCH_K1(t->K1, return (diag_launch<0, K1, MODE>(t, smp_traj, mean, s, ldb_s, inc_s, times, init_time,
                                                           init_pos, init_vel, pred_pairs, diag_max, reg_rel, grad_logp,
                                                           logp, info, grad_mean, grad_s, ldb_gs, inc_gs, B, T, P, st)));

@@ -73,7 +73,10 @@ class Tables:
         self.handle = handle.value
         self.num_pc = _lib.load().tce_prodmp_tables_num_pc(self.handle)
         # one of the five shapes with fused / uniform-grid likelihood kernels (else: staged kernels, see ops_seglik.compiled)
-        self.compiled = _lib.load().tce_seglik_compiled(self.handle) == 1
+        status = _lib.load().tce_seglik_compiled(self.handle)
+        self.compiled = status == 1
+        # the dense (full-covariance) likelihood takes this shape (Dp <= 64); the diagonal one takes every shape
+        self.dense_likelihood = status >= 0
 
     def export(self):
         """fp64 tables as CPU tensors (for tests / inspection)."""
@@ -1267,6 +1270,244 @@ def _pkd_backward(ctx, g, g_state, g_info):
 
 
 proj_kl_diag.register_autograd(_pkd_backward, setup_context=_pkd_setup)
+
+
+# --------------------------------------------------------------------------------------------------
+# (4b) diagonal factors (std_only policies): the dense ops above specialised to L = diag(s), one warp per episode,
+# n <= 1024.  Factors are [B or 1, n, n] tensors read on their diagonals only (any strides); gradients are dense
+# [B, n, n] buffers that are zero off the diagonal, as for proj_kl_diag.
+# --------------------------------------------------------------------------------------------------
+def _diag_pair(L: Tensor, L_o: Tensor) -> Tuple[int, int, int, int]:
+    ldb, inc = diag_strides(L)
+    ldb_o, inc_o = diag_strides(L_o, "L_o")
+    if L_o.shape[0] not in (1, L.shape[0]) or L_o.shape[-1] != L.shape[-1]:
+        raise TceError("L_o must be [B, n, n] or [1, n, n] with the n of L")
+    return ldb, inc, ldb_o, inc_o
+
+
+@torch.library.custom_op("tce::gauss_stats_diag", mutates_args=())
+def gauss_stats_diag(mean: Optional[Tensor], L: Tensor, mean_o: Optional[Tensor], L_o: Tensor) -> Tensor:
+    """``gauss_stats`` of diagonal factors -> [B, 5] fp64; ``mean`` = ``mean_o`` = None: zero mean difference.  B is the
+    batch of ``mean`` (else of ``L``); a [1, n, n] factor is broadcast.  Differentiable w.r.t. ``mean`` and ``L``."""
+    B = mean.shape[0] if mean is not None else L.shape[0]
+    if L.shape[0] not in (1, B):
+        raise TceError("L must be [B, n, n] or [1, n, n]")
+    ldb, inc, ldb_o, inc_o = _diag_pair(L, L_o)
+    if mean is not None:
+        mean, mean_o = _chk(mean), _chk(mean_o)
+    out = torch.empty(B, 5, device=L.device, dtype=torch.float64)
+    _lib.call("tce_gauss_stats_diag", _p(mean), _p(mean_o), _p(L), ldb, inc, _p(L_o), ldb_o, inc_o, _p(out), B,
+              L.shape[-1], _stream())
+    return out
+
+
+@gauss_stats_diag.register_fake
+def _(mean, L, mean_o, L_o):
+    return L.new_empty(mean.shape[0] if mean is not None else L.shape[0], 5, dtype=torch.float64)
+
+
+@torch.library.custom_op("tce::gauss_stats_diag_bwd", mutates_args=())
+def gauss_stats_diag_bwd(grad_out: Tensor, mean: Optional[Tensor], L: Tensor, mean_o: Optional[Tensor],
+                         L_o: Tensor) -> Tuple[Tensor, Tensor]:
+    """-> (d / d mean [B, n] (empty without a mean), d / d L [B, n, n] diagonal) from d loss / d stats [B, 5]."""
+    g = _chk(grad_out, torch.float64, "grad_out")
+    B = g.shape[0]
+    ldb, inc, ldb_o, inc_o = _diag_pair(L, L_o)
+    g_mean = torch.empty(B, L.shape[-1], device=L.device, dtype=torch.float32) if mean is not None else L.new_empty(0)
+    if mean is not None:
+        mean, mean_o = _chk(mean), _chk(mean_o)
+    n = L.shape[-1]
+    g_L = torch.zeros(B, n, n, device=L.device, dtype=torch.float32)
+    _lib.call("tce_gauss_stats_diag_bwd", _p(mean), _p(mean_o), _p(L), ldb, inc, _p(L_o), ldb_o, inc_o, _p(g),
+              _p(g_mean) if mean is not None else None, _p(g_L), n * n, n + 1, B, n, _stream())
+    return g_mean, g_L
+
+
+@gauss_stats_diag_bwd.register_fake
+def _(grad_out, mean, L, mean_o, L_o):
+    B, n = grad_out.shape[0], L.shape[-1]
+    return (L.new_empty(B, n) if mean is not None else L.new_empty(0)), L.new_empty(B, n, n)
+
+
+def _gsd_setup(ctx, inputs, output):
+    ctx.save_for_backward(*inputs)
+
+
+def _gsd_backward(ctx, g):
+    mean, L, mean_o, L_o = ctx.saved_tensors
+    g_mean, g_L = gauss_stats_diag_bwd(g.contiguous(), mean, L, mean_o, L_o)
+    if L.shape[0] != g_L.shape[0]:                     # one factor broadcast over the batch
+        g_L = g_L.sum(dim=0, keepdim=True)
+    return (g_mean if mean is not None and ctx.needs_input_grad[0] else None,
+            g_L if ctx.needs_input_grad[1] else None, None, None)
+
+
+gauss_stats_diag.register_autograd(_gsd_backward, setup_context=_gsd_setup)
+
+
+@torch.library.custom_op("tce::gauss_maha_diag", mutates_args=())
+def gauss_maha_diag(mean: Tensor, mean_o: Tensor, L_o: Tensor) -> Tensor:
+    """``gauss_maha`` with a diagonal factor L_o [B or 1, n, n] -> [B] fp64 (no triangular solve or inverse).
+    Differentiable w.r.t. ``mean`` and ``mean_o``; L_o is data, as in ``gauss_stats``."""
+    mean, mean_o = _chk(mean), _chk(mean_o)
+    B, n = mean.shape
+    ldb_o, inc_o = diag_strides(L_o, "L_o")
+    if L_o.shape[0] not in (1, B) or L_o.shape[-1] != n:
+        raise TceError("L_o must be [B, n, n] or [1, n, n]")
+    out = torch.empty(B, device=mean.device, dtype=torch.float64)
+    _lib.call("tce_gauss_stats_diag", _p(mean), _p(mean_o), None, 0, 0, _p(L_o), ldb_o, inc_o, _p(out), B, n, _stream())
+    return out
+
+
+@gauss_maha_diag.register_fake
+def _(mean, mean_o, L_o):
+    return mean.new_empty(mean.shape[0], dtype=torch.float64)
+
+
+@torch.library.custom_op("tce::gauss_maha_diag_bwd", mutates_args=())
+def gauss_maha_diag_bwd(grad: Tensor, mean: Tensor, mean_o: Tensor, L_o: Tensor) -> Tensor:
+    mean, mean_o = _chk(mean), _chk(mean_o)
+    g = _chk(grad, torch.float64, "grad")
+    ldb_o, inc_o = diag_strides(L_o, "L_o")
+    g_mean = torch.empty_like(mean)
+    _lib.call("tce_gauss_stats_diag_bwd", _p(mean), _p(mean_o), None, 0, 0, _p(L_o), ldb_o, inc_o, _p(g), _p(g_mean),
+              None, 0, 0, mean.shape[0], mean.shape[1], _stream())
+    return g_mean
+
+
+@gauss_maha_diag_bwd.register_fake
+def _(grad, mean, mean_o, L_o):
+    return torch.empty_like(mean)
+
+
+def _gmd_setup(ctx, inputs, output):
+    ctx.save_for_backward(*inputs)
+
+
+def _gmd_backward(ctx, g):
+    mean, mean_o, L_o = ctx.saved_tensors
+    g_mean = gauss_maha_diag_bwd(g, mean, mean_o, L_o)
+    return (g_mean if ctx.needs_input_grad[0] else None, -g_mean if ctx.needs_input_grad[1] else None, None)
+
+
+gauss_maha_diag.register_autograd(_gmd_backward, setup_context=_gmd_setup)
+
+
+@torch.library.custom_op("tce::proj_cov_diag", mutates_args=())
+def proj_cov_diag(kind: int, L: Tensor, L_o: Tensor, eps_cov: float, scale_prec: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """Frobenius (kind 0, ``proj_frob_cov``) / W2 (kind 1, ``proj_w2_cov``) covariance projection of diagonal factors
+    -> (out [Bc, n, n] diagonal, save_sc [Bc, 4] fp64 {eta, active, cp, 0}, info [Bc] int32)."""
+    ldb, inc, ldb_o, inc_o = _diag_pair(L, L_o)
+    Bc, n = L.shape[0], L.shape[-1]
+    out, ldb_out, inc_out = _dense_diag_grad(L)
+    sc = torch.empty(Bc, 4, device=L.device, dtype=torch.float64)
+    info = torch.zeros(Bc, device=L.device, dtype=torch.int32)
+    if kind == 0:
+        _lib.call("tce_proj_frob_diag_fwd", _p(L), ldb, inc, _p(L_o), ldb_o, inc_o, float(eps_cov), _p(out), ldb_out,
+                  inc_out, _p(sc), _p(info), Bc, n, _stream())
+    else:
+        _lib.call("tce_proj_w2_diag_fwd", _p(L), ldb, inc, _p(L_o), ldb_o, inc_o, float(eps_cov), int(scale_prec),
+                  _p(out), ldb_out, inc_out, _p(sc), Bc, n, _stream())
+    return out, sc, info
+
+
+@proj_cov_diag.register_fake
+def _(kind, L, L_o, eps_cov, scale_prec):
+    Bc, n = L.shape[0], L.shape[-1]
+    return L.new_empty(Bc, n, n), L.new_empty(Bc, 4, dtype=torch.float64), L.new_empty(Bc, dtype=torch.int32)
+
+
+@torch.library.custom_op("tce::proj_cov_diag_bwd", mutates_args=())
+def proj_cov_diag_bwd(grad_out: Tensor, kind: int, L: Tensor, L_o: Tensor, sc: Tensor, eps_cov: float,
+                      scale_prec: bool) -> Tensor:
+    ldb, inc, ldb_o, inc_o = _diag_pair(L, L_o)
+    ldb_g, inc_g = diag_strides(grad_out, "grad_out")
+    sc = _chk(sc, torch.float64, "save_sc")
+    g, ldb_gs, inc_gs = _dense_diag_grad(L)
+    Bc, n = L.shape[0], L.shape[-1]
+    if kind == 0:
+        _lib.call("tce_proj_frob_diag_bwd", _p(L), ldb, inc, _p(L_o), ldb_o, inc_o, float(eps_cov), _p(sc),
+                  _p(grad_out), ldb_g, inc_g, _p(g), ldb_gs, inc_gs, Bc, n, _stream())
+    else:
+        _lib.call("tce_proj_w2_diag_bwd", _p(L), ldb, inc, _p(L_o), ldb_o, inc_o, float(eps_cov), int(scale_prec),
+                  _p(sc), _p(grad_out), ldb_g, inc_g, _p(g), ldb_gs, inc_gs, Bc, n, _stream())
+    return g
+
+
+@proj_cov_diag_bwd.register_fake
+def _(grad_out, kind, L, L_o, sc, eps_cov, scale_prec):
+    return L.new_empty(L.shape[0], L.shape[-1], L.shape[-1])
+
+
+def _pcd_setup(ctx, inputs, output):
+    kind, L, L_o, eps_cov, scale_prec = inputs
+    ctx.save_for_backward(L, L_o, output[1])
+    ctx.kind, ctx.eps_cov, ctx.scale_prec = kind, eps_cov, scale_prec
+    ctx.set_materialize_grads(False)
+
+
+def _pcd_backward(ctx, g, g_sc, g_info):
+    if g is None:
+        return None, None, None, None, None
+    L, L_o, sc = ctx.saved_tensors
+    return None, proj_cov_diag_bwd(g, ctx.kind, L, L_o, sc, ctx.eps_cov, ctx.scale_prec), None, None, None
+
+
+proj_cov_diag.register_autograd(_pcd_backward, setup_context=_pcd_setup)
+
+
+def proj_frob_diag(L: Tensor, L_o: Tensor, eps_cov: float) -> Tuple[Tensor, Tensor, Tensor]:
+    """``proj_frob_cov`` of diagonal factors -> (out, save_sc, info)."""
+    return proj_cov_diag(0, L, L_o, eps_cov, False)
+
+
+def proj_w2_diag(L: Tensor, L_o: Tensor, eps_cov: float, scale_prec: bool) -> Tuple[Tensor, Tensor]:
+    """``proj_w2_cov`` of diagonal factors -> (out, save_sc)."""
+    return proj_cov_diag(1, L, L_o, eps_cov, scale_prec)[:2]
+
+
+@torch.library.custom_op("tce::cov_distance_diag", mutates_args=())
+def cov_distance_diag(kind: int, L: Tensor, L_o: Tensor, scale_prec: bool) -> Tensor:
+    """``cov_distance`` of diagonal factors -> [Bc] fp64, differentiable w.r.t. L."""
+    ldb, inc, ldb_o, inc_o = _diag_pair(L, L_o)
+    val = torch.empty(L.shape[0], device=L.device, dtype=torch.float64)
+    _lib.call("tce_cov_distance_diag", int(kind), _p(L), ldb, inc, _p(L_o), ldb_o, inc_o, int(scale_prec), None,
+              _p(val), None, 0, 0, L.shape[0], L.shape[-1], _stream())
+    return val
+
+
+@cov_distance_diag.register_fake
+def _(kind, L, L_o, scale_prec):
+    return L.new_empty(L.shape[0], dtype=torch.float64)
+
+
+@torch.library.custom_op("tce::cov_distance_diag_bwd", mutates_args=())
+def cov_distance_diag_bwd(grad_val: Tensor, kind: int, L: Tensor, L_o: Tensor, scale_prec: bool) -> Tensor:
+    ldb, inc, ldb_o, inc_o = _diag_pair(L, L_o)
+    g = _chk(grad_val, torch.float64, "grad_val")
+    out, ldb_out, inc_out = _dense_diag_grad(L)
+    _lib.call("tce_cov_distance_diag", int(kind), _p(L), ldb, inc, _p(L_o), ldb_o, inc_o, int(scale_prec), _p(g), None,
+              _p(out), ldb_out, inc_out, L.shape[0], L.shape[-1], _stream())
+    return out
+
+
+@cov_distance_diag_bwd.register_fake
+def _(grad_val, kind, L, L_o, scale_prec):
+    return L.new_empty(L.shape[0], L.shape[-1], L.shape[-1])
+
+
+def _cdd_setup(ctx, inputs, output):
+    kind, L, L_o, scale_prec = inputs
+    ctx.save_for_backward(L, L_o)
+    ctx.kind, ctx.scale_prec = kind, scale_prec
+
+
+def _cdd_backward(ctx, g):
+    L, L_o = ctx.saved_tensors
+    return None, cov_distance_diag_bwd(g.contiguous(), ctx.kind, L, L_o, ctx.scale_prec), None, None
+
+
+cov_distance_diag.register_autograd(_cdd_backward, setup_context=_cdd_setup)
 
 
 @torch.library.custom_op("tce::proj_frob_cov", mutates_args=())

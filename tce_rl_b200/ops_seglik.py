@@ -557,13 +557,18 @@ def seglik_diag_bwd(grad_logp: Tensor, smp_traj: Tensor, mean: Tensor, L: Tensor
     pairs = _chk(pred_pairs, torch.int64, "pred_pairs")
     ldb, inc = diag_strides(L)
     B, T = times.shape
-    g_mean = torch.empty(B, mean.shape[-1], device=mean.device, dtype=torch.float32)
+    n = mean.shape[-1]
+    g_mean = torch.empty(B, n, device=mean.device, dtype=torch.float32)
     g_L, ldb_g, inc_g = _dense_diag_grad(L)
     if B == 0:
         return g_mean, g_L
+    shared = L.shape[0] == 1 and B > 1            # one factor for the batch: per-episode gradients, then their sum
+    g_s = torch.empty(B, n, device=mean.device, dtype=torch.float32) if shared else g_L
     _lib.call("tce_seglik_diag_bwd", tables, _p(smp_traj), _p(mean), _p(L), ldb, inc, _p(times), _p(init_time),
-              _p(init_pos), _p(init_vel), _p(pairs), _p(diag_max), float(reg_rel), _p(grad_logp), _p(g_mean), _p(g_L),
-              ldb_g, inc_g, B, T, pairs.shape[0], _stream())
+              _p(init_pos), _p(init_vel), _p(pairs), _p(diag_max), float(reg_rel), _p(grad_logp), _p(g_mean), _p(g_s),
+              n if shared else ldb_g, 1 if shared else inc_g, B, T, pairs.shape[0], _stream())
+    if shared:
+        g_L.diagonal(dim1=-2, dim2=-1).copy_(g_s.sum(dim=0, keepdim=True))
     return g_mean, g_L
 
 

@@ -171,24 +171,33 @@ class TemporalCorrelatedPolicy(BlackBoxPolicy):
     def log_prob(self, smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel, **kwargs):
         """TCE segment-wise likelihood [B, P] (temporal_correlated_policy.py:104-203)."""
         pred_pairs = kwargs["pred_pairs"]
-        if self._per_episode_diag(params_L, times.shape[0]):
-            return ops.seg_logprob_diag(smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel,
+        diag_L = self._diag_factor(params_L, times.shape[0])
+        if diag_L is not None:
+            return ops.seg_logprob_diag(smp_traj, params_mean, diag_L, times, init_time, init_pos, init_vel,
                                         pred_pairs, self.mp.tables)
         return ops.seg_logprob(smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel, pred_pairs,
                                self.mp.tables)
 
-    def _per_episode_diag(self, params_L, batch):
-        """std_only with one factor per episode: the block-diagonal (2 x 2 per DoF) likelihood.  A factor shared by
-        the batch keeps the shared-covariance path, which forms the trajectory covariance once per batch."""
-        return self.is_diag and ops.shared_factor(params_L, batch) is None
+    def _diag_factor(self, params_L, batch):
+        """The factor to hand to the block-diagonal (2 x 2 per DoF) likelihood, or None for the dense likelihood.
+        std_only with one factor per episode: ``params_L``.  A std_only factor shared by the batch keeps the
+        shared-covariance path, which forms the trajectory covariance once per batch, at the shapes its kernels take
+        (Dp <= 64); at larger shapes the diagonal likelihood reads the ONE factor for every episode (stride 0)."""
+        if not self.is_diag:
+            return None
+        first = ops.shared_factor(params_L, batch)
+        if first is None:
+            return params_L
+        return None if self.mp.tables.dense_likelihood else first
 
     def segment_surrogate(self, smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel, pred_pairs,
                           log_prob_old, advantages):
         """Fused ``log_prob`` + ``surrogate_loss`` (temporal_correlated_agent.py:538-550,718-739): returns
         (-mean(exp(lp_new - lp_old) * adv), mean importance ratio, lp_new) from two kernels, backward = one.
-        Per-episode diagonal factors: the diagonal likelihood, then the surrogate formula of the agent on its log-probs."""
-        if self._per_episode_diag(params_L, times.shape[0]):
-            lp = ops.seg_logprob_diag(smp_traj, params_mean, params_L, times, init_time, init_pos, init_vel, pred_pairs,
+        Diagonal likelihood (``_diag_factor``): its log-probs, then the surrogate formula of the agent on them."""
+        diag_L = self._diag_factor(params_L, times.shape[0])
+        if diag_L is not None:
+            lp = ops.seg_logprob_diag(smp_traj, params_mean, diag_L, times, init_time, init_pos, init_vel, pred_pairs,
                                       self.mp.tables)
             ratio = (lp - log_prob_old).exp()
             return -(ratio * advantages).mean(), ratio.mean().detach(), lp.detach()

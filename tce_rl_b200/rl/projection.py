@@ -53,9 +53,11 @@ def _helper_stream(device):
 
 
 def _maha(policy, mean, mean_o, L_o, linv=None):
-    """|L_o^-1 (mean - mean_o)|^2 [B] fp64.  One shared covariance (non-contextual policy): invert the factor once
-    (``linv``: an inverse already formed in this epoch, see ``shared_inverse``) and use matrix-vector products
-    per episode instead of two triangular solves."""
+    """|L_o^-1 (mean - mean_o)|^2 [B] fp64.  Diagonal factors: elementwise.  One shared covariance (non-contextual
+    policy): invert the factor once (``linv``: an inverse already formed in this epoch, see ``shared_inverse``) and use
+    matrix-vector products per episode instead of two triangular solves."""
+    if policy.is_diag:
+        return ops.gauss_maha_diag(mean, mean_o, L_o)
     if not (_shared(policy, L_o) and L_o.is_cuda):
         return ops.gauss_maha(mean, mean_o, L_o)
     return ops.gauss_maha_shared(mean, mean_o, linv if linv is not None else shared_inverse(L_o))
@@ -66,13 +68,20 @@ def shared_inverse(L_o):
     return ops.tri_inverse(_first(L_o).detach().contiguous())[0]
 
 
+def _factor_stats(policy, L, L_o):
+    """gauss_stats of the covariance factors only (zero mean difference) [Bc, 5]."""
+    if policy.is_diag:
+        return ops.gauss_stats_diag(None, L, None, L_o)
+    zeros = torch.zeros(L.shape[0], L.shape[-1], device=L.device)
+    return ops.gauss_stats(zeros, L.contiguous(), zeros, L_o)
+
+
 def _cov_stats(policy, L, L_o):
     """gauss_stats on the covariance factors only (zero mean difference), broadcast when shared."""
     B = L.shape[0]
     if _shared(policy, L):
         L, L_o = _first(L), _first(L_o)
-    zeros = torch.zeros(L.shape[0], L.shape[-1], device=L.device)
-    st = ops.gauss_stats(zeros, L.contiguous(), zeros, L_o)
+    st = _factor_stats(policy, L, L_o)
     return st.expand(B, -1) if st.shape[0] != B else st
 
 
@@ -381,17 +390,17 @@ class BaseProjectionLayer:
         cur, helper = torch.cuda.current_stream(), _helper_stream(p[0].device)
         helper.wait_stream(cur)
         with torch.cuda.stream(helper):                                    # mean part beside the covariance part
-            linv = shared_inverse(target[1])
-            ready = torch.cuda.Event()
-            ready.record()
-            # the KL layer's backward needs the inverse of exactly this factor (its own output): hand it over
-            self._output_inverse = (linv, ready, _first(target[1]).data_ptr())
+            linv = None
+            if not policy.is_diag:
+                linv = shared_inverse(target[1])
+                ready = torch.cuda.Event()
+                ready.record()
+                # the KL layer's backward needs the inverse of exactly this factor (its own output): hand it over
+                self._output_inverse = (linv, ready, _first(target[1]).data_ptr())
             maha = _maha(policy, p[0], target[0], target[1], linv=linv)
             maha.record_stream(cur)
-        L1, Lt1 = _first(p[1]), _first(target[1])
         with_cov = self._with_cov(policy, set_variance)
-        zeros = torch.zeros(1, L1.shape[-1], device=L1.device)
-        st = ops.gauss_stats(zeros, L1.contiguous(), zeros, Lt1)          # [1, 5]
+        st = _factor_stats(policy, _first(p[1]), _first(target[1]))      # [1, 5]
         cur.wait_stream(helper)
         loss, mean_diff, cov_diff, shape, volume = _SharedKLLoss.apply(
             maha, st, float(self.trust_region_coeff), bool(with_cov), int(p[0].shape[-1]), p[0].dtype)
@@ -511,7 +520,7 @@ class KLProjectionLayer(BaseProjectionLayer):
         return loss
 
     def _mean_part(self, policy, p, q):
-        linv = shared_inverse(q[1]) if (_shared(policy, q[1]) and q[1].is_cuda) else None
+        linv = shared_inverse(q[1]) if (_shared(policy, q[1]) and q[1].is_cuda and not policy.is_diag) else None
         self._old_linv = linv                                   # reused by the logging branch of the same epoch
         return 0.5 * _maha(policy, p[0], q[0], q[1], linv=linv)
 
@@ -551,15 +560,17 @@ class KLProjectionLayer(BaseProjectionLayer):
 class FrobeniusProjectionLayer(BaseProjectionLayer):
     projects = True
 
-    def _mean_dist(self, p, q):
+    def _mean_dist(self, policy, p, q):
         if self.scale_prec:
-            return ops.gauss_maha(p[0], q[0], q[1])
+            return ops.gauss_maha_diag(p[0], q[0], q[1]) if policy.is_diag else ops.gauss_maha(p[0], q[0], q[1])
         return ((q[0] - p[0]) ** 2).sum(-1).to(torch.float64)
 
     def _mean_part(self, policy, p, q):
-        return self._mean_dist(p, q)
+        return self._mean_dist(policy, p, q)
 
     def _cov_projection(self, policy, L, L_old):
+        if policy.is_diag:
+            return ops.proj_frob_diag(L, L_old, self.cov_bound)[0]
         return ops.proj_frob_cov(L.contiguous(), L_old, self.cov_bound)[0]
 
     def _cov_dist(self, policy, kind, L, L_o, scale_prec):
@@ -567,27 +578,36 @@ class FrobeniusProjectionLayer(BaseProjectionLayer):
         B = L.shape[0]
         if _shared(policy, L):
             L, L_o = _first(L), _first(L_o)
-        val = ops.cov_distance(kind, L.contiguous(), L_o, scale_prec)
+        if policy.is_diag:
+            val = ops.cov_distance_diag(kind, L, L_o, scale_prec)
+        else:
+            val = ops.cov_distance(kind, L.contiguous(), L_o, scale_prec)
         return val.expand(B) if val.shape[0] != B else val
 
     def trust_region_value(self, policy, p, q):
-        return self._mean_dist(p, q), self._cov_dist(policy, 0, p[1], q[1], False)
+        return self._mean_dist(policy, p, q), self._cov_dist(policy, 0, p[1], q[1], False)
 
     def get_trust_region_loss(self, policy, p, proj_p, set_variance=None):
         target = (proj_p[0].detach(), proj_p[1].detach())
-        diff = self._mean_dist(p, target)
+        diff = self._mean_dist(policy, p, target)
         if self._with_cov(policy, set_variance):               # squared L difference instead of the Frobenius metric
             Lp, Lt = (_first(p[1]), _first(target[1])) if _shared(policy, p[1]) else (p[1], target[1])
-            diff = diff + (Lp - Lt).pow(2).sum([-1, -2]).to(torch.float64)
+            if policy.is_diag:                                 # (zero off the diagonal)
+                Lp, Lt = Lp.diagonal(dim1=-2, dim2=-1), Lt.diagonal(dim1=-2, dim2=-1)
+                diff = diff + (Lp - Lt).pow(2).sum(-1).to(torch.float64)
+            else:
+                diff = diff + (Lp - Lt).pow(2).sum([-1, -2]).to(torch.float64)
         return (diff.mean() * self.trust_region_coeff).to(p[0].dtype)
 
 
 class WassersteinProjectionLayer(FrobeniusProjectionLayer):
     def _cov_projection(self, policy, L, L_old):
+        if policy.is_diag:
+            return ops.proj_w2_diag(L, L_old, self.cov_bound, self.scale_prec)[0]
         return ops.proj_w2_cov(L.contiguous(), L_old, self.cov_bound, self.scale_prec)[0]
 
     def trust_region_value(self, policy, p, q):
-        return self._mean_dist(p, q), self._cov_dist(policy, 1, p[1], q[1], self.scale_prec)
+        return self._mean_dist(policy, p, q), self._cov_dist(policy, 1, p[1], q[1], self.scale_prec)
 
     def get_trust_region_loss(self, policy, p, proj_p, set_variance=None):
         return BaseProjectionLayer.get_trust_region_loss(self, policy, p, proj_p, set_variance)
