@@ -158,7 +158,8 @@ int tce_gauss_maha_shared(const float *mean, const float *mean_o, const double *
 /* ---- (4a) differentiable trust-region projections ------------------------------------------------------
  * Replace the trust_region_projections layers (BruceGeLi/trust-region-layers@TCE_ICLR24) created by
  * projection_factory (mprl/rl/projection/__init__.py:19-40) and called at
- * temporal_correlated_agent.py:530-533; KL covariance part replaces cpp_projection (ITPAL).  n <= 64.
+ * temporal_correlated_agent.py:530-533; KL covariance part replaces cpp_projection (ITPAL).  n <= 64
+ * (64 < n <= 128: the *_ws entry points below).
  *
  * mean projection (all layers): mean_part [B] fp64 is the layer's mean distance (1/2 maha for KL, maha or
  * squared Euclidean otherwise); proj = (mean + w mean_o) / (1 + w), w = sqrt(mean_part / eps) - 1 where
@@ -270,6 +271,65 @@ int tce_proj_w2_cov_bwd(const float *L, const float *L_o, int64_t ldb_Lo, double
  * otherwise grad_L [B,n,n] = grad_val[b] * d val / d L (used by get_trust_region_loss).                 */
 int tce_cov_distance(int kind, const float *L, const float *L_o, int64_t ldb_Lo, int scale_prec,
                      const double *grad_val, double *val, float *grad_L, int64_t B, int n, void *stream);
+
+/* ---- 64 < n <= 128: the same entry points with a caller-owned workspace --------------------------------------
+ * The entry points above (and tce_gauss_stats(_bwd), tce_tri_inverse) keep n <= 64 and return
+ * TCE_ERR_UNSUPPORTED_SHAPE above it.  Each has a *_ws twin with the same arguments and `work` inserted before
+ * `stream`: with work != NULL it also takes 64 < n <= 128, where the n x n fp64 buffers of a CTA live in a slice of
+ * `work` instead of shared memory; at n <= 64 it runs the shared-memory kernels and ignores `work`.
+ * tce_proj_work_bytes(B, n) is the size of `work` (0 where none is needed): min(B, number of SMs) slices of six padded
+ * fp64 matrices, so it does not grow with B (a batch runs as consecutive launches of at most that many CTAs).  `work` must stay
+ * untouched until the call's kernels have run (stream order); `save` and every other argument are as above.    */
+size_t tce_proj_work_bytes(int64_t B, int n);
+int tce_gauss_stats_ws(const float *mean, const float *L, int64_t ldb_L, const float *mean_o, const float *L_o,
+                       int64_t ldb_Lo, double *out, int64_t B, int n, double *work, void *stream);
+int tce_gauss_stats_bwd_ws(const float *mean, const float *L, int64_t ldb_L, const float *mean_o, const float *L_o,
+                           int64_t ldb_Lo, const double *grad_out, float *grad_mean, float *grad_L, int64_t B, int n,
+                           double *work, void *stream);
+int tce_tri_inverse_ws(const float *L, int64_t ldb, double *Linv, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_cov_fwd_ws(const float *L, const float *L_o, double eps_cov, float *proj_L, double *save,
+                           int32_t *info, int warm_start, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_cov_bwd_ws(const float *L, const float *proj_L, const float *grad_out, const double *save,
+                           float *grad_L, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_entropy_fwd_ws(const float *L, const float *L_o, double eps_cov, const double *beta,
+                               int64_t ldb_beta, int equality, float *proj_L, float *out_L, double *save,
+                               int32_t *info, int warm_start, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_entropy_bwd_ws(const float *L, const float *proj_L, const float *grad_out, const double *save,
+                               float *grad_L, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_entropy_bwd_inv_ws(const float *L, const float *proj_L, const float *grad_out, const double *save,
+                                   const double *out_inv, float *grad_L, int64_t B, int n, double *work,
+                                   void *stream);
+int tce_proj_kl_entropy_bwd_tr_ws(const float *L, const float *proj_L, const float *grad_out, const double *save,
+                                  double tr_coeff, float *grad_L, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_bwd_sigma_ws(const float *L, const double *grad_sigma, const double *save, int fused_entropy,
+                             double tr_coeff, float *grad_L, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_entropy_fwd_sigma_vec_ws(const float *vec, int64_t ldb_vec, float min_std, float *L_built,
+                                         const float *L_o, double eps_cov, const double *beta, int64_t ldb_beta,
+                                         int equality, float *proj_L, float *out_L, double *save, int32_t *info,
+                                         int warm_start, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_bwd_sigma_k_vec_ws(const float *L, const float *vec, int64_t ldb_vec, const double *grad_sigma,
+                                   const double *save, int fused_entropy, double tr_coeff, float *grad_vec, int64_t B,
+                                   int n, double *work, void *stream);
+int tce_proj_kl_bwd_prep_ws(double *save, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_bwd_sigma_k_ws(const float *L, const double *grad_sigma, const double *save, int fused_entropy,
+                               double tr_coeff, float *grad_L, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_entropy_fwd_sigma_ws(const float *L, const float *L_o, double eps_cov, const double *beta,
+                                     int64_t ldb_beta, int equality, float *proj_L, float *out_L, double *save,
+                                     int32_t *info, int warm_start, int64_t B, int n, double *work, void *stream);
+int tce_proj_kl_entropy_fwd_chol_ws(const double *save, float *proj_L, float *out_L, double *out_inv, int32_t *info,
+                                    int64_t B, int n, double *work, void *stream);
+int tce_proj_frob_cov_fwd_ws(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, float *proj_L,
+                             double *save_sc, int32_t *info, int64_t B, int n, double *work, void *stream);
+int tce_proj_frob_cov_bwd_ws(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, const float *proj_L,
+                             const float *grad_out, const double *save_sc, float *grad_L, int64_t B, int n,
+                             double *work, void *stream);
+int tce_proj_w2_cov_fwd_ws(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, int scale_prec,
+                           float *proj_L, double *save_sc, int64_t B, int n, double *work, void *stream);
+int tce_proj_w2_cov_bwd_ws(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, int scale_prec,
+                           const float *grad_out, float *grad_L, int64_t B, int n, double *work, void *stream);
+int tce_cov_distance_ws(int kind, const float *L, const float *L_o, int64_t ldb_Lo, int scale_prec,
+                        const double *grad_val, double *val, float *grad_L, int64_t B, int n, double *work,
+                        void *stream);
 
 /* ---- (4b) the same for DIAGONAL factors (std_only policies) ---------------------------------------------------
  * L = diag(s), L_o = diag(s_old), each a strided vector as for tce_proj_kl_diag_* (element i of episode b is

@@ -135,6 +135,18 @@ SIGNATURES = {
     "tce_debug_seglik_phase_cycles": (C.c_int, [_P]),
     "tce_bench_fma": (C.c_int, [_I32, _I32, _P, C.POINTER(C.c_double), _P]),
 }
+# The dense projection family at 64 < n <= 128: each entry point's *_ws twin takes the workspace (double *) before the
+# stream; tce_proj_work_bytes(B, n) sizes it.
+PROJ_WS = ("tce_gauss_stats", "tce_gauss_stats_bwd", "tce_tri_inverse", "tce_proj_kl_cov_fwd", "tce_proj_kl_cov_bwd",
+           "tce_proj_kl_entropy_fwd", "tce_proj_kl_entropy_bwd", "tce_proj_kl_entropy_bwd_inv",
+           "tce_proj_kl_entropy_bwd_tr", "tce_proj_kl_bwd_sigma", "tce_proj_kl_bwd_sigma_k", "tce_proj_kl_bwd_prep",
+           "tce_proj_kl_entropy_fwd_sigma", "tce_proj_kl_entropy_fwd_sigma_vec", "tce_proj_kl_bwd_sigma_k_vec",
+           "tce_proj_kl_entropy_fwd_chol", "tce_proj_frob_cov_fwd", "tce_proj_frob_cov_bwd", "tce_proj_w2_cov_fwd",
+           "tce_proj_w2_cov_bwd", "tce_cov_distance")
+for _name in PROJ_WS:
+    _res, _args = SIGNATURES[_name]
+    SIGNATURES[_name + "_ws"] = (_res, _args[:-1] + [_P, _args[-1]])
+SIGNATURES["tce_proj_work_bytes"] = (C.c_size_t, [_I64, _I32])
 
 _lib = None
 

@@ -33,6 +33,24 @@ constexpr int KL_SC = 16;     // scalars saved per matrix by the KL projection: 
 
 __device__ inline int pad_even(int n) { return (n + 1) & ~1; }
 
+// 64 < n <= 128 (the WS instantiations): one padded fp64 matrix is 132 KB at n = 128 and the kernels hold two to six,
+// so a CTA's n x n buffers live in its slice of a caller-owned global workspace (PJ_WS_MATS matrices; L2-resident)
+// while the small scratch -- inverted diagonal blocks, eigenvalues, reductions, Jacobi partials -- stays in shared
+// memory.  A batch runs as consecutive launches of at most #SMs CTAs (pj_ws_waves), each starting at matrix b0, so the
+// workspace is bounded by the number of SMs, not by B.  The la_* routines take the same code with wider register
+// arrays (la_tri_inverse<8>, la_chol<4>, la_jacobi_onesided<2>).  WS = false: the kernels as they run for n <= 64.
+constexpr int PJ_WS_MATS = 6;
+struct PjWs {
+  double *p;
+  long long slice, b0;
+};
+template <bool WS>
+__device__ __forceinline__ long long pj_b(const PjWs &ws) { return WS ? ws.b0 + blockIdx.x : blockIdx.x; }
+template <bool WS>
+__device__ __forceinline__ double *pj_mats(double *sd, const PjWs &ws) { return WS ? ws.p + blockIdx.x * ws.slice : sd; }
+__host__ __device__ constexpr int pj_dinv(bool ws) { return ws ? LA_DINV_DOUBLES_LARGE : LA_DINV_DOUBLES; }
+constexpr int PJ_TU_WS = 8;       // la_tri_inverse outputs per thread at n <= 128 (every WS kernel runs 512 threads)
+
 // Stream `count` contiguous global elements through `sink(e, value)` with FOUR loads in flight per thread: a
 // plain `for (e...) smem[f(e)] = src[e]` loop is not unrolled (runtime trip count, index arithmetic in the
 // body) and pays one full memory latency per iteration -- 4 to 16 dependent round trips per matrix.
@@ -89,6 +107,7 @@ __device__ inline double block_sum(double v, double *red) {   // red: >= 32 doub
 // grad_A (sym) of a Cholesky factor P with upstream G (lower): Sbar = sym(P^-T Phi(P^T G) P^-1)
 // P in bP, G in bG; result in bM (full symmetric); bP and bG are destroyed.  P^-1 by recursive doubling and
 // two GEMMs instead of two triangular solves with n right-hand sides.
+template <int TU = 4>
 __device__ inline void chol_backward(Mat bP, Mat bG, Mat bM, double *inv_diag, int n) {
   // M = Phi(P^T G)  (lower, halved diagonal, zero above)
   la_gemm(bM, bP.T(), bG, n, n, n, TRI_UPPER, TRI_LOWER, TRI_FULL, 1.0, 0.0);
@@ -97,7 +116,7 @@ __device__ inline void chol_backward(Mat bP, Mat bG, Mat bM, double *inv_diag, i
     if (j > i) bM(i, j) = 0.0; else if (i == j) bM(i, j) *= 0.5;
   }
   __syncthreads();
-  la_tri_inverse(bP, bG, inv_diag, n);                                              // bG = P^-1 (G is consumed)
+  la_tri_inverse<TU>(bP, bG, inv_diag, n);                                          // bG = P^-1 (G is consumed)
   la_gemm(bP, bM, bG, n, n, n, TRI_LOWER, TRI_LOWER, TRI_FULL, 1.0, 0.0);           // Phi P^-1 (P is consumed)
   la_gemm(bM, bG.T(), bP, n, n, n, TRI_UPPER, TRI_FULL, TRI_FULL, 1.0, 0.0);        // X = P^-T Phi P^-1
   for (int e = threadIdx.x; e < n * n; e += blockDim.x) {
@@ -119,16 +138,18 @@ __device__ inline void chol_backward(Mat bP, Mat bG, Mat bM, double *inv_diag, i
 // bwd: given gout[b][5] -> grad_mean[b] (n), grad_L[b] (n x n lower)
 //   d maha / d mean = 2 Sigma_o^-1 (mean - mean_o) ; d tr / d L = 2 Sigma_o^-1 L ; d logdet / d L_ii = 2 / L_ii ;
 //   d entropy / d L_ii = 1 / L_ii
+template <bool WS>
 __global__ void __launch_bounds__(PJ_THREADS)
 gauss_kl_kernel(const float *__restrict__ mean, const float *__restrict__ L, long long ldb_L,
                 const float *__restrict__ mean_o, const float *__restrict__ L_o, long long ldb_Lo,
                 double *__restrict__ out, const double *__restrict__ gout, float *__restrict__ grad_mean,
-                float *__restrict__ grad_L, int n, int mean_only) {
+                float *__restrict__ grad_L, int n, int mean_only, PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1;
-  Mat Lo{sd, LD, 1}, W{sd + m * LD, LD, 1};
-  double *inv_diag = sd + 2 * m * LD, *red = inv_diag + LA_DINV_DOUBLES;
-  const long long b = blockIdx.x;
+  double *mb = pj_mats<WS>(sd, ws);
+  Mat Lo{mb, LD, 1}, W{mb + m * LD, LD, 1};
+  double *inv_diag = WS ? sd : sd + 2 * m * LD, *red = inv_diag + pj_dinv(WS);
+  const long long b = pj_b<WS>(ws);
   load_lower_d(Lo, L_o + b * ldb_Lo, n, m);
   // W = [L | diff] : n x (n+1)
   for (int e = threadIdx.x; e < m * m; e += blockDim.x) {
@@ -352,15 +373,17 @@ maha_warp_kernel(const float *__restrict__ mean, const float *__restrict__ mean_
 // Shared-covariance variants (non-contextual policy: every episode has the same L_o).  L_o^-1 is formed once
 // (tri_inverse_kernel, fp64) and the two triangular solves per episode become dense matrix-vector products
 // without a dependent chain: one warp per episode, Linv staged once per CTA (row stride n | 1).
-__global__ void __launch_bounds__(256)
-tri_inverse_kernel(const float *__restrict__ L, long long ldb, double *__restrict__ Linv, int n) {
+template <bool WS>
+__global__ void __launch_bounds__(WS ? 512 : 256)
+tri_inverse_kernel(const float *__restrict__ L, long long ldb, double *__restrict__ Linv, int n, PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1, MS = m * LD;
-  Mat A{sd, LD, 1}, X{sd + MS, LD, 1};
-  double *dinv = sd + 2 * MS;
-  const long long b = blockIdx.x;
+  double *mb = pj_mats<WS>(sd, ws);
+  Mat A{mb, LD, 1}, X{mb + MS, LD, 1};
+  double *dinv = WS ? sd : sd + 2 * MS;
+  const long long b = pj_b<WS>(ws);
   load_lower_d(A, L + b * ldb, n, m);
-  la_tri_inverse(A, X, dinv, n);
+  la_tri_inverse<WS ? PJ_TU_WS : 4>(A, X, dinv, n);
   double *out = Linv + (size_t)b * n * n;
   for (int e = threadIdx.x; e < n * n; e += blockDim.x) {
     const int i = e / n, j = e - i * n;
@@ -752,6 +775,7 @@ __device__ __forceinline__ void store_full_rows(double *__restrict__ dst, Mat M,
     for (int j = lane; j < n; j += 32) dst[(size_t)i * n + j] = M(i, j);
 }
 
+template <bool WS>
 __global__ void __launch_bounds__(KL_THREADS)
 proj_kl_cov_fwd_kernel(const float *__restrict__ L, const float *__restrict__ L_o, double eps_cov,
                        float *__restrict__ proj_L, double *__restrict__ save_M, double *__restrict__ save_U,
@@ -760,19 +784,21 @@ proj_kl_cov_fwd_kernel(const float *__restrict__ L, const float *__restrict__ L_
                        const double *__restrict__ beta,
                        long long ldb_beta, int entropy_eq, float *__restrict__ out_L, int split,
                        const float *__restrict__ vec, long long ldb_vec, float min_std, float *__restrict__ L_built,
-                       int compact) {
+                       int compact, PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1, MS = m * LD;
+  double *mb = pj_mats<WS>(sd, ws);                                                   // (WS: never `compact`)
   // Four buffers: b0 = Lt throughout, b3 = Lo -> W -> U~.  `compact` (batches: two CTAs of 256 threads per SM instead of
   // one of 512, so that one matrix's Jacobi phase -- four busy warps -- runs beside another's GEMMs): THREE buffers;
   // Lo is staged where Lt^-1 goes next, W = Lt^-1 (basis) overwrites Lt, and the warps that idle during the Jacobi
   // iteration fetch Lt again into the buffer the start basis has left (bL: where Lt is once U~ exists).
-  Mat b0{sd, LD, 1}, b1{sd + MS, LD, 1}, b2{sd + 2 * MS, LD, 1}, b3{compact ? sd : sd + 3 * MS, LD, 1};
+  Mat b0{mb, LD, 1}, b1{mb + MS, LD, 1}, b2{mb + 2 * MS, LD, 1}, b3{compact ? mb : mb + 3 * MS, LD, 1};
   Mat bLo = compact ? b2 : b3, bL = compact ? b1 : b0, bS = compact ? b0 : b1;       // bS: Sigma of an identity step
-  double *dinv = sd + (compact ? 3 : 4) * MS, *lam = dinv + LA_DINV_DOUBLES, *nrm = lam + m,
-         *red = nrm + LA_JACOBI_SCRATCH;                                                               // red: >= 48
+  double *dinv = WS ? sd : sd + (compact ? 3 : 4) * MS, *lam = dinv + pj_dinv(WS), *nrm = lam + m,
+         *red = nrm + (WS ? LA_JACOBI_SCRATCH_LARGE : LA_JACOBI_SCRATCH);                              // red: >= 48
+  constexpr int JS = WS ? 2 : 1, JR = WS ? 8 : LA_JACOBI_ROWS;                      // Jacobi pair slots, rows per thread
   __shared__ int s_bad;
-  const long long b = blockIdx.x;
+  const long long b = pj_b<WS>(ws);
   const size_t off = (size_t)b * n * n;
   // `vec` != NULL: the policy head is fused in -- Lt is built from the covariance vector (softplus(v_i) + min_std on the
   // diagonal, strictly-lower entries row-major behind the first n: abstract_policy.py:166-187) and also written to
@@ -830,7 +856,7 @@ proj_kl_cov_fwd_kernel(const float *__restrict__ L, const float *__restrict__ L_
     __syncthreads();
   }
   KL_STAMP(1);
-  la_tri_inverse(b0, b2, dinv, n);                                                 // Lt^-1 (kept for the backward)
+  la_tri_inverse<WS ? PJ_TU_WS : 4>(b0, b2, dinv, n);                             // Lt^-1 (kept for the backward)
   KL_STAMP(10);
   zero_padding(b3, n, m);
   la_gemm(b3, b2, b1, n, n, n, TRI_LOWER, warm ? TRI_FULL : TRI_LOWER, TRI_FULL, 1.0, 0.0);   // W (or W Q_prev)
@@ -843,13 +869,13 @@ proj_kl_cov_fwd_kernel(const float *__restrict__ L, const float *__restrict__ L_
       bL(i, j) = (i < n && j <= i) ? (double)Lt[(size_t)i * n + j] : 0.0;
     }
   };
-  const int sweeps = la_jacobi_onesided(b3, lam, nrm, n, [&](int t, int nt) {
+  const int sweeps = la_jacobi_onesided<JS>(b3, lam, nrm, n, [&](int t, int nt) {
     if (nt >= 32) {
       store_full_rows(save_Li + off, b2, n, t, nt);
       if (compact) refetch_Lt(t, nt);
     }
   });                                                                               // b3 = U~
-  if ((int)blockDim.x - 32 * ((n + LA_JACOBI_ROWS - 1) / LA_JACOBI_ROWS) < 32) {    // (no idle warp: all of them do it now)
+  if ((int)blockDim.x - 32 * ((n + JR - 1) / JR) < 32) {                           // (no idle warp: all of them do it now)
     store_full_rows(save_Li + off, b2, n, threadIdx.x, blockDim.x);
     if (compact) refetch_Lt(threadIdx.x, blockDim.x);
     __syncthreads();
@@ -965,7 +991,7 @@ proj_kl_cov_fwd_kernel(const float *__restrict__ L, const float *__restrict__ L_
   }
   __syncthreads();                                                                  // ... before chol overwrites it
   KL_STAMP(7);
-  la_chol(b1, n, &s_bad);
+  la_chol<WS ? 4 : 2>(b1, n, &s_bad);
   KL_STAMP(8);
   const double alpha = tail_scalars([&](int i, double) { return log(b1(i, i)); }, true);
   store_lower_f(out, b1, n, 1.0);
@@ -975,15 +1001,17 @@ proj_kl_cov_fwd_kernel(const float *__restrict__ L, const float *__restrict__ L_
 }
 
 // Second half of a `split` forward: proj_L = chol(Sigma_proj) from the state, out_L = alpha * proj_L.
+template <bool WS>
 __global__ void __launch_bounds__(KL_THREADS)
 kl_chol_kernel(const double *__restrict__ save_Sig, const double *__restrict__ save_sc, float *__restrict__ proj_L,
-               float *__restrict__ out_L, double *__restrict__ out_inv, int32_t *__restrict__ info, int n) {
+               float *__restrict__ out_L, double *__restrict__ out_inv, int32_t *__restrict__ info, int n, PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1, MS = m * LD;
-  Mat b0{sd, LD, 1}, b1{sd + MS, LD, 1};
-  double *dinv = sd + 2 * MS;
+  double *mb = pj_mats<WS>(sd, ws);
+  Mat b0{mb, LD, 1}, b1{mb + MS, LD, 1};
+  double *dinv = WS ? sd : sd + 2 * MS;
   __shared__ int s_bad;
-  const long long b = blockIdx.x;
+  const long long b = pj_b<WS>(ws);
   const size_t off = (size_t)b * n * n;
   const double alpha = save_sc[b * KL_SC + 4];
   if (save_sc[b * KL_SC + 1] == 0.0) {                // inactive projection: the first half wrote the identity result
@@ -992,14 +1020,14 @@ kl_chol_kernel(const double *__restrict__ save_Sig, const double *__restrict__ s
   } else {
     if (threadIdx.x == 0) s_bad = 0;
     load_full_d(b0, save_Sig + off, n, m);
-    la_chol(b0, n, &s_bad);
+    la_chol<WS ? 4 : 2>(b0, n, &s_bad);
     store_lower_f(proj_L + off, b0, n, 1.0);
     if (out_L) store_lower_f(out_L + off, b0, n, alpha);
     if (info && threadIdx.x == 0) info[b] = s_bad;
   }
   if (out_inv) {                                      // (alpha P)^-1, fp64 lower: the trust-region loss's Mahalanobis term
     __syncthreads();
-    la_tri_inverse(b0, b1, dinv, n);
+    la_tri_inverse<WS ? PJ_TU_WS : 4>(b0, b1, dinv, n);
     const double ia = 1.0 / alpha;
     for (int e = threadIdx.x; e < n * n; e += blockDim.x) {
       const int i = e / n, j = e - i * n;
@@ -1016,17 +1044,19 @@ kl_chol_kernel(const double *__restrict__ save_Sig, const double *__restrict__ s
 //   etabar = sum_i Ft_ii (rho_i - (1+eta) rho_i^2) ;  grad_Lt = -2 tril(Lt^-T U~ Nt U~^T)
 // with U~ = Lt^-1 M and Lt^-1 saved by the forward.  No triangular solves: P^-1 by recursive doubling
 // (la_tri_inverse), everything else is fp64 tensor-core GEMMs (la_gemm) on four shared buffers.
+template <bool WS>
 __global__ void __launch_bounds__(KL_THREADS)
 proj_kl_cov_bwd_kernel(const float *__restrict__ L, const float *__restrict__ proj_L, const float *__restrict__ gout,
                        const double *__restrict__ save_M, const double *__restrict__ save_U,
                        const double *__restrict__ save_Li, const double *__restrict__ save_lam,
                        const double *__restrict__ save_sc, float *__restrict__ grad_L, int n, int fused_entropy,
-                       const double *__restrict__ out_inv, double tr_coeff, int compact) {
+                       const double *__restrict__ out_inv, double tr_coeff, int compact, PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1, MS = m * LD;
-  Mat b0{sd, LD, 1}, b1{sd + MS, LD, 1}, b2{sd + 2 * MS, LD, 1}, b3{sd + 3 * MS, LD, 1};     // b3: not with `compact`
-  double *dinv = sd + (compact ? 3 : 4) * MS, *lam = dinv + LA_DINV_DOUBLES, *rho = lam + m, *red = rho + m;
-  const long long b = blockIdx.x;
+  double *mb = pj_mats<WS>(sd, ws);
+  Mat b0{mb, LD, 1}, b1{mb + MS, LD, 1}, b2{mb + 2 * MS, LD, 1}, b3{mb + 3 * MS, LD, 1};     // b3: not with `compact`
+  double *dinv = WS ? sd : sd + (compact ? 3 : 4) * MS, *lam = dinv + pj_dinv(WS), *rho = lam + m, *red = rho + m;
+  const long long b = pj_b<WS>(ws);
   const size_t off = (size_t)b * n * n;
   float *gl = grad_L + off;
   (void)L;
@@ -1087,7 +1117,7 @@ proj_kl_cov_bwd_kernel(const float *__restrict__ L, const float *__restrict__ pr
   };
   if (compact) {
     __syncthreads();                                                               // Phi complete, G consumed
-    if (out_inv) load_out_inv(b1); else la_tri_inverse(b0, b1, dinv, n);           // P^-1 (over G)
+    if (out_inv) load_out_inv(b1); else la_tri_inverse<WS ? PJ_TU_WS : 4>(b0, b1, dinv, n);   // P^-1 (over G)
     la_gemm(b0, b2, b1, n, n, n, TRI_LOWER, TRI_LOWER, TRI_LOWER, 1.0, 0.0);       // Phi P^-1 (over P; lower x lower)
     for (int e = threadIdx.x; e < n * n; e += blockDim.x) {                        // (its strict upper triangle is zero)
       const int i = e / n, j = e - i * n;
@@ -1100,7 +1130,7 @@ proj_kl_cov_bwd_kernel(const float *__restrict__ L, const float *__restrict__ pr
     la_gemm(b2, b0.T(), b1, n, n, n, TRI_FULL, TRI_FULL, TRI_FULL, 1.0, 0.0);      // F' = M^T S' M ; Ft = sym(F')
   } else {
     load_full_d(b1, save_M + off, n, m);                                           // M (G is consumed)
-    if (out_inv) load_out_inv(b3); else la_tri_inverse(b0, b3, dinv, n);           // P^-1
+    if (out_inv) load_out_inv(b3); else la_tri_inverse<WS ? PJ_TU_WS : 4>(b0, b3, dinv, n);   // P^-1
     la_gemm(b0, b3, b1, n, n, n, TRI_LOWER, TRI_FULL, TRI_FULL, 1.0, 0.0);         // Y = P^-1 M (P is consumed)
     la_gemm(b3, b2, b0, n, n, n, TRI_LOWER, TRI_FULL, TRI_FULL, 1.0, 0.0);         // Phi Y
     la_gemm(b1, b0.T(), b3, n, n, n, TRI_FULL, TRI_FULL, TRI_FULL, 1.0, 0.0);      // F' = Y^T Phi Y ; Ft = sym(F')
@@ -1147,13 +1177,15 @@ proj_kl_cov_bwd_kernel(const float *__restrict__ L, const float *__restrict__ pr
 // K = Lt^-T U~ : the part of the covariance-space backward that does not depend on the incoming gradient.  Launched
 // right after the forward on the covariance stream it runs while the segment likelihood is busy and takes one GEMM and
 // one matrix load off the backward's critical path.
+template <bool WS>
 __global__ void __launch_bounds__(KL_THREADS)
 kl_bwd_prep_kernel(const double *__restrict__ save_U, const double *__restrict__ save_Li, const double *__restrict__ save_sc,
-                   double *__restrict__ save_K, int n) {
+                   double *__restrict__ save_K, int n, PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1, MS = m * LD;
-  Mat b0{sd, LD, 1}, b1{sd + MS, LD, 1}, b2{sd + 2 * MS, LD, 1};
-  const long long b = blockIdx.x;
+  double *mb = pj_mats<WS>(sd, ws);
+  Mat b0{mb, LD, 1}, b1{mb + MS, LD, 1}, b2{mb + 2 * MS, LD, 1};
+  const long long b = pj_b<WS>(ws);
   const size_t off = (size_t)b * n * n;
   if (save_sc[b * KL_SC + 1] == 0.0) return;                                        // identity step: K is not used
   {
@@ -1180,6 +1212,7 @@ kl_bwd_prep_kernel(const double *__restrict__ save_U, const double *__restrict__
   store_full_rows(save_K + off, b2, n, threadIdx.x, blockDim.x);
 }
 
+template <bool WS>
 __global__ void __launch_bounds__(KL_THREADS)
 proj_kl_cov_bwd_sigma_kernel(const float *__restrict__ L, const double *__restrict__ gsig,
                              const double *__restrict__ save_M, const double *__restrict__ save_U,
@@ -1187,13 +1220,14 @@ proj_kl_cov_bwd_sigma_kernel(const float *__restrict__ L, const double *__restri
                              const double *__restrict__ save_lam, const double *__restrict__ save_sc,
                              const double *__restrict__ save_K, float *__restrict__ grad_L, int n, int fused_entropy,
                              double tr_coeff, const float *__restrict__ vec, long long ldb_vec,
-                             float *__restrict__ grad_vec) {
+                             float *__restrict__ grad_vec, PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1, MS = m * LD;
-  Mat b0{sd, LD, 1}, b1{sd + MS, LD, 1}, b2{sd + 2 * MS, LD, 1}, b3{sd + 3 * MS, LD, 1}, b4{sd + 4 * MS, LD, 1},
-      b5{sd + 5 * MS, LD, 1};
-  double *dinv = sd + 6 * MS, *lam = dinv + LA_DINV_DOUBLES, *rho = lam + m, *red = rho + m;
-  const long long b = blockIdx.x;
+  double *mb = pj_mats<WS>(sd, ws);
+  Mat b0{mb, LD, 1}, b1{mb + MS, LD, 1}, b2{mb + 2 * MS, LD, 1}, b3{mb + 3 * MS, LD, 1}, b4{mb + 4 * MS, LD, 1},
+      b5{mb + 5 * MS, LD, 1};
+  double *dinv = WS ? sd : sd + 6 * MS, *lam = dinv + pj_dinv(WS), *rho = lam + m, *red = rho + m;
+  const long long b = pj_b<WS>(ws);
   const size_t off = (size_t)b * n * n;
   float *gl = grad_L ? grad_L + off : nullptr;
   // grad_vec != NULL: the adjoint of the policy head is fused in (head_bwd_kernel): the gradient is written w.r.t. the
@@ -1326,15 +1360,18 @@ proj_kl_cov_bwd_sigma_kernel(const float *__restrict__ L, const double *__restri
 // =====================================================================================================
 // Frobenius covariance projection
 // =====================================================================================================
+template <bool WS>
 __global__ void __launch_bounds__(PJ_THREADS)
 proj_frob_cov_fwd_kernel(const float *__restrict__ L, const float *__restrict__ L_o, long long ldb_Lo, double eps_cov,
-                         float *__restrict__ proj_L, double *__restrict__ save_sc, int32_t *__restrict__ info, int n) {
+                         float *__restrict__ proj_L, double *__restrict__ save_sc, int32_t *__restrict__ info, int n,
+                         PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1, MS = m * LD;
-  Mat b0{sd, LD, 1}, b1{sd + MS, LD, 1}, b2{sd + 2 * MS, LD, 1};
-  double *red = sd + 3 * MS;
+  double *mb = pj_mats<WS>(sd, ws);
+  Mat b0{mb, LD, 1}, b1{mb + MS, LD, 1}, b2{mb + 2 * MS, LD, 1};
+  double *red = WS ? sd : sd + 3 * MS;
   __shared__ int s_bad;
-  const long long b = blockIdx.x;
+  const long long b = pj_b<WS>(ws);
   const size_t off = (size_t)b * n * n;
   if (threadIdx.x == 0) s_bad = 0;
   load_lower_d(b0, L + off, n, m);
@@ -1356,20 +1393,22 @@ proj_frob_cov_fwd_kernel(const float *__restrict__ L, const float *__restrict__ 
   const double a = 1.0 / (1.0 + eta + 1e-16);
   for (int e = threadIdx.x; e < n * n; e += blockDim.x) b1(e / n, e % n) = (b1(e / n, e % n) + eta * b2(e / n, e % n)) * a;
   __syncthreads();
-  la_chol(b1, n, &s_bad);
+  la_chol<WS ? 4 : 2>(b1, n, &s_bad);
   store_lower_f(out, b1, n, 1.0);
   if (info && threadIdx.x == 0) info[b] = s_bad;
 }
 
+template <bool WS>
 __global__ void __launch_bounds__(PJ_THREADS)
 proj_frob_cov_bwd_kernel(const float *__restrict__ L, const float *__restrict__ L_o, long long ldb_Lo, double eps_cov,
                          const float *__restrict__ proj_L, const float *__restrict__ gout,
-                         const double *__restrict__ save_sc, float *__restrict__ grad_L, int n) {
+                         const double *__restrict__ save_sc, float *__restrict__ grad_L, int n, PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1, MS = m * LD;
-  Mat b0{sd, LD, 1}, b1{sd + MS, LD, 1}, b2{sd + 2 * MS, LD, 1}, b3{sd + 3 * MS, LD, 1};
-  double *inv_diag = sd + 4 * MS, *red = inv_diag + LA_DINV_DOUBLES;
-  const long long b = blockIdx.x;
+  double *mb = pj_mats<WS>(sd, ws);
+  Mat b0{mb, LD, 1}, b1{mb + MS, LD, 1}, b2{mb + 2 * MS, LD, 1}, b3{mb + 3 * MS, LD, 1};
+  double *inv_diag = WS ? sd : sd + 4 * MS, *red = inv_diag + pj_dinv(WS);
+  const long long b = pj_b<WS>(ws);
   const size_t off = (size_t)b * n * n;
   float *gl = grad_L + off;
   const double eta = save_sc[b * 4];
@@ -1379,7 +1418,7 @@ proj_frob_cov_bwd_kernel(const float *__restrict__ L, const float *__restrict__ 
   }
   load_lower_d(b0, proj_L + off, n, m);
   load_lower_d(b1, gout + off, n, m);
-  chol_backward(b0, b1, b2, inv_diag, n);                                          // b2 = Sbar_new (sym)
+  chol_backward<WS ? PJ_TU_WS : 4>(b0, b1, b2, inv_diag, n);                       // b2 = Sbar_new (sym)
   load_lower_d(b1, L + off, n, m);
   la_gemm(b3, b1, b1.T(), n, n, n, TRI_LOWER, TRI_UPPER, TRI_FULL, 1.0, 0.0);     // Sigma
   load_lower_d(b1, L_o + b * ldb_Lo, n, m);
@@ -1410,22 +1449,24 @@ proj_frob_cov_bwd_kernel(const float *__restrict__ L, const float *__restrict__ 
 // =====================================================================================================
 // cov_part: scale_prec ? tr(I + A Sigma A - 2 A R) : tr(Sigma_o + Sigma - 2 S R), A = S^-1, S = L_o, R = L
 // mode 0: forward (proj + scalars); mode 1: backward
+template <bool WS>
 __global__ void __launch_bounds__(PJ_THREADS)
 proj_w2_cov_kernel(const float *__restrict__ L, const float *__restrict__ L_o, long long ldb_Lo, double eps_cov,
                    int scale_prec, const float *__restrict__ gout, float *__restrict__ out, double *__restrict__ save_sc,
-                   int n) {
+                   int n, PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1, MS = m * LD;
-  Mat R{sd, LD, 1}, S{sd + MS, LD, 1}, A{sd + 2 * MS, LD, 1}, T{sd + 3 * MS, LD, 1}, U{sd + 4 * MS, LD, 1};
-  double *inv_diag = sd + 5 * MS, *red = inv_diag + LA_DINV_DOUBLES;
-  const long long b = blockIdx.x;
+  double *mb = pj_mats<WS>(sd, ws);
+  Mat R{mb, LD, 1}, S{mb + MS, LD, 1}, A{mb + 2 * MS, LD, 1}, T{mb + 3 * MS, LD, 1}, U{mb + 4 * MS, LD, 1};
+  double *inv_diag = WS ? sd : sd + 5 * MS, *red = inv_diag + pj_dinv(WS);
+  const long long b = pj_b<WS>(ws);
   const size_t off = (size_t)b * n * n;
   load_lower_d(R, L + off, n, m);
   load_lower_d(S, L_o + b * ldb_Lo, n, m);
   double cp;
   if (scale_prec) {
     zero_padding(A, n, m);
-    la_tri_inverse(S, A, inv_diag, n);                                             // A = S^-1 (lower)
+    la_tri_inverse<WS ? PJ_TU_WS : 4>(S, A, inv_diag, n);                         // A = S^-1 (lower)
     la_gemm(T, A, R, n, n, n, TRI_LOWER, TRI_LOWER, TRI_FULL, 1.0, 0.0);           // T = A R (lower)
     la_gemm(U, A.T(), R, n, n, n, TRI_UPPER, TRI_LOWER, TRI_FULL, 1.0, 0.0);       // U = A^T R
     double v = 0.0;
@@ -1492,15 +1533,17 @@ proj_w2_cov_kernel(const float *__restrict__ L, const float *__restrict__ L_o, l
 
 // gradient of the W2 / Frobenius covariance distances themselves (needed by the trust-region loss):
 // value only (gval == nullptr) or gradient w.r.t. L scaled by gval[b]
+template <bool WS>
 __global__ void __launch_bounds__(PJ_THREADS)
 cov_distance_kernel(int kind /*0 frob, 1 w2*/, const float *__restrict__ L, const float *__restrict__ L_o,
                     long long ldb_Lo, int scale_prec, const double *__restrict__ gval, double *__restrict__ val,
-                    float *__restrict__ grad_L, int n) {
+                    float *__restrict__ grad_L, int n, PjWs ws) {
   extern __shared__ double sd[];
   const int m = pad_even(n), LD = m + 1, MS = m * LD;
-  Mat R{sd, LD, 1}, S{sd + MS, LD, 1}, A{sd + 2 * MS, LD, 1}, T{sd + 3 * MS, LD, 1}, U{sd + 4 * MS, LD, 1};
-  double *inv_diag = sd + 5 * MS, *red = inv_diag + LA_DINV_DOUBLES;
-  const long long b = blockIdx.x;
+  double *mb = pj_mats<WS>(sd, ws);
+  Mat R{mb, LD, 1}, S{mb + MS, LD, 1}, A{mb + 2 * MS, LD, 1}, T{mb + 3 * MS, LD, 1}, U{mb + 4 * MS, LD, 1};
+  double *inv_diag = WS ? sd : sd + 5 * MS, *red = inv_diag + pj_dinv(WS);
+  const long long b = pj_b<WS>(ws);
   const size_t off = (size_t)b * n * n;
   load_lower_d(R, L + off, n, m);
   load_lower_d(S, L_o + b * ldb_Lo, n, m);
@@ -1521,7 +1564,7 @@ cov_distance_kernel(int kind /*0 frob, 1 w2*/, const float *__restrict__ L, cons
     }
   } else if (scale_prec) {
     zero_padding(A, n, m);
-    la_tri_inverse(S, A, inv_diag, n);
+    la_tri_inverse<WS ? PJ_TU_WS : 4>(S, A, inv_diag, n);
     la_gemm(T, A, R, n, n, n, TRI_LOWER, TRI_LOWER, TRI_FULL, 1.0, 0.0);
     la_gemm(U, A.T(), R, n, n, n, TRI_UPPER, TRI_LOWER, TRI_FULL, 1.0, 0.0);
     for (int e = threadIdx.x; e < n * n; e += blockDim.x) {
@@ -1589,37 +1632,86 @@ int set_smem(K kernel, size_t smem) {
   return TCE_OK;
 }
 
+size_t pj_ws_smem(int n) {             // the WS instantiations' shared memory: scratch only
+  const int m = (n + 1) & ~1;
+  return sizeof(double) * ((size_t)LA_DINV_DOUBLES_LARGE + LA_JACOBI_SCRATCH_LARGE + 8 * m + 256);
+}
+long long pj_ws_slice(int n) { const long long m = (n + 1) & ~1; return PJ_WS_MATS * m * (m + 1); }
+long long pj_ws_ctas(int64_t B) { return B < num_sms_proj() ? B : num_sms_proj(); }
+
+// The WS instantiation of a kernel over B matrices: launches of pj_ws_ctas(B) CTAs (as many as SMs; 512 threads of up to 128
+// registers), CTA i of every wave on slice i of `work`.  The launches of one stream run in order, so a wave reuses the
+// slices of the previous one.  launch(grid, ws) issues one launch.
+template <typename K, typename Launch>
+int pj_ws_waves(K kernel, int64_t B, int n, double *work, const char *where, void *stream, Launch launch) {
+  (void)stream;
+  int rc = set_smem(kernel, pj_smem_exclusive(pj_ws_smem(n), B));
+  if (rc) return rc;
+  const long long G = pj_ws_ctas(B);
+  for (long long b0 = 0; b0 < B; b0 += G) {
+    launch((unsigned)(B - b0 < G ? B - b0 : G), PjWs{work, pj_ws_slice(n), b0});
+    TCE_CHECK_LAUNCH(where);
+  }
+  return TCE_OK;
+}
+
 }  // namespace
 
-#define PJ_CHECK_N(n) if ((n) < 1 || (n) > 64) return TCE_ERR_UNSUPPORTED_SHAPE
+// n <= 64 on the shared-memory kernels; 64 < n <= 128 only with a workspace (the *_ws entry points)
+#define PJ_CHECK_N(n, work) if ((n) < 1 || (n) > ((work) ? 128 : 64)) return TCE_ERR_UNSUPPORTED_SHAPE
+#define PJ_WS(n, work) ((n) > 64 && (work))
+
+extern "C" size_t tce_proj_work_bytes(int64_t B, int n) {
+  if (B <= 0 || n <= 64 || n > 128) return 0;
+  return sizeof(double) * (size_t)pj_ws_ctas(B) * (size_t)pj_ws_slice(n);
+}
+
+static int gauss_stats_launch(const float *mean, const float *L, int64_t ldb_L, const float *mean_o, const float *L_o,
+                              int64_t ldb_Lo, double *out, const double *grad_out, float *grad_mean, float *grad_L,
+                              int64_t B, int n, double *work, void *stream) {
+  const int mean_only = grad_out ? (grad_L ? 0 : 1) : (L ? 0 : 1);
+  if (PJ_WS(n, work))
+    return pj_ws_waves(gauss_kl_kernel<true>, B, n, work, "gauss_kl_kernel<ws>", stream, [&](unsigned g, PjWs ws) {
+      gauss_kl_kernel<true><<<g, PJ_THREADS, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(
+          mean, L, ldb_L, mean_o, L_o, ldb_Lo, out, grad_out, grad_mean, grad_L, n, mean_only, ws);
+    });
+  const size_t smem = pj_smem(n, 2);      // NOT exclusive: these run beside the likelihood kernels (trust-region loss,
+  int rc = set_smem(gauss_kl_kernel<false>, smem);   // logging) and must fit into the first CTA slot that frees up
+  if (rc) return rc;
+  gauss_kl_kernel<false><<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(mean, L, ldb_L, mean_o, L_o, ldb_Lo, out,
+                                                                                 grad_out, grad_mean, grad_L, n, mean_only,
+                                                                                 PjWs{});
+  TCE_CHECK_LAUNCH(grad_out ? "gauss_kl_kernel(bwd)" : "gauss_kl_kernel");
+  return TCE_OK;
+}
+
+extern "C" int tce_gauss_stats_ws(const float *mean, const float *L, int64_t ldb_L, const float *mean_o,
+                                  const float *L_o, int64_t ldb_Lo, double *out, int64_t B, int n, double *work,
+                                  void *stream) {
+  if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
+  if (!mean || !mean_o || !L_o || !out || B < 0) return TCE_ERR_INVALID_ARGUMENT;
+  PJ_CHECK_N(n, work);
+  return gauss_stats_launch(mean, L, ldb_L, mean_o, L_o, ldb_Lo, out, nullptr, nullptr, nullptr, B, n, work, stream);
+}
 
 extern "C" int tce_gauss_stats(const float *mean, const float *L, int64_t ldb_L, const float *mean_o,
                                const float *L_o, int64_t ldb_Lo, double *out, int64_t B, int n, void *stream) {
+  return tce_gauss_stats_ws(mean, L, ldb_L, mean_o, L_o, ldb_Lo, out, B, n, nullptr, stream);
+}
+
+extern "C" int tce_gauss_stats_bwd_ws(const float *mean, const float *L, int64_t ldb_L, const float *mean_o,
+                                      const float *L_o, int64_t ldb_Lo, const double *grad_out, float *grad_mean,
+                                      float *grad_L, int64_t B, int n, double *work, void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
-  if (!mean || !mean_o || !L_o || !out || B < 0) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
-  const size_t smem = pj_smem(n, 2);      // NOT exclusive: these run beside the likelihood kernels (trust-region loss,
-  int rc = set_smem(gauss_kl_kernel, smem);   // logging) and must fit into the first CTA slot that frees up
-  if (rc) return rc;
-  gauss_kl_kernel<<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(mean, L, ldb_L, mean_o, L_o, ldb_Lo, out,
-                                                                          nullptr, nullptr, nullptr, n, L ? 0 : 1);
-  TCE_CHECK_LAUNCH("gauss_kl_kernel");
-  return TCE_OK;
+  if (!mean || !mean_o || !L_o || !grad_out || B < 0 || (grad_L && !L)) return TCE_ERR_INVALID_ARGUMENT;
+  PJ_CHECK_N(n, work);
+  return gauss_stats_launch(mean, L, ldb_L, mean_o, L_o, ldb_Lo, nullptr, grad_out, grad_mean, grad_L, B, n, work, stream);
 }
 
 extern "C" int tce_gauss_stats_bwd(const float *mean, const float *L, int64_t ldb_L, const float *mean_o,
                                    const float *L_o, int64_t ldb_Lo, const double *grad_out, float *grad_mean,
                                    float *grad_L, int64_t B, int n, void *stream) {
-  if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
-  if (!mean || !mean_o || !L_o || !grad_out || B < 0 || (grad_L && !L)) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
-  const size_t smem = pj_smem(n, 2);      // NOT exclusive: these run beside the likelihood kernels (trust-region loss,
-  int rc = set_smem(gauss_kl_kernel, smem);   // logging) and must fit into the first CTA slot that frees up
-  if (rc) return rc;
-  gauss_kl_kernel<<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(mean, L, ldb_L, mean_o, L_o, ldb_Lo, nullptr,
-                                                                          grad_out, grad_mean, grad_L, n, grad_L ? 0 : 1);
-  TCE_CHECK_LAUNCH("gauss_kl_kernel(bwd)");
-  return TCE_OK;
+  return tce_gauss_stats_bwd_ws(mean, L, ldb_L, mean_o, L_o, ldb_Lo, grad_out, grad_mean, grad_L, B, n, nullptr, stream);
 }
 
 static int maha_launch(const float *mean, const float *mean_o, const float *L_o, int64_t ldb_Lo, const double *grad_out,
@@ -1682,16 +1774,25 @@ extern "C" int tce_gauss_maha_bwd_full(const float *mean, const float *mean_o, c
   return maha_launch(mean, mean_o, L_o, ldb_Lo, grad_out, nullptr, grad_mean, grad_L, B, n, stream);
 }
 
-extern "C" int tce_tri_inverse(const float *L, int64_t ldb, double *Linv, int64_t B, int n, void *stream) {
+extern "C" int tce_tri_inverse_ws(const float *L, int64_t ldb, double *Linv, int64_t B, int n, double *work,
+                                  void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if (!L || !Linv || B < 0) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
+  PJ_CHECK_N(n, work);
+  if (PJ_WS(n, work))
+    return pj_ws_waves(tri_inverse_kernel<true>, B, n, work, "tri_inverse_kernel<ws>", stream, [&](unsigned g, PjWs ws) {
+      tri_inverse_kernel<true><<<g, 512, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(L, ldb, Linv, n, ws);
+    });
   const size_t smem = pj_smem(n, 2);
-  int rc = set_smem(tri_inverse_kernel, smem);
+  int rc = set_smem(tri_inverse_kernel<false>, smem);
   if (rc) return rc;
-  tri_inverse_kernel<<<(unsigned)B, 256, smem, (cudaStream_t)stream>>>(L, ldb, Linv, n);
+  tri_inverse_kernel<false><<<(unsigned)B, 256, smem, (cudaStream_t)stream>>>(L, ldb, Linv, n, PjWs{});
   TCE_CHECK_LAUNCH("tri_inverse_kernel");
   return TCE_OK;
+}
+
+extern "C" int tce_tri_inverse(const float *L, int64_t ldb, double *Linv, int64_t B, int n, void *stream) {
+  return tce_tri_inverse_ws(L, ldb, Linv, B, n, nullptr, stream);
 }
 
 extern "C" int tce_gauss_maha_shared(const float *mean, const float *mean_o, const double *Linv, const double *grad_out,
@@ -1801,235 +1902,381 @@ extern "C" size_t tce_proj_kl_save_doubles(int64_t B, int n) { return (size_t)B 
 
 static int kl_fwd_launch(const float *L, const float *L_o, double eps_cov, const double *beta, int64_t ldb_beta,
                          int equality, float *proj_L, float *out_L, double *save, int32_t *info, int warm_start,
-                         int64_t B, int n, void *stream, int split = 0, const float *vec = nullptr,
+                         int64_t B, int n, void *stream, double *work, int split = 0, const float *vec = nullptr,
                          int64_t ldb_vec = 0, float min_std = 0.f, float *L_built = nullptr) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if ((!L && !vec) || (vec && !L_built) || !L_o || !proj_L || !save || B < 0 || !(eps_cov > 0))
     return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
+  PJ_CHECK_N(n, work);
+  const size_t nn = (size_t)B * n * n;
+  double *M = save, *U = M + nn, *Li = U + nn, *Sig = Li + nn, *lam = Sig + nn, *sc = lam + (size_t)B * n;
+  if (PJ_WS(n, work))
+    return pj_ws_waves(proj_kl_cov_fwd_kernel<true>, B, n, work, "proj_kl_cov_fwd_kernel<ws>", stream, [&](unsigned g, PjWs ws) {
+      proj_kl_cov_fwd_kernel<true><<<g, KL_THREADS, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(
+          L, L_o, eps_cov, proj_L, M, U, Li, Sig, lam, sc, info, n, warm_start, beta, (long long)ldb_beta, equality, out_L,
+          split, vec, (long long)ldb_vec, min_std, L_built, 0, ws);
+    });
   // more matrices than SMs: two CTAs of 256 threads per SM on three buffers each (`compact`), else one of 512 on four
   const int compact = B > num_sms_proj();
   const size_t smem = pj_smem_exclusive(pj_smem(n, compact ? 3 : 4) + sizeof(double) * LA_JACOBI_SCRATCH, B);
-  int rc = set_smem(proj_kl_cov_fwd_kernel, compact ? pj_smem(n, 4) + sizeof(double) * LA_JACOBI_SCRATCH : smem);
+  int rc = set_smem(proj_kl_cov_fwd_kernel<false>, compact ? pj_smem(n, 4) + sizeof(double) * LA_JACOBI_SCRATCH : smem);
   if (rc) return rc;
-  const size_t nn = (size_t)B * n * n;
-  double *M = save, *U = M + nn, *Li = U + nn, *Sig = Li + nn, *lam = Sig + nn, *sc = lam + (size_t)B * n;
-  proj_kl_cov_fwd_kernel<<<(unsigned)B, compact ? KL_THREADS / 2 : KL_THREADS, smem, (cudaStream_t)stream>>>(
+  proj_kl_cov_fwd_kernel<false><<<(unsigned)B, compact ? KL_THREADS / 2 : KL_THREADS, smem, (cudaStream_t)stream>>>(
       L, L_o, eps_cov, proj_L, M, U, Li, Sig, lam, sc, info, n, warm_start, beta, (long long)ldb_beta, equality, out_L,
-      split, vec, (long long)ldb_vec, min_std, L_built, compact);
+      split, vec, (long long)ldb_vec, min_std, L_built, compact, PjWs{});
   TCE_CHECK_LAUNCH("proj_kl_cov_fwd_kernel");
   return TCE_OK;
 }
 
 static int kl_bwd_launch(const float *L, const float *proj_L, const float *grad_out, const double *save, float *grad_L,
-                         int64_t B, int n, int fused_entropy, void *stream, const double *out_inv = nullptr,
-                         double tr_coeff = 0.0) {
+                         int64_t B, int n, int fused_entropy, void *stream, double *work,
+                         const double *out_inv = nullptr, double tr_coeff = 0.0) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if (!L || !proj_L || !grad_out || !save || !grad_L || B < 0) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
-  const int compact = B > num_sms_proj();      // as kl_fwd_launch: two 256-thread CTAs per SM
-  const size_t smem = pj_smem_exclusive(pj_smem(n, compact ? 3 : 4), B);
-  int rc = set_smem(proj_kl_cov_bwd_kernel, compact ? pj_smem(n, 4) : smem);
-  if (rc) return rc;
+  PJ_CHECK_N(n, work);
   const size_t nn = (size_t)B * n * n;
   const double *M = save, *U = M + nn, *Li = U + nn, *lam = Li + 2 * nn, *sc = lam + (size_t)B * n;
-  proj_kl_cov_bwd_kernel<<<(unsigned)B, compact ? KL_THREADS / 2 : KL_THREADS, smem, (cudaStream_t)stream>>>(
-      L, proj_L, grad_out, M, U, Li, lam, sc, grad_L, n, fused_entropy, out_inv, tr_coeff, compact);
+  if (PJ_WS(n, work))
+    return pj_ws_waves(proj_kl_cov_bwd_kernel<true>, B, n, work, "proj_kl_cov_bwd_kernel<ws>", stream, [&](unsigned g, PjWs ws) {
+      proj_kl_cov_bwd_kernel<true><<<g, KL_THREADS, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(
+          L, proj_L, grad_out, M, U, Li, lam, sc, grad_L, n, fused_entropy, out_inv, tr_coeff, 0, ws);
+    });
+  const int compact = B > num_sms_proj();      // as kl_fwd_launch: two 256-thread CTAs per SM
+  const size_t smem = pj_smem_exclusive(pj_smem(n, compact ? 3 : 4), B);
+  int rc = set_smem(proj_kl_cov_bwd_kernel<false>, compact ? pj_smem(n, 4) : smem);
+  if (rc) return rc;
+  proj_kl_cov_bwd_kernel<false><<<(unsigned)B, compact ? KL_THREADS / 2 : KL_THREADS, smem, (cudaStream_t)stream>>>(
+      L, proj_L, grad_out, M, U, Li, lam, sc, grad_L, n, fused_entropy, out_inv, tr_coeff, compact, PjWs{});
   TCE_CHECK_LAUNCH("proj_kl_cov_bwd_kernel");
   return TCE_OK;
 }
 
+/* Every entry point below has a *_ws twin that takes `work` (tce_proj_work_bytes(B, n) bytes, 8-byte aligned) as its
+ * second-to-last argument: with it, 64 < n <= 128 runs on the workspace instantiations; n <= 64 ignores it. */
+extern "C" int tce_proj_kl_cov_fwd_ws(const float *L, const float *L_o, double eps_cov, float *proj_L, double *save,
+                                      int32_t *info, int warm_start, int64_t B, int n, double *work, void *stream) {
+  return kl_fwd_launch(L, L_o, eps_cov, nullptr, 0, 0, proj_L, nullptr, save, info, warm_start, B, n, stream, work);
+}
 extern "C" int tce_proj_kl_cov_fwd(const float *L, const float *L_o, double eps_cov, float *proj_L, double *save,
                                    int32_t *info, int warm_start, int64_t B, int n, void *stream) {
-  return kl_fwd_launch(L, L_o, eps_cov, nullptr, 0, 0, proj_L, nullptr, save, info, warm_start, B, n, stream);
+  return tce_proj_kl_cov_fwd_ws(L, L_o, eps_cov, proj_L, save, info, warm_start, B, n, nullptr, stream);
 }
 
+extern "C" int tce_proj_kl_cov_bwd_ws(const float *L, const float *proj_L, const float *grad_out, const double *save,
+                                      float *grad_L, int64_t B, int n, double *work, void *stream) {
+  return kl_bwd_launch(L, proj_L, grad_out, save, grad_L, B, n, 0, stream, work);
+}
 extern "C" int tce_proj_kl_cov_bwd(const float *L, const float *proj_L, const float *grad_out, const double *save,
                                    float *grad_L, int64_t B, int n, void *stream) {
-  return kl_bwd_launch(L, proj_L, grad_out, save, grad_L, B, n, 0, stream);
+  return tce_proj_kl_cov_bwd_ws(L, proj_L, grad_out, save, grad_L, B, n, nullptr, stream);
 }
 
+extern "C" int tce_proj_kl_entropy_fwd_ws(const float *L, const float *L_o, double eps_cov, const double *beta,
+                                          int64_t ldb_beta, int equality, float *proj_L, float *out_L, double *save,
+                                          int32_t *info, int warm_start, int64_t B, int n, double *work, void *stream) {
+  if (B != 0 && (!beta || !out_L)) return TCE_ERR_INVALID_ARGUMENT;
+  return kl_fwd_launch(L, L_o, eps_cov, beta, ldb_beta, equality, proj_L, out_L, save, info, warm_start, B, n, stream,
+                       work);
+}
 extern "C" int tce_proj_kl_entropy_fwd(const float *L, const float *L_o, double eps_cov, const double *beta,
                                        int64_t ldb_beta, int equality, float *proj_L, float *out_L, double *save,
                                        int32_t *info, int warm_start, int64_t B, int n, void *stream) {
-  if (B != 0 && (!beta || !out_L)) return TCE_ERR_INVALID_ARGUMENT;
-  return kl_fwd_launch(L, L_o, eps_cov, beta, ldb_beta, equality, proj_L, out_L, save, info, warm_start, B, n, stream);
+  return tce_proj_kl_entropy_fwd_ws(L, L_o, eps_cov, beta, ldb_beta, equality, proj_L, out_L, save, info, warm_start, B,
+                                    n, nullptr, stream);
 }
 
 /* The forward in two launches: _sigma writes the state (Sigma_proj, alpha, ...; for an inactive projection also the
  * outputs), _chol forms proj_L = chol(Sigma_proj) and out_L = alpha proj_L from it.  What only needs Sigma (stage 1
  * of the likelihood) can start after the first.                                                           */
+extern "C" int tce_proj_kl_entropy_fwd_sigma_ws(const float *L, const float *L_o, double eps_cov, const double *beta,
+                                                int64_t ldb_beta, int equality, float *proj_L, float *out_L,
+                                                double *save, int32_t *info, int warm_start, int64_t B, int n,
+                                                double *work, void *stream) {
+  if (B != 0 && !out_L) return TCE_ERR_INVALID_ARGUMENT;        /* beta == NULL: no entropy control (bound -inf) */
+  return kl_fwd_launch(L, L_o, eps_cov, beta, ldb_beta, equality, proj_L, out_L, save, info, warm_start, B, n, stream,
+                       work, 1);
+}
 extern "C" int tce_proj_kl_entropy_fwd_sigma(const float *L, const float *L_o, double eps_cov, const double *beta,
                                              int64_t ldb_beta, int equality, float *proj_L, float *out_L,
                                              double *save, int32_t *info, int warm_start, int64_t B, int n,
                                              void *stream) {
-  if (B != 0 && !out_L) return TCE_ERR_INVALID_ARGUMENT;        /* beta == NULL: no entropy control (bound -inf) */
-  return kl_fwd_launch(L, L_o, eps_cov, beta, ldb_beta, equality, proj_L, out_L, save, info, warm_start, B, n, stream,
-                       1);
+  return tce_proj_kl_entropy_fwd_sigma_ws(L, L_o, eps_cov, beta, ldb_beta, equality, proj_L, out_L, save, info,
+                                          warm_start, B, n, nullptr, stream);
 }
 
 /* tce_proj_kl_entropy_fwd_sigma with the policy head fused in: the unprojected factor is built from the covariance
  * vector(s) `vec` (batch stride ldb_vec, 0 = one shared vector) inside the kernel and also written to L_built [B,n,n]. */
+extern "C" int tce_proj_kl_entropy_fwd_sigma_vec_ws(const float *vec, int64_t ldb_vec, float min_std, float *L_built,
+                                                    const float *L_o, double eps_cov, const double *beta,
+                                                    int64_t ldb_beta, int equality, float *proj_L, float *out_L,
+                                                    double *save, int32_t *info, int warm_start, int64_t B, int n,
+                                                    double *work, void *stream) {
+  if (B != 0 && (!out_L || !vec)) return TCE_ERR_INVALID_ARGUMENT;
+  return kl_fwd_launch(nullptr, L_o, eps_cov, beta, ldb_beta, equality, proj_L, out_L, save, info, warm_start, B, n, stream,
+                       work, 1, vec, ldb_vec, min_std, L_built);
+}
 extern "C" int tce_proj_kl_entropy_fwd_sigma_vec(const float *vec, int64_t ldb_vec, float min_std, float *L_built,
                                                  const float *L_o, double eps_cov, const double *beta, int64_t ldb_beta,
                                                  int equality, float *proj_L, float *out_L, double *save, int32_t *info,
                                                  int warm_start, int64_t B, int n, void *stream) {
-  if (B != 0 && (!out_L || !vec)) return TCE_ERR_INVALID_ARGUMENT;
-  return kl_fwd_launch(nullptr, L_o, eps_cov, beta, ldb_beta, equality, proj_L, out_L, save, info, warm_start, B, n, stream,
-                       1, vec, ldb_vec, min_std, L_built);
+  return tce_proj_kl_entropy_fwd_sigma_vec_ws(vec, ldb_vec, min_std, L_built, L_o, eps_cov, beta, ldb_beta, equality,
+                                              proj_L, out_L, save, info, warm_start, B, n, nullptr, stream);
 }
 
-extern "C" int tce_proj_kl_entropy_fwd_chol(const double *save, float *proj_L, float *out_L, double *out_inv,
-                                            int32_t *info, int64_t B, int n, void *stream) {
+extern "C" int tce_proj_kl_entropy_fwd_chol_ws(const double *save, float *proj_L, float *out_L, double *out_inv,
+                                               int32_t *info, int64_t B, int n, double *work, void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if (!save || !proj_L || B < 0) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
-  const size_t smem = pj_smem_exclusive(pj_smem(n, 2), B);
-  int rc = set_smem(kl_chol_kernel, smem);
-  if (rc) return rc;
+  PJ_CHECK_N(n, work);
   const size_t nn = (size_t)B * n * n;
   const double *Sig = save + 3 * nn, *sc = save + 4 * nn + (size_t)B * n;
-  kl_chol_kernel<<<(unsigned)B, KL_THREADS, smem, (cudaStream_t)stream>>>(Sig, sc, proj_L, out_L, out_inv, info, n);
+  if (PJ_WS(n, work))
+    return pj_ws_waves(kl_chol_kernel<true>, B, n, work, "kl_chol_kernel<ws>", stream, [&](unsigned g, PjWs ws) {
+      kl_chol_kernel<true><<<g, KL_THREADS, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(
+          Sig, sc, proj_L, out_L, out_inv, info, n, ws);
+    });
+  const size_t smem = pj_smem_exclusive(pj_smem(n, 2), B);
+  int rc = set_smem(kl_chol_kernel<false>, smem);
+  if (rc) return rc;
+  kl_chol_kernel<false><<<(unsigned)B, KL_THREADS, smem, (cudaStream_t)stream>>>(Sig, sc, proj_L, out_L, out_inv, info, n,
+                                                                                PjWs{});
   TCE_CHECK_LAUNCH("kl_chol_kernel");
   return TCE_OK;
 }
+extern "C" int tce_proj_kl_entropy_fwd_chol(const double *save, float *proj_L, float *out_L, double *out_inv,
+                                            int32_t *info, int64_t B, int n, void *stream) {
+  return tce_proj_kl_entropy_fwd_chol_ws(save, proj_L, out_L, out_inv, info, B, n, nullptr, stream);
+}
 
+extern "C" int tce_proj_kl_entropy_bwd_ws(const float *L, const float *proj_L, const float *grad_out, const double *save,
+                                          float *grad_L, int64_t B, int n, double *work, void *stream) {
+  return kl_bwd_launch(L, proj_L, grad_out, save, grad_L, B, n, 1, stream, work);
+}
 extern "C" int tce_proj_kl_entropy_bwd(const float *L, const float *proj_L, const float *grad_out, const double *save,
                                        float *grad_L, int64_t B, int n, void *stream) {
-  return kl_bwd_launch(L, proj_L, grad_out, save, grad_L, B, n, 1, stream);
+  return tce_proj_kl_entropy_bwd_ws(L, proj_L, grad_out, save, grad_L, B, n, nullptr, stream);
 }
 
 /* tce_proj_kl_entropy_bwd + the gradient of tr_coeff * KL_cov(N(L L^T) || N(Sigma_out detached)) (trust-region loss). */
+extern "C" int tce_proj_kl_entropy_bwd_tr_ws(const float *L, const float *proj_L, const float *grad_out,
+                                             const double *save, double tr_coeff, float *grad_L, int64_t B, int n,
+                                             double *work, void *stream) {
+  return kl_bwd_launch(L, proj_L, grad_out, save, grad_L, B, n, 1, stream, work, nullptr, tr_coeff);
+}
 extern "C" int tce_proj_kl_entropy_bwd_tr(const float *L, const float *proj_L, const float *grad_out, const double *save,
                                           double tr_coeff, float *grad_L, int64_t B, int n, void *stream) {
-  return kl_bwd_launch(L, proj_L, grad_out, save, grad_L, B, n, 1, stream, nullptr, tr_coeff);
+  return tce_proj_kl_entropy_bwd_tr_ws(L, proj_L, grad_out, save, tr_coeff, grad_L, B, n, nullptr, stream);
 }
 
 /* Backward of tce_proj_kl_cov_fwd (fused_entropy = 0) / tce_proj_kl_entropy_fwd* (fused_entropy = 1) given the gradient
  * w.r.t. the OUTPUT COVARIANCE Sigma_out = alpha^2 Sigma_proj [B,n,n] (symmetric, fp64) instead of w.r.t. its factor.  */
 static int kl_bwd_sigma_launch(const float *L, const double *grad_sigma, const double *save, int fused_entropy,
-                               double tr_coeff, float *grad_L, int64_t B, int n, void *stream, int use_K,
+                               double tr_coeff, float *grad_L, int64_t B, int n, void *stream, double *work, int use_K,
                                const float *vec = nullptr, int64_t ldb_vec = 0, float *grad_vec = nullptr) {
   if (B == 0) return TCE_OK;
   if (!L || !grad_sigma || !save || (!grad_L && !grad_vec) || (grad_vec && !vec) || B < 0) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
-  const size_t smem = pj_smem_exclusive(pj_smem(n, 6), B);
-  int rc = set_smem(proj_kl_cov_bwd_sigma_kernel, smem);
-  if (rc) return rc;
+  PJ_CHECK_N(n, work);
   const size_t nn = (size_t)B * n * n;
   const double *M = save, *U = M + nn, *Li = U + nn, *Sig = Li + nn, *lam = Sig + nn, *sc = lam + (size_t)B * n;
   const double *K = use_K ? sc + (size_t)B * KL_SC : nullptr;
-  proj_kl_cov_bwd_sigma_kernel<<<(unsigned)B, KL_THREADS, smem, (cudaStream_t)stream>>>(L, grad_sigma, M, U, Li, Sig, lam,
-                                                                                       sc, K, grad_L, n, fused_entropy, tr_coeff,
-                                                                                       vec, (long long)ldb_vec, grad_vec);
+  if (PJ_WS(n, work))
+    return pj_ws_waves(proj_kl_cov_bwd_sigma_kernel<true>, B, n, work, "proj_kl_cov_bwd_sigma_kernel<ws>", stream,
+                       [&](unsigned g, PjWs ws) {
+      proj_kl_cov_bwd_sigma_kernel<true><<<g, KL_THREADS, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(
+          L, grad_sigma, M, U, Li, Sig, lam, sc, K, grad_L, n, fused_entropy, tr_coeff, vec, (long long)ldb_vec, grad_vec,
+          ws);
+    });
+  const size_t smem = pj_smem_exclusive(pj_smem(n, 6), B);
+  int rc = set_smem(proj_kl_cov_bwd_sigma_kernel<false>, smem);
+  if (rc) return rc;
+  proj_kl_cov_bwd_sigma_kernel<false><<<(unsigned)B, KL_THREADS, smem, (cudaStream_t)stream>>>(
+      L, grad_sigma, M, U, Li, Sig, lam, sc, K, grad_L, n, fused_entropy, tr_coeff, vec, (long long)ldb_vec, grad_vec,
+      PjWs{});
   TCE_CHECK_LAUNCH("proj_kl_cov_bwd_sigma_kernel");
   return TCE_OK;
 }
 
+extern "C" int tce_proj_kl_bwd_sigma_ws(const float *L, const double *grad_sigma, const double *save, int fused_entropy,
+                                        double tr_coeff, float *grad_L, int64_t B, int n, double *work, void *stream) {
+  return kl_bwd_sigma_launch(L, grad_sigma, save, fused_entropy, tr_coeff, grad_L, B, n, stream, work, 0);
+}
 extern "C" int tce_proj_kl_bwd_sigma(const float *L, const double *grad_sigma, const double *save, int fused_entropy,
                                      double tr_coeff, float *grad_L, int64_t B, int n, void *stream) {
-  return kl_bwd_sigma_launch(L, grad_sigma, save, fused_entropy, tr_coeff, grad_L, B, n, stream, 0);
+  return tce_proj_kl_bwd_sigma_ws(L, grad_sigma, save, fused_entropy, tr_coeff, grad_L, B, n, nullptr, stream);
 }
 
 /* K = Lt^-T U~ into the state (needs only the forward's outputs); then tce_proj_kl_bwd_sigma_k is tce_proj_kl_bwd_sigma
  * with one GEMM and one load less on its critical path.  The pair must see the state of the SAME forward.      */
-extern "C" int tce_proj_kl_bwd_prep(double *save, int64_t B, int n, void *stream) {
+extern "C" int tce_proj_kl_bwd_prep_ws(double *save, int64_t B, int n, double *work, void *stream) {
   if (B == 0) return TCE_OK;
   if (!save || B < 0) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
-  const size_t smem = pj_smem_exclusive(pj_smem(n, 3), B);
-  int rc = set_smem(kl_bwd_prep_kernel, smem);
-  if (rc) return rc;
+  PJ_CHECK_N(n, work);
   const size_t nn = (size_t)B * n * n;
   double *U = save + nn, *Li = U + nn, *sc = save + 4 * nn + (size_t)B * n, *K = sc + (size_t)B * KL_SC;
-  kl_bwd_prep_kernel<<<(unsigned)B, KL_THREADS, smem, (cudaStream_t)stream>>>(U, Li, sc, K, n);
+  if (PJ_WS(n, work))
+    return pj_ws_waves(kl_bwd_prep_kernel<true>, B, n, work, "kl_bwd_prep_kernel<ws>", stream, [&](unsigned g, PjWs ws) {
+      kl_bwd_prep_kernel<true><<<g, KL_THREADS, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(U, Li, sc, K,
+                                                                                                             n, ws);
+    });
+  const size_t smem = pj_smem_exclusive(pj_smem(n, 3), B);
+  int rc = set_smem(kl_bwd_prep_kernel<false>, smem);
+  if (rc) return rc;
+  kl_bwd_prep_kernel<false><<<(unsigned)B, KL_THREADS, smem, (cudaStream_t)stream>>>(U, Li, sc, K, n, PjWs{});
   TCE_CHECK_LAUNCH("kl_bwd_prep_kernel");
   return TCE_OK;
 }
+extern "C" int tce_proj_kl_bwd_prep(double *save, int64_t B, int n, void *stream) {
+  return tce_proj_kl_bwd_prep_ws(save, B, n, nullptr, stream);
+}
 
+extern "C" int tce_proj_kl_bwd_sigma_k_ws(const float *L, const double *grad_sigma, const double *save, int fused_entropy,
+                                          double tr_coeff, float *grad_L, int64_t B, int n, double *work, void *stream) {
+  return kl_bwd_sigma_launch(L, grad_sigma, save, fused_entropy, tr_coeff, grad_L, B, n, stream, work, 1);
+}
 extern "C" int tce_proj_kl_bwd_sigma_k(const float *L, const double *grad_sigma, const double *save, int fused_entropy,
                                        double tr_coeff, float *grad_L, int64_t B, int n, void *stream) {
-  return kl_bwd_sigma_launch(L, grad_sigma, save, fused_entropy, tr_coeff, grad_L, B, n, stream, 1);
+  return tce_proj_kl_bwd_sigma_k_ws(L, grad_sigma, save, fused_entropy, tr_coeff, grad_L, B, n, nullptr, stream);
 }
 
 /* ..._k with the adjoint of the policy head fused in: the result is the gradient w.r.t. the covariance vector(s)
  * [B, n + n(n-1)/2] (overwritten), L = the factor tce_proj_kl_entropy_fwd_sigma_vec built from `vec`.           */
+extern "C" int tce_proj_kl_bwd_sigma_k_vec_ws(const float *L, const float *vec, int64_t ldb_vec, const double *grad_sigma,
+                                              const double *save, int fused_entropy, double tr_coeff, float *grad_vec,
+                                              int64_t B, int n, double *work, void *stream) {
+  return kl_bwd_sigma_launch(L, grad_sigma, save, fused_entropy, tr_coeff, nullptr, B, n, stream, work, 1, vec, ldb_vec,
+                             grad_vec);
+}
 extern "C" int tce_proj_kl_bwd_sigma_k_vec(const float *L, const float *vec, int64_t ldb_vec, const double *grad_sigma,
                                            const double *save, int fused_entropy, double tr_coeff, float *grad_vec,
                                            int64_t B, int n, void *stream) {
-  return kl_bwd_sigma_launch(L, grad_sigma, save, fused_entropy, tr_coeff, nullptr, B, n, stream, 1, vec, ldb_vec, grad_vec);
+  return tce_proj_kl_bwd_sigma_k_vec_ws(L, vec, ldb_vec, grad_sigma, save, fused_entropy, tr_coeff, grad_vec, B, n,
+                                        nullptr, stream);
 }
 
+extern "C" int tce_proj_kl_entropy_bwd_inv_ws(const float *L, const float *proj_L, const float *grad_out,
+                                              const double *save, const double *out_inv, float *grad_L, int64_t B,
+                                              int n, double *work, void *stream) {
+  if (B != 0 && !out_inv) return TCE_ERR_INVALID_ARGUMENT;
+  return kl_bwd_launch(L, proj_L, grad_out, save, grad_L, B, n, 1, stream, work, out_inv);
+}
 extern "C" int tce_proj_kl_entropy_bwd_inv(const float *L, const float *proj_L, const float *grad_out,
                                            const double *save, const double *out_inv, float *grad_L, int64_t B, int n,
                                            void *stream) {
-  if (B != 0 && !out_inv) return TCE_ERR_INVALID_ARGUMENT;
-  return kl_bwd_launch(L, proj_L, grad_out, save, grad_L, B, n, 1, stream, out_inv);
+  return tce_proj_kl_entropy_bwd_inv_ws(L, proj_L, grad_out, save, out_inv, grad_L, B, n, nullptr, stream);
 }
 
-extern "C" int tce_proj_frob_cov_fwd(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, float *proj_L,
-                                     double *save_sc, int32_t *info, int64_t B, int n, void *stream) {
+extern "C" int tce_proj_frob_cov_fwd_ws(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, float *proj_L,
+                                        double *save_sc, int32_t *info, int64_t B, int n, double *work, void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if (!L || !L_o || !proj_L || !save_sc || B < 0 || !(eps_cov > 0)) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
+  PJ_CHECK_N(n, work);
+  if (PJ_WS(n, work))
+    return pj_ws_waves(proj_frob_cov_fwd_kernel<true>, B, n, work, "proj_frob_cov_fwd_kernel<ws>", stream,
+                       [&](unsigned g, PjWs ws) {
+      proj_frob_cov_fwd_kernel<true><<<g, PJ_THREADS, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(
+          L, L_o, ldb_Lo, eps_cov, proj_L, save_sc, info, n, ws);
+    });
   const size_t smem = pj_smem_exclusive(pj_smem(n, 3), B);
-  int rc = set_smem(proj_frob_cov_fwd_kernel, smem);
+  int rc = set_smem(proj_frob_cov_fwd_kernel<false>, smem);
   if (rc) return rc;
-  proj_frob_cov_fwd_kernel<<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(L, L_o, ldb_Lo, eps_cov, proj_L, save_sc, info, n);
+  proj_frob_cov_fwd_kernel<false><<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(L, L_o, ldb_Lo, eps_cov, proj_L,
+                                                                                          save_sc, info, n, PjWs{});
   TCE_CHECK_LAUNCH("proj_frob_cov_fwd_kernel");
   return TCE_OK;
 }
+extern "C" int tce_proj_frob_cov_fwd(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, float *proj_L,
+                                     double *save_sc, int32_t *info, int64_t B, int n, void *stream) {
+  return tce_proj_frob_cov_fwd_ws(L, L_o, ldb_Lo, eps_cov, proj_L, save_sc, info, B, n, nullptr, stream);
+}
 
-extern "C" int tce_proj_frob_cov_bwd(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov,
-                                     const float *proj_L, const float *grad_out, const double *save_sc, float *grad_L,
-                                     int64_t B, int n, void *stream) {
+extern "C" int tce_proj_frob_cov_bwd_ws(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov,
+                                        const float *proj_L, const float *grad_out, const double *save_sc,
+                                        float *grad_L, int64_t B, int n, double *work, void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if (!L || !L_o || !proj_L || !grad_out || !save_sc || !grad_L || B < 0) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
+  PJ_CHECK_N(n, work);
+  if (PJ_WS(n, work))
+    return pj_ws_waves(proj_frob_cov_bwd_kernel<true>, B, n, work, "proj_frob_cov_bwd_kernel<ws>", stream,
+                       [&](unsigned g, PjWs ws) {
+      proj_frob_cov_bwd_kernel<true><<<g, PJ_THREADS, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(
+          L, L_o, ldb_Lo, eps_cov, proj_L, grad_out, save_sc, grad_L, n, ws);
+    });
   const size_t smem = pj_smem_exclusive(pj_smem(n, 4), B);
-  int rc = set_smem(proj_frob_cov_bwd_kernel, smem);
+  int rc = set_smem(proj_frob_cov_bwd_kernel<false>, smem);
   if (rc) return rc;
-  proj_frob_cov_bwd_kernel<<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(L, L_o, ldb_Lo, eps_cov, proj_L, grad_out, save_sc, grad_L, n);
+  proj_frob_cov_bwd_kernel<false><<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(L, L_o, ldb_Lo, eps_cov, proj_L,
+                                                                                          grad_out, save_sc, grad_L, n,
+                                                                                          PjWs{});
   TCE_CHECK_LAUNCH("proj_frob_cov_bwd_kernel");
   return TCE_OK;
 }
+extern "C" int tce_proj_frob_cov_bwd(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov,
+                                     const float *proj_L, const float *grad_out, const double *save_sc, float *grad_L,
+                                     int64_t B, int n, void *stream) {
+  return tce_proj_frob_cov_bwd_ws(L, L_o, ldb_Lo, eps_cov, proj_L, grad_out, save_sc, grad_L, B, n, nullptr, stream);
+}
 
-extern "C" int tce_proj_w2_cov_fwd(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, int scale_prec,
-                                   float *proj_L, double *save_sc, int64_t B, int n, void *stream) {
+static int w2_launch(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, int scale_prec,
+                     const float *grad_out, float *out, double *save_sc, int64_t B, int n, double *work, void *stream) {
+  PJ_CHECK_N(n, work);
+  if (PJ_WS(n, work))
+    return pj_ws_waves(proj_w2_cov_kernel<true>, B, n, work, "proj_w2_cov_kernel<ws>", stream, [&](unsigned g, PjWs ws) {
+      proj_w2_cov_kernel<true><<<g, PJ_THREADS, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(
+          L, L_o, ldb_Lo, eps_cov, scale_prec, grad_out, out, save_sc, n, ws);
+    });
+  const size_t smem = pj_smem_exclusive(pj_smem(n, 5), B);
+  int rc = set_smem(proj_w2_cov_kernel<false>, smem);
+  if (rc) return rc;
+  proj_w2_cov_kernel<false><<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(L, L_o, ldb_Lo, eps_cov, scale_prec,
+                                                                                    grad_out, out, save_sc, n, PjWs{});
+  TCE_CHECK_LAUNCH(grad_out ? "proj_w2_cov_kernel(bwd)" : "proj_w2_cov_kernel");
+  return TCE_OK;
+}
+
+extern "C" int tce_proj_w2_cov_fwd_ws(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, int scale_prec,
+                                      float *proj_L, double *save_sc, int64_t B, int n, double *work, void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if (!L || !L_o || !proj_L || !save_sc || B < 0 || !(eps_cov > 0)) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
-  const size_t smem = pj_smem_exclusive(pj_smem(n, 5), B);
-  int rc = set_smem(proj_w2_cov_kernel, smem);
-  if (rc) return rc;
-  proj_w2_cov_kernel<<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(L, L_o, ldb_Lo, eps_cov, scale_prec, nullptr, proj_L, save_sc, n);
-  TCE_CHECK_LAUNCH("proj_w2_cov_kernel");
-  return TCE_OK;
+  return w2_launch(L, L_o, ldb_Lo, eps_cov, scale_prec, nullptr, proj_L, save_sc, B, n, work, stream);
+}
+extern "C" int tce_proj_w2_cov_fwd(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, int scale_prec,
+                                   float *proj_L, double *save_sc, int64_t B, int n, void *stream) {
+  return tce_proj_w2_cov_fwd_ws(L, L_o, ldb_Lo, eps_cov, scale_prec, proj_L, save_sc, B, n, nullptr, stream);
 }
 
-extern "C" int tce_proj_w2_cov_bwd(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, int scale_prec,
-                                   const float *grad_out, float *grad_L, int64_t B, int n, void *stream) {
+extern "C" int tce_proj_w2_cov_bwd_ws(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, int scale_prec,
+                                      const float *grad_out, float *grad_L, int64_t B, int n, double *work,
+                                      void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if (!L || !L_o || !grad_out || !grad_L || B < 0) return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
-  const size_t smem = pj_smem_exclusive(pj_smem(n, 5), B);
-  int rc = set_smem(proj_w2_cov_kernel, smem);
-  if (rc) return rc;
-  proj_w2_cov_kernel<<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(L, L_o, ldb_Lo, eps_cov, scale_prec, grad_out, grad_L, nullptr, n);
-  TCE_CHECK_LAUNCH("proj_w2_cov_kernel(bwd)");
-  return TCE_OK;
+  return w2_launch(L, L_o, ldb_Lo, eps_cov, scale_prec, grad_out, grad_L, nullptr, B, n, work, stream);
+}
+extern "C" int tce_proj_w2_cov_bwd(const float *L, const float *L_o, int64_t ldb_Lo, double eps_cov, int scale_prec,
+                                   const float *grad_out, float *grad_L, int64_t B, int n, void *stream) {
+  return tce_proj_w2_cov_bwd_ws(L, L_o, ldb_Lo, eps_cov, scale_prec, grad_out, grad_L, B, n, nullptr, stream);
 }
 
-extern "C" int tce_cov_distance(int kind, const float *L, const float *L_o, int64_t ldb_Lo, int scale_prec,
-                                const double *grad_val, double *val, float *grad_L, int64_t B, int n, void *stream) {
+extern "C" int tce_cov_distance_ws(int kind, const float *L, const float *L_o, int64_t ldb_Lo, int scale_prec,
+                                   const double *grad_val, double *val, float *grad_L, int64_t B, int n, double *work,
+                                   void *stream) {
   if (B == 0) return TCE_OK;              /* empty shard: pointers may be NULL */
   if (kind < 0 || kind > 1 || !L || !L_o || B < 0 || (grad_val && !grad_L) || (!grad_val && !val))
     return TCE_ERR_INVALID_ARGUMENT;
-  PJ_CHECK_N(n);
+  PJ_CHECK_N(n, work);
+  if (PJ_WS(n, work))
+    return pj_ws_waves(cov_distance_kernel<true>, B, n, work, "cov_distance_kernel<ws>", stream, [&](unsigned g, PjWs ws) {
+      cov_distance_kernel<true><<<g, PJ_THREADS, pj_smem_exclusive(pj_ws_smem(n), B), (cudaStream_t)stream>>>(
+          kind, L, L_o, ldb_Lo, scale_prec, grad_val, val, grad_L, n, ws);
+    });
   const size_t smem = pj_smem_exclusive(pj_smem(n, 5), B);
-  int rc = set_smem(cov_distance_kernel, smem);
+  int rc = set_smem(cov_distance_kernel<false>, smem);
   if (rc) return rc;
-  cov_distance_kernel<<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(kind, L, L_o, ldb_Lo, scale_prec, grad_val, val, grad_L, n);
+  cov_distance_kernel<false><<<(unsigned)B, PJ_THREADS, smem, (cudaStream_t)stream>>>(kind, L, L_o, ldb_Lo, scale_prec,
+                                                                                     grad_val, val, grad_L, n, PjWs{});
   TCE_CHECK_LAUNCH("cov_distance_kernel");
   return TCE_OK;
+}
+extern "C" int tce_cov_distance(int kind, const float *L, const float *L_o, int64_t ldb_Lo, int scale_prec,
+                                const double *grad_val, double *val, float *grad_L, int64_t B, int n, void *stream) {
+  return tce_cov_distance_ws(kind, L, L_o, ldb_Lo, scale_prec, grad_val, val, grad_L, B, n, nullptr, stream);
 }

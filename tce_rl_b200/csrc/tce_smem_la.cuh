@@ -1,5 +1,7 @@
-// Small dense linear algebra on shared-memory matrices (fp64), executed cooperatively by one CTA.
-// Building blocks of the trust-region projection kernels (n <= 64: Dp = 63 / 36 / 28 / 12).
+// Small dense linear algebra on fp64 matrices, executed cooperatively by one CTA.
+// Building blocks of the trust-region projection kernels: n <= 64 (Dp = 63 / 36 / 28 / 12) on shared-memory
+// matrices, and 64 < n <= 128 on matrices in a global workspace (a `Mat` is a generic pointer; the template
+// arguments that size register arrays and scratch for n <= 128 are noted at each routine).
 // Every routine is called by ALL threads of the CTA and ends with __syncthreads().
 #pragma once
 #include "tce_common.cuh"
@@ -92,6 +94,7 @@ __device__ inline void la_gemm(Mat C, Mat A, Mat B, int m, int n, int k, int a_t
 
 constexpr int LA_NB = 8;                              // block size of the blocked triangular routines
 constexpr int LA_DINV_DOUBLES = 8 * LA_NB * LA_NB;    // scratch for the inverted diagonal blocks (n <= 64)
+constexpr int LA_DINV_DOUBLES_LARGE = 16 * LA_NB * LA_NB;   // (n <= 128)
 
 // dinv[bk][i][j] = inverse of the bk-th LA_NB x LA_NB diagonal block of the lower-triangular L (zeros above
 // the diagonal).  One warp per block, lane j < 8 builds column j.
@@ -122,6 +125,8 @@ __device__ inline void la_diag_block_inverses(Mat L, double *dinv, int n) {
 }
 
 // X <- L^-1 for a lower-triangular L (n <= 64, X must not alias L; dinv: LA_DINV_DOUBLES doubles of scratch).
+// U: outputs per thread of one merge level; U = 4 covers n <= 64 with 256 threads, U = 8 covers n <= 128 with 512
+// (dinv: LA_DINV_DOUBLES_LARGE).
 // Recursive doubling instead of forward substitution: the 8x8 diagonal blocks are inverted directly, then
 // blocks of width w = 8, 16, 32 are merged pairwise,
 //   [A1 0; C A2]^-1 = [A1^-1 0; -A2^-1 C A1^-1  A2^-1],
@@ -129,6 +134,7 @@ __device__ inline void la_diag_block_inverses(Mat L, double *dinv, int n) {
 // (scripts/ubench/gemm.cu gives the cycles), where the blocked substitution needs 8 dependent block rows (~25k
 // cycles with n right-hand sides).  A solve with n right-hand sides is then ONE triangular GEMM.  For the factors met here (covariance factors,
 // condition ~1e2) the explicit inverse loses nothing measurable in fp64.  Needs blockDim.x >= 256.
+template <int U = 4>
 __device__ inline void la_tri_inverse(Mat L, Mat X, double *dinv, int n) {
   la_diag_block_inverses(L, dinv, n);
   for (int e = threadIdx.x; e < n * n; e += blockDim.x) {
@@ -138,10 +144,10 @@ __device__ inline void la_tri_inverse(Mat L, Mat X, double *dinv, int n) {
   __syncthreads();
   for (int lw = 3; (1 << lw) < n; ++lw) {
     const int w = 1 << lw, npair = (n + 2 * w - 1) >> (lw + 1), nout = npair << (2 * lw);
-    double v[4];
+    double v[U];
     // T = C A1^-1 into the (still zero) block below the diagonal: T(i, j) = sum_{k >= j} L(i, k) A1inv(k, j)
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int o = threadIdx.x + u * (int)blockDim.x;
       v[u] = 0.0;
       if (o < nout) {
@@ -158,7 +164,7 @@ __device__ inline void la_tri_inverse(Mat L, Mat X, double *dinv, int n) {
       }
     }
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int o = threadIdx.x + u * (int)blockDim.x;
       if (o < nout) {
         const int pr = o >> (2 * lw), rem = o & ((1 << (2 * lw)) - 1), ii = rem >> lw, jj = rem & (w - 1);
@@ -169,7 +175,7 @@ __device__ inline void la_tri_inverse(Mat L, Mat X, double *dinv, int n) {
     __syncthreads();
     // block <- -A2^-1 T (in place: every output is formed in a register before anything is overwritten)
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int o = threadIdx.x + u * (int)blockDim.x;
       v[u] = 0.0;
       if (o < nout) {
@@ -186,7 +192,7 @@ __device__ inline void la_tri_inverse(Mat L, Mat X, double *dinv, int n) {
     }
     __syncthreads();
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int o = threadIdx.x + u * (int)blockDim.x;
       if (o < nout) {
         const int pr = o >> (2 * lw), rem = o & ((1 << (2 * lw)) - 1), ii = rem >> lw, jj = rem & (w - 1);
@@ -292,19 +298,27 @@ __device__ inline void la_trsm_lower_t(Mat L, const double *dinv, Mat X, int n, 
   }
 }
 
-// in-place blocked Cholesky of the lower triangle of A (n <= 64; the upper triangle is scratch on exit); *bad
+// in-place blocked Cholesky of the lower triangle of A (n <= 32 S; the upper triangle is scratch on exit); *bad
 // (shared int, pre-set to 0) receives the 1-based index of the first non-positive pivot.  Per block of 8
 // columns: warp 0 factors the whole panel (rows r0..n-1) in REGISTERS -- lane l holds rows l and l + 32, pivots
 // and multipliers travel by shuffle, one rsqrt per column -- then everybody applies the rank-8 update to the
-// trailing matrix with la_gemm (k = 8).  Two barriers per 8 columns.
+// trailing matrix with la_gemm (k = 8).  Two barriers per 8 columns.  S = 4 (rows l + 32 s, s < 4): n <= 128.
+template <int S>
+__device__ __forceinline__ double la_chol_pick(const double (&p)[S][LA_NB], int j, int row) {   // p[row / 32][j]
+  static_assert(S == 2 || S == 4, "rows l + 32 s, s < 2 or s < 4");
+  if constexpr (S == 2) return row >= 32 ? p[1][j] : p[0][j];
+  else return row >= 64 ? (row >= 96 ? p[3][j] : p[2][j]) : (row >= 32 ? p[1][j] : p[0][j]);
+}
+
+template <int S = 2>
 __device__ inline void la_chol(Mat A, int n, int *bad) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int r0 = 0; r0 < n; r0 += LA_NB) {
     const int nb = min(LA_NB, n - r0);
     if (warp == 0) {
-      double p[2][LA_NB];
+      double p[S][LA_NB];
 #pragma unroll
-      for (int s = 0; s < 2; ++s)
+      for (int s = 0; s < S; ++s)
 #pragma unroll
         for (int c = 0; c < LA_NB; ++c) {
           const int row = lane + 32 * s;
@@ -314,7 +328,7 @@ __device__ inline void la_chol(Mat A, int n, int *bad) {
       for (int j = 0; j < LA_NB; ++j) {
         if (j < nb) {                                               // uniform
           const int col = r0 + j;
-          const double djj = __shfl_sync(0xffffffffu, col >= 32 ? p[1][j] : p[0][j], col & 31);
+          const double djj = __shfl_sync(0xffffffffu, la_chol_pick<S>(p, j, col), col & 31);
           if (lane == 0 && !(djj > 0.0) && *bad == 0) *bad = col + 1;
           // 1/sqrt: fp32 MUFU seed + two fp64 Newton steps (1e-7 -> 1e-14 -> rounding); the library rsqrt(double)
           // is a ~40-instruction subroutine on the critical path of every column
@@ -322,18 +336,18 @@ __device__ inline void la_chol(Mat A, int n, int *bad) {
           inv = inv * fma(-0.5 * djj, inv * inv, 1.5);
           inv = inv * fma(-0.5 * djj, inv * inv, 1.5);
 #pragma unroll
-          for (int s = 0; s < 2; ++s) p[s][j] = (lane + 32 * s == col) ? djj * inv : p[s][j] * inv;
+          for (int s = 0; s < S; ++s) p[s][j] = (lane + 32 * s == col) ? djj * inv : p[s][j] * inv;
 #pragma unroll
           for (int c = j + 1; c < LA_NB; ++c) {
             const int rc = r0 + c;                                  // L(rc, col) sits in lane rc % 32
-            const double lcj = __shfl_sync(0xffffffffu, rc >= 32 ? p[1][j] : p[0][j], rc & 31);
-            p[0][c] = fma(-p[0][j], lcj, p[0][c]);
-            p[1][c] = fma(-p[1][j], lcj, p[1][c]);
+            const double lcj = __shfl_sync(0xffffffffu, la_chol_pick<S>(p, j, rc), rc & 31);
+#pragma unroll
+            for (int s = 0; s < S; ++s) p[s][c] = fma(-p[s][j], lcj, p[s][c]);
           }
         }
       }
 #pragma unroll
-      for (int s = 0; s < 2; ++s)
+      for (int s = 0; s < S; ++s)
 #pragma unroll
         for (int c = 0; c < LA_NB; ++c) {
           const int row = lane + 32 * s;
@@ -403,44 +417,74 @@ constexpr float LA_JACOBI_TOL2 = 1e-7f;
 
 struct LaNoIdle { __device__ void operator()(int, int) const {} };
 
+// Two pair slots per lane (S = 2, n <= 128): 16 warps of 8 rows, lane t holds pair slots t and 32 + t.  Levels of
+// width <= 32 run on each slot as above; the first level (width 64) shifts Q around the ring of both slots (lane 31 of
+// one slot takes lane 0 of the other) and its trade of column sets is a swap of registers.  127 steps meet all 8128
+// pairs; partials are combined over 16 warps in a fixed order.  scratch: LA_JACOBI_SCRATCH_LARGE doubles.
+constexpr int LA_JACOBI_SCRATCH_LARGE = 2 * 2 * 16 * 32;
+
+__device__ __forceinline__ double la_combine16(const double *col) {
+  double v[8];
+#pragma unroll
+  for (int k = 0; k < 8; ++k) v[k] = col[64 * k] + col[64 * k + 32];
+  return ((v[0] + v[1]) + (v[2] + v[3])) + ((v[4] + v[5]) + (v[6] + v[7]));
+}
+
 // idle(t, nt): executed by the nt threads of the warps that hold no rows (t = 0..nt-1) while the others iterate;
 // it must not touch W, lam or scratch and must not synchronise.
-template <typename Idle = LaNoIdle>
+template <int S = 1, typename Idle = LaNoIdle>
 __device__ inline int la_jacobi_onesided(Mat W, double *lam, double *scratch, int n, Idle idle = Idle()) {
+  static_assert(S == 1 || S == 2, "one or two pair slots per lane");
+  constexpr int R = S == 1 ? LA_JACOBI_ROWS : 8;                     // rows per thread
+  constexpr int SLOT = 512, BUF = S == 1 ? 256 : 1024;                // scratch offsets: second slot, second buffer
+  constexpr int NSCR = S == 1 ? LA_JACOBI_SCRATCH : LA_JACOBI_SCRATCH_LARGE;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int nw = (n + LA_JACOBI_ROWS - 1) / LA_JACOBI_ROWS, nbar = nw * 32;   // warps that hold rows
-  int w0 = 1;                                          // pair slots: power of two >= ceil(n / 2), <= 32
+  const int nw = (n + R - 1) / R, nbar = nw * 32;                     // warps that hold rows
+  int w0 = 1;                                          // pair slots: power of two >= ceil(n / 2), <= 32 S
   while (2 * w0 < n) w0 <<= 1;
   int sweeps = 0;
-  for (int i = threadIdx.x; i < LA_JACOBI_SCRATCH; i += blockDim.x) scratch[i] = 0.0;   // warps >= nw add 0
+  for (int i = threadIdx.x; i < NSCR; i += blockDim.x) scratch[i] = 0.0;   // warps >= nw add 0
   __syncthreads();
   if (warp < nw) {
     double *mine = scratch + warp * 32 + lane;         // this thread's partial; its lane's column of partials
     const double *col = scratch + lane;
-    int idp = lane, idq = w0 + lane;                   // column ids (>= n or lane >= w0: zero padding)
-    if (lane >= w0) idp = idq = n;
-    double xp[LA_JACOBI_ROWS], xq[LA_JACOBI_ROWS];
+    auto combine = [](const double *c) { if constexpr (S == 1) return la_combine(c); else return la_combine16(c); };
+    int idp[S], idq[S];                                // column ids (>= n or slot >= w0: zero padding)
 #pragma unroll
-    for (int i = 0; i < LA_JACOBI_ROWS; ++i) {
-      const int r = warp * LA_JACOBI_ROWS + i;
-      xp[i] = (idp < n && r < n) ? W(r, idp) : 0.0;
-      xq[i] = (idq < n && r < n) ? W(r, idq) : 0.0;
+    for (int s = 0; s < S; ++s) {
+      const int t = 32 * s + lane;
+      idp[s] = t; idq[s] = w0 + t;
+      if (t >= w0) idp[s] = idq[s] = n;
     }
-    double ap, aq;
+    double xp[S][R], xq[S][R];
+#pragma unroll
+    for (int s = 0; s < S; ++s)
+#pragma unroll
+      for (int i = 0; i < R; ++i) {
+        const int r = warp * R + i;
+        xp[s][i] = (idp[s] < n && r < n) ? W(r, idp[s]) : 0.0;
+        xq[s][i] = (idq[s] < n && r < n) ? W(r, idq[s]) : 0.0;
+      }
+    double ap[S], aq[S];
     bool done = false;
     for (;;) {
       // exact squared norms (once per sweep: bounds the drift of the closed-form fp32 updates)
-      double sp = 0.0, sq = 0.0;
 #pragma unroll
-      for (int i = 0; i < LA_JACOBI_ROWS; ++i) { sp = fma(xp[i], xp[i], sp); sq = fma(xq[i], xq[i], sq); }
-      mine[0] = sp;
-      mine[256] = sq;
+      for (int s = 0; s < S; ++s) {
+        double sp = 0.0, sq = 0.0;
+#pragma unroll
+        for (int i = 0; i < R; ++i) { sp = fma(xp[s][i], xp[s][i], sp); sq = fma(xq[s][i], xq[s][i], sq); }
+        mine[SLOT * s] = sp;
+        mine[SLOT * s + BUF] = sq;
+      }
       la_named_barrier(nbar);
-      ap = la_combine(col);
-      aq = la_combine(col + 256);
+#pragma unroll
+      for (int s = 0; s < S; ++s) { ap[s] = combine(col + SLOT * s); aq[s] = combine(col + SLOT * s + BUF); }
       la_named_barrier(nbar);                          // the step buffers alias these partial sums
       if (done || sweeps == 40) break;
-      float a = (float)ap, b = (float)aq;
+      float a[S], b[S];
+#pragma unroll
+      for (int s = 0; s < S; ++s) { a[s] = (float)ap[s]; b[s] = (float)aq[s]; }
       int big = 0;      // some pair was still correlated above the tolerance when it was visited in this sweep
 #ifdef TCE_PROFILE
       float cmax2 = 0.f;
@@ -452,69 +496,117 @@ __device__ inline int la_jacobi_onesided(Mat W, double *lam, double *scratch, in
 #pragma unroll 1
       for (int w = w0; w >= 1; w >>= 1) {
 #pragma unroll 1
-        for (int k = 0; k < w; ++k, buf ^= 256) {
+        for (int k = 0; k < w; ++k, buf ^= BUF) {
           JP(4);
-          double g0 = 0.0, g1 = 0.0;
 #pragma unroll
-          for (int i = 0; i < LA_JACOBI_ROWS; i += 2) { g0 = fma(xp[i], xq[i], g0); g1 = fma(xp[i + 1], xq[i + 1], g1); }
-          mine[buf] = g0 + g1;
+          for (int s = 0; s < S; ++s) {
+            double g0 = 0.0, g1 = 0.0;
+#pragma unroll
+            for (int i = 0; i < R; i += 2) { g0 = fma(xp[s][i], xq[s][i], g0); g1 = fma(xp[s][i + 1], xq[s][i + 1], g1); }
+            mine[SLOT * s + buf] = g0 + g1;
+          }
           JP(0);
           la_named_barrier(nbar);
           JP(1);
-          const float g = (float)la_combine(col + buf);
+          double c[S], sn[S];
+          float nb[S];
+#pragma unroll
+          for (int s = 0; s < S; ++s) {
+            const float g = (float)combine(col + SLOT * s + buf);
 #ifdef JAC_PROF
-          if (g == 123.456f) jp[0]++;
+            if (g == 123.456f) jp[0]++;
 #endif
-          JP(2);
-          double c = 1.0, sn = 0.0;
-          float na = a, nb = b;
-          const float g2 = g * g, ab = a * b;
-          if (g2 > LA_JACOBI_TOL2 * ab) big = 1;
+            JP(2);
+            c[s] = 1.0; sn[s] = 0.0;
+            float na = a[s];
+            nb[s] = b[s];
+            const float g2 = g * g, ab = a[s] * b[s];
+            if (g2 > LA_JACOBI_TOL2 * ab) big = 1;
 #ifdef TCE_PROFILE
-          if (ab > 0.f) cmax2 = fmaxf(cmax2, g2 / ab);
+            if (ab > 0.f) cmax2 = fmaxf(cmax2, g2 / ab);
 #endif
-          if (g2 > 1e-24f * ab) {
-            // tan(theta) = 2g / (d + sgn(d) sqrt(d^2 + 4 g^2)), d = b - a: three MUFU ops, no IEEE fix-ups
-            const float d = b - a, s4 = fmaf(d, d, 4.0f * g2);
-            const float r = s4 * la_rsqrt_approx(s4);
-            const float tf = 2.0f * g * la_rcp_approx(d + copysignf(r, d));
-            const float c0 = la_rsqrt_approx(fmaf(tf, tf, 1.0f));
-            const double t = (double)tf, hh = fma(t, t, 1.0);
-            c = (double)c0;
-            c = c * fma(-0.5 * hh, c * c, 1.5);        // one Newton step: c^2 (1 + t^2) = 1 to ~1e-14
-            sn = c * t;
-            const float sf = c0 * tf, cs2 = 2.0f * c0 * sf * g;   // |c x - s y|^2, |s x + c y|^2 (fp32)
-            na = c0 * c0 * a + sf * sf * b - cs2;
-            nb = sf * sf * a + c0 * c0 * b + cs2;
-          }
-          a = na;
+            if (g2 > 1e-24f * ab) {
+              // tan(theta) = 2g / (d + sgn(d) sqrt(d^2 + 4 g^2)), d = b - a: three MUFU ops, no IEEE fix-ups
+              const float d = b[s] - a[s], s4 = fmaf(d, d, 4.0f * g2);
+              const float r = s4 * la_rsqrt_approx(s4);
+              const float tf = 2.0f * g * la_rcp_approx(d + copysignf(r, d));
+              const float c0 = la_rsqrt_approx(fmaf(tf, tf, 1.0f));
+              const double t = (double)tf, hh = fma(t, t, 1.0);
+              c[s] = (double)c0;
+              c[s] = c[s] * fma(-0.5 * hh, c[s] * c[s], 1.5);   // one Newton step: c^2 (1 + t^2) = 1 to ~1e-14
+              sn[s] = c[s] * t;
+              const float sf = c0 * tf, cs2 = 2.0f * c0 * sf * g;   // |c x - s y|^2, |s x + c y|^2 (fp32)
+              na = c0 * c0 * a[s] + sf * sf * b[s] - cs2;
+              nb[s] = sf * sf * a[s] + c0 * c0 * b[s] + cs2;
+            }
+            a[s] = na;
 #ifdef JAC_PROF
-          if (sn == 123.456) jp[0]++;
+            if (sn[s] == 123.456) jp[0]++;
 #endif
+          }
           JP(3);
           // rotate, then ring-shift Q inside the segment (not after the last step of a level: Q then stays
           // shifted by w - 1, which is as good a start for the next level; a shift by 0 keeps the code branch-free)
           const int src = lane + (k + 1 < w ? 1 : 0);
+          if (S == 1 || w <= 32) {
 #pragma unroll
-          for (int i = 0; i < LA_JACOBI_ROWS; ++i) {
-            const double np = fma(c, xp[i], -sn * xq[i]), nq = fma(sn, xp[i], c * xq[i]);
-            xp[i] = np;
-            xq[i] = __shfl_sync(0xffffffffu, nq, src, w);
+            for (int s = 0; s < S; ++s) {
+#pragma unroll
+              for (int i = 0; i < R; ++i) {
+                const double np = fma(c[s], xp[s][i], -sn[s] * xq[s][i]), nq = fma(sn[s], xp[s][i], c[s] * xq[s][i]);
+                xp[s][i] = np;
+                xq[s][i] = __shfl_sync(0xffffffffu, nq, src, w);
+              }
+              b[s] = __shfl_sync(0xffffffffu, nb[s], src, w);
+            }
+          } else {                                     // width 64: one ring over both slots
+            const bool cross = lane == 31 && k + 1 < w;
+#pragma unroll
+            for (int i = 0; i < R; ++i) {
+              double q[S];
+#pragma unroll
+              for (int s = 0; s < S; ++s) {
+                const double np = fma(c[s], xp[s][i], -sn[s] * xq[s][i]), nq = fma(sn[s], xp[s][i], c[s] * xq[s][i]);
+                xp[s][i] = np;
+                q[s] = __shfl_sync(0xffffffffu, nq, src);
+              }
+              xq[0][i] = cross ? q[S - 1] : q[0];
+              xq[S - 1][i] = cross ? q[0] : q[S - 1];
+            }
+            const float f0 = __shfl_sync(0xffffffffu, nb[0], src), f1 = __shfl_sync(0xffffffffu, nb[S - 1], src);
+            b[0] = cross ? f1 : f0;
+            b[S - 1] = cross ? f0 : f1;
           }
-          b = __shfl_sync(0xffffffffu, nb, src, w);
         }
-        idq = __shfl_sync(0xffffffffu, idq, lane + w - 1, w);
-        if (w > 1) {                                   // trade column sets between the halves of the segment
-          const int hw = w >> 1;
-          const bool upper = (lane & hw) != 0;
+        if (S == 1 || w <= 32) {
 #pragma unroll
-          for (int i = 0; i < LA_JACOBI_ROWS; ++i) {
-            const double got = __shfl_xor_sync(0xffffffffu, upper ? xp[i] : xq[i], hw);
-            if (upper) xp[i] = got; else xq[i] = got;
+          for (int s = 0; s < S; ++s) idq[s] = __shfl_sync(0xffffffffu, idq[s], lane + w - 1, w);
+        } else {                                       // position p takes p - 1 of the 64-ring
+          const int i0 = __shfl_sync(0xffffffffu, idq[0], lane + 31), i1 = __shfl_sync(0xffffffffu, idq[S - 1], lane + 31);
+          idq[0] = lane == 0 ? i1 : i0;
+          idq[S - 1] = lane == 0 ? i0 : i1;
+        }
+        if (w > 1) {                                   // trade column sets between the halves of the segment
+          if (S == 2 && w == 64) {                     // lower half = slot 0, upper half = slot 1
+#pragma unroll
+            for (int i = 0; i < R; ++i) { const double t = xq[0][i]; xq[0][i] = xp[S - 1][i]; xp[S - 1][i] = t; }
+            const float ft = b[0]; b[0] = a[S - 1]; a[S - 1] = ft;
+            const int it = idq[0]; idq[0] = idp[S - 1]; idp[S - 1] = it;
+          } else {
+            const int hw = w >> 1;
+            const bool upper = (lane & hw) != 0;
+#pragma unroll
+            for (int s = 0; s < S; ++s) {
+#pragma unroll
+              for (int i = 0; i < R; ++i) {
+                const double got = __shfl_xor_sync(0xffffffffu, upper ? xp[s][i] : xq[s][i], hw);
+                if (upper) xp[s][i] = got; else xq[s][i] = got;
+              }
+              const float fgot = __shfl_xor_sync(0xffffffffu, upper ? a[s] : b[s], hw);
+              const int igot = __shfl_xor_sync(0xffffffffu, upper ? idp[s] : idq[s], hw);
+              if (upper) { a[s] = fgot; idp[s] = igot; } else { b[s] = fgot; idq[s] = igot; }
+            }
           }
-          const float fgot = __shfl_xor_sync(0xffffffffu, upper ? a : b, hw);
-          const int igot = __shfl_xor_sync(0xffffffffu, upper ? idp : idq, hw);
-          if (upper) { a = fgot; idp = igot; } else { b = fgot; idq = igot; }
         }
       }
 #ifdef JAC_PROF
@@ -533,14 +625,19 @@ __device__ inline int la_jacobi_onesided(Mat W, double *lam, double *scratch, in
       done = !__any_sync(0xffffffffu, big);            // identical in every warp (same data, same code)
     }
 #pragma unroll
-    for (int i = 0; i < LA_JACOBI_ROWS; ++i) {
-      const int r = warp * LA_JACOBI_ROWS + i;
-      if (idp < n && r < n) W(r, idp) = xp[i];
-      if (idq < n && r < n) W(r, idq) = xq[i];
-    }
+    for (int s = 0; s < S; ++s)
+#pragma unroll
+      for (int i = 0; i < R; ++i) {
+        const int r = warp * R + i;
+        if (idp[s] < n && r < n) W(r, idp[s]) = xp[s][i];
+        if (idq[s] < n && r < n) W(r, idq[s]) = xq[s][i];
+      }
     if (warp == 0) {
-      if (idp < n) lam[idp] = ap;
-      if (idq < n) lam[idq] = aq;
+#pragma unroll
+      for (int s = 0; s < S; ++s) {
+        if (idp[s] < n) lam[idp[s]] = ap[s];
+        if (idq[s] < n) lam[idq[s]] = aq[s];
+      }
     }
   } else {
     idle((int)threadIdx.x - nbar, (int)blockDim.x - nbar);

@@ -24,6 +24,18 @@ def _stream() -> int:
     return torch.cuda.current_stream().cuda_stream
 
 
+def _pcall(name: str, *args) -> None:
+    """Call an entry point of the dense projection family, whose last two arguments are (B, n).  Above n = 64 its
+    *_ws twin runs, on a workspace from the caching allocator (stream-ordered: freed for reuse after the launch)."""
+    B, n = args[-2], args[-1]
+    if n <= 64:
+        _lib.call(name, *args, _stream())
+        return
+    nbytes = _lib.load().tce_proj_work_bytes(B, n)
+    work = torch.empty(max(nbytes // 8, 1), device=torch.cuda.current_device(), dtype=torch.float64)
+    _lib.call(name + "_ws", *args, _p(work), _stream())
+
+
 def _p(t: Optional[Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
@@ -363,7 +375,7 @@ def gauss_stats(mean: Tensor, L: Tensor, mean_o: Tensor, L_o: Tensor) -> Tensor:
     L_o, ldbo = _batched_matrix(L_o, "L_o")
     B, n = mean.shape
     out = torch.empty(B, 5, device=mean.device, dtype=torch.float64)
-    _lib.call("tce_gauss_stats", _p(mean), _p(L), ldb, _p(mean_o), _p(L_o), ldbo, _p(out), B, n, _stream())
+    _pcall("tce_gauss_stats", _p(mean), _p(L), ldb, _p(mean_o), _p(L_o), ldbo, _p(out), B, n)
     return out
 
 
@@ -756,7 +768,7 @@ def tri_inverse(L: Tensor) -> Tensor:
     L = _chk(L, name="L")
     Bc, n = L.shape[0], L.shape[-1]
     out = torch.empty(Bc, n, n, device=L.device, dtype=torch.float64)
-    _lib.call("tce_tri_inverse", _p(L), n * n, _p(out), Bc, n, _stream())
+    _pcall("tce_tri_inverse", _p(L), n * n, _p(out), Bc, n)
     return out
 
 
@@ -834,8 +846,8 @@ def gauss_stats_bwd(grad_out: Tensor, mean: Tensor, L: Tensor, mean_o: Tensor, L
     B, n = mean.shape
     g_mean = torch.empty_like(mean)
     g_L = torch.empty(B, n, n, device=mean.device, dtype=torch.float32) if need_L else mean.new_empty(0)
-    _lib.call("tce_gauss_stats_bwd", _p(mean), _p(Lc), ldb, _p(mean_o), _p(L_oc), ldbo, _p(g), _p(g_mean),
-              _p(g_L) if need_L else None, B, n, _stream())
+    _pcall("tce_gauss_stats_bwd", _p(mean), _p(Lc), ldb, _p(mean_o), _p(L_oc), ldbo, _p(g), _p(g_mean),
+              _p(g_L) if need_L else None, B, n)
     return g_mean, g_L
 
 
@@ -988,8 +1000,7 @@ def proj_kl_cov_fwd(L: Tensor, L_o: Tensor, eps_cov: float, state: Tensor, warm:
         raise TceError("state must come from ops.kl_state(batch, n, device)")
     out = torch.empty_like(L)
     info = torch.empty(Bc, device=L.device, dtype=torch.int32)
-    _lib.call("tce_proj_kl_cov_fwd", _p(L), _p(L_o), float(eps_cov), _p(out), _p(state), _p(info), int(warm), Bc, n,
-              _stream())
+    _pcall("tce_proj_kl_cov_fwd", _p(L), _p(L_o), float(eps_cov), _p(out), _p(state), _p(info), int(warm), Bc, n)
     return out, info
 
 
@@ -1002,7 +1013,7 @@ def _(L, L_o, eps_cov, state, warm):
 def proj_kl_cov_bwd(grad_out: Tensor, L: Tensor, proj_L: Tensor, state: Tensor) -> Tensor:
     g, L, proj_L = _chk(grad_out), _chk(L), _chk(proj_L)
     out = torch.empty_like(L)
-    _lib.call("tce_proj_kl_cov_bwd", _p(L), _p(proj_L), _p(g), _p(state), _p(out), L.shape[0], L.shape[-1], _stream())
+    _pcall("tce_proj_kl_cov_bwd", _p(L), _p(proj_L), _p(g), _p(state), _p(out), L.shape[0], L.shape[-1])
     return out
 
 
@@ -1059,17 +1070,16 @@ def proj_kl_entropy_fwd(L: Tensor, L_o: Tensor, eps_cov: float, state: Tensor, w
     out, proj = torch.empty_like(L), torch.empty_like(L)
     info = torch.empty(Bc, device=L.device, dtype=torch.int32)
     if split:
-        _lib.call("tce_proj_kl_entropy_fwd_sigma", _p(L), _p(L_o), float(eps_cov), _p(beta),
-                  0 if beta.numel() == 1 else 1, int(equality), _p(proj), _p(out), _p(state), _p(info), int(warm), Bc, n,
-                  _stream())
+        _pcall("tce_proj_kl_entropy_fwd_sigma", _p(L), _p(L_o), float(eps_cov), _p(beta),
+                  0 if beta.numel() == 1 else 1, int(equality), _p(proj), _p(out), _p(state), _p(info), int(warm), Bc, n)
         ev = torch.cuda.Event()
         ev.record()
         SIGMA_READY[id(state)] = ev
         out_inv = torch.empty(Bc, n, n, device=L.device, dtype=torch.float64)     # (out_L)^-1 for the trust-region loss
-        _lib.call("tce_proj_kl_entropy_fwd_chol", _p(state), _p(proj), _p(out), _p(out_inv), _p(info), Bc, n, _stream())
+        _pcall("tce_proj_kl_entropy_fwd_chol", _p(state), _p(proj), _p(out), _p(out_inv), _p(info), Bc, n)
         return out, proj, info, out_inv
-    _lib.call("tce_proj_kl_entropy_fwd", _p(L), _p(L_o), float(eps_cov), _p(beta), 0 if beta.numel() == 1 else 1,
-              int(equality), _p(proj), _p(out), _p(state), _p(info), int(warm), Bc, n, _stream())
+    _pcall("tce_proj_kl_entropy_fwd", _p(L), _p(L_o), float(eps_cov), _p(beta), 0 if beta.numel() == 1 else 1,
+              int(equality), _p(proj), _p(out), _p(state), _p(info), int(warm), Bc, n)
     return out, proj, info, L.new_empty(0, dtype=torch.float64)
 
 
@@ -1089,11 +1099,10 @@ def proj_kl_entropy_bwd(grad_out: Tensor, L: Tensor, proj_L: Tensor, state: Tens
         inv = _chk(out_inv, torch.float64, "out_inv")
         if inv.numel() != L.numel():
             raise TceError("out_inv must have the shape of L")
-        _lib.call("tce_proj_kl_entropy_bwd_inv", _p(L), _p(proj_L), _p(g), _p(state), _p(inv), _p(out), L.shape[0],
-                  L.shape[-1], _stream())
+        _pcall("tce_proj_kl_entropy_bwd_inv", _p(L), _p(proj_L), _p(g), _p(state), _p(inv), _p(out), L.shape[0],
+                  L.shape[-1])
     else:
-        _lib.call("tce_proj_kl_entropy_bwd", _p(L), _p(proj_L), _p(g), _p(state), _p(out), L.shape[0], L.shape[-1],
-                  _stream())
+        _pcall("tce_proj_kl_entropy_bwd", _p(L), _p(proj_L), _p(g), _p(state), _p(out), L.shape[0], L.shape[-1])
     return out
 
 
@@ -1107,8 +1116,8 @@ def proj_kl_entropy_bwd_tr(grad_out: Tensor, L: Tensor, proj_L: Tensor, state: T
     """``proj_kl_entropy_bwd`` + the gradient of tr_coeff * KL_cov(N(L L^T) || N(Sigma_out detached)) per matrix."""
     g, L, proj_L = _chk(grad_out), _chk(L), _chk(proj_L)
     out = torch.empty_like(L)
-    _lib.call("tce_proj_kl_entropy_bwd_tr", _p(L), _p(proj_L), _p(g), _p(state), float(tr_coeff), _p(out), L.shape[0],
-              L.shape[-1], _stream())
+    _pcall("tce_proj_kl_entropy_bwd_tr", _p(L), _p(proj_L), _p(g), _p(state), float(tr_coeff), _p(out), L.shape[0],
+              L.shape[-1])
     return out
 
 
@@ -1126,8 +1135,8 @@ def proj_kl_bwd_sigma(grad_sigma: Tensor, L: Tensor, state: Tensor, fused_entrop
     if g.numel() != L.numel():
         raise TceError("grad_sigma must have the shape of L")
     out = torch.empty_like(L)
-    _lib.call("tce_proj_kl_bwd_sigma", _p(L), _p(g), _p(state), int(fused_entropy), float(tr_coeff), _p(out),
-              L.shape[0], L.shape[-1], _stream())
+    _pcall("tce_proj_kl_bwd_sigma", _p(L), _p(g), _p(state), int(fused_entropy), float(tr_coeff), _p(out),
+              L.shape[0], L.shape[-1])
     return out
 
 
@@ -1518,7 +1527,7 @@ def proj_frob_cov(L: Tensor, L_o: Tensor, eps_cov: float) -> Tuple[Tensor, Tenso
     out = torch.empty_like(L)
     sc = torch.empty(Bc, 4, device=L.device, dtype=torch.float64)
     info = torch.empty(Bc, device=L.device, dtype=torch.int32)
-    _lib.call("tce_proj_frob_cov_fwd", _p(L), _p(L_o), ldbo, float(eps_cov), _p(out), _p(sc), _p(info), Bc, n, _stream())
+    _pcall("tce_proj_frob_cov_fwd", _p(L), _p(L_o), ldbo, float(eps_cov), _p(out), _p(sc), _p(info), Bc, n)
     return out, sc, info
 
 
@@ -1532,8 +1541,8 @@ def proj_frob_cov_bwd(grad_out: Tensor, L: Tensor, L_o: Tensor, proj_L: Tensor, 
     g, L, proj_L = _chk(grad_out), _chk(L), _chk(proj_L)
     L_o, ldbo = _batched_matrix(L_o, "L_o")
     out = torch.empty_like(L)
-    _lib.call("tce_proj_frob_cov_bwd", _p(L), _p(L_o), ldbo, float(eps_cov), _p(proj_L), _p(g), _p(sc), _p(out),
-              L.shape[0], L.shape[-1], _stream())
+    _pcall("tce_proj_frob_cov_bwd", _p(L), _p(L_o), ldbo, float(eps_cov), _p(proj_L), _p(g), _p(sc), _p(out),
+              L.shape[0], L.shape[-1])
     return out
 
 
@@ -1563,8 +1572,7 @@ def proj_w2_cov(L: Tensor, L_o: Tensor, eps_cov: float, scale_prec: bool) -> Tup
     Bc, n = L.shape[0], L.shape[-1]
     out = torch.empty_like(L)
     sc = torch.empty(Bc, 4, device=L.device, dtype=torch.float64)
-    _lib.call("tce_proj_w2_cov_fwd", _p(L), _p(L_o), ldbo, float(eps_cov), int(scale_prec), _p(out), _p(sc), Bc, n,
-              _stream())
+    _pcall("tce_proj_w2_cov_fwd", _p(L), _p(L_o), ldbo, float(eps_cov), int(scale_prec), _p(out), _p(sc), Bc, n)
     return out, sc
 
 
@@ -1578,8 +1586,8 @@ def proj_w2_cov_bwd(grad_out: Tensor, L: Tensor, L_o: Tensor, eps_cov: float, sc
     g, L = _chk(grad_out), _chk(L)
     L_o, ldbo = _batched_matrix(L_o, "L_o")
     out = torch.empty_like(L)
-    _lib.call("tce_proj_w2_cov_bwd", _p(L), _p(L_o), ldbo, float(eps_cov), int(scale_prec), _p(g), _p(out), L.shape[0],
-              L.shape[-1], _stream())
+    _pcall("tce_proj_w2_cov_bwd", _p(L), _p(L_o), ldbo, float(eps_cov), int(scale_prec), _p(g), _p(out), L.shape[0],
+              L.shape[-1])
     return out
 
 
@@ -1608,8 +1616,8 @@ def cov_distance(kind: int, L: Tensor, L_o: Tensor, scale_prec: bool) -> Tensor:
     L = _chk(L, name="L")
     L_o, ldbo = _batched_matrix(L_o, "L_o")
     val = torch.empty(L.shape[0], device=L.device, dtype=torch.float64)
-    _lib.call("tce_cov_distance", int(kind), _p(L), _p(L_o), ldbo, int(scale_prec), None, _p(val), None, L.shape[0],
-              L.shape[-1], _stream())
+    _pcall("tce_cov_distance", int(kind), _p(L), _p(L_o), ldbo, int(scale_prec), None, _p(val), None, L.shape[0],
+              L.shape[-1])
     return val
 
 
@@ -1624,8 +1632,8 @@ def cov_distance_bwd(grad_val: Tensor, kind: int, L: Tensor, L_o: Tensor, scale_
     g = _chk(grad_val, torch.float64)
     L_o, ldbo = _batched_matrix(L_o, "L_o")
     out = torch.empty_like(L)
-    _lib.call("tce_cov_distance", int(kind), _p(L), _p(L_o), ldbo, int(scale_prec), _p(g), None, _p(out), L.shape[0],
-              L.shape[-1], _stream())
+    _pcall("tce_cov_distance", int(kind), _p(L), _p(L_o), ldbo, int(scale_prec), _p(g), None, _p(out), L.shape[0],
+              L.shape[-1])
     return out
 
 

@@ -471,8 +471,7 @@ class KLProjectionLayer(BaseProjectionLayer):
         in the state: the covariance terms of the trust-region loss and of the logging decomposition are closed forms
         of it (``cache``: no gauss_stats launches), the trust-region covariance gradient is added inside the backward
         kernel (``get_trust_region_loss(fold=True)``)."""
-        if (not policy.contextual_std or not self.fuse_entropy or not p[1].is_cuda
-                or (p[1].shape[-1] > 64 and not policy.is_diag)):
+        if not policy.contextual_std or not self.fuse_entropy or not p[1].is_cuda:
             return None
         mean, L = p
         old_mean, old_L = q
