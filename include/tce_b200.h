@@ -58,6 +58,10 @@ typedef struct {
 
 typedef struct tce_tables tce_tables_t;
 
+/* Tables: 1 <= num_dof <= 16, 1 <= num_basis <= 15 and num_dof (num_basis + 1) <= 128, else TCE_ERR_UNSUPPORTED_SHAPE.
+ * The tables are built per basis function and do not depend on num_dof; the trajectory entry points take every shape
+ * the tables accept.                                                                                                  */
+
 int tce_prodmp_tables_create(const tce_mp_cfg *cfg, void *stream, tce_tables_t **out);
 void tce_prodmp_tables_destroy(tce_tables_t *tables);
 int tce_prodmp_tables_num_pc(const tce_tables_t *tables);
@@ -403,11 +407,18 @@ int tce_seglik_bwd(const tce_tables_t *tables, const void *work, const float *L,
                    const float *times, const float *init_time, const int64_t *pred_pairs,
                    const float *upstream, float *grad_mean, float *grad_L, int64_t B, int64_t T, int64_t P,
                    void *stream);
-/* Shapes.  The staged entry points above and below (and the diagonal likelihood) serve every supported shape:
- * 1 <= num_dof <= 8, 2 <= K1 <= 16, Dp = num_dof K1 <= 64.  The five (num_dof, K1) pairs (7, 9), (4, 9), (7, 4), (3, 4)
+/* Shapes.  The staged entry points above and below serve every supported shape of the dense likelihood:
+ * 1 <= num_dof <= 16, 2 <= K1 <= 16, Dp = num_dof K1 <= 64.  The five (num_dof, K1) pairs (7, 9), (4, 9), (7, 4), (3, 4)
  * and (2, 3) have kernels specialised on num_dof and are the only shapes of the fused and uniform-grid entry points
  * (tce_seglik_fused_config ... tce_seglik_uniform_finish); other shapes run the staged kernels with num_dof read from
- * the tables.  Anything else returns TCE_ERR_UNSUPPORTED_SHAPE.
+ * the tables.  tce_seglik_chol factors a segment with one thread for num_dof <= 8 and with one warp (lane r owns row r)
+ * for num_dof = 9..16.  Anything else returns TCE_ERR_UNSUPPORTED_SHAPE.
+ * Segment counts: P is bounded by the shared memory of the gram and backward kernels (200 KB per CTA, both grow by
+ * (2 K1 + 4) doubles per segment); a P past it returns TCE_ERR_UNSUPPORTED_SHAPE before any launch.  Up to
+ * num_dof = 8 the backward also stages the adjoints as fp32 [tri(2 num_dof)][P] in shared memory and refuses a P whose
+ * staging does not fit, as before; above 8 it reads them in fp64 from the workspace where they do not fit, so every
+ * num_dof > 8 shape takes P <= 957 on every covariance layout ((16, 4): P <= 1612 with per-episode factors, 1433 with
+ * a shared covariance; (9, 7): 1074 and 957).
  * tce_seglik_compiled: 1 = one of the five specialised shapes, 0 = supported by the staged path only,
  * TCE_ERR_UNSUPPORTED_SHAPE = outside the supported set.  Host only, no launch.                                      */
 int tce_seglik_compiled(const tce_tables_t *tables);
@@ -436,7 +447,7 @@ int tce_seglik_bwd_shared(const tce_tables_t *tables, const void *work, const fl
  * zero it first; all-reduce(MAX) it between the launches at > 1 GPU).  tce_seglik_diag_fwd: logp [B, P], info [B, P]
  * (optional; first non-positive pivot as in tce_seglik_chol).  tce_seglik_diag_bwd: from grad_logp [B, P],
  * grad_mean [B, Dp] and grad_s (strided, ldb_gs > 0), either may be NULL.  fp64 arithmetic, fixed summation order.
- * Every shape the tables accept (1 <= D <= 8, 2 <= K1 <= 16, Dp up to 128), not only the Dp <= 64 of the dense path. */
+ * Every shape the tables accept (1 <= D <= 16, 2 <= K1 <= 16, Dp <= 128), not only the Dp <= 64 of the dense path. */
 int tce_seglik_diag_max(const tce_tables_t *tables, const float *s, int64_t ldb_s, int64_t inc_s,
                         const float *times, const float *init_time, const int64_t *pred_pairs, double *diag_max,
                         int64_t B, int64_t T, int64_t P, void *stream);

@@ -7,8 +7,9 @@
 #include "../../include/tce_b200.h"
 
 #define TCE_MAX_K1 16   // max parameters per DoF (num_basis + 1)
-#define TCE_MAX_DOF 8
-#define TCE_MAX_DP 64   // max parameters per episode (num_dof * K1) of the likelihood and the projections
+#define TCE_MAX_DOF 16
+#define TCE_MAX_TABLE_DP 128  // max parameters per episode (num_dof * K1) of the tables, trajectories and diagonal likelihood
+#define TCE_MAX_DP 64   // max parameters per episode (num_dof * K1) of the dense likelihood and the projections
 
 // CALL with `K1` a compile-time constant for every K1 the tables accept (2..TCE_MAX_K1); returns
 // TCE_ERR_UNSUPPORTED_SHAPE for anything else.

@@ -309,8 +309,154 @@ seglik_chol_kernel(const double *Cmat, const double *Rres, double *Gout, double 
 }
 
 // =====================================================================================================
+// Stage 2 for N = 2 D in 18..32 (D = 9..16): one warp per segment, lane r owns row r of the packed triangle in
+// registers (every loop fully unrolled over N, rows padded with zeros past the diagonal; lanes >= N idle).  The same
+// arithmetic as seg_factor / seg_adjoint, in the same order where a lane owns the sum (Cholesky, forward substitution,
+// X = S^-1, the rows of C^-1); |z|^2, log det and alpha = X^T z are summed across lanes (xor butterflies, so every lane
+// and every call gets the same bits).  A pivot row or an X row is broadcast with __shfl_sync when the lanes below it
+// need it; X is then stored in a per-warp shared triangle so that lane i can read its column X[k][i].
+// G / A may overwrite C / R (the surrogate passes adj == work): a warp reads its segment before it writes it.
+// =====================================================================================================
+constexpr int CW_WARPS = 8;
+
+template <int N>
+__global__ void __launch_bounds__(CW_WARPS * 32)
+seglik_chol_warp_kernel(const double *Cmat, const double *Rres, double *Gout, double *Aout,
+                        const double *__restrict__ diag_max, double reg_rel, const float *__restrict__ grad_logp,
+                        const float *__restrict__ logp_old, const float *__restrict__ advantage, double grad_scale,
+                        double *__restrict__ loss_acc, float *__restrict__ logp, int32_t *__restrict__ info,
+                        long long BP, int P, int want_grad) {
+  constexpr int NT = tri(N);
+  __shared__ double s_x[CW_WARPS][NT];
+  __shared__ double s_loss[CW_WARPS][2];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const long long gid = (long long)blockIdx.x * CW_WARPS + warp;
+  double loss_part = 0.0, ratio_part = 0.0;
+  if (gid < BP) {                                     // warp-uniform
+    const long long b = gid / P;
+    const int p = (int)(gid % P);
+    const double *Cb = Cmat + (size_t)b * NT * P + p;
+    const double *Rb = Rres + (size_t)b * N * P + p;
+    const bool own = lane < N;
+    const int row0 = own ? tri_idx(lane, 0) : 0;
+    double a[N];
+#pragma unroll
+    for (int k = 0; k < N; ++k) a[k] = (own && k <= lane) ? Cb[(size_t)(row0 + k) * P] : 0.0;
+    double z = own ? Rb[(size_t)lane * P] : 0.0;
+    const double reg = reg_rel * (*diag_max);
+
+    // ---- left-looking Cholesky C + reg I = S S^T (diagonal <- 1/S_jj), z <- S^-1 z column by column
+    int bad = 0;
+    double my_d = 1.0;                                // lane j: its pivot
+#pragma unroll
+    for (int j = 0; j < N; ++j) {
+      double v = a[j];
+      if (lane == j) v += reg;
+#pragma unroll
+      for (int k = 0; k < j; ++k) v = fma(-a[k], __shfl_sync(0xffffffffu, a[k], j), v);   // row j is final left of j
+      const double dj = __shfl_sync(0xffffffffu, v, j);
+      if (!(dj > 0.0) && bad == 0) bad = j + 1;
+      double inv = (double)rsqrtf((float)dj);
+      inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
+      inv = inv * fma(-0.5 * dj, inv * inv, 1.5);
+      if (lane == j) { a[j] = inv; my_d = dj; z *= inv; }
+      else if (own && lane > j) a[j] = v * inv;
+      const double zj = __shfl_sync(0xffffffffu, z, j);
+      if (own && lane > j) z = fma(-a[j], zj, z);
+    }
+    const double half_logdet = warp_sum(own ? 0.5 * log(my_d) : 0.0);
+    const double maha = warp_sum(z * z);
+    const double lp = -0.5 * ((double)N * LN_2PI + maha) - half_logdet;
+    if (lane == 0) {
+      if (logp) logp[gid] = (float)lp;
+      if (info) info[gid] = bad;
+    }
+    if (want_grad) {
+      const SegIO io{grad_logp, logp_old, advantage, logp, info, grad_scale, reg, logp_old ? 2 : 1};
+      double lpart = 0.0, rpart = 0.0;
+      const double g = seg_upstream(io, lp, gid, lpart, rpart);
+      if (lane == 0) { loss_part = lpart; ratio_part = rpart; }
+      // ---- X = S^-1 (right-looking: row k is final once rows < k have been folded in; a[] holds the partial sums)
+#pragma unroll
+      for (int k = 0; k < N; ++k) {
+        if (lane == k) {
+#pragma unroll
+          for (int j = 0; j < k; ++j) a[j] = -a[j] * a[k];
+        }
+        const double s = a[k];
+#pragma unroll
+        for (int j = 0; j <= k; ++j) {
+          const double xkj = __shfl_sync(0xffffffffu, a[j], k);
+          if (own && lane > k) a[j] = j < k ? fma(s, xkj, a[j]) : s * xkj;
+        }
+      }
+      double *xs = s_x[warp];
+#pragma unroll
+      for (int j = 0; j < N; ++j)
+        if (own && j <= lane) xs[row0 + j] = a[j];
+      __syncwarp();
+      // ---- alpha = X^T z and row i of C^-1 = X^T X (sum over k >= i, ascending), G = g/2 (alpha alpha^T - C^-1)
+      double alpha = 0.0, acc[N];
+#pragma unroll
+      for (int j = 0; j < N; ++j) acc[j] = 0.0;
+#pragma unroll
+      for (int k = 0; k < N; ++k) {
+        const bool on = own && k >= lane;
+        const double xki = on ? xs[tri_idx(k, 0) + lane] : 0.0;
+        const double zk = __shfl_sync(0xffffffffu, z, k);
+        if (on) alpha = fma(xki, zk, alpha);
+#pragma unroll
+        for (int j = 0; j <= k; ++j)
+          if (on) acc[j] = fma(xki, xs[tri_idx(k, 0) + j], acc[j]);
+      }
+      double *Gb = Gout + (size_t)b * NT * P + p;
+      double *Ab = Aout + (size_t)b * N * P + p;
+      const double hg = 0.5 * g;
+#pragma unroll
+      for (int j = 0; j < N; ++j) {
+        const double aj = __shfl_sync(0xffffffffu, alpha, j);
+        if (own && j <= lane) Gb[(size_t)(row0 + j) * P] = hg * (alpha * aj - acc[j]);
+      }
+      if (own) Ab[(size_t)lane * P] = g * alpha;
+    }
+  }
+  if (loss_acc) {                                     // lane 0 of each warp holds its segment's parts
+    if (lane == 0) { s_loss[warp][0] = loss_part; s_loss[warp][1] = ratio_part; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      double l = 0.0, r = 0.0;
+      for (int w = 0; w < CW_WARPS; ++w) { l += s_loss[w][0]; r += s_loss[w][1]; }
+      if (r != 0.0) {
+        atomicAdd(loss_acc, l);
+        atomicAdd(loss_acc + 1, r);
+      }
+    }
+  }
+}
+
+// =====================================================================================================
 // Stage 3: backward accumulation.  One CTA per episode.
 // =====================================================================================================
+// The adjoints are staged in shared memory as fp32 [tri(2D)][P].  Above D = 8 the staging is dropped where it would
+// take the CTA past BWD_SMEM_LIMIT (e.g. (16, 4) at P = 128: 270 KB alone); the kernel then reads the fp64 adjoints
+// from the workspace, as the shared-covariance branch always does.  D <= 8 always stages (and refuses a P whose staging
+// does not fit), as it always has.
+constexpr size_t BWD_SMEM_LIMIT = 200 * 1024;
+constexpr int BWD_ALWAYS_STAGED_DOF = 8;
+
+__host__ __device__ inline size_t bwd_smem_bytes(int D, int K1, int P, bool multi, bool stage) {
+  const int Dp = D * K1, N = 2 * D, NT = tri(N), NR = (Dp + 3) & ~3, LD = NR + 1;
+  const int gs_need = (stage && NT * P > Dp * Dp) ? NT * P : Dp * Dp + 1;
+  const size_t g = sizeof(float) * (size_t)((gs_need + 1) & ~1);
+  return g + sizeof(double) * (2 * (size_t)P * K1 + 4 * (size_t)P + 5 + 2 * K1 + 1) + sizeof(float) * 2 * NR * LD +
+         (multi ? sizeof(double) * tri(D) * K1 * K1 : 0) + 16;
+}
+
+// fp32 staging of the adjoints (else: fp64 reads from the workspace); a function of the shape and P only
+__host__ __device__ inline bool bwd_stage(int D, int K1, int P, bool multi) {
+  return D <= BWD_ALWAYS_STAGED_DOF || (!multi && bwd_smem_bytes(D, K1, P, false, true) <= BWD_SMEM_LIMIT);
+}
+
 // DC as for the gram kernel.  With dsig_part != NULL (DC = 0 only) the covariance is ONE matrix for the batch: CTA c
 // owns episodes c, c + gridDim.x, ... (< B), sums upstream * d lp / d Sigma over them in that order and writes the sum
 // in block layout to dsig_part[c][tri(D) K1 K1] (fp64, entry (blk, i, j) = M_{d d'}[i][j], (d, d') = tri_decode(blk));
@@ -327,11 +473,13 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
   const int NR = (Dp + 3) & ~3;              // rows padded to a multiple of 4 for the 4x4 tiles
   const int LD = NR + 1;
   const bool multi = DC == 0 && dsig_part != nullptr;
+  const bool stage = bwd_stage(D, K1, P, multi);
+  const bool from_ws = multi || !stage;            // adjoints read in fp64 from the workspace
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float *Gs = reinterpret_cast<float *>(smem_raw);                // [NT][P] staged adjoints, fp32 (later: out tile)
   // Gs holds NT * P staged adjoints (and later the Dp x Dp output tile); its size is rounded UP to an even number of
-  // floats so that hs is 8-byte aligned and starts after the last adjoint, as bwd_smem() sizes it.
-  const int gs_need = NT * P > Dp * Dp ? NT * P : Dp * Dp + 1;
+  // floats so that hs is 8-byte aligned and starts after the last adjoint, as bwd_smem_bytes() sizes it.
+  const int gs_need = (stage && NT * P > Dp * Dp) ? NT * P : Dp * Dp + 1;
   const int gs_floats = (gs_need + 1) & ~1;
   double *hs = reinterpret_cast<double *>(Gs + gs_floats);       // [2P][K1]
   double *xi = hs + 2 * P * K1;                                   // [2P][2]
@@ -349,7 +497,7 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
 
   SL_STAMP(16);
   if (!multi) load_lower(L + b * ldb_L, Ls, Dp, NR, LD);
-  if (!multi)
+  if (!from_ws)
     for (int e = threadIdx.x; e < NT * P; e += blockDim.x) Gs[e] = (float)Gb[e];
   if (!multi)
     for (int e = threadIdx.x; e < NR * LD; e += blockDim.x) Ms[e] = 0.f;
@@ -383,13 +531,14 @@ seglik_bwd_kernel(TabDev tb, const double *__restrict__ Gmat, const double *__re
     const float *g01 = (d != dd) ? Gs + (size_t)tri_idx(r0, q0 + 1) * P : g10;    // symmetric inside a diagonal block
     // multi: the adjoints are read in fp64 from the workspace.  The batch sum of a shared covariance's gradient
     // cancels (advantages of both signs) far below the size of its terms; fp32-staged adjoints then cost ~1e-3 of it.
+    // (!stage: read from the workspace as well, their staging does not fit.)
     const double *G00 = Gb + (size_t)tri_idx(r0, q0) * P, *G10 = Gb + (size_t)tri_idx(r0 + 1, q0) * P;
     const double *G11 = Gb + (size_t)tri_idx(r0 + 1, q0 + 1) * P;
     const double *G01 = (d != dd) ? Gb + (size_t)tri_idx(r0, q0 + 1) * P : G10;
     for (int p = 0; p < P; ++p) {
       const double a0 = hs[(2 * p) * K1 + i], a1 = hs[(2 * p + 1) * K1 + i];
-      const double w0 = multi ? a0 * G00[p] + a1 * G10[p] : a0 * (double)g00[p] + a1 * (double)g10[p];   // coefficient of h_p0[:]
-      const double w1 = multi ? a0 * G01[p] + a1 * G11[p] : a0 * (double)g01[p] + a1 * (double)g11[p];   // coefficient of h_p1[:]
+      const double w0 = from_ws ? a0 * G00[p] + a1 * G10[p] : a0 * (double)g00[p] + a1 * (double)g10[p];   // coefficient of h_p0[:]
+      const double w1 = from_ws ? a0 * G01[p] + a1 * G11[p] : a0 * (double)g01[p] + a1 * (double)g11[p];   // coefficient of h_p1[:]
 #pragma unroll
       for (int j = 0; j < K1; ++j)
         acc[j] = fma(w0, hs[(2 * p) * K1 + j], fma(w1, hs[(2 * p + 1) * K1 + j], acc[j]));
@@ -636,11 +785,7 @@ size_t gram_smem(int D, int K1, int P) {
   return sizeof(double) * ((size_t)NR * SD + 2 * P * K1 + 4 * P + 5 + 2 * K1 + 1) + sizeof(float) * NR4 * LD + 16;
 }
 size_t bwd_smem(int D, int K1, int P, bool multi) {
-  const int Dp = D * K1, N = 2 * D, NT = tri(N), NR = (Dp + 3) & ~3, LD = NR + 1;
-  const size_t gs_floats = (size_t)(((NT * P > Dp * Dp ? NT * P : Dp * Dp + 1) + 1) & ~1);   // >= the kernel's
-  const size_t g = sizeof(float) * gs_floats;
-  return g + sizeof(double) * (2 * P * K1 + 4 * P + 5 + 2 * K1 + 1) + sizeof(float) * 2 * NR * LD +
-         (multi ? sizeof(double) * tri(D) * K1 * K1 : 0) + 16;
+  return bwd_smem_bytes(D, K1, P, multi, bwd_stage(D, K1, P, multi));
 }
 
 int g_sms = 0;
@@ -684,7 +829,7 @@ int bwd_launch(const tce_tables_t *t, const double *G, const double *A, const fl
                const float *times, const float *init_time, const int64_t *pred_pairs, const float *upstream,
                float *grad_mean, float *grad_L, double *dsig_part, int64_t B, int64_t T, int64_t P, cudaStream_t st) {
   const size_t smem = bwd_smem(t->D, K1, (int)P, dsig_part != nullptr);
-  if (smem > 200 * 1024) return TCE_ERR_UNSUPPORTED_SHAPE;
+  if (smem > BWD_SMEM_LIMIT) return TCE_ERR_UNSUPPORTED_SHAPE;
   TCE_CUDA(cudaFuncSetAttribute(seglik_bwd_kernel<DC, K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
            "bwd smem attr");
   cudaFuncSetAttribute(seglik_bwd_kernel<DC, K1>, cudaFuncAttributePreferredSharedMemoryCarveout,
@@ -718,7 +863,7 @@ int diag_launch(const tce_tables_t *t, const float *smp_traj, const float *mean,
 }  // namespace
 
 // (D, K1) combinations with instantiations specialised on D (and the fused / uniform-grid kernels of
-// tce_seglik_fused.cu); every other shape with 1 <= D <= 8, 2 <= K1 <= 16, D K1 <= 64 runs the DC = 0 instantiations
+// tce_seglik_fused.cu); every other shape with 1 <= D <= 16, 2 <= K1 <= 16, D K1 <= 64 runs the DC = 0 instantiations
 #define TCE_FOR_SHAPES(X) X(7, 9) X(4, 9) X(7, 4) X(3, 4) X(2, 3)
 
 static bool shape_supported(const tce_tables_t *t) {
@@ -728,7 +873,7 @@ static bool shape_supported(const tce_tables_t *t) {
 // The diagonal likelihood keeps no Dp x Dp matrix: its work per (pair, DoF) depends on K1 only, so it takes every
 // shape the tables accept
 static bool diag_shape_supported(const tce_tables_t *t) {
-  return t->D >= 1 && t->D <= TCE_MAX_DOF && t->K1 >= 2 && t->K1 <= TCE_MAX_K1;
+  return t->D >= 1 && t->D <= TCE_MAX_DOF && t->K1 >= 2 && t->K1 <= TCE_MAX_K1 && t->D * t->K1 <= TCE_MAX_TABLE_DP;
 }
 
 extern "C" int tce_seglik_compiled(const tce_tables_t *t) {
@@ -821,6 +966,7 @@ extern "C" int tce_seglik_chol(const tce_tables_t *t, const void *work, void *ad
   const unsigned grid = (unsigned)((BP + CH_THREADS - 1) / CH_THREADS);
   const int want_grad = (grad_logp != nullptr) || (logp_old != nullptr);
   if (want_grad && !adj) return TCE_ERR_INVALID_ARGUMENT;
+  const unsigned wgrid = (unsigned)((BP + CW_WARPS - 1) / CW_WARPS);
   switch (t->D) {
 #define Y(Dv)                                                                                                  \
   case Dv:                                                                                                     \
@@ -830,6 +976,14 @@ extern "C" int tce_seglik_chol(const tce_tables_t *t, const void *work, void *ad
     break;
     Y(1) Y(2) Y(3) Y(4) Y(5) Y(6) Y(7) Y(8)
 #undef Y
+#define W(Dv)                                                                                                  \
+  case Dv:                                                                                                     \
+    seglik_chol_warp_kernel<2 * Dv><<<wgrid, CW_WARPS * 32, 0, st>>>(Cmat, R, G, A, diag_max, reg_rel, grad_logp, \
+                                                                     logp_old, advantage, grad_scale, loss_acc,   \
+                                                                     logp, info, BP, (int)P, want_grad);          \
+    break;
+    W(9) W(10) W(11) W(12) W(13) W(14) W(15) W(16)
+#undef W
     default: return TCE_ERR_UNSUPPORTED_SHAPE;
   }
   TCE_CHECK_LAUNCH("seglik_chol_kernel");

@@ -113,7 +113,8 @@ __global__ void build_tables_kernel(tce_mp_cfg cfg, int n_pc, int K, double *y1,
 extern "C" int tce_prodmp_tables_create(const tce_mp_cfg *cfg, void *stream, tce_tables_t **out) {
   if (!cfg || !out) return TCE_ERR_INVALID_ARGUMENT;
   const int K = cfg->num_basis, K1 = K + 1;
-  if (K < 1 || K1 > TCE_MAX_K1 || cfg->num_dof < 1 || cfg->num_dof > TCE_MAX_DOF) return TCE_ERR_UNSUPPORTED_SHAPE;
+  if (K < 1 || K1 > TCE_MAX_K1 || cfg->num_dof < 1 || cfg->num_dof > TCE_MAX_DOF || cfg->num_dof * K1 > TCE_MAX_TABLE_DP)
+    return TCE_ERR_UNSUPPORTED_SHAPE;
   if (cfg->tau <= 0 || cfg->dt <= 0 || cfg->pre_compute_length_factor < 1) return TCE_ERR_INVALID_ARGUMENT;
   if (K > 1 && K - 2 * cfg->num_basis_outside - 1 <= 0) return TCE_ERR_INVALID_ARGUMENT;
   tce_tables *t = new tce_tables();

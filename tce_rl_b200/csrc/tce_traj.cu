@@ -27,7 +27,7 @@ __device__ __forceinline__ void time_to_index_fast(const TabDev &tb, double inv_
 // shared tile so that the global stores are contiguous 128-bit.  HBM traffic = the algorithmic bytes (params, initial
 // conditions and times are read once, the trajectory is written once).
 constexpr int TW_WARPS = 8;
-template <int K1, int DMAX>
+template <int K1>
 __global__ void __launch_bounds__(TW_WARPS * 32)
 traj_fwd_warp_kernel(TabDev tb, const float *__restrict__ params, const float *__restrict__ times,
                      const float *__restrict__ init_time, const float *__restrict__ init_pos,
@@ -360,8 +360,8 @@ int launch_traj_fwd(const tce_tables *t, const float *params, const float *times
   long long grid = (slabs + TW_WARPS - 1) / TW_WARPS;
   const long long cap = 8LL * num_sms();
   if (grid > cap) grid = cap;
-  const size_t smem_w = (size_t)TW_WARPS * (32 * 2 * t->D + 4) * sizeof(float);
-  traj_fwd_warp_kernel<K1, TCE_MAX_DOF><<<(unsigned)grid, TW_WARPS * 32, smem_w, st>>>(
+  const size_t smem_w = (size_t)TW_WARPS * (32 * 2 * t->D + 4) * sizeof(float);   // <= 33 KB (D <= 16): no opt-in
+  traj_fwd_warp_kernel<K1><<<(unsigned)grid, TW_WARPS * 32, smem_w, st>>>(
       tab_dev(t), params, times, init_time, init_pos, init_vel, traj, B, (int)T);
   TCE_CHECK_LAUNCH("traj_fwd_warp_kernel");
   return TCE_OK;
