@@ -92,6 +92,32 @@ int tce_prodmp_traj_bwd(const tce_tables_t *tables, const float *grad_traj, cons
                         const float *init_time, float *grad_params, float *grad_init_pos,
                         float *grad_init_vel, int64_t B, int64_t T, void *stream);
 
+/* ---- (1b) position covariances and standard deviations on any time grid -------------------------------------------
+ * ProDMP.get_traj_pos_cov / get_traj_pos_std of mp_pytorch for T >= 1 time points per episode.  F = H L [D T, Dp] (rows
+ * DoF-major, time-minor; H block diagonal with the episode's scaled position basis rows), C = F F^T + r I with
+ * r = reg_rel * max over the whole call of diag(F F^T).
+ *   cov_fwd: cov [B, D T, D T];            cov_bwd: grad_cov [B, D T, D T] -> grad_L = tril(H^T (G + G^T) F)
+ *   std_fwd: std [B, T, D] = sqrt(diag C); std_bwd: std, grad_std [B, T, D] -> grad_L
+ * L [B, Dp, Dp] (lower triangle read; batch stride ldb_L >= Dp^2, or 0 = one factor for the batch), times [B, T],
+ * init_time [B].  grad_L is [B, Dp, Dp] per episode, or [Dp, Dp] summed over the batch in a fixed order when
+ * ldb_L = 0 (repeated calls give the same bits).  r is a constant in the backward.  fp64 arithmetic, no host
+ * synchronisation.  Every shape the tables accept (num_dof <= 16, K1 <= 16, Dp <= 128); B = 0 is a no-op.
+ * work: tce_prodmp_traj_cov_work_bytes(tables, B, T, ldb_L, entry) bytes, 16-byte aligned, entry 0 = cov_fwd,
+ * 1 = cov_bwd, 2 = std_fwd, 3 = std_bwd (0: invalid arguments or unsupported shape).                           */
+size_t tce_prodmp_traj_cov_work_bytes(const tce_tables_t *tables, int64_t B, int64_t T, int64_t ldb_L, int entry);
+int tce_prodmp_traj_cov_fwd(const tce_tables_t *tables, const float *L, int64_t ldb_L, const float *times,
+                            const float *init_time, double reg_rel, void *work, float *cov, int64_t B, int64_t T,
+                            void *stream);
+int tce_prodmp_traj_cov_bwd(const tce_tables_t *tables, const float *L, int64_t ldb_L, const float *times,
+                            const float *init_time, const float *grad_cov, void *work, float *grad_L, int64_t B,
+                            int64_t T, void *stream);
+int tce_prodmp_traj_std_fwd(const tce_tables_t *tables, const float *L, int64_t ldb_L, const float *times,
+                            const float *init_time, double reg_rel, void *work, float *std_out, int64_t B, int64_t T,
+                            void *stream);
+int tce_prodmp_traj_std_bwd(const tce_tables_t *tables, const float *L, int64_t ldb_L, const float *times,
+                            const float *init_time, const float *std_in, const float *grad_std, void *work,
+                            float *grad_L, int64_t B, int64_t T, void *stream);
+
 /* ---- (2) Gaussian policy over the MP parameters -----------------------------------------------------
  * out = mean + L eps : MultivariateNormal(loc, scale_tril).rsample (black_box_policy.py:82-84 and
  * mp_pytorch sample_trajectories).  eps [B, n] is injected when not NULL, otherwise drawn in-kernel

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtce_b200.so")
-SOURCES = ["tce_tables.cu", "tce_traj.cu", "tce_seglik.cu", "tce_seglik_fused.cu", "tce_gauss.cu", "tce_adv.cu", "tce_proj.cu", "tce_proj_diag.cu", "tce_adam.cu", "tce_epoch.cu", "tce_p2p.cu", "tce_bench.cu"]
+SOURCES = ["tce_tables.cu", "tce_traj.cu", "tce_traj_cov.cu", "tce_seglik.cu", "tce_seglik_fused.cu", "tce_gauss.cu", "tce_adv.cu", "tce_proj.cu", "tce_proj_diag.cu", "tce_adam.cu", "tce_epoch.cu", "tce_p2p.cu", "tce_bench.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 

@@ -40,6 +40,11 @@ SIGNATURES = {
     "tce_prodmp_traj_fwd": (C.c_int, [_P] * 7 + [_I64, _I64, _P]),
     "tce_prodmp_traj_fwd_uniform": (C.c_int, [_P] * 8 + [_I64, _I64, _P]),
     "tce_prodmp_traj_bwd": (C.c_int, [_P] * 7 + [_I64, _I64, _P]),
+    "tce_prodmp_traj_cov_work_bytes": (C.c_size_t, [_P, _I64, _I64, _I64, _I32]),
+    "tce_prodmp_traj_cov_fwd": (C.c_int, [_P, _P, _I64, _P, _P, _D, _P, _P, _I64, _I64, _P]),
+    "tce_prodmp_traj_cov_bwd": (C.c_int, [_P, _P, _I64, _P, _P, _P, _P, _P, _I64, _I64, _P]),
+    "tce_prodmp_traj_std_fwd": (C.c_int, [_P, _P, _I64, _P, _P, _D, _P, _P, _I64, _I64, _P]),
+    "tce_prodmp_traj_std_bwd": (C.c_int, [_P, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _I64, _P]),
     "tce_mvn_rsample": (C.c_int, [_P, _P, _I64, _P, _U64, _U64, _P, _I64, _I32, _P]),
     "tce_chol_fwd": (C.c_int, [_P, _P, _P, _I64, _I32, _P]),
     "tce_chol_bwd": (C.c_int, [_P, _P, _P, _I64, _I32, _P]),

@@ -2,13 +2,13 @@
 
 Reference construction: ``get_mp`` (mprl/util/util_mp.py:11-46); reference call sites:
 mprl/rl/policy/temporal_correlated_policy.py:76-92,188-192.  Everything is evaluated by the CUDA
-kernels (``tce::prodmp_traj``, ``tce::mvn_rsample``, the gram stage of ``tce::seglik``).
+kernels (``tce::prodmp_traj``, ``tce::mvn_rsample``, ``tce::traj_pos_cov``, ``tce::traj_pos_std``).
 """
 from __future__ import annotations
 
 import torch
 
-from . import _lib, ops
+from . import ops, ops_seglik
 
 
 class ProDMP:
@@ -103,36 +103,44 @@ class ProDMP:
         self.update_inputs(*old)
         return pos, vel
 
+    def _pos_cov_inputs(self):
+        """times [n, T], init_time [n] and params_L as [n, Dp, Dp], or as the ONE [1, Dp, Dp] matrix behind a
+        broadcast (stride-0) factor, so that a shared factor is neither copied nor given a per-episode gradient."""
+        times, lead = self._flat(self.times, 1)
+        n, Dp = times.shape[0], self.num_dof * self.num_basis_g
+        L = self.params_L
+        if L.dim() > 2 and tuple(L.shape[:-2]) != tuple(lead):
+            L = L.expand(*lead, Dp, Dp)
+        if L.dim() > 3:
+            L = L.reshape(-1, Dp, Dp)
+        shared = ops_seglik.shared_factor(L, n)
+        if shared is not None:
+            L = shared
+        elif L.dim() != 3 or L.shape[0] != n:
+            raise ValueError(f"params_L must broadcast to [*a, {Dp}, {Dp}] over times [*a, T], got {list(L.shape)}")
+        return times, self.init_time.reshape(-1), L, lead
+
     def get_traj_pos_cov(self, times=None, params_L=None, init_time=None, init_pos=None, init_vel=None,
                          reg: float = 1e-4):
-        """[*a, 2D, 2D] trajectory covariance for TWO time points per entry (the only shape TCE uses):
-        H (L L^T) H^T + reg * max diag over the whole batch * I."""
+        """[*a, D*T, D*T] covariance of the positions at the times [*a, T] (rows DoF-major, time-minor) under the
+        parameter distribution N(., L L^T): H (L L^T) H^T + reg * max diag over the whole call * I.  Any time grid
+        (TCE passes pairs, [*a] = [B, P]); differentiable w.r.t. params_L.  One factor may be broadcast over the
+        batch (stride-0 expand): it is read once and its gradient is summed over the batch."""
         self.update_inputs(times, None, params_L, init_time, init_pos, init_vel)
-        times2, lead = self._flat(self.times, 1)
-        if times2.shape[-1] != 2:
-            raise NotImplementedError("get_traj_pos_cov is provided for time pairs only (TCE segments)")
-        n = times2.shape[0]
-        D, Dp = self.num_dof, self.num_dof * self.num_basis_g
-        L3 = self.params_L.reshape(-1, Dp, Dp)
-        it = self.init_time.reshape(-1).contiguous()
-        zeros = torch.zeros(n, Dp, device=times2.device)
-        zpos = torch.zeros(n, D, device=times2.device)
-        pairs = torch.tensor([[0, 1]], device=times2.device, dtype=torch.int64)
-        smp = torch.zeros(n, 2, 2 * D, device=times2.device)
-        work = ops._work(self.tables.handle, n, 1, times2.device)
-        dmax = torch.zeros(1, device=times2.device, dtype=torch.float64)
-        Lc, ldb = ops._batched_matrix(L3)
-        _lib.call("tce_seglik_gram", self.tables.handle, smp.data_ptr(), zeros.data_ptr(), Lc.data_ptr(), ldb,
-                  times2.contiguous().data_ptr(), it.data_ptr(), zpos.data_ptr(), zpos.data_ptr(), pairs.data_ptr(),
-                  work.data_ptr(), dmax.data_ptr(), n, 2, 1, ops._stream())
-        N = 2 * D
-        tri = work[:n * N * (N + 1) // 2].reshape(n, N * (N + 1) // 2)
-        r, c = torch.tril_indices(N, N, device=times2.device)
-        cov = torch.zeros(n, N, N, device=times2.device, dtype=torch.float64)
-        cov[:, r, c] = tri
-        cov[:, c, r] = tri
-        cov = cov + torch.eye(N, device=cov.device, dtype=cov.dtype) * (dmax * reg)
-        return cov.to(torch.float32).reshape(*lead, N, N)
+        times2, it, L, lead = self._pos_cov_inputs()
+        cov = ops.traj_pos_cov(L, times2, it, self.tables.handle, self.num_dof, float(reg))
+        return cov.reshape(*lead, *cov.shape[-2:])
+
+    def get_traj_pos_std(self, times=None, params_L=None, init_time=None, init_pos=None, init_vel=None,
+                         flat_shape=False, reg: float = 1e-4):
+        """Standard deviations of the positions, sqrt(diag(get_traj_pos_cov)) with the same regulariser, without
+        forming the covariance: [*a, T, D], or [*a, D*T] DoF-major with ``flat_shape``.  Differentiable w.r.t.
+        params_L."""
+        self.update_inputs(times, None, params_L, init_time, init_pos, init_vel)
+        times2, it, L, lead = self._pos_cov_inputs()
+        std = ops.traj_pos_std(L, times2, it, self.tables.handle, self.num_dof, float(reg))
+        std = std.reshape(*lead, *std.shape[-2:])
+        return std.transpose(-1, -2).reshape(*lead, -1) if flat_shape else std
 
 
 def get_mp(**kwargs) -> ProDMP:

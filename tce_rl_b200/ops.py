@@ -199,6 +199,140 @@ def _traj_backward(ctx, grad):
 prodmp_traj.register_autograd(_traj_backward, setup_context=_traj_setup)
 
 
+# (1b) position covariances / standard deviations (mp.ProDMP.get_traj_pos_cov / get_traj_pos_std)
+# --------------------------------------------------------------------------------------------------
+_TRAJ_COV_FWD, _TRAJ_COV_BWD, _TRAJ_STD_FWD, _TRAJ_STD_BWD = range(4)     # `entry` of tce_prodmp_traj_cov_work_bytes
+
+
+def _traj_factor(L: Tensor, B: int) -> Tuple[Tensor, int]:
+    """(storage, batch stride) of L: [B, Dp, Dp] per episode, or [1, Dp, Dp] shared by the batch (stride 0)."""
+    if not L.is_cuda or L.dtype != torch.float32 or L.dim() != 3 or L.shape[0] not in (1, B):
+        raise TceError(f"L must be a CUDA float32 [B or 1, Dp, Dp] tensor with B = {B}, got {list(L.shape)}")
+    n = L.shape[-1]
+    return L.contiguous(), (0 if L.shape[0] == 1 and B > 1 else n * n)
+
+
+def _traj_work(tables: int, B: int, T: int, ldb: int, entry: int, device) -> Tensor:
+    nbytes = _lib.load().tce_prodmp_traj_cov_work_bytes(tables, B, T, ldb, entry)
+    return torch.empty(max(nbytes // 8, 1), device=device, dtype=torch.float64)
+
+
+@torch.library.custom_op("tce::traj_pos_cov", mutates_args=())
+def traj_pos_cov(L: Tensor, times: Tensor, init_time: Tensor, tables: int, num_dof: int, reg: float) -> Tensor:
+    """Position covariance [B, D T, D T] (rows DoF-major) of N(., L L^T) at times [B, T]: H L L^T H^T + r I,
+    r = reg * max of its diagonal over the batch.  L: [B, Dp, Dp] or [1, Dp, Dp] shared."""
+    times, init_time = _chk(times, name="times"), _chk(init_time, name="init_time")
+    B, T = times.shape
+    L, ldb = _traj_factor(L, B)
+    cov = torch.empty(B, num_dof * T, num_dof * T, device=times.device, dtype=torch.float32)
+    if B == 0:
+        return cov
+    work = _traj_work(tables, B, T, ldb, _TRAJ_COV_FWD, times.device)
+    _lib.call("tce_prodmp_traj_cov_fwd", tables, _p(L), ldb, _p(times), _p(init_time), float(reg), _p(work), _p(cov),
+              B, T, _stream())
+    return cov
+
+
+@traj_pos_cov.register_fake
+def _(L, times, init_time, tables, num_dof, reg):
+    B, T = times.shape
+    return times.new_empty(B, num_dof * T, num_dof * T)
+
+
+@torch.library.custom_op("tce::traj_pos_cov_bwd", mutates_args=())
+def traj_pos_cov_bwd(grad: Tensor, L: Tensor, times: Tensor, init_time: Tensor, tables: int) -> Tensor:
+    grad, times, init_time = _chk(grad, name="grad"), _chk(times), _chk(init_time)
+    B, T = times.shape
+    L, ldb = _traj_factor(L, B)
+    g_L = torch.empty(L.shape, device=L.device, dtype=torch.float32)
+    if B == 0:
+        return g_L.zero_()
+    work = _traj_work(tables, B, T, ldb, _TRAJ_COV_BWD, times.device)
+    _lib.call("tce_prodmp_traj_cov_bwd", tables, _p(L), ldb, _p(times), _p(init_time), _p(grad), _p(work), _p(g_L), B,
+              T, _stream())
+    return g_L
+
+
+@traj_pos_cov_bwd.register_fake
+def _(grad, L, times, init_time, tables):
+    return L.new_empty(L.shape)
+
+
+def _traj_cov_setup(ctx, inputs, output):
+    L, times, init_time, tables, num_dof, reg = inputs
+    ctx.save_for_backward(L, times, init_time)
+    ctx.tables = tables
+    ctx.set_materialize_grads(False)
+
+
+def _traj_cov_backward(ctx, g):
+    if g is None:
+        return (None,) * 6
+    L, times, init_time = ctx.saved_tensors
+    return traj_pos_cov_bwd(g.contiguous(), L, times, init_time, ctx.tables), None, None, None, None, None
+
+
+traj_pos_cov.register_autograd(_traj_cov_backward, setup_context=_traj_cov_setup)
+
+
+@torch.library.custom_op("tce::traj_pos_std", mutates_args=())
+def traj_pos_std(L: Tensor, times: Tensor, init_time: Tensor, tables: int, num_dof: int, reg: float) -> Tensor:
+    """Position standard deviations [B, T, D] = sqrt of the diagonal of ``traj_pos_cov`` (same regulariser), without
+    forming the covariance."""
+    times, init_time = _chk(times, name="times"), _chk(init_time, name="init_time")
+    B, T = times.shape
+    L, ldb = _traj_factor(L, B)
+    out = torch.empty(B, T, num_dof, device=times.device, dtype=torch.float32)
+    if B == 0:
+        return out
+    work = _traj_work(tables, B, T, ldb, _TRAJ_STD_FWD, times.device)
+    _lib.call("tce_prodmp_traj_std_fwd", tables, _p(L), ldb, _p(times), _p(init_time), float(reg), _p(work), _p(out),
+              B, T, _stream())
+    return out
+
+
+@traj_pos_std.register_fake
+def _(L, times, init_time, tables, num_dof, reg):
+    B, T = times.shape
+    return times.new_empty(B, T, num_dof)
+
+
+@torch.library.custom_op("tce::traj_pos_std_bwd", mutates_args=())
+def traj_pos_std_bwd(grad: Tensor, std: Tensor, L: Tensor, times: Tensor, init_time: Tensor, tables: int) -> Tensor:
+    grad, std, times, init_time = _chk(grad, name="grad"), _chk(std), _chk(times), _chk(init_time)
+    B, T = times.shape
+    L, ldb = _traj_factor(L, B)
+    g_L = torch.empty(L.shape, device=L.device, dtype=torch.float32)
+    if B == 0:
+        return g_L.zero_()
+    work = _traj_work(tables, B, T, ldb, _TRAJ_STD_BWD, times.device)
+    _lib.call("tce_prodmp_traj_std_bwd", tables, _p(L), ldb, _p(times), _p(init_time), _p(std), _p(grad), _p(work),
+              _p(g_L), B, T, _stream())
+    return g_L
+
+
+@traj_pos_std_bwd.register_fake
+def _(grad, std, L, times, init_time, tables):
+    return L.new_empty(L.shape)
+
+
+def _traj_std_setup(ctx, inputs, output):
+    L, times, init_time, tables, num_dof, reg = inputs
+    ctx.save_for_backward(output, L, times, init_time)
+    ctx.tables = tables
+    ctx.set_materialize_grads(False)
+
+
+def _traj_std_backward(ctx, g):
+    if g is None:
+        return (None,) * 6
+    std, L, times, init_time = ctx.saved_tensors
+    return traj_pos_std_bwd(g.contiguous(), std, L, times, init_time, ctx.tables), None, None, None, None, None
+
+
+traj_pos_std.register_autograd(_traj_std_backward, setup_context=_traj_std_setup)
+
+
 # --------------------------------------------------------------------------------------------------
 # (2) Gaussian sampling, Cholesky, head, stats
 # --------------------------------------------------------------------------------------------------
@@ -389,8 +523,8 @@ def _(mean, L, mean_o, L_o):
 # --------------------------------------------------------------------------------------------------
 # Two implementations of the likelihood.  A shared covariance runs the fused kernels in ops_seglik.py (re-exported at
 # the end of this module); per-episode factors run the STAGED ops below (gram / chol / bwd with an fp64 HBM workspace,
-# see ops_seglik.PER_EPISODE_STAGED).  The staged gram kernel also serves mp.ProDMP.get_traj_pos_cov, and the tests use
-# the staged ops as an independent reference for the fused kernels.
+# see ops_seglik.PER_EPISODE_STAGED).  The tests use the staged ops as an independent reference for the fused kernels.
+# (mp.ProDMP.get_traj_pos_cov runs its own kernels: tce::traj_pos_cov above.)
 from .ops_seglik import (set_regulariser_group, _reduce_diag_max, unit_seed, sync_uniform,  # noqa: E402
                          diag_strides, _dense_diag_grad)
 
